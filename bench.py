@@ -17,6 +17,7 @@ templates of config 3 split over the N ranks (the replicated 1.5 ms build is its
   parity : the benched top-10 equals the CPU oracle's (checked outside the timed region)
   config4 / config5 : templates/s of the wide 4K search, scenes/s of the multi-scene batch
   --impl reference : the CPU oracle (port of the reference, all host threads), whole job per step.
+  --dump-outputs DIR : after the timed steps, the outputs of the last step as DIR/<name>.npy (see dump_outputs).
 
 Prints ONE JSON line on rank 0.
 """
@@ -104,6 +105,21 @@ def load_traffic():
         return {}
 
 
+MAP_SAMPLE_PER_PLANE = 1 << 17   # 30 planes x 128 Ki values x 4 B = 15.7 MB of the 995 MB map
+
+
+def dump_outputs(out_dir, fm, top):
+    """What a caller of the timed step receives from it: the top-10 matches and the DT3 map they were searched in.
+    The map is too large to store whole, so a fixed, seeded sample of positions of every plane stands for it."""
+    os.makedirs(out_dir, exist_ok=True)
+    idx = np.random.default_rng(0).integers(0, fm.height * fm.width, (fm.depth, MAP_SAMPLE_PER_PLANE))
+    arrays = {"top10_tmpl_idx": top["tmpl_idx"].astype(np.float64), "top10_score": top["score"],
+              "top10_transform": top["transform"].reshape(-1, 2, 3),
+              "dt3_map_sample": np.stack([fm.plane(d).reshape(-1)[idx[d]] for d in range(fm.depth)])}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
+
+
 def oracle_job(scene, tmpls, nthreads=0):
     """The CPU oracle (port of the reference, ThreadPool decomposition) on the WHOLE job: one full map build + the
     search / penalize / sort of every template.  Returns timings and the penalised match list."""
@@ -163,7 +179,13 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the config-4 / config-5 / strong-scaling legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the top-10 and a seeded sample of the DT3 map of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 timed path")
     # stdout carries exactly one JSON line: libraries that print to fd 1 (NCCL's version banner) are sent to stderr
     global _JSON_OUT
     sys.stdout.flush()
@@ -267,6 +289,8 @@ def main():
     sampler.start()
     ms_res, top_res, launches, prof = timed(step_resident, args.steps, args.warmup, profile=True)
     stats = fm.last_search_stats()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, fm, top_res)
     ms_e2e, top_e2e, _, _ = timed(step_e2e, args.steps, args.warmup)
     clocks = sampler.stop()
 

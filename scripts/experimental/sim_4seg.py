@@ -1,5 +1,5 @@
-import sys, numpy as np
-sys.path.insert(0, '/root/repo')
+import os, sys, numpy as np
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), '..', '..'))
 from oracle import fdcm_oracle as orc
 BIG = 0xFFFF
 def fdiv(N, D): return N // D
