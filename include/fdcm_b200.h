@@ -160,7 +160,13 @@ fdcm_status fdcm_templates_lengths(const fdcm_templates* t, float* lengths);
  * (un-shifted), as in the reference; n_scene == 0 yields no matches (defaultmatch.cpp:40) and
  * n_scene == FDCM_SCENE_RESIDENT (scene_xyxy ignored) searches the scene the map was built from, which is
  * already resident on the device.  out: capacity records; *n_out = number written (or required
- * when FDCM_ERR_CAPACITY). */
+ * when FDCM_ERR_CAPACITY).
+ * Template size limit: the search kernel keeps the aligned copy of the longest template of the set in shared memory,
+ * 16 L + round_up(L, 16) bytes per hypothesis in flight and at least one per block.  On a device with S bytes of opt-in
+ * shared memory per block (cudaDevAttrMaxSharedMemoryPerBlockOptin; 232448 on a B200) the longest template may have
+ * L lines with 16 L + round_up(L, 16) <= S: 13673 lines on a B200.  A set holding a longer template fails with
+ * FDCM_ERR_INVALID (the message states the limit); so do fdcm_optimize and fdcm_search_scenes.  Templates of up to
+ * S / 68 lines (3418 on a B200) run 4 hypotheses per block, longer ones 2 or 1. */
 #define FDCM_SCENE_RESIDENT (-1)
 fdcm_status fdcm_search(const fdcm_dt3* map, const fdcm_templates* templates, const float* scene_xyxy, int32_t n_scene,
                         const fdcm_search_params* params, fdcm_match* out, int64_t capacity, int64_t* n_out);

@@ -1458,6 +1458,18 @@ static fdcm_status exchange_empty(const fdcm_dt3* m, fdcm_comm* comm, int k, fdc
     return finish_topk(m, comm, k, s, nullptr, out, capacity, n_out);
 }
 
+// The search kernel stages the longest template of a set in shared memory, at least one warp's worth per block: a set
+// holding a template longer than one warp can stage within the device's per-block opt-in limit cannot be searched.
+static fdcm_status search_smem_optin(int device, int max_lines, int* smem_optin) {
+    CUDA_TRY(cudaDeviceGetAttribute(smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device));
+    const int limit = search_max_template_lines(*smem_optin);
+    if (max_lines > limit)
+        return fail(FDCM_ERR_INVALID, "template of " + std::to_string(max_lines) + " lines: the search takes at most " +
+                                          std::to_string(limit) + " lines per template on this device (" +
+                                          std::to_string(*smem_optin) + " bytes of shared memory per block)");
+    return FDCM_OK;
+}
+
 static fdcm_status search_impl(const fdcm_dt3* m, const fdcm_templates* tc, const float* scene, int32_t n_scene,
                                const fdcm_search_params* p, fdcm_match* out, int64_t capacity, int64_t* n_out, fdcm_comm* comm) {
     if (!m || !tc || !p || !n_out) return fail(FDCM_ERR_INVALID, "null argument");
@@ -1488,6 +1500,8 @@ static fdcm_status search_impl(const fdcm_dt3* m, const fdcm_templates* tc, cons
     cudaStream_t s;
     if (fdcm_status st = get_stream(m->device, &s)) return st;
     if (fdcm_status st = templates_ready(t, s)) return st;
+    int smem_optin = 0;
+    if (fdcm_status st = search_smem_optin(m->device, t->max_lines, &smem_optin)) return st;
 
     // ---- host prep: scene length order (defaultsearch.cpp:32-36) and hypothesis offsets ----
     const SceneFilter flt{p->concentric != 0, p->center_x, p->center_y, p->low_radius, p->high_radius};
@@ -1598,9 +1612,8 @@ static fdcm_status search_impl(const fdcm_dt3* m, const fdcm_templates* tc, cons
     }
     {
         KernelScope k("search", 0.0, s);
-        launch_search(map_view(m), m->table_dev, tv, sv, sl, so, s);
+        CUDA_TRY(launch_search(map_view(m), m->table_dev, tv, sv, sl, so, smem_optin, s));
     }
-    CUDA_TRY(cudaGetLastError());
 
     unsigned long long counters[3] = {0, 0, 0};
     fdcm_status result = FDCM_OK;
@@ -1815,6 +1828,8 @@ extern "C" fdcm_status fdcm_optimize(const fdcm_dt3* m, const float* tmpl_lines,
     if (fdcm_status st = get_stream(m->device, &s)) return st;
     int max_lines = 1;
     for (int t = 0; t < n_tmpl; ++t) max_lines = std::max(max_lines, tmpl_offsets[t + 1] - tmpl_offsets[t]);
+    int smem_optin = 0;
+    if (fdcm_status st = search_smem_optin(m->device, max_lines, &smem_optin)) return st;
     DevBuf dl, doff, dal, drec, dval, dcnt;
     auto cleanup = [&]() { for (DevBuf* b : {&dl, &doff, &dal, &drec, &dval, &dcnt}) b->release(); };
     std::vector<fdcm_match> rec((size_t)n_tmpl);
@@ -1845,9 +1860,8 @@ extern "C" fdcm_status fdcm_optimize(const fdcm_dt3* m, const float* tmpl_lines,
         so.valid = dval.as<uint8_t>();
         so.counters = dcnt.as<unsigned long long>();
         KernelScope k("optimize", 0.0, s);
-        launch_search(map_view(m), m->table_dev, tv, sv, sl, so, s);
+        e = launch_search(map_view(m), m->table_dev, tv, sv, sl, so, smem_optin, s);
     }
-    if (e == cudaSuccess) e = cudaGetLastError();
     if (e == cudaSuccess) e = cudaMemcpyAsync(rec.data(), drec.p, (size_t)n_tmpl * sizeof(fdcm_match), cudaMemcpyDeviceToHost, s);
     if (e == cudaSuccess) e = cudaMemcpyAsync(has_value, dval.p, (size_t)n_tmpl, cudaMemcpyDeviceToHost, s);
     if (e == cudaSuccess) e = cudaStreamSynchronize(s);

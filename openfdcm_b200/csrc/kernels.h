@@ -113,8 +113,12 @@ void launch_search_order(const TemplatesView& tv, const SceneView& sv, const Sea
                          int32_t* d_idx, int32_t* d_perm, void* d_temp, size_t temp_bytes, float minx, float miny, int cells_x,
                          int key_bits, int4* d_hyp, cudaStream_t s);
 
-void launch_search(const MapView& map, const SlopeTableDev& table, const TemplatesView& tv, const SceneView& sv,
-                   const SearchLaunch& sl, const SearchOutputs& out, cudaStream_t s);
+// Every warp stages the aligned longest template of the set in shared memory: a block runs 4, 2 or 1 warps, whichever
+// fits smem_optin (the device's cudaDevAttrMaxSharedMemoryPerBlockOptin).  search_max_template_lines(smem_optin) is the
+// longest template one warp can take; launch_search returns cudaErrorInvalidValue above it.
+int search_max_template_lines(int smem_optin);
+cudaError_t launch_search(const MapView& map, const SlopeTableDev& table, const TemplatesView& tv, const SceneView& sv,
+                          const SearchLaunch& sl, const SearchOutputs& out, int smem_optin, cudaStream_t s);
 
 // top-K smallest (score, index) among valid records; returns via d_out (k records) and d_n_out
 void launch_topk(const fdcm_match* d_rec, const uint8_t* d_valid, int64_t n, int k, float* d_ws_score, int64_t* d_ws_idx,

@@ -384,14 +384,32 @@ __global__ void __launch_bounds__(128, 6) search_warp_kernel(const __grid_consta
     }
 }
 
-void launch_search(const MapView& map, const SlopeTableDev& table, const TemplatesView& tv, const SceneView& sv,
-                   const SearchLaunch& sl, const SearchOutputs& out, cudaStream_t s) {
-    if (sl.n_hyp <= 0) return;
-    const int threads = 128, hyps = threads / 32;
-    const size_t smem = (size_t)hyps * ((size_t)tv.max_lines * 16 + (((size_t)tv.max_lines + 15) & ~(size_t)15));
-    if (smem > 48 * 1024) cudaFuncSetAttribute(search_warp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+// shared memory one warp of search_warp_kernel stages a template of max_lines lines in
+static size_t search_smem_per_warp(int max_lines) { return (size_t)max_lines * 16 + (((size_t)max_lines + 15) & ~(size_t)15); }
+
+int search_max_template_lines(int smem_optin) {
+    int L = smem_optin / 17;
+    while (search_smem_per_warp(L + 1) <= (size_t)smem_optin) ++L;
+    while (L > 0 && search_smem_per_warp(L) > (size_t)smem_optin) --L;
+    return L;
+}
+
+cudaError_t launch_search(const MapView& map, const SlopeTableDev& table, const TemplatesView& tv, const SceneView& sv,
+                          const SearchLaunch& sl, const SearchOutputs& out, int smem_optin, cudaStream_t s) {
+    if (sl.n_hyp <= 0) return cudaSuccess;
+    // 4 warps per block; long templates halve that until the block's staging fits the device's opt-in shared memory
+    const size_t per_warp = search_smem_per_warp(tv.max_lines);
+    int hyps = 4;
+    while (hyps > 1 && (size_t)hyps * per_warp > (size_t)smem_optin) hyps >>= 1;
+    const size_t smem = (size_t)hyps * per_warp;
+    if (smem > (size_t)smem_optin) return cudaErrorInvalidValue;   // callers reject such templates first
+    if (smem > 48 * 1024) {
+        const cudaError_t e = cudaFuncSetAttribute(search_warp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+    }
     const unsigned grid = (unsigned)((sl.n_hyp + hyps - 1) / hyps);
-    search_warp_kernel<<<grid, threads, smem, s>>>(map, table, tv, sv, sl, out);
+    search_warp_kernel<<<grid, hyps * 32, smem, s>>>(map, table, tv, sv, sl, out);
+    return cudaGetLastError();
 }
 
 // =============================================================================================

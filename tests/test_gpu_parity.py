@@ -72,7 +72,7 @@ def test_edge_masks_and_bins_bit_exact():
         assert np.array_equal(g.mask(d), (c.plane(d) == 0).astype(np.uint8)), f"edge mask of plane {d}"
 
 
-@pytest.mark.parametrize("depth", [1, 4, 7, 30])
+@pytest.mark.parametrize("depth", [1, 4, 7, 30, 64])   # 64: the largest depth, fills the propagation tables exactly
 def test_other_depths(depth):
     scene = synth_scene(200, 150, 40, seed=5)
     g = fdcm.build_cuda_featuremap(scene, fdcm.Dt3CudaParameters(depth, 3.0, 2.2, fdcm.distance.L2))
