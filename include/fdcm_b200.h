@@ -170,6 +170,38 @@ fdcm_status fdcm_templates_lengths(const fdcm_templates* t, float* lengths);
 #define FDCM_SCENE_RESIDENT (-1)
 fdcm_status fdcm_search(const fdcm_dt3* map, const fdcm_templates* templates, const float* scene_xyxy, int32_t n_scene,
                         const fdcm_search_params* params, fdcm_match* out, int64_t capacity, int64_t* n_out);
+/* ---- distinct top-K (beyond the reference) -------------------------------------------------
+ * Many hypotheses of one template converge on the same pose, so a plain top-K is mostly repeats.  The *_select entry
+ * points run the search like fdcm_search (top_k > 0, penalty, ConcentricRange and tmpl_idx_base as there) and then
+ * select on the device, from the valid matches ordered by ascending (score, hypothesis index), NaN as +inf:
+ * walk that order with an accepted list A (empty at first) and accept a candidate b iff
+ *   |A| < top_k, and
+ *   max_per_template == 0 or A holds fewer than max_per_template matches of b's template, and
+ *   radius == 0 or no a in A with near(a, b) has (across_templates || a's template == b's template);
+ * the result is A in acceptance order.  max_per_template == 0 and radius == 0 give exactly fdcm_search's top-K.
+ * near(a, b), in fp32 without contraction: the anchor of a template is the centre of the bounding box of its 2L end
+ * points ((min + max) * 0.5f per axis; (0, 0) for an empty template), the anchor of a match with transform T is
+ * ((T0*ax + T1*ay) + T2, (T3*ax + T4*ay) + T5); near holds iff dx*dx + dy*dy <= radius*radius for the difference of the
+ * two anchors and either max_angle >= 3.14159274f or Ta0*Tb0 + Ta3*Tb3 >= (float)cos((double)max_angle) (a reversed
+ * hypothesis carries -R, a rotation by pi).
+ * Cost: with across_templates == 0 every template is walked by its own warp (each rule only involves matches of one
+ * template, so this is the global walk); with across_templates != 0 one thread block walks the sorted list, worst case
+ * H x top_k anchor tests for H hypotheses, and top_k may not exceed FDCM_SELECT_MAX_ACROSS (the accepted list lives in
+ * shared memory).  Invalid parameters (top_k < 1, max_per_template < 0, radius negative or not finite, max_angle
+ * negative or NaN, that bound) fail with FDCM_ERR_INVALID. */
+#define FDCM_SELECT_MAX_ACROSS 1024
+typedef struct fdcm_select_params {      /* 16 bytes */
+    int32_t max_per_template;   /* > 0: at most this many matches of one template; 0: no cap */
+    float radius;               /* > 0: suppression radius (pixels) between match anchors; 0: no suppression */
+    float max_angle;            /* radians; with radius > 0, suppress only within this rotation; >= pi: any rotation */
+    int32_t across_templates;   /* 0: a match suppresses matches of its own template only; 1: of every template */
+} fdcm_select_params;
+fdcm_status fdcm_search_select(const fdcm_dt3* map, const fdcm_templates* templates, const float* scene_xyxy, int32_t n_scene,
+                               const fdcm_search_params* params, const fdcm_select_params* select,
+                               fdcm_match* out, int64_t capacity, int64_t* n_out);
+/* anchors of n_tmpl templates (CSR like fdcm_template_lengths), n_tmpl (x, y) pairs; host only */
+fdcm_status fdcm_template_anchors(const float* tmpl_lines, const int32_t* tmpl_offsets, int32_t n_tmpl, float* anchors_xy);
+
 /* optimize(optimizer, templates, alignments, featuremap) (matching/optimizestrategy.h:62-64; BatchOptimize:
  * batchoptimize.cpp:6-123, batch_size == 0: DefaultOptimize, defaultoptimize.cpp:6-93).  The templates are used
  * as given (already aligned); alignments: n_tmpl (x,y) pairs.  Outputs per template: has_value (0 = nullopt),
@@ -232,6 +264,10 @@ fdcm_status fdcm_scene_batch_create(const fdcm_dt3_params* params, int32_t devic
 fdcm_status fdcm_scene_batch_destroy(fdcm_scene_batch* batch);
 fdcm_status fdcm_search_scenes(fdcm_scene_batch* batch, const float* scene_lines, const int32_t* scene_offsets, int32_t n_scenes,
                                const fdcm_templates* templates, const fdcm_search_params* params, fdcm_match* out, int32_t* n_out);
+/* the same with the distinct top-K selection of fdcm_search_select in every scene */
+fdcm_status fdcm_search_scenes_select(fdcm_scene_batch* batch, const float* scene_lines, const int32_t* scene_offsets, int32_t n_scenes,
+                                      const fdcm_templates* templates, const fdcm_search_params* params,
+                                      const fdcm_select_params* select, fdcm_match* out, int32_t* n_out);
 
 /* ---- multi-GPU (SURVEY.md 8e): one process per GPU, templates sharded by tmpl_idx, NCCL over NVLink ------------
  * The reference has no distributed code; these entry points are what a multi-GPU host (C++ or Python) calls instead of
@@ -252,6 +288,12 @@ fdcm_status fdcm_comm_shard(int32_t n_items, int32_t rank, int32_t world, int32_
 fdcm_status fdcm_comm_search_topk(fdcm_comm* comm, const fdcm_dt3* map, const fdcm_templates* shard, const float* scene_xyxy,
                                   int32_t n_scene, const fdcm_search_params* params, fdcm_match* out, int64_t capacity,
                                   int64_t* n_out);
+/* fdcm_comm_search_topk with the distinct top-K selection of fdcm_search_select.  Only across_templates == 0: each rank's
+ * accepted list is then the global one restricted to its templates, so the same exchange yields the global result;
+ * across_templates != 0 fails with FDCM_ERR_INVALID (suppression across ranks does not decompose). */
+fdcm_status fdcm_comm_search_select(fdcm_comm* comm, const fdcm_dt3* map, const fdcm_templates* shard, const float* scene_xyxy,
+                                    int32_t n_scene, const fdcm_search_params* params, const fdcm_select_params* select,
+                                    fdcm_match* out, int64_t capacity, int64_t* n_out);
 /* the same with this rank's shard given as host templates (like fdcm_search_host: uploaded into a reusable device set) */
 fdcm_status fdcm_comm_search_host_topk(fdcm_comm* comm, const fdcm_dt3* map, const float* tmpl_lines, const int32_t* tmpl_offsets,
                                        int32_t n_tmpl, const float* scene_xyxy, int32_t n_scene, const fdcm_search_params* params,

@@ -232,6 +232,38 @@ inline std::vector<Match> searchTopK(const DefaultSearch& s, const BatchOptimize
     return detail::search((int)o.batchSize, s, fm, templates, scene, FDCM_PENALTY_EXPONENTIAL, pen.tau, k);
 }
 
+// distinct top-K (beyond the reference; rules of fdcm_search_select): at most maxPerTemplate matches of one template
+// (0: no cap), and with radius > 0 no two matches whose template anchors lie within radius pixels at a rotation
+// difference within maxAngle (>= pi: any), counted within one template unless acrossTemplates
+struct DistinctMatches {
+    int maxPerTemplate{0};
+    float radius{0.f};
+    float maxAngle{3.14159265358979323846f};
+    bool acrossTemplates{false};
+};
+inline std::vector<Match> searchTopK(const DefaultSearch& s, const BatchOptimize& o, const ExponentialPenalty& pen, const Dt3Cuda& fm,
+                                     const std::vector<LineArray>& templates, const LineArray& scene, int k, const DistinctMatches& select) {
+    std::vector<float> flat;
+    std::vector<int32_t> off;
+    detail::pack(templates, flat, off);
+    fdcm_templates* ts = nullptr;
+    check(fdcm_templates_create(flat.data(), off.data(), (int32_t)templates.size(), fm.info().device, &ts));
+    const std::unique_ptr<fdcm_templates, fdcm_status (*)(fdcm_templates*)> owner(ts, fdcm_templates_release);
+    const fdcm_search_params p{(int32_t)s.max_tmpl_lines, (int32_t)s.max_scene_lines, (int32_t)o.batchSize, FDCM_PENALTY_EXPONENTIAL,
+                               pen.tau, k, 0, 0, 0.f, 0.f, 0.f, 0.f};
+    const fdcm_select_params q{select.maxPerTemplate, select.radius, select.maxAngle, select.acrossTemplates ? 1 : 0};
+    std::vector<fdcm_match> rec((size_t)std::max(k, 1));
+    int64_t n = 0;
+    check(fdcm_search_select(fm.handle(), ts, scene.data(), (int32_t)(scene.size() / 4), &p, &q, rec.data(), (int64_t)rec.size(), &n));
+    std::vector<Match> out((size_t)n);
+    for (int64_t i = 0; i < n; ++i) {
+        out[(size_t)i].tmplIdx = rec[(size_t)i].tmpl_idx;
+        out[(size_t)i].score = rec[(size_t)i].score;
+        for (int c = 0; c < 6; ++c) out[(size_t)i].transform[(size_t)c] = rec[(size_t)i].transform[c];
+    }
+    return out;
+}
+
 // ---- PenaltyStrategy concept, template lengths, sort ----------------------------------------------
 inline std::vector<float> getTemplateLengths(const std::vector<LineArray>& templates) {   // core/math.h:319-324
     std::vector<float> flat, len(templates.size());

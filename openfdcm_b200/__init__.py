@@ -11,6 +11,7 @@ fallback.
 """
 import ctypes as C
 import enum
+import math
 
 import numpy as np
 
@@ -21,7 +22,8 @@ from ._lib import MATCH_DTYPE, FdcmError, check, lib, ptr
 __all__ = [
     "distance", "Dt3CudaParameters", "Dt3Cuda", "build_cuda_featuremap", "ThreadPool", "DefaultSearch", "ConcentricRangeStrategy",
     "BatchOptimize", "DefaultOptimize", "DefaultMatch", "DefaultPenalty", "ExponentialPenalty", "Match",
-    "TemplateSet", "SceneBatch", "search", "search_topk", "penalize", "get_template_lengths", "sort_matches", "evaluate",
+    "TemplateSet", "SceneBatch", "DistinctMatches", "search", "search_topk", "penalize", "get_template_lengths",
+    "get_template_anchors", "sort_matches", "evaluate",
     "minmax_translation", "get_feature_size", "establish_search_strategy", "optimize", "read", "write", "FdcmError", "MATCH_DTYPE",
 ]
 
@@ -305,7 +307,28 @@ class TemplateSet:
         return out
 
 
-def _search_raw(featuremap, templates, scene, searcher, optimizer, penalty=None, top_k=0, tmpl_idx_base=0):
+class DistinctMatches:
+    """Distinct top-K (beyond the reference): from the matches in ascending (score, hypothesis) order, keep a match only
+    while fewer than `top_k` are kept, fewer than `max_per_template` of its template are kept (0: no cap) and, with
+    `radius` > 0, no kept match lies near it: template anchors (bounding-box centres) mapped by the two transforms within
+    `radius` pixels and rotations within `max_angle` radians (>= pi: any rotation), counting kept matches of its own
+    template only unless `across_templates` (at most top-k 1024 then).  Exact rules: include/fdcm_b200.h."""
+
+    def __init__(self, max_per_template=0, radius=0.0, max_angle=math.pi, across_templates=False):
+        self.max_per_template = int(max_per_template)
+        self.radius = float(radius)
+        self.max_angle = float(max_angle)
+        self.across_templates = bool(across_templates)
+
+    def _params(self):
+        return _lib.SelectParams(self.max_per_template, self.radius, self.max_angle, 1 if self.across_templates else 0)
+
+    def __repr__(self):
+        return (f"<DistinctMatches: max_per_template={self.max_per_template}, radius={self.radius}, max_angle={self.max_angle}, "
+                f"across_templates={self.across_templates}>")
+
+
+def _search_raw(featuremap, templates, scene, searcher, optimizer, penalty=None, top_k=0, tmpl_idx_base=0, select=None):
     if not isinstance(featuremap, Dt3Cuda):
         raise TypeError("the CUDA search needs a Dt3Cuda feature map (build_cuda_featuremap)")
     tset = templates if isinstance(templates, TemplateSet) else TemplateSet(templates, featuremap.device)
@@ -318,12 +341,17 @@ def _search_raw(featuremap, templates, scene, searcher, optimizer, penalty=None,
                           searcher.low_boundary if conc else 0.0, searcher.high_boundary if conc else 0.0)
     if tset.n_tmpl == 0:
         return np.zeros(0, MATCH_DTYPE)
-    cap = int(top_k) if top_k > 0 else 2 * tset.n_tmpl * max(1, min(searcher.max_tmpl_lines, tset.max_lines)) * max(
+    cap = int(top_k) if top_k > 0 or select is not None else 2 * tset.n_tmpl * max(1, min(searcher.max_tmpl_lines, tset.max_lines)) * max(
         1, searcher.max_scene_lines)
     out = np.zeros(max(cap, 1), MATCH_DTYPE)
     n = C.c_int64(0)
-    check(lib().fdcm_search(featuremap._h, tset._h, ptr(s), _lib.FDCM_SCENE_RESIDENT if s is None else s.shape[0], C.byref(p), ptr(out),
-                            out.shape[0], C.byref(n)))
+    n_scene = _lib.FDCM_SCENE_RESIDENT if s is None else s.shape[0]
+    if select is None:
+        check(lib().fdcm_search(featuremap._h, tset._h, ptr(s), n_scene, C.byref(p), ptr(out), out.shape[0], C.byref(n)))
+    else:
+        sp = select._params()
+        check(lib().fdcm_search_select(featuremap._h, tset._h, ptr(s), n_scene, C.byref(p), C.byref(sp), ptr(out), out.shape[0],
+                                       C.byref(n)))
     return out[: n.value]
 
 
@@ -332,9 +360,10 @@ def search(matcher, searcher, optimizer, featuremap, templates, scene):
     return _to_matches(_search_raw(featuremap, templates, scene, searcher, optimizer))
 
 
-def search_topk(featuremap, templates, scene, searcher, optimizer, penalty=None, k=10, tmpl_idx_base=0):
-    """Fused search -> penalize -> top-k on the device; returns a MATCH_DTYPE record array (ascending score)."""
-    return _search_raw(featuremap, templates, scene, searcher, optimizer, penalty, k, tmpl_idx_base).copy()
+def search_topk(featuremap, templates, scene, searcher, optimizer, penalty=None, k=10, tmpl_idx_base=0, *, select=None):
+    """Fused search -> penalize -> top-k on the device; returns a MATCH_DTYPE record array (ascending score).
+    select: a DistinctMatches for the distinct top-k (the kept matches in acceptance order, also ascending score)."""
+    return _search_raw(featuremap, templates, scene, searcher, optimizer, penalty, k, tmpl_idx_base, select).copy()
 
 
 def search_all(featuremap, templates, scene, searcher, optimizer, penalty=None, tmpl_idx_base=0):
@@ -359,8 +388,8 @@ class SceneBatch:
         if h and lib is not None:   # (module globals are gone when the interpreter shuts down)
             lib().fdcm_scene_batch_destroy(h)
 
-    def search_topk(self, scenes, templates, searcher, optimizer, penalty=None, k=10, tmpl_idx_base=0):
-        """-> list (one per scene) of MATCH_DTYPE arrays (ascending score)."""
+    def search_topk(self, scenes, templates, searcher, optimizer, penalty=None, k=10, tmpl_idx_base=0, *, select=None):
+        """-> list (one per scene) of MATCH_DTYPE arrays (ascending score); select: a DistinctMatches, like search_topk."""
         tset = templates if isinstance(templates, TemplateSet) else TemplateSet(templates, self.device)
         flat, off = _pack(scenes)
         p = _lib.SearchParams(searcher.max_tmpl_lines, searcher.max_scene_lines, int(optimizer.batch_size),
@@ -369,7 +398,11 @@ class SceneBatch:
         n = len(off) - 1
         out = np.zeros((max(n, 1), int(k)), MATCH_DTYPE)
         cnt = np.zeros(max(n, 1), np.int32)
-        check(lib().fdcm_search_scenes(self._h, ptr(flat), ptr(off), n, tset._h, C.byref(p), ptr(out), ptr(cnt)))
+        if select is None:
+            check(lib().fdcm_search_scenes(self._h, ptr(flat), ptr(off), n, tset._h, C.byref(p), ptr(out), ptr(cnt)))
+        else:
+            sp = select._params()
+            check(lib().fdcm_search_scenes_select(self._h, ptr(flat), ptr(off), n, tset._h, C.byref(p), C.byref(sp), ptr(out), ptr(cnt)))
         return [out[i, : cnt[i]].copy() for i in range(n)]
 
 
@@ -390,6 +423,15 @@ def get_template_lengths(templates):
     out = np.zeros(len(off) - 1, np.float32)
     check(lib().fdcm_template_lengths(ptr(flat), ptr(off), len(off) - 1, ptr(out)))
     return out.tolist()
+
+
+def get_template_anchors(templates):
+    """Anchor of every template for DistinctMatches: the centre of the bounding box of its line end points, (0, 0) when
+    empty; an (n_tmpl, 2) float32 array."""
+    flat, off = _pack(templates)
+    out = np.zeros((len(off) - 1, 2), np.float32)
+    check(lib().fdcm_template_anchors(ptr(flat), ptr(off), len(off) - 1, ptr(out)))
+    return out
 
 
 def sort_matches(matches):

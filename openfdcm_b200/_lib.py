@@ -27,6 +27,10 @@ class SearchParams(C.Structure):
                 ("low_radius", C.c_float), ("high_radius", C.c_float)]
 
 
+class SelectParams(C.Structure):
+    _fields_ = [("max_per_template", C.c_int32), ("radius", C.c_float), ("max_angle", C.c_float), ("across_templates", C.c_int32)]
+
+
 class Dt3Info(C.Structure):
     _fields_ = [("depth", C.c_int32), ("width", C.c_int32), ("height", C.c_int32), ("pitch", C.c_int32),
                 ("scene_translation", C.c_float * 2), ("distance", C.c_int32), ("device", C.c_int32),
@@ -65,6 +69,9 @@ SIGNATURES = {
     "fdcm_templates_release": (C.c_int, [_P]),
     "fdcm_templates_lengths": (C.c_int, [_P, _P]),
     "fdcm_search": (C.c_int, [_P, _P, _P, C.c_int32, C.POINTER(SearchParams), _P, C.c_int64, C.POINTER(C.c_int64)]),
+    "fdcm_search_select": (C.c_int, [_P, _P, _P, C.c_int32, C.POINTER(SearchParams), C.POINTER(SelectParams), _P, C.c_int64,
+                                     C.POINTER(C.c_int64)]),
+    "fdcm_template_anchors": (C.c_int, [_P, _P, C.c_int32, _P]),
     "fdcm_optimize": (C.c_int, [_P, _P, _P, C.c_int32, _P, C.c_int32, _P, _P, _P]),
     "fdcm_search_host": (C.c_int, [_P, _P, _P, C.c_int32, _P, C.c_int32, C.POINTER(SearchParams), _P, C.c_int64,
                                    C.POINTER(C.c_int64)]),
@@ -92,6 +99,8 @@ SIGNATURES = {
     "fdcm_comm_info": (C.c_int, [_P, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     "fdcm_comm_shard": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     "fdcm_comm_search_topk": (C.c_int, [_P, _P, _P, _P, C.c_int32, C.POINTER(SearchParams), _P, C.c_int64, C.POINTER(C.c_int64)]),
+    "fdcm_comm_search_select": (C.c_int, [_P, _P, _P, _P, C.c_int32, C.POINTER(SearchParams), C.POINTER(SelectParams), _P, C.c_int64,
+                                          C.POINTER(C.c_int64)]),
     "fdcm_comm_search_host_topk": (C.c_int, [_P, _P, _P, _P, C.c_int32, _P, C.c_int32, C.POINTER(SearchParams), _P, C.c_int64,
                                              C.POINTER(C.c_int64)]),
     "fdcm_comm_rebuild_broadcast": (C.c_int, [_P, _P, _P, C.c_int32, C.c_int32]),
@@ -99,6 +108,7 @@ SIGNATURES = {
     "fdcm_scene_batch_create": (C.c_int, [C.POINTER(Dt3Params), C.c_int32, C.POINTER(_P)]),
     "fdcm_scene_batch_destroy": (C.c_int, [_P]),
     "fdcm_search_scenes": (C.c_int, [_P, _P, _P, C.c_int32, _P, C.POINTER(SearchParams), _P, _P]),
+    "fdcm_search_scenes_select": (C.c_int, [_P, _P, _P, C.c_int32, _P, C.POINTER(SearchParams), C.POINTER(SelectParams), _P, _P]),
 }
 
 

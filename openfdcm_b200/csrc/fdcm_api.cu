@@ -290,6 +290,7 @@ struct fdcm_dt3 {
     mutable std::mutex search_mutex;
     mutable DevBuf s_scene, s_sorted_len, s_sorted_idx, s_hyp_off, s_rec, s_valid, s_hyp, s_counters, s_topk_score, s_topk_idx,
         s_topk_out, s_topk_n, s_keys, s_keys2, s_idx, s_perm, s_sort_tmp;
+    mutable DevBuf s_sel_keys, s_sel_keys2, s_sel_vals, s_sel_vals2, s_sel_surv, s_sel_acc, s_sel_tmp;   // distinct top-K
     mutable float s_scene_min[2] = {0.f, 0.f}, s_scene_max[2] = {0.f, 0.f};   // bbox of the resident search scene
     mutable std::mutex host_tset_mutex;
     mutable fdcm_templates* host_tset = nullptr;   // reusable template set of fdcm_search_host
@@ -311,7 +312,8 @@ struct fdcm_dt3 {
         cudaSetDevice(device);
         for (DevBuf* b : {&planes, &mask, &stack, &lines, &bins, &band_info, &band_spill, &integ_items, &s_scene, &s_sorted_len, &s_sorted_idx, &s_hyp_off, &s_rec,
                           &s_valid, &s_hyp, &s_counters, &s_topk_score, &s_topk_idx, &s_topk_out, &s_topk_n, &s_keys, &s_keys2, &s_idx,
-                          &s_perm, &s_sort_tmp})
+                          &s_perm, &s_sort_tmp, &s_sel_keys, &s_sel_keys2, &s_sel_vals, &s_sel_vals2, &s_sel_surv, &s_sel_acc,
+                          &s_sel_tmp})
             b->release();
         if (h_pinned) cudaFreeHost(h_pinned);
         if (ev_fork) cudaEventDestroy(ev_fork);
@@ -1029,7 +1031,8 @@ struct fdcm_templates {
     std::vector<float> lengths;       // getTemplateLengths
     PinnedVec<float> h_line_len;      // host scratch kept for reloads (pinned: uploaded every fdcm_search_host)
     PinnedVec<int32_t> h_argsort;
-    DevBuf lines, offs, argsort, line_len, denom;
+    PinnedVec<float> h_anchors;       // 2 per template (fdcm_template_anchors)
+    DevBuf lines, offs, argsort, line_len, denom, anchors;
     int denom_kind = -1;
     float denom_tau = 0.f;
     std::mutex mu;
@@ -1051,7 +1054,7 @@ struct fdcm_templates {
         cudaSetDevice(device);
         if (ready) cudaEventDestroy(ready);
         if (h_stage) cudaFreeHost(h_stage);
-        for (DevBuf* b : {&lines, &offs, &argsort, &line_len, &denom}) b->release();
+        for (DevBuf* b : {&lines, &offs, &argsort, &line_len, &denom, &anchors}) b->release();
     }
 };
 
@@ -1137,6 +1140,19 @@ void fdcm_dt3::destroy_host_tset() {
     host_tset = nullptr;
 }
 
+// anchor of a template for the distinct top-K: centre of the bounding box of its 2 L end points, (0, 0) when empty
+static void template_anchor(const float* lines, int L, float* xy) {
+    if (L <= 0) { xy[0] = xy[1] = 0.f; return; }
+    float mnx = lines[0], mxx = lines[0], mny = lines[1], mxy = lines[1];
+    for (int i = 0; i < 2 * L; ++i) {
+        const float x = lines[2 * (size_t)i], y = lines[2 * (size_t)i + 1];
+        mnx = std::min(mnx, x); mxx = std::max(mxx, x);
+        mny = std::min(mny, y); mxy = std::max(mxy, y);
+    }
+    xy[0] = (mnx + mxx) * 0.5f;
+    xy[1] = (mny + mxy) * 0.5f;
+}
+
 // need_ranks: how many leading entries of every template's length order the caller will read (DefaultSearch only aligns the
 // max_tmpl_lines longest lines, defaultsearch.cpp:35-38); <= 0: the whole order.  When the need_ranks + 1 largest lengths
 // of a template are pairwise distinct, the leading ranks of ANY correct descending sort are the same as std::sort's, and a
@@ -1144,11 +1160,12 @@ void fdcm_dt3::destroy_host_tset() {
 // keys depends on the algorithm.  (Host cores are shared by all ranks of a node: at 8 GPUs per 16 cores the full sort of
 // 5000 templates per step no longer hid behind the map build.)
 static void template_host_prep(const float* tl, const int32_t* off, int32_t T, float* line_len /* off[T] */,
-                               int32_t* argsort /* off[T] */, std::vector<float>& lengths, int need_ranks = 0) {
+                               int32_t* argsort /* off[T] */, float* anchors /* 2 T */, std::vector<float>& lengths, int need_ranks = 0) {
     lengths.resize((size_t)T);
     auto work = [&](int t0, int t1) {
         for (int t = t0; t < t1; ++t) {
             const int l0 = off[t], L = off[t + 1] - off[t];
+            template_anchor(tl + 4 * (size_t)l0, L, anchors + 2 * (size_t)t);
             float* len = line_len + l0;
             int32_t* idx = argsort + l0;
             for (int i = 0; i < L; ++i) {
@@ -1229,16 +1246,20 @@ static fdcm_status templates_load(fdcm_templates* t, const float* tmpl_lines, co
     for (int i = 0; i < n_tmpl; ++i) t->max_lines = std::max(t->max_lines, tmpl_offsets[i + 1] - tmpl_offsets[i]);
     CUDA_TRY(t->h_line_len.resize((size_t)std::max<int64_t>(n, 1)));
     CUDA_TRY(t->h_argsort.resize((size_t)std::max<int64_t>(n, 1)));
-    template_host_prep(tmpl_lines, tmpl_offsets, n_tmpl, t->h_line_len.data(), t->h_argsort.data(), t->lengths, need_ranks);
+    CUDA_TRY(t->h_anchors.resize((size_t)std::max<int32_t>(2 * n_tmpl, 2)));
+    template_host_prep(tmpl_lines, tmpl_offsets, n_tmpl, t->h_line_len.data(), t->h_argsort.data(), t->h_anchors.data(), t->lengths,
+                       need_ranks);
     cudaError_t e = t->lines.reserve(std::max<size_t>(16, (size_t)n * 16));
     if (e == cudaSuccess) e = t->offs.reserve((size_t)(n_tmpl + 1) * 4);
     if (e == cudaSuccess) e = t->argsort.reserve(std::max<size_t>(4, (size_t)n * 4));
     if (e == cudaSuccess) e = t->line_len.reserve(std::max<size_t>(4, (size_t)n * 4));
     if (e == cudaSuccess) e = t->denom.reserve(std::max<size_t>(4, (size_t)n_tmpl * 4));
+    if (e == cudaSuccess) e = t->anchors.reserve(std::max<size_t>(8, (size_t)n_tmpl * 8));
     if (e == cudaSuccess && n) e = cudaMemcpyAsync(t->lines.p, tmpl_lines, (size_t)n * 16, cudaMemcpyHostToDevice, s);
     if (e == cudaSuccess) e = cudaMemcpyAsync(t->offs.p, tmpl_offsets, (size_t)(n_tmpl + 1) * 4, cudaMemcpyHostToDevice, s);
     if (e == cudaSuccess && n) e = cudaMemcpyAsync(t->argsort.p, t->h_argsort.data(), (size_t)n * 4, cudaMemcpyHostToDevice, s);
     if (e == cudaSuccess && n) e = cudaMemcpyAsync(t->line_len.p, t->h_line_len.data(), (size_t)n * 4, cudaMemcpyHostToDevice, s);
+    if (e == cudaSuccess && n_tmpl) e = cudaMemcpyAsync(t->anchors.p, t->h_anchors.data(), (size_t)n_tmpl * 8, cudaMemcpyHostToDevice, s);
     // no host synchronisation needed: pageable sources are staged by the runtime before the call returns
     if (e == cudaSuccess) e = cudaEventRecord(t->ready, s);
     if (e != cudaSuccess)
@@ -1277,6 +1298,16 @@ extern "C" fdcm_status fdcm_templates_release(fdcm_templates* t) {
 extern "C" fdcm_status fdcm_templates_lengths(const fdcm_templates* t, float* lengths) {
     if (!t || !lengths) return fail(FDCM_ERR_INVALID, "null argument");
     std::memcpy(lengths, t->lengths.data(), t->lengths.size() * sizeof(float));
+    return FDCM_OK;
+}
+
+extern "C" fdcm_status fdcm_template_anchors(const float* tl, const int32_t* off, int32_t T, float* anchors_xy) {
+    if (T < 0 || !off || (T > 0 && !anchors_xy)) return fail(FDCM_ERR_INVALID, "null argument");
+    for (int t = 0; t < T; ++t) {
+        if (off[t + 1] < off[t]) return fail(FDCM_ERR_INVALID, "template offsets must be non-decreasing");
+        if (off[t + 1] > off[t] && !tl) return fail(FDCM_ERR_INVALID, "tmpl_lines is null");
+    }
+    for (int t = 0; t < T; ++t) template_anchor(tl + 4 * (size_t)off[t], off[t + 1] - off[t], anchors_xy + 2 * (size_t)t);
     return FDCM_OK;
 }
 
@@ -1470,10 +1501,83 @@ static fdcm_status search_smem_optin(int device, int max_lines, int* smem_optin)
     return FDCM_OK;
 }
 
+// parameters of the distinct top-K (fdcm_search_select)
+static fdcm_status check_select(const fdcm_select_params* q, int32_t top_k, bool comm) {
+    if (top_k < 1) return fail(FDCM_ERR_INVALID, "distinct top-K: top_k must be >= 1");
+    if (q->max_per_template < 0) return fail(FDCM_ERR_INVALID, "distinct top-K: max_per_template must be >= 0");
+    if (!(q->radius >= 0.f) || !std::isfinite(q->radius)) return fail(FDCM_ERR_INVALID, "distinct top-K: radius must be finite and >= 0");
+    if (!(q->max_angle >= 0.f)) return fail(FDCM_ERR_INVALID, "distinct top-K: max_angle must be >= 0 (and not NaN)");
+    if (q->across_templates && comm)
+        return fail(FDCM_ERR_INVALID, "distinct top-K: across_templates is not supported by the multi-GPU search (it does not decompose over template shards)");
+    if (q->across_templates && top_k > FDCM_SELECT_MAX_ACROSS)
+        return fail(FDCM_ERR_INVALID, "distinct top-K: across_templates takes top_k <= " + std::to_string(FDCM_SELECT_MAX_ACROSS));
+    return FDCM_OK;
+}
+
+// Distinct top-K over the records the search kernel just queued on `s`: writes s_topk_out / s_topk_n like the top-K kernels
+static fdcm_status run_select(const fdcm_dt3* m, const fdcm_templates* t, const fdcm_search_params* p, const fdcm_select_params* q,
+                              int64_t H, cudaStream_t s) {
+    if (H >= ((int64_t)1 << 31)) return fail(FDCM_ERR_INVALID, "distinct top-K: more than 2^31 - 1 hypotheses");
+    SelectLaunch sp;
+    sp.rec = m->s_rec.as<fdcm_match>();
+    sp.valid = m->s_valid.as<uint8_t>();
+    sp.hyp_off = m->s_hyp_off.as<int64_t>();
+    sp.anchors = t->anchors.as<float2>();
+    sp.n_hyp = H;
+    sp.n_tmpl = t->n_tmpl;
+    sp.tmpl_idx_base = p->tmpl_idx_base;
+    sp.top_k = p->top_k;
+    sp.cap = q->max_per_template;
+    sp.radius_on = q->radius > 0.f;
+    sp.r2 = q->radius * q->radius;
+    sp.any_angle = q->max_angle >= 3.14159274f;
+    sp.cos_thr = (float)std::cos((double)q->max_angle);
+    const bool within = q->across_templates == 0;
+    const size_t tmp = select_temp_bytes(H);
+    CUDA_TRY(m->s_sel_keys.reserve((size_t)H * 8));
+    CUDA_TRY(m->s_sel_keys2.reserve((size_t)H * 8));
+    CUDA_TRY(m->s_sel_vals.reserve((size_t)H * 4));
+    CUDA_TRY(m->s_sel_vals2.reserve((size_t)H * 4));
+    CUDA_TRY(m->s_sel_tmp.reserve(std::max<size_t>(tmp, 16)));
+    uint64_t* keys = m->s_sel_keys.as<uint64_t>();
+    uint64_t* sorted_keys = m->s_sel_keys2.as<uint64_t>();
+    int32_t* iota = m->s_sel_vals.as<int32_t>();
+    int32_t* sorted_h = m->s_sel_vals2.as<int32_t>();
+    {
+        KernelScope k("select_sort", 0.0, s, 1);   // our key kernel; the CUB radix-sort launches are library code
+        launch_select_sort(sp, within, keys, sorted_keys, iota, sorted_h, m->s_sel_tmp.p, tmp, s);
+    }
+    fdcm_match* d_out = m->s_topk_out.as<fdcm_match>();
+    int* d_n = m->s_topk_n.as<int>();
+    if (within) {
+        CUDA_TRY(m->s_sel_surv.reserve((size_t)H * 4));
+        if (sp.radius_on) CUDA_TRY(m->s_sel_acc.reserve((size_t)H * 16));
+        {
+            KernelScope k("select_greedy", 0.0, s);
+            launch_select_greedy(sp, sorted_keys, sorted_h, m->s_sel_surv.as<uint32_t>(), m->s_sel_acc.as<float4>(), s);
+        }
+        // the unsorted keys and the per-template order are free again: they take the global sort of the survivors
+        KernelScope k("select_topk", 0.0, s, 1);
+        launch_select_topk(sp, m->s_sel_surv.as<uint32_t>(), reinterpret_cast<uint32_t*>(keys), iota, sorted_h, m->s_sel_tmp.p, tmp, d_out,
+                           d_n, s);
+    } else {
+        KernelScope k("select_walk", 0.0, s);
+        launch_select_walk(sp, sorted_keys, sorted_h, d_out, d_n, s);
+    }
+    CUDA_TRY(cudaGetLastError());
+    return FDCM_OK;
+}
+
+// sel: distinct top-K (fdcm_search_select); nullptr for the plain search
 static fdcm_status search_impl(const fdcm_dt3* m, const fdcm_templates* tc, const float* scene, int32_t n_scene,
-                               const fdcm_search_params* p, fdcm_match* out, int64_t capacity, int64_t* n_out, fdcm_comm* comm) {
+                               const fdcm_search_params* p, fdcm_match* out, int64_t capacity, int64_t* n_out, fdcm_comm* comm,
+                               const fdcm_select_params* sel) {
     if (!m || !tc || !p || !n_out) return fail(FDCM_ERR_INVALID, "null argument");
     *n_out = 0;
+    if (sel)
+        if (fdcm_status st = check_select(sel, p->top_k, comm != nullptr)) return st;
+    // caps and radius both off: the selection is the plain top-K
+    if (sel && sel->max_per_template == 0 && !(sel->radius > 0.f)) sel = nullptr;
     if (comm && p->top_k <= 0) return fail(FDCM_ERR_INVALID, "the multi-GPU search needs top_k > 0");
 #define FDCM_NO_LOCAL_MATCHES() do { if (comm) return exchange_empty(m, comm, p->top_k, out, capacity, n_out); return FDCM_OK; } while (0)
     if (p->max_tmpl_lines < 0 || p->max_scene_lines < 0 || p->batch_size < 0 || p->top_k < 0 || p->penalty_kind < 0 ||
@@ -1619,17 +1723,23 @@ static fdcm_status search_impl(const fdcm_dt3* m, const fdcm_templates* tc, cons
     fdcm_status result = FDCM_OK;
     if (p->top_k > 0) {
         const int k = p->top_k;
-        const int blocks = topk_ws_blocks(H);
-        CUDA_TRY(m->s_topk_score.reserve((size_t)blocks * k * 4));
-        CUDA_TRY(m->s_topk_idx.reserve((size_t)blocks * k * 8));
-        CUDA_TRY(m->s_topk_out.reserve((size_t)k * sizeof(fdcm_match)));
-        CUDA_TRY(m->s_topk_n.reserve(4));
-        {
-            KernelScope ks("topk", 0.0, s, 2);   // two kernels in this scope
-            launch_topk(so.rec, so.valid, H, k, m->s_topk_score.as<float>(), m->s_topk_idx.as<int64_t>(), blocks,
-                        m->s_topk_out.as<fdcm_match>(), m->s_topk_n.as<int>(), s);
+        if (sel) {
+            CUDA_TRY(m->s_topk_out.reserve((size_t)k * sizeof(fdcm_match)));
+            CUDA_TRY(m->s_topk_n.reserve(4));
+            if (fdcm_status st = run_select(m, t, p, sel, H, s)) return st;
+        } else {
+            const int blocks = topk_ws_blocks(H);
+            CUDA_TRY(m->s_topk_score.reserve((size_t)blocks * k * 4));
+            CUDA_TRY(m->s_topk_idx.reserve((size_t)blocks * k * 8));
+            CUDA_TRY(m->s_topk_out.reserve((size_t)k * sizeof(fdcm_match)));
+            CUDA_TRY(m->s_topk_n.reserve(4));
+            {
+                KernelScope ks("topk", 0.0, s, 2);   // two kernels in this scope
+                launch_topk(so.rec, so.valid, H, k, m->s_topk_score.as<float>(), m->s_topk_idx.as<int64_t>(), blocks,
+                            m->s_topk_out.as<fdcm_match>(), m->s_topk_n.as<int>(), s);
+            }
+            CUDA_TRY(cudaGetLastError());
         }
-        CUDA_TRY(cudaGetLastError());
         result = finish_topk(m, comm, k, s, counters, out, capacity, n_out);
         if (result != FDCM_OK && result != FDCM_ERR_CAPACITY) return result;
     } else {
@@ -1667,7 +1777,14 @@ static fdcm_status search_impl(const fdcm_dt3* m, const fdcm_templates* tc, cons
 
 extern "C" fdcm_status fdcm_search(const fdcm_dt3* m, const fdcm_templates* tc, const float* scene, int32_t n_scene,
                                    const fdcm_search_params* p, fdcm_match* out, int64_t capacity, int64_t* n_out) {
-    return search_impl(m, tc, scene, n_scene, p, out, capacity, n_out, nullptr);
+    return search_impl(m, tc, scene, n_scene, p, out, capacity, n_out, nullptr, nullptr);
+}
+
+extern "C" fdcm_status fdcm_search_select(const fdcm_dt3* m, const fdcm_templates* tc, const float* scene, int32_t n_scene,
+                                          const fdcm_search_params* p, const fdcm_select_params* select, fdcm_match* out, int64_t capacity,
+                                          int64_t* n_out) {
+    if (!select) return fail(FDCM_ERR_INVALID, "select is null");
+    return search_impl(m, tc, scene, n_scene, p, out, capacity, n_out, nullptr, select);
 }
 
 // fdcm_search of this rank's template shard (params->tmpl_idx_base = first global index of the shard) followed by the
@@ -1676,7 +1793,15 @@ extern "C" fdcm_status fdcm_comm_search_topk(fdcm_comm* comm, const fdcm_dt3* m,
                                              int32_t n_scene, const fdcm_search_params* p, fdcm_match* out, int64_t capacity,
                                              int64_t* n_out) {
     if (!comm) return fail(FDCM_ERR_INVALID, "comm is null");
-    return search_impl(m, shard, scene, n_scene, p, out, capacity, n_out, comm);
+    return search_impl(m, shard, scene, n_scene, p, out, capacity, n_out, comm, nullptr);
+}
+
+extern "C" fdcm_status fdcm_comm_search_select(fdcm_comm* comm, const fdcm_dt3* m, const fdcm_templates* shard, const float* scene,
+                                               int32_t n_scene, const fdcm_search_params* p, const fdcm_select_params* select,
+                                               fdcm_match* out, int64_t capacity, int64_t* n_out) {
+    if (!comm) return fail(FDCM_ERR_INVALID, "comm is null");
+    if (!select) return fail(FDCM_ERR_INVALID, "select is null");
+    return search_impl(m, shard, scene, n_scene, p, out, capacity, n_out, comm, select);
 }
 
 // Scene feature map on every rank without building it everywhere: all ranks run the O(#lines) host preparation of the same
@@ -1780,8 +1905,9 @@ static fdcm_status batch_queue_build(fdcm_scene_batch* b, int slot, const float*
     return FDCM_OK;
 }
 
-extern "C" fdcm_status fdcm_search_scenes(fdcm_scene_batch* b, const float* scene_lines, const int32_t* scene_offsets, int32_t n_scenes,
-                                          const fdcm_templates* templates, const fdcm_search_params* p, fdcm_match* out, int32_t* n_out) {
+static fdcm_status search_scenes_impl(fdcm_scene_batch* b, const float* scene_lines, const int32_t* scene_offsets, int32_t n_scenes,
+                                      const fdcm_templates* templates, const fdcm_search_params* p, const fdcm_select_params* sel,
+                                      fdcm_match* out, int32_t* n_out) {
     if (!b || !p || n_scenes < 0) return fail(FDCM_ERR_INVALID, "bad argument");
     if (n_scenes == 0) return FDCM_OK;
     if (!scene_offsets || !templates || !out || !n_out) return fail(FDCM_ERR_INVALID, "null argument");
@@ -1804,11 +1930,26 @@ extern "C" fdcm_status fdcm_search_scenes(fdcm_scene_batch* b, const float* scen
         CUDA_TRY(cudaStreamWaitEvent(main_s, b->built[slot], 0));
         int64_t n = 0;
         fdcm_search_params ps = *p;
-        const fdcm_status st = search_impl(b->maps[slot], templates, nullptr, FDCM_SCENE_RESIDENT, &ps, out + (size_t)s * p->top_k, p->top_k, &n, nullptr);
+        const fdcm_status st = search_impl(b->maps[slot], templates, nullptr, FDCM_SCENE_RESIDENT, &ps, out + (size_t)s * p->top_k, p->top_k, &n, nullptr,
+                                           sel);
         if (st != FDCM_OK) return st;
         n_out[s] = (int32_t)n;
     }
     return FDCM_OK;
+}
+
+extern "C" fdcm_status fdcm_search_scenes(fdcm_scene_batch* b, const float* scene_lines, const int32_t* scene_offsets, int32_t n_scenes,
+                                          const fdcm_templates* templates, const fdcm_search_params* p, fdcm_match* out, int32_t* n_out) {
+    return search_scenes_impl(b, scene_lines, scene_offsets, n_scenes, templates, p, nullptr, out, n_out);
+}
+
+extern "C" fdcm_status fdcm_search_scenes_select(fdcm_scene_batch* b, const float* scene_lines, const int32_t* scene_offsets, int32_t n_scenes,
+                                                 const fdcm_templates* templates, const fdcm_search_params* p, const fdcm_select_params* select,
+                                                 fdcm_match* out, int32_t* n_out) {
+    if (!select) return fail(FDCM_ERR_INVALID, "select is null");
+    if (p)
+        if (fdcm_status st = check_select(select, p->top_k, false)) return st;
+    return search_scenes_impl(b, scene_lines, scene_offsets, n_scenes, templates, p, select, out, n_out);
 }
 
 // optimize(optimizer, templates, alignments, featuremap) (matching/optimizestrategy.h:62-64;
@@ -1900,7 +2041,7 @@ static fdcm_status search_host_impl(const fdcm_dt3* m, const float* tmpl_lines, 
     static const int32_t zero_off[1] = {0};
     // (this template set lives for this one search: only the ranks DefaultSearch / ConcentricRange will read are ordered)
     if (fdcm_status st = templates_load(m->host_tset, tmpl_lines, n_tmpl ? tmpl_offsets : zero_off, n_tmpl, s, p ? p->max_tmpl_lines : 0)) return st;
-    return search_impl(m, m->host_tset, scene, n_scene, p, out, capacity, n_out, comm);
+    return search_impl(m, m->host_tset, scene, n_scene, p, out, capacity, n_out, comm, nullptr);
 }
 
 extern "C" fdcm_status fdcm_search_host(const fdcm_dt3* m, const float* tmpl_lines, const int32_t* tmpl_offsets, int32_t n_tmpl,

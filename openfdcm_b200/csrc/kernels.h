@@ -128,6 +128,40 @@ int topk_ws_blocks(int64_t n);
 void launch_topk_merge(const fdcm_match* d_gathered, int n_cand, int k, fdcm_match* d_out, int* d_n_out, cudaStream_t s);
 void launch_topk_invalid(fdcm_match* d_out, int k, int* d_n_out, cudaStream_t s);
 
+// distinct top-K (fdcm_search_select): selection over the records / valid flags the search kernel left in HBM
+struct SelectLaunch {
+    const fdcm_match* rec;       // n_hyp records, valid ones written by the search
+    const uint8_t* valid;        // n_hyp flags
+    const int64_t* hyp_off;      // n_tmpl + 1: the hypotheses of template t are [hyp_off[t], hyp_off[t+1])
+    const float2* anchors;       // n_tmpl template anchors (bounding-box centres)
+    int64_t n_hyp;
+    int32_t n_tmpl, tmpl_idx_base;
+    int32_t top_k;
+    int32_t cap;                 // max_per_template (0: none)
+    int32_t radius_on, any_angle;
+    float r2, cos_thr;           // radius * radius, (float)cos((double)max_angle)
+};
+constexpr int kSelectMaxAcross = FDCM_SELECT_MAX_ACROSS;   // accepted list of the across-template walk (shared memory)
+// bytes of CUB scratch the select sorts need for n_hyp (< 2^31) hypotheses
+size_t select_temp_bytes(int64_t n_hyp);
+// 1. one order-preserving key per hypothesis (score, NaN as +inf; 0xFFFFFFFF for an invalid one) and its stable radix sort
+//    with the hypothesis index as value (vals_in receives the identity).  by_template: 64-bit keys (template << 32 | key),
+//    so that the hypotheses of template t keep their range [hyp_off[t], hyp_off[t+1]) in (score, h) order; otherwise the
+//    high half is 0: one global (score, h) order.
+void launch_select_sort(const SelectLaunch& p, bool by_template, uint64_t* keys_in, uint64_t* keys_out, int32_t* vals_in,
+                        int32_t* vals_out, void* d_temp, size_t temp_bytes, cudaStream_t s);
+// 2a. across_templates == 0: one warp walks each template's sorted range and writes the key of every accepted hypothesis to
+//     surv_keys (0xFFFFFFFF elsewhere); acc: n_hyp x 16 B of accepted anchors, read only with a radius
+void launch_select_greedy(const SelectLaunch& p, const uint64_t* sorted_keys, const int32_t* sorted_h, uint32_t* surv_keys, float4* acc,
+                          cudaStream_t s);
+// 3a. the first top_k survivors in (score, h) order: stable sort of surv_keys (values: the identity in vals_in), gather
+void launch_select_topk(const SelectLaunch& p, const uint32_t* surv_keys, uint32_t* keys_out, const int32_t* vals_in, int32_t* vals_out,
+                        void* d_temp, size_t temp_bytes, fdcm_match* d_out, int* d_n_out, cudaStream_t s);
+// 2b. across_templates != 0 (top_k <= kSelectMaxAcross): one block walks the global order, accepted list in shared memory
+void launch_select_walk(const SelectLaunch& p, const uint64_t* sorted_keys, const int32_t* sorted_h, fdcm_match* d_out, int* d_n_out,
+                        cudaStream_t s);
+// d_out[0, top_k) + *d_n_out are written like the top-K kernels' (unused slots: tmpl_idx -1, score +inf).
+
 void launch_evaluate(const MapView& map, const SlopeTableDev& table, const float4* d_lines, const int32_t* d_toff,
                      const float2* d_transl, const int32_t* d_troff, const int32_t* d_owner, int64_t n_scores,
                      float* d_scores, cudaStream_t s);

@@ -245,16 +245,30 @@ PYBIND11_MODULE(_openfdcm_cuda, m) {
           "matcher"_a, "searcher"_a, "optimizer"_a, "featuremap"_a, "templates"_a, "scene"_a,
           "Search for optimal matches between the templates and the scene");
 
+    py::class_<DistinctMatches>(m, "DistinctMatches")
+        .def(py::init([](int max_per_template, float radius, float max_angle, bool across_templates) {
+                 return DistinctMatches{max_per_template, radius, max_angle, across_templates};
+             }), "max_per_template"_a = 0, "radius"_a = 0.f, "max_angle"_a = 3.14159265358979323846f, "across_templates"_a = false)
+        .def_readwrite("max_per_template", &DistinctMatches::maxPerTemplate)
+        .def_readwrite("radius", &DistinctMatches::radius)
+        .def_readwrite("max_angle", &DistinctMatches::maxAngle)
+        .def_readwrite("across_templates", &DistinctMatches::acrossTemplates)
+        .def("__repr__", [](const DistinctMatches& a) {
+            return "<DistinctMatches: max_per_template=" + std::to_string(a.maxPerTemplate) + ", radius=" + std::to_string(a.radius) +
+                   ", max_angle=" + std::to_string(a.maxAngle) + ", across_templates=" + (a.acrossTemplates ? "True" : "False") + ">";
+        });
+
     m.def("search_topk",
           [](const Dt3Cuda& featuremap, const std::vector<LinesIn>& templates, const LinesIn& scene, const DefaultSearch& searcher,
-             const BatchOptimize& optimizer, const ExponentialPenalty& penalty, int k) {
+             const BatchOptimize& optimizer, const ExponentialPenalty& penalty, int k, const std::optional<DistinctMatches>& select) {
               const auto t = to_templates(templates);
               const auto s = to_lines(scene);
               py::gil_scoped_release release;
+              if (select) return searchTopK(searcher, optimizer, penalty, featuremap, t, s, k, *select);
               return searchTopK(searcher, optimizer, penalty, featuremap, t, s, k);
           },
-          "featuremap"_a, "templates"_a, "scene"_a, "searcher"_a, "optimizer"_a, "penalty"_a, "k"_a = 10,
-          "Fused search -> penalize -> top-k on the device (ascending score)");
+          "featuremap"_a, "templates"_a, "scene"_a, "searcher"_a, "optimizer"_a, "penalty"_a, "k"_a = 10, py::kw_only(), "select"_a = py::none(),
+          "Fused search -> penalize -> top-k on the device (ascending score); select: DistinctMatches for the distinct top-k");
 
     m.def("penalize",
           [](const PenaltyStrategy& penalty, const std::vector<Match>& matches, const std::vector<float>& templatelengths) {

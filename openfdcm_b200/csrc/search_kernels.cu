@@ -570,6 +570,221 @@ void launch_topk(const fdcm_match* d_rec, const uint8_t* d_valid, int64_t n, int
 }
 
 // =============================================================================================
+// Distinct top-K (fdcm_search_select, beyond the reference): greedy walk of the valid matches in (score, h) order that
+// caps the matches per template and suppresses matches whose anchors lie within a radius (and a rotation) of an accepted
+// one.  Semantics in include/fdcm_b200.h; the keys below order exactly like the top-K kernels' (score, h) comparison.
+// =============================================================================================
+constexpr uint32_t kInvalidKey = 0xFFFFFFFFu;
+
+// order-preserving 32-bit key of a score: NaN as +inf (0xFF800000, still below kInvalidKey), -0 as +0
+__device__ __forceinline__ uint32_t score_key(float s) {
+    if (s != s) s = INFINITY;
+    if (s == 0.f) s = 0.f;
+    const uint32_t u = __float_as_uint(s);
+    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+
+// anchor of a match and the first column of its rotation: (px, py, T0, T3)
+__device__ __forceinline__ float4 match_anchor(const fdcm_match& m, float2 a) {
+    return make_float4((m.transform[0] * a.x + m.transform[1] * a.y) + m.transform[2],
+                       (m.transform[3] * a.x + m.transform[4] * a.y) + m.transform[5], m.transform[0], m.transform[3]);
+}
+
+// near(a, b) of the header (the build has no FMA contraction, so this is the fp32 expression as written)
+__device__ __forceinline__ bool anchors_near(const float4 a, const float4 b, const SelectLaunch& p) {
+    const float dx = a.x - b.x, dy = a.y - b.y;
+    if (!(dx * dx + dy * dy <= p.r2)) return false;
+    return p.any_angle || a.z * b.z + a.w * b.w >= p.cos_thr;
+}
+
+__device__ __forceinline__ void write_invalid(fdcm_match* out) {
+    fdcm_match m;
+    m.tmpl_idx = -1;
+    m.score = INFINITY;
+    for (int i = 0; i < 6; ++i) m.transform[i] = 0.f;
+    *out = m;
+}
+
+__global__ void select_key_kernel(const __grid_constant__ SelectLaunch p, bool by_template, uint64_t* __restrict__ keys,
+                                  int32_t* __restrict__ vals) {
+    const long long h = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (h >= p.n_hyp) return;
+    const uint32_t k = p.valid[h] ? score_key(p.rec[h].score) : kInvalidKey;
+    uint64_t t = 0;
+    if (by_template) {   // largest t with hyp_off[t] <= h
+        int lo = 0, hi = p.n_tmpl;
+        while (hi - lo > 1) {
+            const int mid = (lo + hi) >> 1;
+            if (p.hyp_off[mid] <= h) lo = mid; else hi = mid;
+        }
+        t = (uint64_t)lo;
+    }
+    keys[h] = t << 32 | k;
+    vals[h] = (int32_t)h;
+}
+
+size_t select_temp_bytes(int64_t n_hyp) {
+    size_t b64 = 0, b32 = 0;
+    cub::DeviceRadixSort::SortPairs(nullptr, b64, (const uint64_t*)nullptr, (uint64_t*)nullptr, (const int32_t*)nullptr,
+                                    (int32_t*)nullptr, (int)n_hyp);
+    cub::DeviceRadixSort::SortPairs(nullptr, b32, (const uint32_t*)nullptr, (uint32_t*)nullptr, (const int32_t*)nullptr,
+                                    (int32_t*)nullptr, (int)n_hyp);
+    return b64 > b32 ? b64 : b32;
+}
+
+void launch_select_sort(const SelectLaunch& p, bool by_template, uint64_t* keys_in, uint64_t* keys_out, int32_t* vals_in,
+                        int32_t* vals_out, void* d_temp, size_t temp_bytes, cudaStream_t s) {
+    select_key_kernel<<<(unsigned)((p.n_hyp + 255) / 256), 256, 0, s>>>(p, by_template, keys_in, vals_in);
+    int end_bit = 32;
+    if (by_template)
+        while (p.n_tmpl > 1 && ((int64_t)1 << (end_bit - 32)) < p.n_tmpl) ++end_bit;
+    // radix sort is stable: equal keys keep ascending h
+    cub::DeviceRadixSort::SortPairs(d_temp, temp_bytes, keys_in, keys_out, vals_in, vals_out, (int)p.n_hyp, 0, end_bit, s);
+}
+
+// One warp per template.  Every rule of the walk involves matches of one template only when across_templates == 0, so
+// walking each template's range on its own and keeping the survivors' global (score, h) order (launch_select_topk) gives
+// exactly the walk over the global order.  The warp takes its sorted range 32 candidates at a time: each lane tests its
+// candidate against the template's accepted anchors, then the chunk is settled in order (the first live lane is accepted
+// and removes the live lanes near it).  The walk ends at min(cap, top_k) accepted or at the first invalid key.
+__global__ void __launch_bounds__(128) select_greedy_kernel(const __grid_constant__ SelectLaunch p, const uint64_t* __restrict__ skeys,
+                                                            const int32_t* __restrict__ sh, uint32_t* __restrict__ surv_keys,
+                                                            float4* __restrict__ acc) {
+    const int lane = threadIdx.x & 31;
+    const int t = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (t >= p.n_tmpl) return;   // whole warp
+    const long long b = p.hyp_off[t], e = p.hyp_off[t + 1];
+    const int lim = p.cap > 0 ? min(p.cap, p.top_k) : p.top_k;
+    const float2 anchor = p.anchors[t];
+    int n_acc = 0;
+    for (long long base = b; base < e && n_acc < lim; base += 32) {
+        const long long i = base + lane;
+        const uint32_t key = i < e ? (uint32_t)skeys[i] : kInvalidKey;
+        bool live = key != kInvalidKey;
+        const bool last_chunk = __ballot_sync(0xffffffffu, i < e && !live) != 0u;
+        const int h = live ? sh[i] : 0;
+        float4 me = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (live && p.radius_on) {
+            me = match_anchor(p.rec[h], anchor);
+            for (int j = 0; j < n_acc && live; ++j) live = !anchors_near(acc[b + j], me, p);
+        }
+        for (;;) {
+            const unsigned alive = __ballot_sync(0xffffffffu, live);
+            if (alive == 0u || n_acc == lim) break;
+            const int ld = __ffs(alive) - 1;
+            const float4 a = make_float4(__shfl_sync(0xffffffffu, me.x, ld), __shfl_sync(0xffffffffu, me.y, ld),
+                                         __shfl_sync(0xffffffffu, me.z, ld), __shfl_sync(0xffffffffu, me.w, ld));
+            if (lane == ld) {
+                surv_keys[h] = key;
+                if (p.radius_on) acc[b + n_acc] = me;
+                live = false;
+            } else if (live && p.radius_on && anchors_near(a, me, p)) {
+                live = false;
+            }
+            ++n_acc;
+        }
+        __syncwarp();   // the accepted anchors written above are read by every lane in the next chunk
+        if (last_chunk) break;
+    }
+}
+
+void launch_select_greedy(const SelectLaunch& p, const uint64_t* sorted_keys, const int32_t* sorted_h, uint32_t* surv_keys, float4* acc,
+                          cudaStream_t s) {
+    cudaMemsetAsync(surv_keys, 0xFF, (size_t)p.n_hyp * 4, s);
+    select_greedy_kernel<<<(unsigned)((p.n_tmpl + 3) / 4), 128, 0, s>>>(p, sorted_keys, sorted_h, surv_keys, acc);
+}
+
+__global__ void select_gather_kernel(const uint32_t* __restrict__ skeys, const int32_t* __restrict__ sh, long long n,
+                                     const fdcm_match* __restrict__ rec, int k, fdcm_match* __restrict__ out, int* __restrict__ n_out) {
+    __shared__ int s_n;
+    if (threadIdx.x == 0) s_n = 0;
+    __syncthreads();
+    int mine = 0;
+    for (int q = threadIdx.x; q < k; q += blockDim.x) {
+        if (q < n && skeys[q] != kInvalidKey) {
+            out[q] = rec[sh[q]];
+            ++mine;
+        } else {
+            write_invalid(out + q);
+        }
+    }
+    atomicAdd(&s_n, mine);
+    __syncthreads();
+    if (threadIdx.x == 0) *n_out = s_n;
+}
+
+void launch_select_topk(const SelectLaunch& p, const uint32_t* surv_keys, uint32_t* keys_out, const int32_t* vals_in, int32_t* vals_out,
+                        void* d_temp, size_t temp_bytes, fdcm_match* d_out, int* d_n_out, cudaStream_t s) {
+    cub::DeviceRadixSort::SortPairs(d_temp, temp_bytes, surv_keys, keys_out, vals_in, vals_out, (int)p.n_hyp, 0, 32, s);
+    select_gather_kernel<<<1, 256, 0, s>>>(keys_out, vals_out, p.n_hyp, p.rec, p.top_k, d_out, d_n_out);
+}
+
+// across_templates != 0: one block walks the global (score, h) order blockDim candidates at a time.  Every thread tests its
+// candidate against the accepted list in shared memory (anchor, rotation, template: the per-template count for the cap is
+// taken in the same pass), then the chunk is settled in order like the warp version above.  Worst case H x top_k tests.
+__global__ void __launch_bounds__(1024) select_walk_kernel(const __grid_constant__ SelectLaunch p, const uint64_t* __restrict__ skeys,
+                                                           const int32_t* __restrict__ sh, fdcm_match* __restrict__ out,
+                                                           int* __restrict__ n_out) {
+    __shared__ float4 s_acc[kSelectMaxAcross];
+    __shared__ int s_tmpl[kSelectMaxAcross];
+    __shared__ unsigned s_live[32];
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, n_warps = blockDim.x >> 5;
+    int n_acc = 0;   // uniform
+    for (long long base = 0; base < p.n_hyp && n_acc < p.top_k; base += blockDim.x) {
+        const long long i = base + tid;
+        const uint32_t key = i < p.n_hyp ? (uint32_t)skeys[i] : kInvalidKey;
+        bool live = key != kInvalidKey;
+        const bool last_chunk = __syncthreads_or(!live) != 0;
+        int h = 0, t = -1, same = 0;
+        float4 me = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (live) {
+            h = sh[i];
+            const fdcm_match m = p.rec[h];
+            t = m.tmpl_idx - p.tmpl_idx_base;
+            me = match_anchor(m, p.anchors[t]);
+            for (int j = 0; j < n_acc && live; ++j) {
+                same += s_tmpl[j] == t;
+                live = !(p.radius_on && anchors_near(s_acc[j], me, p));
+            }
+            if (p.cap > 0 && same >= p.cap) live = false;
+        }
+        for (;;) {
+            const unsigned m = __ballot_sync(0xffffffffu, live);
+            if (lane == 0) s_live[warp] = m;
+            __syncthreads();
+            int ld = -1;
+            for (int w = 0; w < n_warps; ++w)
+                if (s_live[w]) { ld = w * 32 + __ffs(s_live[w]) - 1; break; }
+            if (ld < 0) break;   // uniform
+            if (tid == ld) {
+                s_acc[n_acc] = me;
+                s_tmpl[n_acc] = t;
+                out[n_acc] = p.rec[h];
+                live = false;
+            }
+            __syncthreads();
+            const float4 a = s_acc[n_acc];
+            const int at = s_tmpl[n_acc];
+            ++n_acc;
+            if (n_acc == p.top_k) break;   // uniform
+            if (live) {
+                same += at == t;
+                if ((p.cap > 0 && same >= p.cap) || (p.radius_on && anchors_near(a, me, p))) live = false;
+            }
+        }
+        __syncthreads();   // s_live is rewritten by the next chunk
+        if (last_chunk) break;
+    }
+    for (int q = n_acc + tid; q < p.top_k; q += blockDim.x) write_invalid(out + q);
+    if (tid == 0) *n_out = n_acc;
+}
+
+void launch_select_walk(const SelectLaunch& p, const uint64_t* sorted_keys, const int32_t* sorted_h, fdcm_match* d_out, int* d_n_out,
+                        cudaStream_t s) {
+    select_walk_kernel<<<1, 1024, 0, s>>>(p, sorted_keys, sorted_h, d_out, d_n_out);
+}
+
+// =============================================================================================
 // evaluate<Dt3Cpu> (dt3cpu.cpp:126-179) as a standalone entry point: one thread per (template, translation)
 // =============================================================================================
 __global__ void __launch_bounds__(128) evaluate_kernel(const __grid_constant__ MapView map,

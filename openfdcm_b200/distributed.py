@@ -52,8 +52,9 @@ class Communicator:
         check(lib().fdcm_comm_shard(int(n_items), self.rank, self.world, C.byref(b), C.byref(e)))
         return b.value, e.value
 
-    def search_topk(self, featuremap, shard, scene, searcher, optimizer, penalty, k, tmpl_idx_base):
-        """Search this rank's shard (a TemplateSet) and return the GLOBAL top-k (same on every rank)."""
+    def search_topk(self, featuremap, shard, scene, searcher, optimizer, penalty, k, tmpl_idx_base, *, select=None):
+        """Search this rank's shard (a TemplateSet) and return the GLOBAL top-k (same on every rank).  select: a
+        DistinctMatches without across_templates (the distinct top-k of the whole template set)."""
         from . import _records
         s = None if scene is None else _records(scene)
         p = _lib.SearchParams(searcher.max_tmpl_lines, searcher.max_scene_lines, int(optimizer.batch_size),
@@ -61,8 +62,13 @@ class Communicator:
                               int(k), int(tmpl_idx_base), 0, 0.0, 0.0, 0.0, 0.0)
         out = np.zeros(int(k), MATCH_DTYPE)
         n = C.c_int64(0)
-        check(lib().fdcm_comm_search_topk(self._h, featuremap._h, shard._h, ptr(s), _lib.FDCM_SCENE_RESIDENT if s is None else s.shape[0],
-                                          C.byref(p), ptr(out), int(k), C.byref(n)))
+        n_scene = _lib.FDCM_SCENE_RESIDENT if s is None else s.shape[0]
+        if select is None:
+            check(lib().fdcm_comm_search_topk(self._h, featuremap._h, shard._h, ptr(s), n_scene, C.byref(p), ptr(out), int(k), C.byref(n)))
+        else:
+            sp = select._params()
+            check(lib().fdcm_comm_search_select(self._h, featuremap._h, shard._h, ptr(s), n_scene, C.byref(p), C.byref(sp), ptr(out), int(k),
+                                                C.byref(n)))
         return out[: n.value].copy()
 
     def rebuild_broadcast(self, featuremap, scene, root=0):
