@@ -202,6 +202,60 @@ fdcm_status fdcm_search_select(const fdcm_dt3* map, const fdcm_templates* templa
 /* anchors of n_tmpl templates (CSR like fdcm_template_lengths), n_tmpl (x, y) pairs; host only */
 fdcm_status fdcm_template_anchors(const float* tmpl_lines, const int32_t* tmpl_offsets, int32_t n_tmpl, float* anchors_xy);
 
+/* ---- pose refinement (beyond the reference) -----------------------------------------------------
+ * A search match aligns one template line with one scene line, so its rotation is that scene line's direction and its
+ * translation moves along that line only.  Refinement walks a coarse-to-fine grid of rotations and 2-D translations
+ * around each match and keeps the pose with the lowest evaluate<Dt3Cpu> score over all template lines.
+ * It minimises that score and nothing else.  At sub-pixel and 0.01 rad scales the score is not lowest at the true pose
+ * (a noise-free instance scores far lower a pixel or 0.01 rad away), so refinement was measured to INCREASE the error
+ * against known poses, also when started at the exact pose (DESIGN.md section 4).
+ * Rules, in fp32 without contraction, in the order written.  For a match with transform M = (m0..m5) and template t:
+ *   1. Centre.  The walk starts with C = M.  At every level the rotation centre is p = C applied to the anchor a of t
+ *      (fdcm_template_anchors): px = (c0*ax + c1*ay) + c2, py = (c3*ax + c4*ay) + c5.
+ *   2. Grid of level l (0-based): i in [-rot_steps, rot_steps], k and j in [-trans_steps, trans_steps];
+ *      ci = (float)cos((double)i * ((double)rot_step / 2^l)), si likewise with sin (host C library);
+ *      h = trans_step * 2^-l, dx = (float)j * h, dy = (float)k * h.
+ *   3. Candidate P.  i != 0: P0 = ci*c0 - si*c3, P1 = ci*c1 - si*c4, P3 = si*c0 + ci*c3, P4 = si*c1 + ci*c4,
+ *      ux = c2 - px, uy = c5 - py, P2 = ((ci*ux - si*uy) + px) + dx, P5 = ((si*ux + ci*uy) + py) + dy.
+ *      i == 0 keeps C's rotation: P = (c0, c1, c2 + dx, c3, c4, c5 + dy).  The grid point (0, 0, 0) is C itself.
+ *   4. Score of P: evaluate<Dt3Cpu>(map, {R_P tmpl}, {(P2, P5)}) (fdcm_dt3_evaluate): end point (x, y) -> (P0*x + P1*y,
+ *      P3*x + P4*y); orientation bin from the slope of the rotated line; lookups (int)(r + (shift + P2)); Eigen's sum
+ *      order.  P is valid iff no entry of P and no rotated end point is NaN and every rotated end point has
+ *      0 <= rx + (shift_x + P2) <= W - 1 and 0 <= ry + (shift_y + P5) <= H - 1 (an empty template: any P without NaN).
+ *      Invalid poses are neither evaluated nor read.
+ *   5. Walk.  The grid points by ascending i*i + k*k + j*j (the centre first), equal distances in ascending (i, k, j).
+ *      A valid candidate replaces the running best iff there is none yet or its score is lower (NaN as +inf, strict: ties
+ *      keep the earlier candidate, so the centre wins ties and a plateau of equal scores resolves to its point nearest
+ *      the centre).  The best of level l is the centre of level l + 1; a level without a valid pose keeps C.
+ *   6. Result.  tmpl_idx unchanged; the transform is the final best pose; the score is its raw score, divided by the
+ *      search's penalty denominator (host powf of the template length) when a penalty is given.  No valid pose at any
+ *      level: transform M, score NaN.  Output i is the refinement of input i (not re-sorted; fdcm_sort_matches re-ranks).
+ * Invalid parameters (levels < 1, rot_steps or trans_steps outside 0..FDCM_REFINE_MAX_STEPS, a negative or non-finite
+ * step, a null refine pointer, a template longer than the search accepts) fail with FDCM_ERR_INVALID; a tmpl_idx -
+ * tmpl_idx_base outside the template set fails with FDCM_ERR_OUT_OF_RANGE.
+ * Cost per level and match: (2 rot_steps + 1)(2 trans_steps + 1)^2 poses of 2 L map gathers each. */
+#define FDCM_REFINE_MAX_STEPS 15
+typedef struct fdcm_refine_params {      /* 20 bytes */
+    int32_t levels;             /* >= 1: coarse-to-fine levels; steps halve at every level */
+    int32_t rot_steps;          /* n_r: rotations i * rot_step / 2^l, i in [-n_r, n_r] */
+    float rot_step;             /* radians */
+    int32_t trans_steps;        /* n_t: translations (j, k) * trans_step / 2^l, j, k in [-n_t, n_t] */
+    float trans_step;           /* pixels */
+} fdcm_refine_params;
+/* refine n host matches (search output or from elsewhere) against a map and a resident template set; n == 0 is no error */
+fdcm_status fdcm_refine_matches(const fdcm_dt3* map, const fdcm_templates* templates, int32_t tmpl_idx_base, int32_t penalty_kind,
+                                float penalty_tau, const fdcm_refine_params* refine, const fdcm_match* in, int64_t n,
+                                fdcm_match* out);
+/* fdcm_search (top_k > 0) or, with select != NULL, fdcm_search_select, then refinement of the selected matches on the
+ * device and one download: byte-identical to fdcm_refine_matches applied to their output */
+fdcm_status fdcm_search_refine(const fdcm_dt3* map, const fdcm_templates* templates, const float* scene_xyxy, int32_t n_scene,
+                               const fdcm_search_params* params, const fdcm_select_params* select,
+                               const fdcm_refine_params* refine, fdcm_match* out, int64_t capacity, int64_t* n_out);
+/* the candidate transforms of one level (0 <= level < levels) in grid order, 6 floats each,
+ * (2 rot_steps + 1)(2 trans_steps + 1)^2 of them; host-only parity hook */
+fdcm_status fdcm_refine_poses(const float transform[6], const float anchor[2], const fdcm_refine_params* refine, int32_t level,
+                              float* out);
+
 /* optimize(optimizer, templates, alignments, featuremap) (matching/optimizestrategy.h:62-64; BatchOptimize:
  * batchoptimize.cpp:6-123, batch_size == 0: DefaultOptimize, defaultoptimize.cpp:6-93).  The templates are used
  * as given (already aligned); alignments: n_tmpl (x,y) pairs.  Outputs per template: has_value (0 = nullopt),

@@ -264,6 +264,88 @@ inline std::vector<Match> searchTopK(const DefaultSearch& s, const BatchOptimize
     return out;
 }
 
+// pose refinement (beyond the reference; rules of fdcm_refine_matches): coarse-to-fine rotations about the template anchor
+// and 2-D translations around each match, keeping the pose of lowest score over all template lines.  It minimises the
+// evaluate score only, which was measured to increase the error against known poses (see fdcm_b200.h).
+struct PoseRefinement {
+    int levels{3};
+    int rotSteps{4};
+    float rotStep{0.01f};
+    int transSteps{4};
+    float transStep{1.f};
+};
+namespace detail {
+inline fdcm_refine_params refine_params(const PoseRefinement& r) {
+    return fdcm_refine_params{r.levels, r.rotSteps, r.rotStep, r.transSteps, r.transStep};
+}
+inline std::vector<Match> to_matches(const std::vector<fdcm_match>& rec, int64_t n) {
+    std::vector<Match> out((size_t)n);
+    for (int64_t i = 0; i < n; ++i) {
+        out[(size_t)i].tmplIdx = rec[(size_t)i].tmpl_idx;
+        out[(size_t)i].score = rec[(size_t)i].score;
+        for (int c = 0; c < 6; ++c) out[(size_t)i].transform[(size_t)c] = rec[(size_t)i].transform[c];
+    }
+    return out;
+}
+inline std::vector<Match> search_refine(const DefaultSearch& s, const BatchOptimize& o, const ExponentialPenalty& pen, const Dt3Cuda& fm,
+                                        const std::vector<LineArray>& templates, const LineArray& scene, int k, const DistinctMatches* select,
+                                        const PoseRefinement& refine) {
+    std::vector<float> flat;
+    std::vector<int32_t> off;
+    pack(templates, flat, off);
+    fdcm_templates* ts = nullptr;
+    check(fdcm_templates_create(flat.data(), off.data(), (int32_t)templates.size(), fm.info().device, &ts));
+    const std::unique_ptr<fdcm_templates, fdcm_status (*)(fdcm_templates*)> owner(ts, fdcm_templates_release);
+    const fdcm_search_params p{(int32_t)s.max_tmpl_lines, (int32_t)s.max_scene_lines, (int32_t)o.batchSize, FDCM_PENALTY_EXPONENTIAL,
+                               pen.tau, k, 0, 0, 0.f, 0.f, 0.f, 0.f};
+    fdcm_select_params q{};
+    if (select) q = fdcm_select_params{select->maxPerTemplate, select->radius, select->maxAngle, select->acrossTemplates ? 1 : 0};
+    const fdcm_refine_params r = refine_params(refine);
+    std::vector<fdcm_match> rec((size_t)std::max(k, 1));
+    int64_t n = 0;
+    check(fdcm_search_refine(fm.handle(), ts, scene.data(), (int32_t)(scene.size() / 4), &p, select ? &q : nullptr, &r, rec.data(),
+                             (int64_t)rec.size(), &n));
+    return to_matches(rec, n);
+}
+inline std::vector<Match> refine_matches(const Dt3Cuda& fm, const std::vector<LineArray>& templates, const std::vector<Match>& matches,
+                                         const PoseRefinement& refine, int penalty_kind, float tau) {
+    std::vector<float> flat;
+    std::vector<int32_t> off;
+    pack(templates, flat, off);
+    fdcm_templates* ts = nullptr;
+    check(fdcm_templates_create(flat.data(), off.data(), (int32_t)templates.size(), fm.info().device, &ts));
+    const std::unique_ptr<fdcm_templates, fdcm_status (*)(fdcm_templates*)> owner(ts, fdcm_templates_release);
+    std::vector<fdcm_match> rec(matches.size());
+    for (size_t i = 0; i < matches.size(); ++i) {
+        rec[i].tmpl_idx = matches[i].tmplIdx;
+        rec[i].score = matches[i].score;
+        for (int c = 0; c < 6; ++c) rec[i].transform[c] = matches[i].transform[(size_t)c];
+    }
+    const fdcm_refine_params r = refine_params(refine);
+    check(fdcm_refine_matches(fm.handle(), ts, 0, penalty_kind, tau, &r, rec.data(), (int64_t)rec.size(), rec.data()));
+    return to_matches(rec, (int64_t)rec.size());
+}
+}   // namespace detail
+// fused search -> top-k (or distinct top-k) -> pose refinement on the device; not re-sorted (sortMatches re-ranks)
+inline std::vector<Match> searchTopK(const DefaultSearch& s, const BatchOptimize& o, const ExponentialPenalty& pen, const Dt3Cuda& fm,
+                                     const std::vector<LineArray>& templates, const LineArray& scene, int k, const PoseRefinement& refine) {
+    return detail::search_refine(s, o, pen, fm, templates, scene, k, nullptr, refine);
+}
+inline std::vector<Match> searchTopK(const DefaultSearch& s, const BatchOptimize& o, const ExponentialPenalty& pen, const Dt3Cuda& fm,
+                                     const std::vector<LineArray>& templates, const LineArray& scene, int k, const DistinctMatches& select,
+                                     const PoseRefinement& refine) {
+    return detail::search_refine(s, o, pen, fm, templates, scene, k, &select, refine);
+}
+// refinement of any match list (tmplIdx indexes `templates`); without a penalty the scores are raw
+inline std::vector<Match> refineMatches(const Dt3Cuda& fm, const std::vector<LineArray>& templates, const std::vector<Match>& matches,
+                                        const PoseRefinement& refine) {
+    return detail::refine_matches(fm, templates, matches, refine, FDCM_PENALTY_NONE, 0.f);
+}
+inline std::vector<Match> refineMatches(const Dt3Cuda& fm, const std::vector<LineArray>& templates, const std::vector<Match>& matches,
+                                        const PoseRefinement& refine, const ExponentialPenalty& pen) {
+    return detail::refine_matches(fm, templates, matches, refine, FDCM_PENALTY_EXPONENTIAL, pen.tau);
+}
+
 // ---- PenaltyStrategy concept, template lengths, sort ----------------------------------------------
 inline std::vector<float> getTemplateLengths(const std::vector<LineArray>& templates) {   // core/math.h:319-324
     std::vector<float> flat, len(templates.size());

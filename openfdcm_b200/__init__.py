@@ -22,7 +22,7 @@ from ._lib import MATCH_DTYPE, FdcmError, check, lib, ptr
 __all__ = [
     "distance", "Dt3CudaParameters", "Dt3Cuda", "build_cuda_featuremap", "ThreadPool", "DefaultSearch", "ConcentricRangeStrategy",
     "BatchOptimize", "DefaultOptimize", "DefaultMatch", "DefaultPenalty", "ExponentialPenalty", "Match",
-    "TemplateSet", "SceneBatch", "DistinctMatches", "search", "search_topk", "penalize", "get_template_lengths",
+    "TemplateSet", "SceneBatch", "DistinctMatches", "PoseRefinement", "search", "search_topk", "refine_matches", "penalize", "get_template_lengths",
     "get_template_anchors", "sort_matches", "evaluate",
     "minmax_translation", "get_feature_size", "establish_search_strategy", "optimize", "read", "write", "FdcmError", "MATCH_DTYPE",
 ]
@@ -328,7 +328,29 @@ class DistinctMatches:
                 f"across_templates={self.across_templates}>")
 
 
-def _search_raw(featuremap, templates, scene, searcher, optimizer, penalty=None, top_k=0, tmpl_idx_base=0, select=None):
+class PoseRefinement:
+    """Pose refinement (beyond the reference): around each match, `levels` coarse-to-fine grids of rotations
+    i * rot_step / 2^l about the template anchor (|i| <= rot_steps) and translations (j, k) * trans_step / 2^l
+    (|j|, |k| <= trans_steps); every level keeps the pose with the lowest evaluate<Dt3Cpu> score over all template lines,
+    the centre on ties.  It minimises that score only: at sub-pixel and 0.01 rad scales the score is not lowest at the
+    true pose, and refinement was measured to increase the error against known poses.  Exact rules: include/fdcm_b200.h."""
+
+    def __init__(self, levels=3, rot_steps=4, rot_step=0.01, trans_steps=4, trans_step=1.0):
+        self.levels = int(levels)
+        self.rot_steps = int(rot_steps)
+        self.rot_step = float(rot_step)
+        self.trans_steps = int(trans_steps)
+        self.trans_step = float(trans_step)
+
+    def _params(self):
+        return _lib.RefineParams(self.levels, self.rot_steps, self.rot_step, self.trans_steps, self.trans_step)
+
+    def __repr__(self):
+        return (f"<PoseRefinement: levels={self.levels}, rot_steps={self.rot_steps}, rot_step={self.rot_step}, "
+                f"trans_steps={self.trans_steps}, trans_step={self.trans_step}>")
+
+
+def _search_raw(featuremap, templates, scene, searcher, optimizer, penalty=None, top_k=0, tmpl_idx_base=0, select=None, refine=None):
     if not isinstance(featuremap, Dt3Cuda):
         raise TypeError("the CUDA search needs a Dt3Cuda feature map (build_cuda_featuremap)")
     tset = templates if isinstance(templates, TemplateSet) else TemplateSet(templates, featuremap.device)
@@ -346,7 +368,11 @@ def _search_raw(featuremap, templates, scene, searcher, optimizer, penalty=None,
     out = np.zeros(max(cap, 1), MATCH_DTYPE)
     n = C.c_int64(0)
     n_scene = _lib.FDCM_SCENE_RESIDENT if s is None else s.shape[0]
-    if select is None:
+    if refine is not None:
+        sp = None if select is None else C.byref(select._params())
+        check(lib().fdcm_search_refine(featuremap._h, tset._h, ptr(s), n_scene, C.byref(p), sp, C.byref(refine._params()), ptr(out),
+                                       out.shape[0], C.byref(n)))
+    elif select is None:
         check(lib().fdcm_search(featuremap._h, tset._h, ptr(s), n_scene, C.byref(p), ptr(out), out.shape[0], C.byref(n)))
     else:
         sp = select._params()
@@ -360,10 +386,30 @@ def search(matcher, searcher, optimizer, featuremap, templates, scene):
     return _to_matches(_search_raw(featuremap, templates, scene, searcher, optimizer))
 
 
-def search_topk(featuremap, templates, scene, searcher, optimizer, penalty=None, k=10, tmpl_idx_base=0, *, select=None):
+def search_topk(featuremap, templates, scene, searcher, optimizer, penalty=None, k=10, tmpl_idx_base=0, *, select=None, refine=None):
     """Fused search -> penalize -> top-k on the device; returns a MATCH_DTYPE record array (ascending score).
-    select: a DistinctMatches for the distinct top-k (the kept matches in acceptance order, also ascending score)."""
-    return _search_raw(featuremap, templates, scene, searcher, optimizer, penalty, k, tmpl_idx_base, select).copy()
+    select: a DistinctMatches for the distinct top-k (the kept matches in acceptance order, also ascending score).
+    refine: a PoseRefinement applied to the selected matches on the device, equal to refine_matches of the unrefined
+    result (same order: re-rank with sort_matches); it lowers the score, not the pose error (see PoseRefinement)."""
+    return _search_raw(featuremap, templates, scene, searcher, optimizer, penalty, k, tmpl_idx_base, select, refine).copy()
+
+
+def refine_matches(featuremap, templates, matches, refine, penalty=None, tmpl_idx_base=0):
+    """Pose refinement of any match list against a feature map and a template set (list or TemplateSet); returns a
+    MATCH_DTYPE array, entry i refining matches[i], scored like search_topk with the same penalty.  Each pose moves to the
+    lowest evaluate<Dt3Cpu> score of its grid, which is not a more accurate pose (see PoseRefinement)."""
+    if not isinstance(featuremap, Dt3Cuda):
+        raise TypeError("refine_matches needs a Dt3Cuda feature map (build_cuda_featuremap)")
+    tset = templates if isinstance(templates, TemplateSet) else TemplateSet(templates, featuremap.device)
+    rec = _to_records(matches)
+    out = np.zeros(max(rec.shape[0], 1), MATCH_DTYPE)
+    st = lib().fdcm_refine_matches(featuremap._h, tset._h, int(tmpl_idx_base), 0 if penalty is None else penalty.kind,
+                                   0.0 if penalty is None else float(penalty.tau), C.byref(refine._params()), ptr(rec), rec.shape[0],
+                                   ptr(out))
+    if st == _lib.FDCM_ERR_OUT_OF_RANGE:
+        raise IndexError(lib().fdcm_last_error().decode())
+    check(st)
+    return out[: rec.shape[0]].copy()
 
 
 def search_all(featuremap, templates, scene, searcher, optimizer, penalty=None, tmpl_idx_base=0):

@@ -31,6 +31,11 @@ class SelectParams(C.Structure):
     _fields_ = [("max_per_template", C.c_int32), ("radius", C.c_float), ("max_angle", C.c_float), ("across_templates", C.c_int32)]
 
 
+class RefineParams(C.Structure):
+    _fields_ = [("levels", C.c_int32), ("rot_steps", C.c_int32), ("rot_step", C.c_float), ("trans_steps", C.c_int32),
+                ("trans_step", C.c_float)]
+
+
 class Dt3Info(C.Structure):
     _fields_ = [("depth", C.c_int32), ("width", C.c_int32), ("height", C.c_int32), ("pitch", C.c_int32),
                 ("scene_translation", C.c_float * 2), ("distance", C.c_int32), ("device", C.c_int32),
@@ -72,6 +77,10 @@ SIGNATURES = {
     "fdcm_search_select": (C.c_int, [_P, _P, _P, C.c_int32, C.POINTER(SearchParams), C.POINTER(SelectParams), _P, C.c_int64,
                                      C.POINTER(C.c_int64)]),
     "fdcm_template_anchors": (C.c_int, [_P, _P, C.c_int32, _P]),
+    "fdcm_refine_matches": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_float, C.POINTER(RefineParams), _P, C.c_int64, _P]),
+    "fdcm_search_refine": (C.c_int, [_P, _P, _P, C.c_int32, C.POINTER(SearchParams), C.POINTER(SelectParams), C.POINTER(RefineParams), _P,
+                                     C.c_int64, C.POINTER(C.c_int64)]),
+    "fdcm_refine_poses": (C.c_int, [_P, _P, C.POINTER(RefineParams), C.c_int32, _P]),
     "fdcm_optimize": (C.c_int, [_P, _P, _P, C.c_int32, _P, C.c_int32, _P, _P, _P]),
     "fdcm_search_host": (C.c_int, [_P, _P, _P, C.c_int32, _P, C.c_int32, C.POINTER(SearchParams), _P, C.c_int64,
                                    C.POINTER(C.c_int64)]),

@@ -291,6 +291,7 @@ struct fdcm_dt3 {
     mutable DevBuf s_scene, s_sorted_len, s_sorted_idx, s_hyp_off, s_rec, s_valid, s_hyp, s_counters, s_topk_score, s_topk_idx,
         s_topk_out, s_topk_n, s_keys, s_keys2, s_idx, s_perm, s_sort_tmp;
     mutable DevBuf s_sel_keys, s_sel_keys2, s_sel_vals, s_sel_vals2, s_sel_surv, s_sel_acc, s_sel_tmp;   // distinct top-K
+    mutable DevBuf s_ref_state, s_ref_keys, s_ref_io, s_ref_denom;   // pose refinement
     mutable float s_scene_min[2] = {0.f, 0.f}, s_scene_max[2] = {0.f, 0.f};   // bbox of the resident search scene
     mutable std::mutex host_tset_mutex;
     mutable fdcm_templates* host_tset = nullptr;   // reusable template set of fdcm_search_host
@@ -313,7 +314,7 @@ struct fdcm_dt3 {
         for (DevBuf* b : {&planes, &mask, &stack, &lines, &bins, &band_info, &band_spill, &integ_items, &s_scene, &s_sorted_len, &s_sorted_idx, &s_hyp_off, &s_rec,
                           &s_valid, &s_hyp, &s_counters, &s_topk_score, &s_topk_idx, &s_topk_out, &s_topk_n, &s_keys, &s_keys2, &s_idx,
                           &s_perm, &s_sort_tmp, &s_sel_keys, &s_sel_keys2, &s_sel_vals, &s_sel_vals2, &s_sel_surv, &s_sel_acc,
-                          &s_sel_tmp})
+                          &s_sel_tmp, &s_ref_state, &s_ref_keys, &s_ref_io, &s_ref_denom})
             b->release();
         if (h_pinned) cudaFreeHost(h_pinned);
         if (ev_fork) cudaEventDestroy(ev_fork);
@@ -1568,10 +1569,71 @@ static fdcm_status run_select(const fdcm_dt3* m, const fdcm_templates* t, const 
     return FDCM_OK;
 }
 
-// sel: distinct top-K (fdcm_search_select); nullptr for the plain search
+// parameters of the pose refinement (fdcm_refine_matches, fdcm_search_refine)
+static fdcm_status check_refine(const fdcm_refine_params* r) {
+    if (!r) return fail(FDCM_ERR_INVALID, "refine is null");
+    if (r->levels < 1) return fail(FDCM_ERR_INVALID, "pose refinement: levels must be >= 1");
+    if (r->rot_steps < 0 || r->rot_steps > FDCM_REFINE_MAX_STEPS || r->trans_steps < 0 || r->trans_steps > FDCM_REFINE_MAX_STEPS)
+        return fail(FDCM_ERR_INVALID, "pose refinement: rot_steps and trans_steps must be in 0.." + std::to_string(FDCM_REFINE_MAX_STEPS));
+    if (!(r->rot_step >= 0.f) || !std::isfinite(r->rot_step) || !(r->trans_step >= 0.f) || !std::isfinite(r->trans_step))
+        return fail(FDCM_ERR_INVALID, "pose refinement: rot_step and trans_step must be finite and >= 0");
+    return FDCM_OK;
+}
+
+// the host table of one level: ci, si of every rotation index and the translation step
+static void refine_level_table(const fdcm_refine_params* r, int level, RefineLevel* lv) {
+    const double step = (double)r->rot_step / std::ldexp(1.0, level);
+    for (int i = -r->rot_steps; i <= r->rot_steps; ++i) {
+        lv->ci[i + r->rot_steps] = (float)std::cos((double)i * step);
+        lv->si[i + r->rot_steps] = (float)std::sin((double)i * step);
+    }
+    lv->h = r->trans_step * std::ldexp(1.0f, -level);
+}
+
+// at most this many matches per call: the evaluation grid has (2 rot_steps + 1) blocks per match
+static constexpr int64_t kRefineMaxMatches = ((int64_t)1 << 31) / kRefineSide;
+
+// Refinement of the n (or *d_n <= n) matches at d_in, queued on `s`; the refined records go to d_out (which may be d_in)
+static fdcm_status run_refine(const fdcm_dt3* m, const fdcm_templates* t, int32_t tmpl_idx_base, const float* d_denom,
+                              const fdcm_refine_params* r, const fdcm_match* d_in, const int* d_n, int n, fdcm_match* d_out,
+                              int smem_optin, cudaStream_t s) {
+    CUDA_TRY(m->s_ref_state.reserve((size_t)n * sizeof(RefineState)));
+    CUDA_TRY(m->s_ref_keys.reserve((size_t)n * 8));
+    RefineLaunch rl;
+    rl.in = d_in;
+    rl.d_n = d_n;
+    rl.n = n;
+    rl.lines = t->lines.as<float4>();
+    rl.offsets = t->offs.as<int32_t>();
+    rl.anchors = t->anchors.as<float2>();
+    rl.denom = d_denom;
+    rl.tmpl_idx_base = tmpl_idx_base;
+    rl.n_r = r->rot_steps;
+    rl.n_t = r->trans_steps;
+    rl.state = m->s_ref_state.as<RefineState>();
+    rl.keys = m->s_ref_keys.as<unsigned long long>();
+    {
+        KernelScope k("refine_init", 0.0, s);
+        launch_refine_init(rl, s);
+    }
+    for (int level = 0; level < r->levels; ++level) {
+        RefineLevel lv{};
+        refine_level_table(r, level, &lv);
+        {
+            KernelScope k("refine_eval", 0.0, s);
+            CUDA_TRY(launch_refine_eval(map_view(m), m->table_dev, rl, lv, t->max_lines, smem_optin, s));
+        }
+        KernelScope k("refine_advance", 0.0, s);
+        launch_refine_advance(rl, lv, level + 1 == r->levels ? d_out : nullptr, s);
+    }
+    CUDA_TRY(cudaGetLastError());
+    return FDCM_OK;
+}
+
+// sel: distinct top-K (fdcm_search_select); ref: pose refinement of the top-K (fdcm_search_refine); nullptr when not asked
 static fdcm_status search_impl(const fdcm_dt3* m, const fdcm_templates* tc, const float* scene, int32_t n_scene,
                                const fdcm_search_params* p, fdcm_match* out, int64_t capacity, int64_t* n_out, fdcm_comm* comm,
-                               const fdcm_select_params* sel) {
+                               const fdcm_select_params* sel, const fdcm_refine_params* ref = nullptr) {
     if (!m || !tc || !p || !n_out) return fail(FDCM_ERR_INVALID, "null argument");
     *n_out = 0;
     if (sel)
@@ -1740,6 +1802,10 @@ static fdcm_status search_impl(const fdcm_dt3* m, const fdcm_templates* tc, cons
             }
             CUDA_TRY(cudaGetLastError());
         }
+        if (ref)
+            if (fdcm_status st = run_refine(m, t, p->tmpl_idx_base, d_denom, ref, m->s_topk_out.as<fdcm_match>(), m->s_topk_n.as<int>(), k,
+                                            m->s_topk_out.as<fdcm_match>(), smem_optin, s))
+                return st;
         result = finish_topk(m, comm, k, s, counters, out, capacity, n_out);
         if (result != FDCM_OK && result != FDCM_ERR_CAPACITY) return result;
     } else {
@@ -1785,6 +1851,84 @@ extern "C" fdcm_status fdcm_search_select(const fdcm_dt3* m, const fdcm_template
                                           int64_t* n_out) {
     if (!select) return fail(FDCM_ERR_INVALID, "select is null");
     return search_impl(m, tc, scene, n_scene, p, out, capacity, n_out, nullptr, select);
+}
+
+extern "C" fdcm_status fdcm_search_refine(const fdcm_dt3* m, const fdcm_templates* tc, const float* scene, int32_t n_scene,
+                                          const fdcm_search_params* p, const fdcm_select_params* select, const fdcm_refine_params* refine,
+                                          fdcm_match* out, int64_t capacity, int64_t* n_out) {
+    if (fdcm_status st = check_refine(refine)) return st;
+    if (!p) return fail(FDCM_ERR_INVALID, "null argument");
+    if (p->top_k < 1 || p->top_k > kRefineMaxMatches)
+        return fail(FDCM_ERR_INVALID, "pose refinement: top_k must be in 1.." + std::to_string(kRefineMaxMatches));
+    return search_impl(m, tc, scene, n_scene, p, out, capacity, n_out, nullptr, select, refine);
+}
+
+extern "C" fdcm_status fdcm_refine_matches(const fdcm_dt3* m, const fdcm_templates* tc, int32_t tmpl_idx_base, int32_t penalty_kind,
+                                           float penalty_tau, const fdcm_refine_params* refine, const fdcm_match* in, int64_t n,
+                                           fdcm_match* out) {
+    if (fdcm_status st = check_refine(refine)) return st;
+    if (!m || !tc || n < 0) return fail(FDCM_ERR_INVALID, "bad argument");
+    if (penalty_kind < 0 || penalty_kind > 2) return fail(FDCM_ERR_INVALID, "bad penalty kind");
+    if (n == 0) return FDCM_OK;
+    if (!in || !out) return fail(FDCM_ERR_INVALID, "null argument");
+    if (n > kRefineMaxMatches) return fail(FDCM_ERR_INVALID, "pose refinement: at most " + std::to_string(kRefineMaxMatches) + " matches per call");
+    if (tc->device != m->device) return fail(FDCM_ERR_INVALID, "templates and feature map live on different devices");
+    if (m->stage != 0) return fail(FDCM_ERR_INVALID, "feature map was built with a debug stage");
+    if (m->dm.D == 0) return fail(FDCM_ERR_INVALID, "refine on an empty feature map");
+    for (int64_t i = 0; i < n; ++i) {
+        const int64_t t = (int64_t)in[i].tmpl_idx - tmpl_idx_base;
+        if (t < 0 || t >= tc->n_tmpl)
+            return fail(FDCM_ERR_OUT_OF_RANGE, "match " + std::to_string(i) + ": tmpl_idx " + std::to_string(in[i].tmpl_idx) +
+                                                   " outside the template set");
+    }
+    fdcm_templates* t = const_cast<fdcm_templates*>(tc);
+    std::lock_guard<std::mutex> lk(m->search_mutex);
+    CUDA_TRY(cudaSetDevice(m->device));
+    cudaStream_t s;
+    if (fdcm_status st = get_stream(m->device, &s)) return st;
+    if (fdcm_status st = templates_ready(t, s)) return st;
+    int smem_optin = 0;
+    if (fdcm_status st = search_smem_optin(m->device, t->max_lines, &smem_optin)) return st;
+    CUDA_TRY(m->s_ref_io.reserve((size_t)n * sizeof(fdcm_match)));
+    CUDA_TRY(cudaMemcpyAsync(m->s_ref_io.p, in, (size_t)n * sizeof(fdcm_match), cudaMemcpyHostToDevice, s));
+    const float* d_denom = nullptr;
+    if (penalty_kind != FDCM_PENALTY_NONE) {   // the search's denominators (penalty_denominator)
+        std::vector<float> den((size_t)t->n_tmpl);
+        for (int i = 0; i < t->n_tmpl; ++i) den[(size_t)i] = penalty_denominator(penalty_kind, penalty_tau, t->lengths[(size_t)i]);
+        CUDA_TRY(m->s_ref_denom.reserve(den.size() * 4));
+        CUDA_TRY(cudaMemcpyAsync(m->s_ref_denom.p, den.data(), den.size() * 4, cudaMemcpyHostToDevice, s));
+        d_denom = m->s_ref_denom.as<float>();
+    }
+    fdcm_match* d_io = m->s_ref_io.as<fdcm_match>();
+    if (fdcm_status st = run_refine(m, t, tmpl_idx_base, d_denom, refine, d_io, nullptr, (int)n, d_io, smem_optin, s)) return st;
+    CUDA_TRY(cudaMemcpyAsync(out, d_io, (size_t)n * sizeof(fdcm_match), cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(cudaStreamSynchronize(s));
+    prof_resolve();
+    return FDCM_OK;
+}
+
+extern "C" fdcm_status fdcm_refine_poses(const float transform[6], const float anchor[2], const fdcm_refine_params* refine, int32_t level,
+                                         float* out) {
+    if (fdcm_status st = check_refine(refine)) return st;
+    if (!transform || !anchor || !out) return fail(FDCM_ERR_INVALID, "null argument");
+    if (level < 0 || level >= refine->levels) return fail(FDCM_ERR_INVALID, "level must be in 0..levels - 1");
+    RefineLevel lv{};
+    refine_level_table(refine, level, &lv);
+    const int n_r = refine->rot_steps, n_t = refine->trans_steps, NT = 2 * n_t + 1;
+    for (int ir = 0; ir < 2 * n_r + 1; ++ir) {
+        const RefineRot R = refine_rotation(transform, anchor[0], anchor[1], ir - n_r, lv.ci[ir], lv.si[ir]);
+        for (int kk = 0; kk < NT; ++kk)
+            for (int jj = 0; jj < NT; ++jj) {
+                float* P = out + 6 * (size_t)((ir * NT + kk) * NT + jj);
+                if (ir == n_r && kk == n_t && jj == n_t) {   // the grid point (0, 0, 0) is C itself
+                    for (int q = 0; q < 6; ++q) P[q] = transform[q];
+                    continue;
+                }
+                P[0] = R.r0; P[1] = R.r1; P[2] = R.bx + (float)(jj - n_t) * lv.h;
+                P[3] = R.r3; P[4] = R.r4; P[5] = R.by + (float)(kk - n_t) * lv.h;
+            }
+    }
+    return FDCM_OK;
 }
 
 // fdcm_search of this rank's template shard (params->tmpl_idx_base = first global index of the shard) followed by the

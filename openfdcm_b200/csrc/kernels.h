@@ -162,6 +162,42 @@ void launch_select_walk(const SelectLaunch& p, const uint64_t* sorted_keys, cons
                         cudaStream_t s);
 // d_out[0, top_k) + *d_n_out are written like the top-K kernels' (unused slots: tmpl_idx -1, score +inf).
 
+// pose refinement (fdcm_refine_matches / fdcm_search_refine; rules in include/fdcm_b200.h)
+constexpr int kRefineSide = 2 * FDCM_REFINE_MAX_STEPS + 1;
+struct RefineLevel {             // host-computed table of one level
+    float ci[kRefineSide], si[kRefineSide];   // index i + rot_steps
+    float h;                     // trans_step * 2^-level
+};
+struct RefineState { float c[6]; float raw; int32_t valid; };   // running centre C, its raw score, any valid pose yet
+struct RefineLaunch {
+    const fdcm_match* in;        // the matches (tmpl_idx, transform M)
+    const int* d_n;              // number of matches on the device (fused path), or nullptr: n
+    int32_t n;                   // slots (the grid covers n matches)
+    const float4* lines;         // template set
+    const int32_t* offsets;
+    const float2* anchors;
+    const float* denom;          // per template penalty denominator, or nullptr
+    int32_t tmpl_idx_base;
+    int32_t n_r, n_t;
+    RefineState* state;          // n
+    unsigned long long* keys;    // n: (score bits << 32 | walk order << 1 | score is NaN) of the level's best, ~0 when none
+};
+// the pose of a grid point with rotation index i (cos ci, sin si) around the anchor (ax, ay) of C, before dx / dy
+struct RefineRot { float r0, r1, r3, r4, bx, by; };
+__host__ __device__ inline RefineRot refine_rotation(const float* c, float ax, float ay, int i, float ci, float si) {
+    if (i == 0) return RefineRot{c[0], c[1], c[3], c[4], c[2], c[5]};
+    const float px = (c[0] * ax + c[1] * ay) + c[2], py = (c[3] * ax + c[4] * ay) + c[5];
+    const float ux = c[2] - px, uy = c[5] - py;
+    return RefineRot{ci * c[0] - si * c[3], ci * c[1] - si * c[4], si * c[0] + ci * c[3], si * c[1] + ci * c[4],
+                     (ci * ux - si * uy) + px, (si * ux + ci * uy) + py};
+}
+void launch_refine_init(const RefineLaunch& p, cudaStream_t s);
+// one level: one block per (match, rotation), one thread per translation (k, j); atomicMin of the key per match
+cudaError_t launch_refine_eval(const MapView& map, const SlopeTableDev& table, const RefineLaunch& p, const RefineLevel& lv,
+                               int max_lines, int smem_optin, cudaStream_t s);
+// the level's argmin becomes the centre; out != nullptr (last level): writes the refined matches
+void launch_refine_advance(const RefineLaunch& p, const RefineLevel& lv, fdcm_match* out, cudaStream_t s);
+
 void launch_evaluate(const MapView& map, const SlopeTableDev& table, const float4* d_lines, const int32_t* d_toff,
                      const float2* d_transl, const int32_t* d_troff, const int32_t* d_owner, int64_t n_scores,
                      float* d_scores, cudaStream_t s);

@@ -258,17 +258,49 @@ PYBIND11_MODULE(_openfdcm_cuda, m) {
                    ", max_angle=" + std::to_string(a.maxAngle) + ", across_templates=" + (a.acrossTemplates ? "True" : "False") + ">";
         });
 
+    py::class_<PoseRefinement>(m, "PoseRefinement")
+        .def(py::init([](int levels, int rot_steps, float rot_step, int trans_steps, float trans_step) {
+                 return PoseRefinement{levels, rot_steps, rot_step, trans_steps, trans_step};
+             }), "levels"_a = 3, "rot_steps"_a = 4, "rot_step"_a = 0.01f, "trans_steps"_a = 4, "trans_step"_a = 1.f)
+        .def_readwrite("levels", &PoseRefinement::levels)
+        .def_readwrite("rot_steps", &PoseRefinement::rotSteps)
+        .def_readwrite("rot_step", &PoseRefinement::rotStep)
+        .def_readwrite("trans_steps", &PoseRefinement::transSteps)
+        .def_readwrite("trans_step", &PoseRefinement::transStep)
+        .def("__repr__", [](const PoseRefinement& a) {
+            return "<PoseRefinement: levels=" + std::to_string(a.levels) + ", rot_steps=" + std::to_string(a.rotSteps) + ", rot_step=" +
+                   std::to_string(a.rotStep) + ", trans_steps=" + std::to_string(a.transSteps) + ", trans_step=" + std::to_string(a.transStep) + ">";
+        });
+
     m.def("search_topk",
           [](const Dt3Cuda& featuremap, const std::vector<LinesIn>& templates, const LinesIn& scene, const DefaultSearch& searcher,
-             const BatchOptimize& optimizer, const ExponentialPenalty& penalty, int k, const std::optional<DistinctMatches>& select) {
+             const BatchOptimize& optimizer, const ExponentialPenalty& penalty, int k, const std::optional<DistinctMatches>& select,
+             const std::optional<PoseRefinement>& refine) {
               const auto t = to_templates(templates);
               const auto s = to_lines(scene);
               py::gil_scoped_release release;
+              if (refine && select) return searchTopK(searcher, optimizer, penalty, featuremap, t, s, k, *select, *refine);
+              if (refine) return searchTopK(searcher, optimizer, penalty, featuremap, t, s, k, *refine);
               if (select) return searchTopK(searcher, optimizer, penalty, featuremap, t, s, k, *select);
               return searchTopK(searcher, optimizer, penalty, featuremap, t, s, k);
           },
           "featuremap"_a, "templates"_a, "scene"_a, "searcher"_a, "optimizer"_a, "penalty"_a, "k"_a = 10, py::kw_only(), "select"_a = py::none(),
-          "Fused search -> penalize -> top-k on the device (ascending score); select: DistinctMatches for the distinct top-k");
+          "refine"_a = py::none(),
+          "Fused search -> penalize -> top-k on the device (ascending score); select: DistinctMatches for the distinct top-k; "
+          "refine: PoseRefinement of the selected matches (not re-sorted; it minimises the score, which was measured to increase the "
+          "error against known poses)");
+
+    m.def("refine_matches",
+          [](const Dt3Cuda& featuremap, const std::vector<LinesIn>& templates, const std::vector<Match>& matches, const PoseRefinement& refine,
+             const std::optional<ExponentialPenalty>& penalty) {
+              const auto t = to_templates(templates);
+              py::gil_scoped_release release;
+              if (penalty) return refineMatches(featuremap, t, matches, refine, *penalty);
+              return refineMatches(featuremap, t, matches, refine);
+          },
+          "featuremap"_a, "templates"_a, "matches"_a, "refine"_a, "penalty"_a = py::none(),
+          "Pose refinement of every match (entry i refines matches[i]) to the lowest evaluate score of its grid, not to a more "
+          "accurate pose; with a penalty, scores are penalised like search_topk");
 
     m.def("penalize",
           [](const PenaltyStrategy& penalty, const std::vector<Match>& matches, const std::vector<float>& templatelengths) {

@@ -785,6 +785,155 @@ void launch_select_walk(const SelectLaunch& p, const uint64_t* sorted_keys, cons
 }
 
 // =============================================================================================
+// Pose refinement (fdcm_refine_matches / fdcm_search_refine, beyond the reference): rules in include/fdcm_b200.h.
+// One block per (match, rotation i): the rotated template and its orientation bins are staged in shared memory once, then
+// thread (k, j) scores the translation (j h, k h), so that with h = 1 the lanes of a row gather runs of adjacent pixels as
+// in the search kernel.  Every thread sums its own candidate in Eigen's order (evaluate<Dt3Cpu>).  The walk's argmin is
+// the minimum of a 64-bit key (score, grid order) over all candidates of a match, taken with one atomicMin per warp.
+// =============================================================================================
+constexpr unsigned long long kNoPose = ~0ull;
+
+__global__ void refine_init_kernel(const __grid_constant__ RefineLaunch p) {
+    const int m = blockIdx.x * blockDim.x + threadIdx.x;
+    if (m >= (p.d_n ? *p.d_n : p.n)) return;
+    RefineState st;
+    for (int q = 0; q < 6; ++q) st.c[q] = p.in[m].transform[q];
+    st.raw = NAN;
+    st.valid = 0;
+    p.state[m] = st;
+    p.keys[m] = kNoPose;
+}
+
+void launch_refine_init(const RefineLaunch& p, cudaStream_t s) {
+    refine_init_kernel<<<(unsigned)((p.n + 127) / 128), 128, 0, s>>>(p);
+}
+
+__global__ void __launch_bounds__(1024) refine_eval_kernel(const __grid_constant__ MapView map,
+                                                           const __grid_constant__ SlopeTableDev table,
+                                                           const __grid_constant__ RefineLaunch p,
+                                                           const __grid_constant__ RefineLevel lv) {
+    // rotated end points float4[L], planes u8[L]: the search's staging size, and no static shared memory, so that every
+    // template the search accepts fits the opt-in limit
+    extern __shared__ __align__(16) uint8_t s_raw[];
+    const int NR = 2 * p.n_r + 1, NT = 2 * p.n_t + 1;
+    const int m = blockIdx.x / NR, ir = blockIdx.x % NR;
+    if (m >= (p.d_n ? *p.d_n : p.n)) return;   // whole block
+    const int tid = threadIdx.x, lane = tid & 31;
+    const RefineState st = p.state[m];
+    const int t = p.in[m].tmpl_idx - p.tmpl_idx_base;
+    const int l0 = p.offsets[t], L = p.offsets[t + 1] - l0;
+    const float2 a = p.anchors[t];
+    const RefineRot R = refine_rotation(st.c, a.x, a.y, ir - p.n_r, lv.ci[ir], lv.si[ir]);
+    float4* apts = reinterpret_cast<float4*>(s_raw);
+    uint8_t* bins = reinterpret_cast<uint8_t*>(apts + L);
+    bool nan = false;
+    for (int q = tid; q < L; q += blockDim.x) {
+        const float4 v = __ldg(p.lines + l0 + q);
+        const float x1 = R.r0 * v.x + R.r1 * v.y, y1 = R.r3 * v.x + R.r4 * v.y;
+        const float x2 = R.r0 * v.z + R.r1 * v.w, y2 = R.r3 * v.z + R.r4 * v.w;
+        nan |= x1 != x1 || y1 != y1 || x2 != x2 || y2 != y2;
+        apts[q] = make_float4(x1, y1, x2, y2);
+        bins[q] = (uint8_t)bin_of_slope_dev(table, (y2 - y1) / (x2 - x1));
+    }
+    nan = __syncthreads_or(nan) != 0;   // also publishes apts / bins
+    // bounding box of the rotated template: every warp reduces the staged points itself (no cross-warp exchange)
+    float mnx = INFINITY, mny = INFINITY, mxx = -INFINITY, mxy = -INFINITY;
+    for (int q = lane; q < L; q += 32) {
+        const float4 e = apts[q];
+        mnx = fminf(mnx, fminf(e.x, e.z)); mxx = fmaxf(mxx, fmaxf(e.x, e.z));
+        mny = fminf(mny, fminf(e.y, e.w)); mxy = fmaxf(mxy, fmaxf(e.y, e.w));
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        mnx = fminf(mnx, __shfl_xor_sync(0xffffffffu, mnx, o)); mxx = fmaxf(mxx, __shfl_xor_sync(0xffffffffu, mxx, o));
+        mny = fminf(mny, __shfl_xor_sync(0xffffffffu, mny, o)); mxy = fmaxf(mxy, __shfl_xor_sync(0xffffffffu, mxy, o));
+    }
+    unsigned long long key = kNoPose;
+    if (tid < NT * NT) {
+        const int kk = tid / NT, jj = tid - kk * NT;
+        const float P2 = R.bx + (float)(jj - p.n_t) * lv.h, P5 = R.by + (float)(kk - p.n_t) * lv.h;
+        const float offx = map.shift_x + P2, offy = map.shift_y + P5;
+        // the rounding of r + off is monotonic in r, so the bounding box decides for every end point
+        bool valid = !nan && !(R.r0 != R.r0 || R.r1 != R.r1 || R.r3 != R.r3 || R.r4 != R.r4 || P2 != P2 || P5 != P5);
+        if (valid && L > 0)
+            valid = 0.f <= mnx + offx && mxx + offx <= (float)(map.dm.W - 1) && 0.f <= mny + offy && mxy + offy <= (float)(map.dm.H - 1);
+        if (valid) {
+            const float* planes = map.planes;
+            const size_t pitch = (size_t)map.dm.pitch, pe = map.dm.plane_elems;
+            const float sc = eigen_sum_lazy(L, [&](int q) {
+                const float4 e = apts[q];
+                const int x1 = (int)(e.x + offx), y1 = (int)(e.y + offy), x2 = (int)(e.z + offx), y2 = (int)(e.w + offy);
+                const float* P = planes + (size_t)bins[q] * pe;
+                return fabsf(__ldg(P + (size_t)y1 * pitch + x1) - __ldg(P + (size_t)y2 * pitch + x2));
+            });
+            // walk order: squared grid distance from the centre (0 only for the centre), then (i, k, j)
+            const int di = ir - p.n_r, dk = kk - p.n_t, dj = jj - p.n_t;
+            const unsigned order = (unsigned)(di * di + dk * dk + dj * dj) << 15 | (unsigned)((ir * NT + kk) * NT + jj);
+            const bool is_nan = sc != sc;
+            key = (unsigned long long)(is_nan ? 0x7F800000u : __float_as_uint(sc)) << 32 | (unsigned long long)(order << 1 | (is_nan ? 1u : 0u));
+        }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        const unsigned long long other = __shfl_xor_sync(0xffffffffu, key, o);
+        key = other < key ? other : key;
+    }
+    if (lane == 0 && key != kNoPose) atomicMin(p.keys + m, key);
+}
+
+static size_t refine_smem_bytes(int max_lines) { return (size_t)max_lines * 16 + (((size_t)max_lines + 15) & ~(size_t)15); }
+
+cudaError_t launch_refine_eval(const MapView& map, const SlopeTableDev& table, const RefineLaunch& p, const RefineLevel& lv,
+                               int max_lines, int smem_optin, cudaStream_t s) {
+    const int NR = 2 * p.n_r + 1, NT = 2 * p.n_t + 1;
+    const int threads = ((NT * NT + 31) / 32) * 32;
+    const size_t smem = refine_smem_bytes(max_lines > 0 ? max_lines : 1);
+    if (smem > (size_t)smem_optin) return cudaErrorInvalidValue;   // callers reject such templates first
+    if (smem > 48 * 1024) {
+        const cudaError_t e = cudaFuncSetAttribute(refine_eval_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+    }
+    refine_eval_kernel<<<(unsigned)((int64_t)p.n * NR), threads, smem, s>>>(map, table, p, lv);
+    return cudaGetLastError();
+}
+
+__global__ void refine_advance_kernel(const __grid_constant__ RefineLaunch p, const __grid_constant__ RefineLevel lv,
+                                      fdcm_match* out) {
+    const int m = blockIdx.x * blockDim.x + threadIdx.x;
+    if (m >= (p.d_n ? *p.d_n : p.n)) return;
+    const int tmpl_idx = p.in[m].tmpl_idx;   // (out may be in)
+    const int t = tmpl_idx - p.tmpl_idx_base;
+    RefineState st = p.state[m];
+    const unsigned long long key = p.keys[m];
+    if (key != kNoPose) {
+        const unsigned order = (unsigned)key >> 1;
+        if ((order >> 15) != 0u) {   // not the centre: recompute the winning pose exactly as refine_eval_kernel did
+            const int NT = 2 * p.n_t + 1, g = (int)(order & 0x7FFFu);
+            const int jj = g % NT, kk = (g / NT) % NT, ir = g / (NT * NT);
+            const float2 a = p.anchors[t];
+            const RefineRot R = refine_rotation(st.c, a.x, a.y, ir - p.n_r, lv.ci[ir], lv.si[ir]);
+            st.c[0] = R.r0; st.c[1] = R.r1; st.c[2] = R.bx + (float)(jj - p.n_t) * lv.h;
+            st.c[3] = R.r3; st.c[4] = R.r4; st.c[5] = R.by + (float)(kk - p.n_t) * lv.h;
+        }
+        st.raw = (key & 1ull) ? NAN : __uint_as_float((unsigned)(key >> 32));
+        st.valid = 1;
+        p.state[m] = st;
+        p.keys[m] = kNoPose;
+    }
+    if (out) {
+        fdcm_match r;
+        r.tmpl_idx = tmpl_idx;
+        r.score = st.valid ? (p.denom ? st.raw / p.denom[t] : st.raw) : NAN;
+        for (int q = 0; q < 6; ++q) r.transform[q] = st.c[q];
+        out[m] = r;
+    }
+}
+
+void launch_refine_advance(const RefineLaunch& p, const RefineLevel& lv, fdcm_match* out, cudaStream_t s) {
+    refine_advance_kernel<<<(unsigned)((p.n + 127) / 128), 128, 0, s>>>(p, lv, out);
+}
+
+// =============================================================================================
 // evaluate<Dt3Cpu> (dt3cpu.cpp:126-179) as a standalone entry point: one thread per (template, translation)
 // =============================================================================================
 __global__ void __launch_bounds__(128) evaluate_kernel(const __grid_constant__ MapView map,
