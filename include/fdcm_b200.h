@@ -256,6 +256,60 @@ fdcm_status fdcm_search_refine(const fdcm_dt3* map, const fdcm_templates* templa
 fdcm_status fdcm_refine_poses(const float transform[6], const float anchor[2], const fdcm_refine_params* refine, int32_t level,
                               float* out);
 
+/* ---- dense pose-grid search (beyond the reference) ----------------------------------------------
+ * The search above only poses a template where one of its longest lines lies on one of the scene's longest lines, so a
+ * broken, merged or missing scene line leaves no hypothesis.  The dense search scores every template at a grid of
+ * rotations about its anchor and translations that put the anchor on a grid of map pixels, keeps the best pose of every
+ * cell of the grid and passes those records through the search's top-K or distinct selection, then optionally refinement.
+ * The grid is finite: before refinement a pose is off by up to stride / 2 px and rot_step / 2 rad, and like refinement
+ * it minimises the evaluate<Dt3Cpu> score, which is not lowest at the true pose at sub-pixel scales.
+ * Rules, in fp32 without contraction.  Map W x H, scene translation shift = (shift_x, shift_y), templates t = 0..T-1:
+ *   1. Rotations r = 0..rotations-1: theta_r = (double)rot_start + r * (double)rot_step, c_r = (float)cos(theta_r),
+ *      s_r = (float)sin(theta_r) (host C library).
+ *   2. Grid.  Map-pixel range [lo_x, hi_x] x [lo_y, hi_y]: [0, W-1] x [0, H-1], or with roi_on and roi = (x0, y0, x1, y1)
+ *      in scene coordinates lo_x = max(0, ceil(x0 + shift_x)), hi_x = min(W-1, floor(x1 + shift_x)) evaluated in double,
+ *      y likewise.  Grid point (u, v) is the map pixel (gx, gy) = (lo_x + u stride, lo_y + v stride), for every such
+ *      point inside the range: nx = (hi_x - lo_x) / stride + 1 per row (0 when lo_x > hi_x), ny likewise.  Grid index
+ *      g = v nx + u (row-major).
+ *   3. Pose with anchor a (fdcm_template_anchors): qx = (float)gx - shift_x, qy = (float)gy - shift_y,
+ *      P = (c, -s, qx - (c*ax - s*ay), s, c, qy - (s*ax + c*ay)).  When c == 1 and s == 0 the end points are used exactly
+ *      as given, without a multiply (-s * y would turn the zero dx of a vertical line negative and flip its orientation
+ *      bin), so the theta = 0 slice is fdcm_dt3_evaluate of the template itself.
+ *   4. Score and validity: refinement rule 4 (rotated end points (P0*x + P1*y, P3*x + P4*y), orientation bin from the
+ *      rotated slope, lookups (int)(r + (shift + P2)), Eigen's sum order; valid iff nothing is NaN and the rotated end
+ *      points lie inside the map); invalid poses are never read.  An empty template has no valid pose.
+ *   5. Cells.  Grid point (u, v) is in cell (cu, cv) = (u / cell, v / cell); cells_x = ceil(nx / cell), cells_y likewise.
+ *      Record h = ((t * rotations + r) * cells_y + cv) * cells_x + cu is valid iff its cell has a valid pose; its pose is
+ *      the valid pose of the cell with the lowest raw score (NaN as +inf), ties to the lowest grid index; its score is the
+ *      raw score, divided by the search's penalty denominator of t (host powf of the template length) when a penalty is
+ *      given (the argmin is taken on the raw score); tmpl_idx = t + tmpl_idx_base.
+ *   6. Output: the valid records like fdcm_search's hypothesis records: the top_k best in (score, h) order, or with select
+ *      the walk of fdcm_search_select; then with refine the refinement of those, byte-identical to fdcm_refine_matches of
+ *      the unrefined output.
+ * Invalid parameters fail with FDCM_ERR_INVALID: rotations outside 1..FDCM_DENSE_MAX_ROTATIONS, stride < 1, cell < 1,
+ * rot_start or rot_step not finite, a region not finite or with x0 > x1 or y0 > y1, top_k < 1, a record count of 2^31
+ * or more (T * rotations * cells_y * cells_x), a template longer than the search accepts, and the select and refine
+ * parameters fdcm_search_refine rejects.  An empty map, an empty template set or a grid without points (a region outside
+ * the map) give no matches.  Cost: T * rotations * nx * ny poses of up to 2 L map gathers each; the dense search is
+ * meant for template sets of hundreds, not thousands. */
+#define FDCM_DENSE_MAX_ROTATIONS 4096
+typedef struct fdcm_dense_params {       /* 40 bytes */
+    int32_t rotations;          /* 1..FDCM_DENSE_MAX_ROTATIONS */
+    float rot_start;            /* radians */
+    float rot_step;             /* radians */
+    int32_t stride;             /* >= 1: map pixels between grid points */
+    int32_t cell;               /* >= 1: grid points per cell side; every cell keeps its best pose */
+    int32_t roi_on;             /* 0: the whole map; 1: the region roi */
+    float roi[4];               /* x0, y0, x1, y1 in scene coordinates (inclusive) */
+} fdcm_dense_params;
+fdcm_status fdcm_search_dense(const fdcm_dt3* map, const fdcm_templates* templates, const fdcm_dense_params* dense, int32_t penalty_kind,
+                              float penalty_tau, int32_t top_k, int32_t tmpl_idx_base, const fdcm_select_params* select,
+                              const fdcm_refine_params* refine, fdcm_match* out, int64_t capacity, int64_t* n_out);
+/* the transforms of rotation `rotation` in grid order, 6 floats each (*n_out = nx * ny; FDCM_ERR_CAPACITY when that exceeds
+ * capacity), and grid_wh = (nx, ny), for a map of W x H with scene translation shift; host-only parity hook */
+fdcm_status fdcm_dense_poses(const fdcm_dense_params* dense, const float anchor[2], const float shift[2], int32_t width, int32_t height,
+                             int32_t rotation, float* out, int64_t capacity, int64_t* n_out, int32_t grid_wh[2]);
+
 /* optimize(optimizer, templates, alignments, featuremap) (matching/optimizestrategy.h:62-64; BatchOptimize:
  * batchoptimize.cpp:6-123, batch_size == 0: DefaultOptimize, defaultoptimize.cpp:6-93).  The templates are used
  * as given (already aligned); alignments: n_tmpl (x,y) pairs.  Outputs per template: has_value (0 = nullopt),

@@ -346,6 +346,55 @@ inline std::vector<Match> refineMatches(const Dt3Cuda& fm, const std::vector<Lin
     return detail::refine_matches(fm, templates, matches, refine, FDCM_PENALTY_EXPONENTIAL, pen.tau);
 }
 
+// dense pose-grid search (beyond the reference; rules of fdcm_search_dense): every template at `rotations` rotations
+// rotStart + r * rotStep about its anchor (rotStep < 0: 2 pi / rotations) and at every stride-th map pixel (or of the
+// region roi = {x0, y0, x1, y1} in scene coordinates when hasRoi); each cell of cell x cell grid points keeps its best pose
+struct DenseSearch {
+    int rotations{72};
+    float rotStart{0.f};
+    float rotStep{-1.f};
+    int stride{2};
+    int cell{8};
+    bool hasRoi{false};
+    std::array<float, 4> roi{{0.f, 0.f, 0.f, 0.f}};
+};
+namespace detail {
+inline std::vector<Match> search_dense(const Dt3Cuda& fm, const std::vector<LineArray>& templates, const DenseSearch& dense, int penalty_kind,
+                                       float tau, int k, const DistinctMatches* select, const PoseRefinement* refine) {
+    std::vector<float> flat;
+    std::vector<int32_t> off;
+    pack(templates, flat, off);
+    fdcm_templates* ts = nullptr;
+    check(fdcm_templates_create(flat.data(), off.data(), (int32_t)templates.size(), fm.info().device, &ts));
+    const std::unique_ptr<fdcm_templates, fdcm_status (*)(fdcm_templates*)> owner(ts, fdcm_templates_release);
+    const float step = dense.rotStep >= 0.f || dense.rotations < 1 ? dense.rotStep : (float)(2.0 * 3.14159265358979323846 / dense.rotations);
+    const fdcm_dense_params d{dense.rotations, dense.rotStart, step, dense.stride, dense.cell, dense.hasRoi ? 1 : 0,
+                              {dense.roi[0], dense.roi[1], dense.roi[2], dense.roi[3]}};
+    fdcm_select_params q{};
+    if (select) q = fdcm_select_params{select->maxPerTemplate, select->radius, select->maxAngle, select->acrossTemplates ? 1 : 0};
+    fdcm_refine_params r{};
+    if (refine) r = refine_params(*refine);
+    std::vector<fdcm_match> rec((size_t)std::max(k, 1));
+    int64_t n = 0;
+    check(fdcm_search_dense(fm.handle(), ts, &d, penalty_kind, tau, k, 0, select ? &q : nullptr, refine ? &r : nullptr, rec.data(),
+                            (int64_t)rec.size(), &n));
+    return to_matches(rec, n);
+}
+}   // namespace detail
+// dense search -> top-k (or distinct top-k) [-> pose refinement] on the device, penalised like searchTopK
+inline std::vector<Match> searchDense(const Dt3Cuda& fm, const std::vector<LineArray>& templates, const DenseSearch& dense,
+                                      const ExponentialPenalty& pen, int k) {
+    return detail::search_dense(fm, templates, dense, FDCM_PENALTY_EXPONENTIAL, pen.tau, k, nullptr, nullptr);
+}
+inline std::vector<Match> searchDense(const Dt3Cuda& fm, const std::vector<LineArray>& templates, const DenseSearch& dense,
+                                      const ExponentialPenalty& pen, int k, const DistinctMatches& select) {
+    return detail::search_dense(fm, templates, dense, FDCM_PENALTY_EXPONENTIAL, pen.tau, k, &select, nullptr);
+}
+inline std::vector<Match> searchDense(const Dt3Cuda& fm, const std::vector<LineArray>& templates, const DenseSearch& dense,
+                                      const ExponentialPenalty& pen, int k, const DistinctMatches* select, const PoseRefinement* refine) {
+    return detail::search_dense(fm, templates, dense, FDCM_PENALTY_EXPONENTIAL, pen.tau, k, select, refine);
+}
+
 // ---- PenaltyStrategy concept, template lengths, sort ----------------------------------------------
 inline std::vector<float> getTemplateLengths(const std::vector<LineArray>& templates) {   // core/math.h:319-324
     std::vector<float> flat, len(templates.size());

@@ -22,7 +22,8 @@ from ._lib import MATCH_DTYPE, FdcmError, check, lib, ptr
 __all__ = [
     "distance", "Dt3CudaParameters", "Dt3Cuda", "build_cuda_featuremap", "ThreadPool", "DefaultSearch", "ConcentricRangeStrategy",
     "BatchOptimize", "DefaultOptimize", "DefaultMatch", "DefaultPenalty", "ExponentialPenalty", "Match",
-    "TemplateSet", "SceneBatch", "DistinctMatches", "PoseRefinement", "search", "search_topk", "refine_matches", "penalize", "get_template_lengths",
+    "TemplateSet", "SceneBatch", "DistinctMatches", "PoseRefinement", "DenseSearch", "search", "search_topk", "search_dense",
+    "refine_matches", "penalize", "get_template_lengths",
     "get_template_anchors", "sort_matches", "evaluate",
     "minmax_translation", "get_feature_size", "establish_search_strategy", "optimize", "read", "write", "FdcmError", "MATCH_DTYPE",
 ]
@@ -350,6 +351,35 @@ class PoseRefinement:
                 f"trans_steps={self.trans_steps}, trans_step={self.trans_step}>")
 
 
+class DenseSearch:
+    """Dense pose-grid search (beyond the reference): every template at `rotations` rotations rot_start + r * rot_step
+    about its anchor (rot_step None: 2 pi / rotations) and at every `stride`-th map pixel of the map, or of the region
+    roi = (x0, y0, x1, y1) in scene coordinates; each cell of cell x cell grid points keeps its best pose.  The grid is
+    finite (pose error up to stride / 2 px and rot_step / 2 rad before refinement) and minimises the evaluate<Dt3Cpu>
+    score, which is not lowest at the true pose at sub-pixel scales.  Exact rules: include/fdcm_b200.h."""
+
+    def __init__(self, rotations=72, rot_start=0.0, rot_step=None, stride=2, cell=8, roi=None):
+        self.rotations = int(rotations)
+        self.rot_start = float(rot_start)
+        if rot_step is None:   # one full turn (rotations < 1 is rejected by the search)
+            rot_step = 2.0 * math.pi / self.rotations if self.rotations > 0 else 0.0
+        self.rot_step = float(rot_step)
+        self.stride = int(stride)
+        self.cell = int(cell)
+        self.roi = None if roi is None else tuple(float(v) for v in roi)
+        if self.roi is not None and len(self.roi) != 4:
+            raise ValueError("roi must be (x0, y0, x1, y1)")
+
+    def _params(self):
+        roi = self.roi or (0.0, 0.0, 0.0, 0.0)
+        return _lib.DenseParams(self.rotations, self.rot_start, self.rot_step, self.stride, self.cell, 0 if self.roi is None else 1,
+                                (C.c_float * 4)(*roi))
+
+    def __repr__(self):
+        return (f"<DenseSearch: rotations={self.rotations}, rot_start={self.rot_start}, rot_step={self.rot_step}, stride={self.stride}, "
+                f"cell={self.cell}, roi={self.roi}>")
+
+
 def _search_raw(featuremap, templates, scene, searcher, optimizer, penalty=None, top_k=0, tmpl_idx_base=0, select=None, refine=None):
     if not isinstance(featuremap, Dt3Cuda):
         raise TypeError("the CUDA search needs a Dt3Cuda feature map (build_cuda_featuremap)")
@@ -410,6 +440,23 @@ def refine_matches(featuremap, templates, matches, refine, penalty=None, tmpl_id
         raise IndexError(lib().fdcm_last_error().decode())
     check(st)
     return out[: rec.shape[0]].copy()
+
+
+def search_dense(featuremap, templates, dense, penalty=None, k=10, tmpl_idx_base=0, *, select=None, refine=None):
+    """Dense pose-grid search on the device (see DenseSearch): the best pose of every (template, rotation, cell), then the
+    top-k in ascending (score, record) order, or with select (a DistinctMatches) the distinct top-k, then with refine (a
+    PoseRefinement) the refinement of those, equal to refine_matches of the unrefined result.  Returns a MATCH_DTYPE array."""
+    if not isinstance(featuremap, Dt3Cuda):
+        raise TypeError("search_dense needs a Dt3Cuda feature map (build_cuda_featuremap)")
+    tset = templates if isinstance(templates, TemplateSet) else TemplateSet(templates, featuremap.device)
+    out = np.zeros(max(int(k), 1), MATCH_DTYPE)
+    n = C.c_int64(0)
+    sp = None if select is None else C.byref(select._params())
+    rp = None if refine is None else C.byref(refine._params())
+    check(lib().fdcm_search_dense(featuremap._h, tset._h, C.byref(dense._params()), 0 if penalty is None else penalty.kind,
+                                  0.0 if penalty is None else float(penalty.tau), int(k), int(tmpl_idx_base), sp, rp, ptr(out), out.shape[0],
+                                  C.byref(n)))
+    return out[: n.value].copy()
 
 
 def search_all(featuremap, templates, scene, searcher, optimizer, penalty=None, tmpl_idx_base=0):

@@ -36,6 +36,11 @@ class RefineParams(C.Structure):
                 ("trans_step", C.c_float)]
 
 
+class DenseParams(C.Structure):
+    _fields_ = [("rotations", C.c_int32), ("rot_start", C.c_float), ("rot_step", C.c_float), ("stride", C.c_int32), ("cell", C.c_int32),
+                ("roi_on", C.c_int32), ("roi", C.c_float * 4)]
+
+
 class Dt3Info(C.Structure):
     _fields_ = [("depth", C.c_int32), ("width", C.c_int32), ("height", C.c_int32), ("pitch", C.c_int32),
                 ("scene_translation", C.c_float * 2), ("distance", C.c_int32), ("device", C.c_int32),
@@ -81,6 +86,10 @@ SIGNATURES = {
     "fdcm_search_refine": (C.c_int, [_P, _P, _P, C.c_int32, C.POINTER(SearchParams), C.POINTER(SelectParams), C.POINTER(RefineParams), _P,
                                      C.c_int64, C.POINTER(C.c_int64)]),
     "fdcm_refine_poses": (C.c_int, [_P, _P, C.POINTER(RefineParams), C.c_int32, _P]),
+    "fdcm_search_dense": (C.c_int, [_P, _P, C.POINTER(DenseParams), C.c_int32, C.c_float, C.c_int32, C.c_int32, C.POINTER(SelectParams),
+                                    C.POINTER(RefineParams), _P, C.c_int64, C.POINTER(C.c_int64)]),
+    "fdcm_dense_poses": (C.c_int, [C.POINTER(DenseParams), _P, _P, C.c_int32, C.c_int32, C.c_int32, _P, C.c_int64, C.POINTER(C.c_int64),
+                                   _P]),
     "fdcm_optimize": (C.c_int, [_P, _P, _P, C.c_int32, _P, C.c_int32, _P, _P, _P]),
     "fdcm_search_host": (C.c_int, [_P, _P, _P, C.c_int32, _P, C.c_int32, C.POINTER(SearchParams), _P, C.c_int64,
                                    C.POINTER(C.c_int64)]),

@@ -292,6 +292,7 @@ struct fdcm_dt3 {
         s_topk_out, s_topk_n, s_keys, s_keys2, s_idx, s_perm, s_sort_tmp;
     mutable DevBuf s_sel_keys, s_sel_keys2, s_sel_vals, s_sel_vals2, s_sel_surv, s_sel_acc, s_sel_tmp;   // distinct top-K
     mutable DevBuf s_ref_state, s_ref_keys, s_ref_io, s_ref_denom;   // pose refinement
+    mutable DevBuf s_dense_keys, s_dense_rot;   // dense pose-grid search (records: s_rec / s_valid / s_hyp_off)
     mutable float s_scene_min[2] = {0.f, 0.f}, s_scene_max[2] = {0.f, 0.f};   // bbox of the resident search scene
     mutable std::mutex host_tset_mutex;
     mutable fdcm_templates* host_tset = nullptr;   // reusable template set of fdcm_search_host
@@ -314,7 +315,7 @@ struct fdcm_dt3 {
         for (DevBuf* b : {&planes, &mask, &stack, &lines, &bins, &band_info, &band_spill, &integ_items, &s_scene, &s_sorted_len, &s_sorted_idx, &s_hyp_off, &s_rec,
                           &s_valid, &s_hyp, &s_counters, &s_topk_score, &s_topk_idx, &s_topk_out, &s_topk_n, &s_keys, &s_keys2, &s_idx,
                           &s_perm, &s_sort_tmp, &s_sel_keys, &s_sel_keys2, &s_sel_vals, &s_sel_vals2, &s_sel_surv, &s_sel_acc,
-                          &s_sel_tmp, &s_ref_state, &s_ref_keys, &s_ref_io, &s_ref_denom})
+                          &s_sel_tmp, &s_ref_state, &s_ref_keys, &s_ref_io, &s_ref_denom, &s_dense_keys, &s_dense_rot})
             b->release();
         if (h_pinned) cudaFreeHost(h_pinned);
         if (ev_fork) cudaEventDestroy(ev_fork);
@@ -1928,6 +1929,184 @@ extern "C" fdcm_status fdcm_refine_poses(const float transform[6], const float a
                 P[3] = R.r3; P[4] = R.r4; P[5] = R.by + (float)(kk - n_t) * lv.h;
             }
     }
+    return FDCM_OK;
+}
+
+// =============================================================================================
+// dense pose-grid search (rules in include/fdcm_b200.h)
+// =============================================================================================
+static fdcm_status check_dense(const fdcm_dense_params* d) {
+    if (!d) return fail(FDCM_ERR_INVALID, "dense is null");
+    if (d->rotations < 1 || d->rotations > FDCM_DENSE_MAX_ROTATIONS)
+        return fail(FDCM_ERR_INVALID, "dense search: rotations must be in 1.." + std::to_string(FDCM_DENSE_MAX_ROTATIONS));
+    if (d->stride < 1 || d->cell < 1) return fail(FDCM_ERR_INVALID, "dense search: stride and cell must be >= 1");
+    if (!std::isfinite(d->rot_start) || !std::isfinite(d->rot_step))
+        return fail(FDCM_ERR_INVALID, "dense search: rot_start and rot_step must be finite");
+    if (d->roi_on) {
+        bool ok = d->roi[0] <= d->roi[2] && d->roi[1] <= d->roi[3];
+        for (int q = 0; q < 4; ++q) ok = ok && std::isfinite(d->roi[q]);
+        if (!ok) return fail(FDCM_ERR_INVALID, "dense search: the region must be finite with x0 <= x1 and y0 <= y1");
+    }
+    return FDCM_OK;
+}
+
+// rule 1: cosine and sine of rotation r
+static void dense_rotation(const fdcm_dense_params* d, int r, float* c, float* s) {
+    const double th = (double)d->rot_start + (double)r * (double)d->rot_step;
+    *c = (float)std::cos(th);
+    *s = (float)std::sin(th);
+}
+
+// rule 2: the grid points of a W x H map with scene translation shift (nx = ny = 0: none)
+struct DenseGrid { int lo_x, lo_y, nx, ny; };
+static DenseGrid dense_grid(const fdcm_dense_params* d, const float shift[2], int W, int H) {
+    double lo[2] = {0.0, 0.0}, hi[2] = {(double)W - 1.0, (double)H - 1.0};
+    if (d->roi_on)
+        for (int a = 0; a < 2; ++a) {
+            lo[a] = std::max(lo[a], std::ceil((double)d->roi[a] + (double)shift[a]));
+            hi[a] = std::min(hi[a], std::floor((double)d->roi[a + 2] + (double)shift[a]));
+        }
+    if (lo[0] > hi[0] || lo[1] > hi[1]) return DenseGrid{0, 0, 0, 0};
+    const int lx = (int)lo[0], ly = (int)lo[1];
+    return DenseGrid{lx, ly, ((int)hi[0] - lx) / d->stride + 1, ((int)hi[1] - ly) / d->stride + 1};
+}
+
+extern "C" fdcm_status fdcm_search_dense(const fdcm_dt3* m, const fdcm_templates* tc, const fdcm_dense_params* dense, int32_t penalty_kind,
+                                         float penalty_tau, int32_t top_k, int32_t tmpl_idx_base, const fdcm_select_params* sel,
+                                         const fdcm_refine_params* ref, fdcm_match* out, int64_t capacity, int64_t* n_out) {
+    if (!m || !tc || !n_out) return fail(FDCM_ERR_INVALID, "null argument");
+    *n_out = 0;
+    if (fdcm_status st = check_dense(dense)) return st;
+    if (penalty_kind < 0 || penalty_kind > 2) return fail(FDCM_ERR_INVALID, "bad penalty kind");
+    if (top_k < 1) return fail(FDCM_ERR_INVALID, "dense search: top_k must be >= 1");
+    if (sel)
+        if (fdcm_status st = check_select(sel, top_k, false)) return st;
+    if (sel && sel->max_per_template == 0 && !(sel->radius > 0.f)) sel = nullptr;   // the plain top-K
+    if (ref) {
+        if (fdcm_status st = check_refine(ref)) return st;
+        if (top_k > kRefineMaxMatches) return fail(FDCM_ERR_INVALID, "pose refinement: top_k must be in 1.." + std::to_string(kRefineMaxMatches));
+    }
+    if (tc->device != m->device) return fail(FDCM_ERR_INVALID, "templates and feature map live on different devices");
+    if (m->stage != 0) return fail(FDCM_ERR_INVALID, "feature map was built with a debug stage");
+    fdcm_templates* t = const_cast<fdcm_templates*>(tc);
+    if (t->n_tmpl == 0 || m->dm.D == 0 || m->dm.W == 0 || m->dm.H == 0) return FDCM_OK;
+    // The records, their valid flags and the per-template offsets go to the search's buffers, so that the selection runs
+    // unchanged; the hypothesis list and the counters of the last fdcm_search (s_hyp, last_n_hyp, last_stats) stay as they are.
+    std::lock_guard<std::mutex> lk(m->search_mutex);
+    CUDA_TRY(cudaSetDevice(m->device));
+    cudaStream_t s;
+    if (fdcm_status st = get_stream(m->device, &s)) return st;
+    if (fdcm_status st = templates_ready(t, s)) return st;
+    int smem_optin = 0;
+    if (fdcm_status st = search_smem_optin(m->device, t->max_lines, &smem_optin)) return st;
+    const DenseGrid g = dense_grid(dense, m->shift, m->dm.W, m->dm.H);
+    if (g.nx == 0 || g.ny == 0) return FDCM_OK;
+    const int cell = std::min(dense->cell, std::max(g.nx, g.ny));   // (a larger cell holds the same points)
+    const int cells_x = (g.nx + cell - 1) / cell, cells_y = (g.ny + cell - 1) / cell;
+    const int64_t per_tmpl = (int64_t)dense->rotations * cells_y * cells_x;
+    const int64_t limit = ((int64_t)1 << 31) - 1;
+    if (per_tmpl > limit || per_tmpl * t->n_tmpl > limit)
+        return fail(FDCM_ERR_INVALID, "dense search: " + std::to_string(per_tmpl) + " records per template x " + std::to_string(t->n_tmpl) +
+                                          " templates; at most 2^31 - 1 records (use fewer rotations or templates, a larger cell or stride, or a region)");
+    const int64_t H = per_tmpl * t->n_tmpl;
+
+    std::vector<int64_t> hyp_off((size_t)t->n_tmpl + 1);
+    for (int i = 0; i <= t->n_tmpl; ++i) hyp_off[(size_t)i] = (int64_t)i * per_tmpl;
+    std::vector<float> rot(2 * (size_t)dense->rotations);
+    for (int r = 0; r < dense->rotations; ++r) dense_rotation(dense, r, &rot[2 * (size_t)r], &rot[2 * (size_t)r + 1]);
+    CUDA_TRY(m->s_rec.reserve((size_t)H * sizeof(fdcm_match)));
+    CUDA_TRY(m->s_valid.reserve((size_t)H));
+    CUDA_TRY(m->s_hyp_off.reserve(hyp_off.size() * 8));
+    CUDA_TRY(m->s_dense_keys.reserve((size_t)H * 8));
+    CUDA_TRY(m->s_dense_rot.reserve(rot.size() * 4));
+    CUDA_TRY(cudaMemcpyAsync(m->s_hyp_off.p, hyp_off.data(), hyp_off.size() * 8, cudaMemcpyHostToDevice, s));
+    CUDA_TRY(cudaMemcpyAsync(m->s_dense_rot.p, rot.data(), rot.size() * 4, cudaMemcpyHostToDevice, s));
+    const float* d_denom = nullptr;
+    if (penalty_kind != FDCM_PENALTY_NONE) {   // the search's denominators (penalty_denominator)
+        std::vector<float> den((size_t)t->n_tmpl);
+        for (int i = 0; i < t->n_tmpl; ++i) den[(size_t)i] = penalty_denominator(penalty_kind, penalty_tau, t->lengths[(size_t)i]);
+        CUDA_TRY(m->s_ref_denom.reserve(den.size() * 4));
+        CUDA_TRY(cudaMemcpyAsync(m->s_ref_denom.p, den.data(), den.size() * 4, cudaMemcpyHostToDevice, s));
+        d_denom = m->s_ref_denom.as<float>();
+    }
+    DenseLaunch dl;
+    dl.lines = t->lines.as<float4>();
+    dl.offsets = t->offs.as<int32_t>();
+    dl.anchors = t->anchors.as<float2>();
+    dl.rot = m->s_dense_rot.as<float2>();
+    dl.denom = d_denom;
+    dl.n_tmpl = t->n_tmpl;
+    dl.rotations = dense->rotations;
+    dl.tmpl_idx_base = tmpl_idx_base;
+    dl.lo_x = g.lo_x;
+    dl.lo_y = g.lo_y;
+    dl.stride = dense->stride;
+    dl.nx = g.nx;
+    dl.ny = g.ny;
+    dl.cell = cell;
+    dl.cells_x = cells_x;
+    dl.cells_y = cells_y;
+    // at least 32 grid rows per block where the cells allow it: the staging of the rotated template is paid once per block
+    const int cell_rows = std::min(cell, g.ny);
+    dl.band = std::max(1, std::min(cells_y, (32 + cell_rows - 1) / cell_rows));
+    dl.n_bands = (cells_y + dl.band - 1) / dl.band;
+    dl.n_rec = H;
+    dl.keys = m->s_dense_keys.as<unsigned long long>();
+    dl.rec = m->s_rec.as<fdcm_match>();
+    dl.valid = m->s_valid.as<uint8_t>();
+    CUDA_TRY(cudaMemsetAsync(dl.keys, 0xFF, (size_t)H * 8, s));
+    {
+        KernelScope k("dense_eval", 0.0, s);
+        CUDA_TRY(launch_dense_eval(map_view(m), m->table_dev, dl, t->max_lines, smem_optin, s));
+    }
+    {
+        KernelScope k("dense_finish", (double)H * (8 + sizeof(fdcm_match) + 1), s);
+        launch_dense_finish(map_view(m), dl, s);
+    }
+    const int k = top_k;
+    CUDA_TRY(m->s_topk_out.reserve((size_t)k * sizeof(fdcm_match)));
+    CUDA_TRY(m->s_topk_n.reserve(4));
+    if (sel) {
+        fdcm_search_params sp{};
+        sp.top_k = k;
+        sp.tmpl_idx_base = tmpl_idx_base;
+        if (fdcm_status st = run_select(m, t, &sp, sel, H, s)) return st;
+    } else {
+        const int blocks = topk_ws_blocks(H);
+        CUDA_TRY(m->s_topk_score.reserve((size_t)blocks * k * 4));
+        CUDA_TRY(m->s_topk_idx.reserve((size_t)blocks * k * 8));
+        KernelScope ks("topk", 0.0, s, 2);   // two kernels in this scope
+        launch_topk(dl.rec, dl.valid, H, k, m->s_topk_score.as<float>(), m->s_topk_idx.as<int64_t>(), blocks, m->s_topk_out.as<fdcm_match>(),
+                    m->s_topk_n.as<int>(), s);
+    }
+    CUDA_TRY(cudaGetLastError());
+    if (ref)
+        if (fdcm_status st = run_refine(m, t, tmpl_idx_base, d_denom, ref, m->s_topk_out.as<fdcm_match>(), m->s_topk_n.as<int>(), k,
+                                        m->s_topk_out.as<fdcm_match>(), smem_optin, s))
+            return st;
+    const fdcm_status result = finish_topk(m, nullptr, k, s, nullptr, out, capacity, n_out);
+    prof_resolve();
+    return result;
+}
+
+extern "C" fdcm_status fdcm_dense_poses(const fdcm_dense_params* dense, const float anchor[2], const float shift[2], int32_t width,
+                                        int32_t height, int32_t rotation, float* out, int64_t capacity, int64_t* n_out, int32_t grid_wh[2]) {
+    if (fdcm_status st = check_dense(dense)) return st;
+    if (!anchor || !shift || !n_out || !grid_wh) return fail(FDCM_ERR_INVALID, "null argument");
+    if (width < 0 || height < 0) return fail(FDCM_ERR_INVALID, "width and height must be >= 0");
+    if (rotation < 0 || rotation >= dense->rotations) return fail(FDCM_ERR_INVALID, "rotation must be in 0..rotations - 1");
+    const DenseGrid g = dense_grid(dense, shift, width, height);
+    grid_wh[0] = g.nx;
+    grid_wh[1] = g.ny;
+    const int64_t n = (int64_t)g.nx * g.ny;
+    *n_out = n;
+    if (n > capacity || (n > 0 && !out)) return fail(FDCM_ERR_CAPACITY, "output buffer too small");
+    float c, s;
+    dense_rotation(dense, rotation, &c, &s);
+    for (int v = 0; v < g.ny; ++v)
+        for (int u = 0; u < g.nx; ++u)
+            dense_pose(c, s, anchor[0], anchor[1], g.lo_x + u * dense->stride, g.lo_y + v * dense->stride, shift[0], shift[1],
+                       out + 6 * ((size_t)v * g.nx + u));
     return FDCM_OK;
 }
 

@@ -198,6 +198,41 @@ cudaError_t launch_refine_eval(const MapView& map, const SlopeTableDev& table, c
 // the level's argmin becomes the centre; out != nullptr (last level): writes the refined matches
 void launch_refine_advance(const RefineLaunch& p, const RefineLevel& lv, fdcm_match* out, cudaStream_t s);
 
+// dense pose-grid search (fdcm_search_dense; rules in include/fdcm_b200.h)
+struct DenseLaunch {
+    const float4* lines;         // template set
+    const int32_t* offsets;
+    const float2* anchors;
+    const float2* rot;           // (c_r, s_r) of every rotation
+    const float* denom;          // per template penalty denominator, or nullptr
+    int32_t n_tmpl, rotations, tmpl_idx_base;
+    int32_t lo_x, lo_y, stride;  // grid point (u, v) is the map pixel (lo_x + u stride, lo_y + v stride)
+    int32_t nx, ny;              // grid points per row / column
+    int32_t cell, cells_x, cells_y;
+    int32_t band;                // cell rows per block of the evaluation kernel
+    int32_t n_bands;             // ceil(cells_y / band)
+    int64_t n_rec;               // n_tmpl * rotations * cells_y * cells_x
+    unsigned long long* keys;    // n_rec: (score bits << 32 | grid index << 1 | score is NaN) of the cell's best, ~0 when none
+    fdcm_match* rec;             // n_rec records and valid flags (the search's record buffers)
+    uint8_t* valid;
+};
+// translation of the grid pose whose anchor lands on map pixel (gx, gy): the same arithmetic on the host and the device
+__host__ __device__ inline float dense_tx(float c, float s, float ax, float ay, int gx, float shift_x) {
+    return ((float)gx - shift_x) - (c * ax - s * ay);
+}
+__host__ __device__ inline float dense_ty(float c, float s, float ax, float ay, int gy, float shift_y) {
+    return ((float)gy - shift_y) - (s * ax + c * ay);
+}
+__host__ __device__ inline void dense_pose(float c, float s, float ax, float ay, int gx, int gy, float shift_x, float shift_y, float* P) {
+    P[0] = c; P[1] = -s; P[2] = dense_tx(c, s, ax, ay, gx, shift_x);
+    P[3] = s; P[4] = c;  P[5] = dense_ty(c, s, ax, ay, gy, shift_y);
+}
+// one block per (template, rotation, band of cell rows); atomicMin of the key per record.  keys must hold ~0 on entry.
+cudaError_t launch_dense_eval(const MapView& map, const SlopeTableDev& table, const DenseLaunch& p, int max_lines, int smem_optin,
+                              cudaStream_t s);
+// keys -> records and valid flags (the winning pose recomputed from its grid index, the penalty applied)
+void launch_dense_finish(const MapView& map, const DenseLaunch& p, cudaStream_t s);
+
 void launch_evaluate(const MapView& map, const SlopeTableDev& table, const float4* d_lines, const int32_t* d_toff,
                      const float2* d_transl, const int32_t* d_troff, const int32_t* d_owner, int64_t n_scores,
                      float* d_scores, cudaStream_t s);

@@ -302,6 +302,40 @@ PYBIND11_MODULE(_openfdcm_cuda, m) {
           "Pose refinement of every match (entry i refines matches[i]) to the lowest evaluate score of its grid, not to a more "
           "accurate pose; with a penalty, scores are penalised like search_topk");
 
+    py::class_<DenseSearch>(m, "DenseSearch")
+        .def(py::init([](int rotations, float rot_start, std::optional<float> rot_step, int stride, int cell,
+                         std::optional<std::array<float, 4>> roi) {
+                 DenseSearch d;
+                 d.rotations = rotations;
+                 d.rotStart = rot_start;
+                 d.rotStep = rot_step ? *rot_step : (rotations > 0 ? (float)(2.0 * 3.14159265358979323846 / rotations) : 0.f);
+                 d.stride = stride;
+                 d.cell = cell;
+                 d.hasRoi = roi.has_value();
+                 if (roi) d.roi = *roi;
+                 return d;
+             }), "rotations"_a = 72, "rot_start"_a = 0.f, "rot_step"_a = py::none(), "stride"_a = 2, "cell"_a = 8, "roi"_a = py::none())
+        .def_readwrite("rotations", &DenseSearch::rotations)
+        .def_readwrite("rot_start", &DenseSearch::rotStart)
+        .def_readwrite("rot_step", &DenseSearch::rotStep)
+        .def_readwrite("stride", &DenseSearch::stride)
+        .def_readwrite("cell", &DenseSearch::cell)
+        .def("__repr__", [](const DenseSearch& a) {
+            return "<DenseSearch: rotations=" + std::to_string(a.rotations) + ", rot_start=" + std::to_string(a.rotStart) + ", rot_step=" +
+                   std::to_string(a.rotStep) + ", stride=" + std::to_string(a.stride) + ", cell=" + std::to_string(a.cell) + ">";
+        });
+
+    m.def("search_dense",
+          [](const Dt3Cuda& featuremap, const std::vector<LinesIn>& templates, const DenseSearch& dense, const ExponentialPenalty& penalty, int k,
+             const std::optional<DistinctMatches>& select, const std::optional<PoseRefinement>& refine) {
+              const auto t = to_templates(templates);
+              py::gil_scoped_release release;
+              return searchDense(featuremap, t, dense, penalty, k, select ? &*select : nullptr, refine ? &*refine : nullptr);
+          },
+          "featuremap"_a, "templates"_a, "dense"_a, "penalty"_a, "k"_a = 10, py::kw_only(), "select"_a = py::none(), "refine"_a = py::none(),
+          "Dense pose-grid search on the device: the best pose of every (template, rotation, cell), then the top-k (ascending score) "
+          "or with select the distinct top-k, then with refine the pose refinement of those");
+
     m.def("penalize",
           [](const PenaltyStrategy& penalty, const std::vector<Match>& matches, const std::vector<float>& templatelengths) {
               return penalize(penalty, matches, templatelengths);

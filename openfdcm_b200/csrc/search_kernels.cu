@@ -793,6 +793,54 @@ void launch_select_walk(const SelectLaunch& p, const uint64_t* sorted_keys, cons
 // =============================================================================================
 constexpr unsigned long long kNoPose = ~0ull;
 
+// Block-wide (every thread calls it): stage the L lines of a template rotated by (r0 r1; r3 r4), or as given when as_given
+// (no multiply touches the coordinates, so no zero changes sign), with their orientation bins in shared memory; then every
+// warp reduces the bounding box of the staged end points itself (no cross-warp exchange, no static shared memory).
+// nan: some staged end point is NaN.
+struct StagedBox { float mnx, mny, mxx, mxy; bool nan; };
+__device__ __forceinline__ StagedBox stage_rotated(const float4* __restrict__ lines, int L, float r0, float r1, float r3, float r4,
+                                                   bool as_given, const SlopeTableDev& table, float4* apts, uint8_t* bins) {
+    const int tid = threadIdx.x, lane = tid & 31;
+    bool nan = false;
+    for (int q = tid; q < L; q += blockDim.x) {
+        const float4 v = __ldg(lines + q);
+        float x1 = v.x, y1 = v.y, x2 = v.z, y2 = v.w;
+        if (!as_given) {
+            x1 = r0 * v.x + r1 * v.y; y1 = r3 * v.x + r4 * v.y;
+            x2 = r0 * v.z + r1 * v.w; y2 = r3 * v.z + r4 * v.w;
+        }
+        nan |= x1 != x1 || y1 != y1 || x2 != x2 || y2 != y2;
+        apts[q] = make_float4(x1, y1, x2, y2);
+        bins[q] = (uint8_t)bin_of_slope_dev(table, (y2 - y1) / (x2 - x1));
+    }
+    StagedBox b;
+    b.nan = __syncthreads_or(nan) != 0;   // also publishes apts / bins
+    b.mnx = INFINITY; b.mny = INFINITY; b.mxx = -INFINITY; b.mxy = -INFINITY;
+    for (int q = lane; q < L; q += 32) {
+        const float4 e = apts[q];
+        b.mnx = fminf(b.mnx, fminf(e.x, e.z)); b.mxx = fmaxf(b.mxx, fmaxf(e.x, e.z));
+        b.mny = fminf(b.mny, fminf(e.y, e.w)); b.mxy = fmaxf(b.mxy, fmaxf(e.y, e.w));
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        b.mnx = fminf(b.mnx, __shfl_xor_sync(0xffffffffu, b.mnx, o)); b.mxx = fmaxf(b.mxx, __shfl_xor_sync(0xffffffffu, b.mxx, o));
+        b.mny = fminf(b.mny, __shfl_xor_sync(0xffffffffu, b.mny, o)); b.mxy = fmaxf(b.mxy, __shfl_xor_sync(0xffffffffu, b.mxy, o));
+    }
+    return b;
+}
+
+// sum of |plane(x1, y1) - plane(x2, y2)| over the staged lines in Eigen's order, every end point offset by (offx, offy)
+__device__ __forceinline__ float staged_score(const MapView& map, const float4* apts, const uint8_t* bins, int L, float offx, float offy) {
+    const float* planes = map.planes;
+    const size_t pitch = (size_t)map.dm.pitch, pe = map.dm.plane_elems;
+    return eigen_sum_lazy(L, [&](int q) {
+        const float4 e = apts[q];
+        const int x1 = (int)(e.x + offx), y1 = (int)(e.y + offy), x2 = (int)(e.z + offx), y2 = (int)(e.w + offy);
+        const float* P = planes + (size_t)bins[q] * pe;
+        return fabsf(__ldg(P + (size_t)y1 * pitch + x1) - __ldg(P + (size_t)y2 * pitch + x2));
+    });
+}
+
 __global__ void refine_init_kernel(const __grid_constant__ RefineLaunch p) {
     const int m = blockIdx.x * blockDim.x + threadIdx.x;
     if (m >= (p.d_n ? *p.d_n : p.n)) return;
@@ -826,46 +874,19 @@ __global__ void __launch_bounds__(1024) refine_eval_kernel(const __grid_constant
     const RefineRot R = refine_rotation(st.c, a.x, a.y, ir - p.n_r, lv.ci[ir], lv.si[ir]);
     float4* apts = reinterpret_cast<float4*>(s_raw);
     uint8_t* bins = reinterpret_cast<uint8_t*>(apts + L);
-    bool nan = false;
-    for (int q = tid; q < L; q += blockDim.x) {
-        const float4 v = __ldg(p.lines + l0 + q);
-        const float x1 = R.r0 * v.x + R.r1 * v.y, y1 = R.r3 * v.x + R.r4 * v.y;
-        const float x2 = R.r0 * v.z + R.r1 * v.w, y2 = R.r3 * v.z + R.r4 * v.w;
-        nan |= x1 != x1 || y1 != y1 || x2 != x2 || y2 != y2;
-        apts[q] = make_float4(x1, y1, x2, y2);
-        bins[q] = (uint8_t)bin_of_slope_dev(table, (y2 - y1) / (x2 - x1));
-    }
-    nan = __syncthreads_or(nan) != 0;   // also publishes apts / bins
-    // bounding box of the rotated template: every warp reduces the staged points itself (no cross-warp exchange)
-    float mnx = INFINITY, mny = INFINITY, mxx = -INFINITY, mxy = -INFINITY;
-    for (int q = lane; q < L; q += 32) {
-        const float4 e = apts[q];
-        mnx = fminf(mnx, fminf(e.x, e.z)); mxx = fmaxf(mxx, fmaxf(e.x, e.z));
-        mny = fminf(mny, fminf(e.y, e.w)); mxy = fmaxf(mxy, fmaxf(e.y, e.w));
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-        mnx = fminf(mnx, __shfl_xor_sync(0xffffffffu, mnx, o)); mxx = fmaxf(mxx, __shfl_xor_sync(0xffffffffu, mxx, o));
-        mny = fminf(mny, __shfl_xor_sync(0xffffffffu, mny, o)); mxy = fmaxf(mxy, __shfl_xor_sync(0xffffffffu, mxy, o));
-    }
+    const StagedBox bb = stage_rotated(p.lines + l0, L, R.r0, R.r1, R.r3, R.r4, false, table, apts, bins);
     unsigned long long key = kNoPose;
     if (tid < NT * NT) {
         const int kk = tid / NT, jj = tid - kk * NT;
         const float P2 = R.bx + (float)(jj - p.n_t) * lv.h, P5 = R.by + (float)(kk - p.n_t) * lv.h;
         const float offx = map.shift_x + P2, offy = map.shift_y + P5;
         // the rounding of r + off is monotonic in r, so the bounding box decides for every end point
-        bool valid = !nan && !(R.r0 != R.r0 || R.r1 != R.r1 || R.r3 != R.r3 || R.r4 != R.r4 || P2 != P2 || P5 != P5);
+        bool valid = !bb.nan && !(R.r0 != R.r0 || R.r1 != R.r1 || R.r3 != R.r3 || R.r4 != R.r4 || P2 != P2 || P5 != P5);
         if (valid && L > 0)
-            valid = 0.f <= mnx + offx && mxx + offx <= (float)(map.dm.W - 1) && 0.f <= mny + offy && mxy + offy <= (float)(map.dm.H - 1);
+            valid = 0.f <= bb.mnx + offx && bb.mxx + offx <= (float)(map.dm.W - 1) && 0.f <= bb.mny + offy &&
+                    bb.mxy + offy <= (float)(map.dm.H - 1);
         if (valid) {
-            const float* planes = map.planes;
-            const size_t pitch = (size_t)map.dm.pitch, pe = map.dm.plane_elems;
-            const float sc = eigen_sum_lazy(L, [&](int q) {
-                const float4 e = apts[q];
-                const int x1 = (int)(e.x + offx), y1 = (int)(e.y + offy), x2 = (int)(e.z + offx), y2 = (int)(e.w + offy);
-                const float* P = planes + (size_t)bins[q] * pe;
-                return fabsf(__ldg(P + (size_t)y1 * pitch + x1) - __ldg(P + (size_t)y2 * pitch + x2));
-            });
+            const float sc = staged_score(map, apts, bins, L, offx, offy);
             // walk order: squared grid distance from the centre (0 only for the centre), then (i, k, j)
             const int di = ir - p.n_r, dk = kk - p.n_t, dj = jj - p.n_t;
             const unsigned order = (unsigned)(di * di + dk * dk + dj * dj) << 15 | (unsigned)((ir * NT + kk) * NT + jj);
@@ -931,6 +952,135 @@ __global__ void refine_advance_kernel(const __grid_constant__ RefineLaunch p, co
 
 void launch_refine_advance(const RefineLaunch& p, const RefineLevel& lv, fdcm_match* out, cudaStream_t s) {
     refine_advance_kernel<<<(unsigned)((p.n + 127) / 128), 128, 0, s>>>(p, lv, out);
+}
+
+// =============================================================================================
+// Dense pose-grid search (fdcm_search_dense, beyond the reference): rules in include/fdcm_b200.h.
+// One block per (template, rotation, band of cell rows) stages the rotated template once (stage_rotated, as refinement
+// does).  The valid poses of a rotation form a rectangle of the grid: the bounding-box test is monotonic in u and in v, so
+// the block finds the valid u and v intervals by bisection and its warps visit only those.  A warp item is 32 consecutive
+// u (adjacent pixels at stride 1) by up to kDenseRowGroup rows of one cell row; each lane keeps the minimum key of its
+// column, then a segmented shuffle reduction takes the minimum over the lanes of one cell and the first lane of every
+// cell does one atomicMin on the cell's record key.
+// =============================================================================================
+constexpr int kDenseThreads = 256;
+constexpr int kDenseRowGroup = 8;
+
+// first i in [0, n) with pred(i) for a predicate that is false, then true; n when there is none
+template <class Pred>
+__device__ __forceinline__ int first_true(int n, Pred pred) {
+    int lo = 0, hi = n;
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (pred(mid)) hi = mid; else lo = mid + 1;
+    }
+    return lo;
+}
+
+__global__ void __launch_bounds__(kDenseThreads) dense_eval_kernel(const __grid_constant__ MapView map,
+                                                                   const __grid_constant__ SlopeTableDev table,
+                                                                   const __grid_constant__ DenseLaunch p) {
+    extern __shared__ __align__(16) uint8_t s_raw[];   // rotated end points float4[L], planes u8[L], as refinement
+    const long long tr = blockIdx.x / p.n_bands;
+    const int band = (int)(blockIdx.x - tr * p.n_bands);
+    const int r = (int)(tr % p.rotations), t = (int)(tr / p.rotations);
+    const int l0 = p.offsets[t], L = p.offsets[t + 1] - l0;
+    if (L == 0) return;   // whole block: an empty template has no records
+    const float2 cs = p.rot[r], a = p.anchors[t];
+    const float c = cs.x, s = cs.y;
+    float4* apts = reinterpret_cast<float4*>(s_raw);
+    uint8_t* bins = reinterpret_cast<uint8_t*>(apts + L);
+    const StagedBox bb = stage_rotated(p.lines + l0, L, c, -s, s, c, c == 1.f && s == 0.f, table, apts, bins);
+    if (bb.nan) return;   // uniform
+    // shift + tx(u) is non-decreasing in u (every rounding step is monotonic): the x test holds on an interval of u, the y
+    // test on an interval of v (NaN translations fail everywhere)
+    const float Wm1 = (float)(map.dm.W - 1), Hm1 = (float)(map.dm.H - 1);
+    const float shx = map.shift_x, shy = map.shift_y, ax = a.x, ay = a.y;
+    const int lo_x = p.lo_x, lo_y = p.lo_y, stride = p.stride;
+    auto offx = [=](int u) { return shx + dense_tx(c, s, ax, ay, lo_x + u * stride, shx); };
+    auto offy = [=](int v) { return shy + dense_ty(c, s, ax, ay, lo_y + v * stride, shy); };
+    const float mnx = bb.mnx, mxx = bb.mxx, mny = bb.mny, mxy = bb.mxy;
+    const int ulo = first_true(p.nx, [=](int u) { return 0.f <= mnx + offx(u); });
+    const int uhi = first_true(p.nx, [=](int u) { return !(mxx + offx(u) <= Wm1); }) - 1;
+    const int vlo = first_true(p.ny, [=](int v) { return 0.f <= mny + offy(v); });
+    const int vhi = first_true(p.ny, [=](int v) { return !(mxy + offy(v) <= Hm1); }) - 1;
+    if (ulo > uhi || vlo > vhi) return;   // uniform
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, n_warps = blockDim.x >> 5;
+    const int n_chunks = (uhi - ulo + 32) / 32;
+    const long long rec0 = ((long long)t * p.rotations + r) * p.cells_y;
+    const int cv1 = min(p.cells_y, (band + 1) * p.band);
+    for (int cv = band * p.band; cv < cv1; ++cv) {
+        const int ra = max(cv * p.cell, vlo), rb = min(cv * p.cell + (p.cell - 1), vhi);
+        if (ra > rb) continue;
+        const int n_items = ((rb - ra) / kDenseRowGroup + 1) * n_chunks;
+        for (int item = warp; item < n_items; item += n_warps) {   // warp-uniform
+            const int grp = item / n_chunks, ch = item - grp * n_chunks;
+            const int u = ulo + ch * 32 + lane;
+            const int va = ra + grp * kDenseRowGroup, vb = min(va + kDenseRowGroup - 1, rb);
+            unsigned long long key = kNoPose;
+            if (u <= uhi) {
+                const float ox = offx(u);
+                for (int v = va; v <= vb; ++v) {
+                    const float sc = staged_score(map, apts, bins, L, ox, offy(v));
+                    const bool is_nan = sc != sc;
+                    const unsigned g = (unsigned)v * (unsigned)p.nx + (unsigned)u;   // grid index (row-major)
+                    const unsigned long long k =
+                        (unsigned long long)(is_nan ? 0x7F800000u : __float_as_uint(sc)) << 32 | (unsigned long long)(g << 1 | (is_nan ? 1u : 0u));
+                    key = k < key ? k : key;
+                }
+            }
+            // segmented minimum: after the step of offset o, lane l holds the minimum over lanes [l, l + 2o) of its cell
+            const int cu = u / p.cell;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const unsigned long long other = __shfl_down_sync(0xffffffffu, key, o);
+                const int ocu = __shfl_down_sync(0xffffffffu, cu, o);
+                if (lane + o < 32 && ocu == cu && other < key) key = other;
+            }
+            const int pcu = __shfl_up_sync(0xffffffffu, cu, 1);
+            if ((lane == 0 || pcu != cu) && key != kNoPose) atomicMin(p.keys + (rec0 + cv) * p.cells_x + cu, key);
+        }
+    }
+}
+
+cudaError_t launch_dense_eval(const MapView& map, const SlopeTableDev& table, const DenseLaunch& p, int max_lines, int smem_optin,
+                              cudaStream_t s) {
+    const size_t smem = refine_smem_bytes(max_lines > 0 ? max_lines : 1);
+    if (smem > (size_t)smem_optin) return cudaErrorInvalidValue;   // callers reject such templates first
+    if (smem > 48 * 1024) {
+        const cudaError_t e = cudaFuncSetAttribute(dense_eval_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+    }
+    const long long blocks = (long long)p.n_tmpl * p.rotations * p.n_bands;   // <= n_rec < 2^31
+    dense_eval_kernel<<<(unsigned)blocks, kDenseThreads, smem, s>>>(map, table, p);
+    return cudaGetLastError();
+}
+
+__global__ void dense_finish_kernel(const __grid_constant__ MapView map, const __grid_constant__ DenseLaunch p) {
+    const long long h = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (h >= p.n_rec) return;
+    const unsigned long long key = p.keys[h];
+    if (key == kNoPose) {
+        p.valid[h] = 0;
+        return;
+    }
+    const long long tr = h / ((long long)p.cells_y * p.cells_x);
+    const int r = (int)(tr % p.rotations), t = (int)(tr / p.rotations);
+    const unsigned g = (unsigned)key >> 1;
+    const int u = (int)(g % (unsigned)p.nx), v = (int)(g / (unsigned)p.nx);
+    const float2 cs = p.rot[r], a = p.anchors[t];
+    fdcm_match m;
+    m.tmpl_idx = t + p.tmpl_idx_base;
+    const float raw = (key & 1ull) ? NAN : __uint_as_float((unsigned)(key >> 32));
+    m.score = p.denom ? raw / p.denom[t] : raw;
+    // the pose dense_eval_kernel scored, recomputed from its grid index
+    dense_pose(cs.x, cs.y, a.x, a.y, p.lo_x + u * p.stride, p.lo_y + v * p.stride, map.shift_x, map.shift_y, m.transform);
+    p.rec[h] = m;
+    p.valid[h] = 1;
+}
+
+void launch_dense_finish(const MapView& map, const DenseLaunch& p, cudaStream_t s) {
+    dense_finish_kernel<<<(unsigned)((p.n_rec + 255) / 256), 256, 0, s>>>(map, p);
 }
 
 // =============================================================================================
