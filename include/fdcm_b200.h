@@ -104,7 +104,8 @@ const char* fdcm_last_error(void);
 int32_t fdcm_abi_version(void);
 fdcm_status fdcm_device_count(int32_t* n);
 /* Run every kernel of this library on a caller-owned CUDA stream (e.g. torch's current stream) of `device`;
- * NULL restores the library's own stream. */
+ * NULL restores the library's own stream.  The change applies to later calls; work already queued on a map (an
+ * asynchronous rebuild or rerun) stays ordered before every later call on that map, whatever stream that call uses. */
 fdcm_status fdcm_set_stream(int32_t device, void* cuda_stream);
 
 /* ---- hot path 1: feature map -------------------------------------------------------------- */
@@ -114,12 +115,13 @@ fdcm_status fdcm_dt3_build(const float* scene_xyxy, int32_t n_lines, const fdcm_
                            int32_t stage, fdcm_dt3** out);
 /* Same map object, new scene: reuses the device allocations when the new map fits. */
 fdcm_status fdcm_dt3_rebuild(fdcm_dt3* map, const float* scene_xyxy, int32_t n_lines);
-/* fdcm_dt3_rebuild without the final wait: returns once the build kernels are queued (stream-ordered before any
- * later call on this map); lets host-side preparation of the following search overlap the device build. */
+/* fdcm_dt3_rebuild without the final wait: returns once the build kernels are queued on the current stream; they are
+ * ordered before any later call on this map, on any stream (the map records an event that every call waits on).  Lets
+ * host-side preparation of the following search overlap the device build. */
 fdcm_status fdcm_dt3_rebuild_async(fdcm_dt3* map, const float* scene_xyxy, int32_t n_lines);
 /* Re-run the build kernels on the scene lines already resident on the device (kernel-only timing). */
 fdcm_status fdcm_dt3_rerun(fdcm_dt3* map);
-/* fdcm_dt3_rerun without the final wait (stream-ordered before any later call on this map). */
+/* fdcm_dt3_rerun without the final wait (ordered before any later call on this map, on any stream). */
 fdcm_status fdcm_dt3_rerun_async(fdcm_dt3* map);
 fdcm_status fdcm_dt3_retain(fdcm_dt3* map);
 fdcm_status fdcm_dt3_release(fdcm_dt3* map);
@@ -132,7 +134,8 @@ fdcm_status fdcm_dt3_download_plane(const fdcm_dt3* map, int32_t plane, float* d
 fdcm_status fdcm_dt3_download_mask(const fdcm_dt3* map, int32_t plane, uint8_t* dst);
 /* orientation plane of each scene line (classifyLines, dt3cpu.h:123-134) */
 fdcm_status fdcm_dt3_scene_bins(const fdcm_dt3* map, int32_t* bins);
-/* raw device pointer of the planes (for zero-copy consumers, e.g. torch.from_blob / NCCL broadcast) */
+/* raw device pointer of the planes (for zero-copy consumers, e.g. torch.from_blob / NCCL broadcast).  Reads through it
+ * are the caller's to order: after an asynchronous rebuild or rerun, read on the stream it was queued on or synchronise. */
 fdcm_status fdcm_dt3_device_ptr(const fdcm_dt3* map, void** planes, uint64_t* n_bytes);
 
 /* minmaxTranslation<Dt3Cpu>(featuremap, tmpl, align_vec) (dt3cpu.cpp:119-124, :30-75) */

@@ -164,23 +164,6 @@ struct KernelScope {   // brackets one kernel launch
     }
 };
 
-static void prof_resolve() {   // call after the stream has been synchronised
-    std::lock_guard<std::mutex> lk(g_mutex);
-    for (auto& p : g_prof_pending) {
-        float ms = 0.f;
-        if (cudaEventElapsedTime(&ms, p.a, p.b) == cudaSuccess) {
-            if (!g_prof.count(p.name)) g_prof_order.push_back(p.name);
-            auto& e = g_prof[p.name];
-            e.total_ms += ms;
-            e.launches += 1;
-            e.bytes = p.bytes;
-        }
-        prof_event_put(p.device, p.a);
-        prof_event_put(p.device, p.b);
-    }
-    g_prof_pending.clear();
-}
-
 extern "C" fdcm_status fdcm_profile_enable(int32_t on) { g_prof_on = on != 0; return FDCM_OK; }
 extern "C" fdcm_status fdcm_profile_reset(void) {
     std::lock_guard<std::mutex> lk(g_mutex);
@@ -188,12 +171,15 @@ extern "C" fdcm_status fdcm_profile_reset(void) {
     g_prof_order.clear();
     return FDCM_OK;
 }
-// scopes of asynchronous calls (fdcm_dt3_rerun_async ...) that have finished by now: nobody synchronised inside the library
-static void prof_resolve_finished() {
+// Accounts the scopes that have finished and keeps the others pending, with their events out of the pool: a call resolves
+// after synchronising its own stream, while scopes of other streams may still run (the next scene's build of a SceneBatch,
+// calls of other threads, asynchronous rebuilds).
+static void prof_resolve() {
     std::lock_guard<std::mutex> lk(g_mutex);
     std::vector<ProfPending> keep;
+    bool not_ready = false;
     for (auto& p : g_prof_pending) {
-        if (cudaEventQuery(p.b) != cudaSuccess) { keep.push_back(p); continue; }
+        if (cudaEventQuery(p.b) != cudaSuccess) { keep.push_back(p); not_ready = true; continue; }
         float ms = 0.f;
         if (cudaEventElapsedTime(&ms, p.a, p.b) == cudaSuccess) {
             if (!g_prof.count(p.name)) g_prof_order.push_back(p.name);
@@ -206,11 +192,13 @@ static void prof_resolve_finished() {
         prof_event_put(p.device, p.b);
     }
     g_prof_pending.swap(keep);
+    // a query of a running scope is not a failure of the caller: it must not surface at its next cudaGetLastError
+    if (not_ready && cudaPeekAtLastError() == cudaErrorNotReady) cudaGetLastError();
 }
 
 extern "C" fdcm_status fdcm_profile_count(int32_t* n) {
     if (!n) return fail(FDCM_ERR_INVALID, "n is null");
-    prof_resolve_finished();
+    prof_resolve();
     std::lock_guard<std::mutex> lk(g_mutex);
     *n = (int32_t)g_prof_order.size();
     return FDCM_OK;
@@ -285,13 +273,23 @@ struct fdcm_dt3 {
     int plan_tables_depth = -1;
     int n_sms = 148;
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;   // fork / join of the second stream inside a build
+    // recorded after everything that writes the map (build, rebuild, rerun, SceneBatch slot build, broadcast); every call that
+    // reads or writes the map makes its stream wait on it, so work queued on another stream stays ordered before it
+    cudaEvent_t ev_written = nullptr;
     bool band_path = false, band_l1 = false;   // which distance-transform formulation this map uses (set by prepare)
     // search workspace (mutable state of the last search on this map)
     mutable std::mutex search_mutex;
     mutable DevBuf s_scene, s_sorted_len, s_sorted_idx, s_hyp_off, s_rec, s_valid, s_hyp, s_counters, s_topk_score, s_topk_idx,
         s_topk_out, s_topk_n, s_keys, s_keys2, s_idx, s_perm, s_sort_tmp;
     mutable DevBuf s_sel_keys, s_sel_keys2, s_sel_vals, s_sel_vals2, s_sel_surv, s_sel_acc, s_sel_tmp;   // distinct top-K
-    mutable DevBuf s_ref_state, s_ref_keys, s_ref_io, s_ref_denom;   // pose refinement
+    mutable DevBuf s_ref_state, s_ref_keys, s_ref_io;   // pose refinement
+    // penalty denominators of the last template set searched on this map, for (the set's load_id, kind, tau): per map and
+    // not per set, because every use of a map is serialised by search_mutex and ends in a host synchronisation, while
+    // searches of other maps sharing the set may still be queued
+    mutable DevBuf s_denom;
+    mutable uint64_t denom_set = 0;
+    mutable int denom_kind = -1;
+    mutable float denom_tau = 0.f;
     mutable DevBuf s_dense_keys, s_dense_rot;   // dense pose-grid search (records: s_rec / s_valid / s_hyp_off)
     mutable float s_scene_min[2] = {0.f, 0.f}, s_scene_max[2] = {0.f, 0.f};   // bbox of the resident search scene
     mutable std::mutex host_tset_mutex;
@@ -315,11 +313,12 @@ struct fdcm_dt3 {
         for (DevBuf* b : {&planes, &mask, &stack, &lines, &bins, &band_info, &band_spill, &integ_items, &s_scene, &s_sorted_len, &s_sorted_idx, &s_hyp_off, &s_rec,
                           &s_valid, &s_hyp, &s_counters, &s_topk_score, &s_topk_idx, &s_topk_out, &s_topk_n, &s_keys, &s_keys2, &s_idx,
                           &s_perm, &s_sort_tmp, &s_sel_keys, &s_sel_keys2, &s_sel_vals, &s_sel_vals2, &s_sel_surv, &s_sel_acc,
-                          &s_sel_tmp, &s_ref_state, &s_ref_keys, &s_ref_io, &s_ref_denom, &s_dense_keys, &s_dense_rot})
+                          &s_sel_tmp, &s_ref_state, &s_ref_keys, &s_ref_io, &s_denom, &s_dense_keys, &s_dense_rot})
             b->release();
         if (h_pinned) cudaFreeHost(h_pinned);
         if (ev_fork) cudaEventDestroy(ev_fork);
         if (ev_join) cudaEventDestroy(ev_join);
+        if (ev_written) cudaEventDestroy(ev_written);
         if (h_scene_stage) cudaFreeHost(h_scene_stage);
         if (scene_stage_ev) cudaEventDestroy(scene_stage_ev);
         destroy_host_tset();
@@ -332,6 +331,20 @@ struct fdcm_dt3 {
 constexpr int64_t kMaxSide = 16384;
 
 struct SceneFilter { bool on; float cx, cy, lo, hi; };
+
+// Ordering of the work on one map across streams: the caller's stream may change between calls (fdcm_set_stream), and a
+// SceneBatch builds on a stream of its own, so stream order alone does not put a call after a queued build of the same map.
+// The caller holds m->search_mutex.
+static fdcm_status map_wait(const fdcm_dt3* m, cudaStream_t s) {
+    if (m->ev_written) CUDA_TRY(cudaStreamWaitEvent(s, m->ev_written, 0));
+    return FDCM_OK;
+}
+// (the first call comes from the map's first build, before the handle is visible to any other call)
+static fdcm_status map_written(fdcm_dt3* m, cudaStream_t s) {
+    if (!m->ev_written) CUDA_TRY(cudaEventCreateWithFlags(&m->ev_written, cudaEventDisableTiming));
+    CUDA_TRY(cudaEventRecord(m->ev_written, s));
+    return FDCM_OK;
+}
 
 // filterInRange (searchstrategies/concentricrange.h:73-84)
 static std::vector<int32_t> filter_in_range(const float* lines, int32_t n, const SceneFilter& f) {
@@ -759,6 +772,7 @@ extern "C" fdcm_status fdcm_dt3_build(const float* scene_xyxy, int32_t n_lines, 
     fdcm_status st = prepare_and_upload(m, scene_xyxy, n_lines, s);
     if (st == FDCM_OK) st = run_build_kernels(m, s);
     if (st == FDCM_OK) st = upload_build_scene(m, scene_xyxy, n_lines, s);
+    if (st == FDCM_OK) st = map_written(m, s);
     if (st == FDCM_OK) {
         cudaError_t e = cudaStreamSynchronize(s);
         if (e != cudaSuccess) st = fail(FDCM_ERR_CUDA, std::string("build: ") + cudaGetErrorString(e));
@@ -794,9 +808,11 @@ static fdcm_status rebuild_impl(fdcm_dt3* m, const float* scene_xyxy, int32_t n_
     cudaStream_t s;
     if (fdcm_status st = get_stream(m->device, &s)) return st;
     std::lock_guard<std::mutex> lk(m->search_mutex);   // a search on this handle must not see a half-replaced map
-    fdcm_status st = prepare_and_upload(m, scene_xyxy, n_lines, s);
+    fdcm_status st = map_wait(m, s);   // an earlier build of this map queued on another stream must not overlap this one
+    if (st == FDCM_OK) st = prepare_and_upload(m, scene_xyxy, n_lines, s);
     if (st == FDCM_OK) st = run_build_kernels(m, s);
     if (st == FDCM_OK) st = upload_build_scene(m, scene_xyxy, n_lines, s);
+    if (st == FDCM_OK) st = map_written(m, s);
     if (st != FDCM_OK) {
         const std::string msg = g_last_error;
         cudaStreamSynchronize(s);
@@ -815,9 +831,10 @@ extern "C" fdcm_status fdcm_dt3_rebuild(fdcm_dt3* m, const float* scene_xyxy, in
     return rebuild_impl(m, scene_xyxy, n_lines, true);
 }
 
-// Same as fdcm_dt3_rebuild but returns as soon as the build kernels are queued on the library stream: the host can
+// Same as fdcm_dt3_rebuild but returns as soon as the build kernels are queued on the current stream: the host can
 // prepare the next call (e.g. the template ordering of fdcm_search_host) while the device builds the map.  Every later
-// call on this map is stream-ordered after the build; errors of the build surface at the next synchronising call.
+// call on this map is ordered after the build, on whichever stream it runs (ev_written); errors of the build surface at
+// the next synchronising call.
 extern "C" fdcm_status fdcm_dt3_rebuild_async(fdcm_dt3* m, const float* scene_xyxy, int32_t n_lines) {
     return rebuild_impl(m, scene_xyxy, n_lines, false);
 }
@@ -827,7 +844,10 @@ extern "C" fdcm_status fdcm_dt3_rerun(fdcm_dt3* m) {
     CUDA_TRY(cudaSetDevice(m->device));
     cudaStream_t s;
     if (fdcm_status st = get_stream(m->device, &s)) return st;
-    fdcm_status st = run_build_kernels(m, s);
+    std::lock_guard<std::mutex> lk(m->search_mutex);
+    fdcm_status st = map_wait(m, s);
+    if (st == FDCM_OK) st = run_build_kernels(m, s);
+    if (st == FDCM_OK) st = map_written(m, s);
     if (st == FDCM_OK) {
         cudaError_t e = cudaStreamSynchronize(s);
         if (e != cudaSuccess) st = fail(FDCM_ERR_CUDA, std::string("rerun: ") + cudaGetErrorString(e));
@@ -841,7 +861,10 @@ extern "C" fdcm_status fdcm_dt3_rerun_async(fdcm_dt3* m) {
     CUDA_TRY(cudaSetDevice(m->device));
     cudaStream_t s;
     if (fdcm_status st = get_stream(m->device, &s)) return st;
-    return run_build_kernels(m, s);
+    std::lock_guard<std::mutex> lk(m->search_mutex);
+    if (fdcm_status st = map_wait(m, s)) return st;
+    if (fdcm_status st = run_build_kernels(m, s)) return st;
+    return map_written(m, s);
 }
 
 extern "C" fdcm_status fdcm_dt3_retain(fdcm_dt3* m) {
@@ -881,8 +904,10 @@ extern "C" fdcm_status fdcm_dt3_download_plane(const fdcm_dt3* m, int32_t plane,
     if (!m || !dst) return fail(FDCM_ERR_INVALID, "null argument");
     if (plane < 0 || plane >= m->dm.D) return fail(FDCM_ERR_INVALID, "plane out of range");
     CUDA_TRY(cudaSetDevice(m->device));
-    cudaStream_t s;   // the stream the build kernels run on: a legacy-stream copy would not be ordered after an async rebuild
+    cudaStream_t s;   // a legacy-stream copy would not be ordered after an async rebuild
     if (fdcm_status st = get_stream(m->device, &s)) return st;
+    std::lock_guard<std::mutex> lk(m->search_mutex);
+    if (fdcm_status st = map_wait(m, s)) return st;
     const float* src = m->planes.as<float>() + (size_t)plane * m->dm.plane_elems;
     CUDA_TRY(cudaMemcpy2DAsync(dst, (size_t)m->dm.W * 4, src, (size_t)m->dm.pitch * 4, (size_t)m->dm.W * 4, m->dm.H,
                                cudaMemcpyDeviceToHost, s));
@@ -896,6 +921,8 @@ extern "C" fdcm_status fdcm_dt3_download_mask(const fdcm_dt3* m, int32_t plane, 
     CUDA_TRY(cudaSetDevice(m->device));
     cudaStream_t s;
     if (fdcm_status st = get_stream(m->device, &s)) return st;
+    std::lock_guard<std::mutex> lk(m->search_mutex);
+    if (fdcm_status st = map_wait(m, s)) return st;
     std::vector<uint32_t> w((size_t)m->dm.H * m->dm.wwords);
     CUDA_TRY(cudaMemcpyAsync(w.data(), m->mask.as<uint32_t>() + (size_t)plane * m->dm.H * m->dm.wwords, w.size() * 4,
                              cudaMemcpyDeviceToHost, s));
@@ -947,6 +974,8 @@ extern "C" fdcm_status fdcm_dt3_evaluate(const fdcm_dt3* m, const float* tmpl_li
     CUDA_TRY(cudaSetDevice(m->device));
     cudaStream_t s;
     if (fdcm_status st = get_stream(m->device, &s)) return st;
+    std::lock_guard<std::mutex> lk(m->search_mutex);
+    if (fdcm_status st = map_wait(m, s)) return st;
     std::vector<int32_t> owner((size_t)n_scores);
     for (int t = 0; t < n_tmpl; ++t)
         for (int i = transl_offsets[t]; i < transl_offsets[t + 1]; ++i) owner[i] = t;
@@ -983,6 +1012,8 @@ extern "C" fdcm_status fdcm_dt3_classify(const fdcm_dt3* m, const float* lines, 
     CUDA_TRY(cudaSetDevice(m->device));
     cudaStream_t s;
     if (fdcm_status st = get_stream(m->device, &s)) return st;
+    std::lock_guard<std::mutex> lk(m->search_mutex);
+    if (fdcm_status st = map_wait(m, s)) return st;
     DevBuf dl, db;
     cudaError_t e = dl.reserve((size_t)n * 16);
     if (e == cudaSuccess) e = db.reserve((size_t)n * 4);
@@ -1034,13 +1065,12 @@ struct fdcm_templates {
     PinnedVec<float> h_line_len;      // host scratch kept for reloads (pinned: uploaded every fdcm_search_host)
     PinnedVec<int32_t> h_argsort;
     PinnedVec<float> h_anchors;       // 2 per template (fdcm_template_anchors)
-    DevBuf lines, offs, argsort, line_len, denom, anchors;
-    int denom_kind = -1;
-    float denom_tau = 0.f;
+    DevBuf lines, offs, argsort, line_len, anchors;
+    uint64_t load_id = 0;             // unique over all loads of all sets: keys the maps' denominator caches
     std::mutex mu;
     // uploads run on the copy stream (they overlap a map build in flight on the main stream); consumers wait on `ready`
     cudaEvent_t ready = nullptr;
-    bool upload_pending = false;
+    std::atomic<bool> upload_pending{false};   // (read by searches of other maps sharing the set)
     void* h_stage = nullptr;          // pinned staging for the small per-search uploads (denominators, hypothesis offsets)
     size_t h_stage_cap = 0;
     cudaError_t stage_reserve(size_t bytes) {
@@ -1056,7 +1086,7 @@ struct fdcm_templates {
         cudaSetDevice(device);
         if (ready) cudaEventDestroy(ready);
         if (h_stage) cudaFreeHost(h_stage);
-        for (DevBuf* b : {&lines, &offs, &argsort, &line_len, &denom, &anchors}) b->release();
+        for (DevBuf* b : {&lines, &offs, &argsort, &line_len, &anchors}) b->release();
     }
 };
 
@@ -1227,8 +1257,10 @@ static fdcm_status templates_ready(fdcm_templates* t, cudaStream_t s) {
     return FDCM_OK;
 }
 
-// Every consumer of a template set is host-synchronous (fdcm_search ends with a stream synchronisation), so no kernel can
-// still be reading the device arrays when they are overwritten here.
+static std::atomic<uint64_t> g_tset_loads{0};
+
+// Only fdcm_templates_create (a new set) and fdcm_search_host (the map's own set, under its host_tset_mutex, after the
+// previous search of that map has synchronised) load a set, so no kernel can still be reading the device arrays here.
 static fdcm_status templates_load(fdcm_templates* t, const float* tmpl_lines, const int32_t* tmpl_offsets, int32_t n_tmpl,
                                   cudaStream_t main_stream, int need_ranks = 0) {
     (void)main_stream;
@@ -1243,7 +1275,7 @@ static fdcm_status templates_load(fdcm_templates* t, const float* tmpl_lines, co
     t->n_tmpl = n_tmpl;
     t->n_lines = n;
     t->max_lines = 0;
-    t->denom_kind = -1;
+    t->load_id = g_tset_loads.fetch_add(1) + 1;
     t->offsets.assign(tmpl_offsets, tmpl_offsets + n_tmpl + 1);
     for (int i = 0; i < n_tmpl; ++i) t->max_lines = std::max(t->max_lines, tmpl_offsets[i + 1] - tmpl_offsets[i]);
     CUDA_TRY(t->h_line_len.resize((size_t)std::max<int64_t>(n, 1)));
@@ -1255,7 +1287,6 @@ static fdcm_status templates_load(fdcm_templates* t, const float* tmpl_lines, co
     if (e == cudaSuccess) e = t->offs.reserve((size_t)(n_tmpl + 1) * 4);
     if (e == cudaSuccess) e = t->argsort.reserve(std::max<size_t>(4, (size_t)n * 4));
     if (e == cudaSuccess) e = t->line_len.reserve(std::max<size_t>(4, (size_t)n * 4));
-    if (e == cudaSuccess) e = t->denom.reserve(std::max<size_t>(4, (size_t)n_tmpl * 4));
     if (e == cudaSuccess) e = t->anchors.reserve(std::max<size_t>(8, (size_t)n_tmpl * 8));
     if (e == cudaSuccess && n) e = cudaMemcpyAsync(t->lines.p, tmpl_lines, (size_t)n * 16, cudaMemcpyHostToDevice, s);
     if (e == cudaSuccess) e = cudaMemcpyAsync(t->offs.p, tmpl_offsets, (size_t)(n_tmpl + 1) * 4, cudaMemcpyHostToDevice, s);
@@ -1491,6 +1522,50 @@ static fdcm_status exchange_empty(const fdcm_dt3* m, fdcm_comm* comm, int k, fdc
     return finish_topk(m, comm, k, s, nullptr, out, capacity, n_out);
 }
 
+// Penalty denominators of set t for (kind, tau) (host powf like the reference) in the map's buffer: written through the
+// pinned staging `stage` on the copy stream `cs` unless the map holds them already.  Nothing else reads that buffer: every
+// earlier use of the map has synchronised (m->search_mutex held), and other maps sharing the set have their own.
+static fdcm_status map_denominators(const fdcm_dt3* m, const fdcm_templates* t, int kind, float tau, float* stage, cudaStream_t cs,
+                                    const float** d_denom) {
+    *d_denom = nullptr;
+    if (kind == FDCM_PENALTY_NONE) return FDCM_OK;
+    if (m->denom_set != t->load_id || m->denom_kind != kind || m->denom_tau != tau) {
+        m->denom_set = 0;
+        CUDA_TRY(m->s_denom.reserve(std::max<size_t>(4, (size_t)t->n_tmpl * 4)));
+        for (int i = 0; i < t->n_tmpl; ++i) stage[i] = penalty_denominator(kind, tau, t->lengths[(size_t)i]);
+        CUDA_TRY(cudaMemcpyAsync(m->s_denom.p, stage, (size_t)t->n_tmpl * 4, cudaMemcpyHostToDevice, cs));
+        m->denom_set = t->load_id;
+        m->denom_kind = kind;
+        m->denom_tau = tau;
+    }
+    *d_denom = m->s_denom.as<float>();
+    return FDCM_OK;
+}
+
+// Small per-call uploads (n_off hypothesis offsets to m->s_hyp_off, the penalty denominators) go through the set's pinned
+// staging on the copy stream, and `s` waits for them: a pageable copy on `s` would first wait for everything queued there,
+// e.g. a map build in flight.  (m->search_mutex held)
+static fdcm_status stage_uploads(const fdcm_dt3* m, fdcm_templates* t, const int64_t* hyp_off, size_t n_off, int kind, float tau,
+                                 cudaStream_t s, const float** d_denom) {
+    std::lock_guard<std::mutex> lk(t->mu);
+    cudaStream_t cs;
+    if (fdcm_status st = get_copy_stream(m->device, &cs)) return st;
+    if (!t->ready) CUDA_TRY(cudaEventCreateWithFlags(&t->ready, cudaEventDisableTiming));
+    else CUDA_TRY(cudaEventSynchronize(t->ready));   // the staging buffer may still feed an earlier upload (other threads)
+    const size_t off_bytes = n_off * 8, den_bytes = (size_t)t->n_tmpl * 4;
+    CUDA_TRY(t->stage_reserve(std::max<size_t>(16, off_bytes + den_bytes)));
+    unsigned char* stage = static_cast<unsigned char*>(t->h_stage);
+    if (off_bytes) {
+        std::memcpy(stage, hyp_off, off_bytes);
+        CUDA_TRY(cudaMemcpyAsync(m->s_hyp_off.p, stage, off_bytes, cudaMemcpyHostToDevice, cs));
+    }
+    if (fdcm_status st = map_denominators(m, t, kind, tau, reinterpret_cast<float*>(stage + off_bytes), cs, d_denom)) return st;
+    CUDA_TRY(cudaEventRecord(t->ready, cs));
+    CUDA_TRY(cudaStreamWaitEvent(s, t->ready, 0));
+    t->upload_pending = false;   // (this event is recorded after any template upload on the same copy stream)
+    return FDCM_OK;
+}
+
 // The search kernel stages the longest template of a set in shared memory, at least one warp's worth per block: a set
 // holding a template longer than one warp can stage within the device's per-block opt-in limit cannot be searched.
 static fdcm_status search_smem_optin(int device, int max_lines, int* smem_optin) {
@@ -1666,6 +1741,7 @@ static fdcm_status search_impl(const fdcm_dt3* m, const fdcm_templates* tc, cons
     CUDA_TRY(cudaSetDevice(m->device));
     cudaStream_t s;
     if (fdcm_status st = get_stream(m->device, &s)) return st;
+    if (fdcm_status st = map_wait(m, s)) return st;
     if (fdcm_status st = templates_ready(t, s)) return st;
     int smem_optin = 0;
     if (fdcm_status st = search_smem_optin(m->device, t->max_lines, &smem_optin)) return st;
@@ -1699,34 +1775,8 @@ static fdcm_status search_impl(const fdcm_dt3* m, const fdcm_templates* tc, cons
     CUDA_TRY(m->s_hyp.reserve((size_t)H * 16));
     CUDA_TRY(m->s_counters.reserve(3 * 8));
 
-    // Small per-search uploads (penalty denominators: host powf like the reference, cached per (kind, tau); hypothesis
-    // offsets) go through pinned staging on the copy stream: a pageable copy on the main stream would first wait for
-    // everything queued there, e.g. a map build in flight.
     const float* d_denom = nullptr;
-    {
-        std::lock_guard<std::mutex> lk2(t->mu);
-        cudaStream_t cs;
-        if (fdcm_status st = get_copy_stream(m->device, &cs)) return st;
-        if (!t->ready) CUDA_TRY(cudaEventCreateWithFlags(&t->ready, cudaEventDisableTiming));
-        else CUDA_TRY(cudaEventSynchronize(t->ready));   // the staging buffer may still feed an earlier upload (other threads)
-        const size_t off_bytes = hyp_off.size() * 8, den_bytes = (size_t)t->n_tmpl * 4;
-        CUDA_TRY(t->stage_reserve(off_bytes + den_bytes));
-        std::memcpy(t->h_stage, hyp_off.data(), off_bytes);
-        CUDA_TRY(cudaMemcpyAsync(m->s_hyp_off.p, t->h_stage, off_bytes, cudaMemcpyHostToDevice, cs));
-        if (p->penalty_kind != FDCM_PENALTY_NONE) {
-            if (t->denom_kind != p->penalty_kind || t->denom_tau != p->penalty_tau) {
-                float* den = reinterpret_cast<float*>(static_cast<unsigned char*>(t->h_stage) + off_bytes);
-                for (int i = 0; i < t->n_tmpl; ++i) den[i] = penalty_denominator(p->penalty_kind, p->penalty_tau, t->lengths[(size_t)i]);
-                CUDA_TRY(cudaMemcpyAsync(t->denom.p, den, den_bytes, cudaMemcpyHostToDevice, cs));
-                t->denom_kind = p->penalty_kind;
-                t->denom_tau = p->penalty_tau;
-            }
-            d_denom = t->denom.as<float>();
-        }
-        CUDA_TRY(cudaEventRecord(t->ready, cs));
-        CUDA_TRY(cudaStreamWaitEvent(s, t->ready, 0));
-        t->upload_pending = false;   // (this event is recorded after any template upload on the same copy stream)
-    }
+    if (fdcm_status st = stage_uploads(m, t, hyp_off.data(), hyp_off.size(), p->penalty_kind, p->penalty_tau, s, &d_denom)) return st;
     CUDA_TRY(cudaMemsetAsync(m->s_counters.p, 0, 3 * 8, s));
 
     TemplatesView tv;
@@ -1887,19 +1937,14 @@ extern "C" fdcm_status fdcm_refine_matches(const fdcm_dt3* m, const fdcm_templat
     CUDA_TRY(cudaSetDevice(m->device));
     cudaStream_t s;
     if (fdcm_status st = get_stream(m->device, &s)) return st;
+    if (fdcm_status st = map_wait(m, s)) return st;
     if (fdcm_status st = templates_ready(t, s)) return st;
     int smem_optin = 0;
     if (fdcm_status st = search_smem_optin(m->device, t->max_lines, &smem_optin)) return st;
     CUDA_TRY(m->s_ref_io.reserve((size_t)n * sizeof(fdcm_match)));
     CUDA_TRY(cudaMemcpyAsync(m->s_ref_io.p, in, (size_t)n * sizeof(fdcm_match), cudaMemcpyHostToDevice, s));
-    const float* d_denom = nullptr;
-    if (penalty_kind != FDCM_PENALTY_NONE) {   // the search's denominators (penalty_denominator)
-        std::vector<float> den((size_t)t->n_tmpl);
-        for (int i = 0; i < t->n_tmpl; ++i) den[(size_t)i] = penalty_denominator(penalty_kind, penalty_tau, t->lengths[(size_t)i]);
-        CUDA_TRY(m->s_ref_denom.reserve(den.size() * 4));
-        CUDA_TRY(cudaMemcpyAsync(m->s_ref_denom.p, den.data(), den.size() * 4, cudaMemcpyHostToDevice, s));
-        d_denom = m->s_ref_denom.as<float>();
-    }
+    const float* d_denom = nullptr;   // the search's denominators
+    if (fdcm_status st = stage_uploads(m, t, nullptr, 0, penalty_kind, penalty_tau, s, &d_denom)) return st;
     fdcm_match* d_io = m->s_ref_io.as<fdcm_match>();
     if (fdcm_status st = run_refine(m, t, tmpl_idx_base, d_denom, refine, d_io, nullptr, (int)n, d_io, smem_optin, s)) return st;
     CUDA_TRY(cudaMemcpyAsync(out, d_io, (size_t)n * sizeof(fdcm_match), cudaMemcpyDeviceToHost, s));
@@ -1996,6 +2041,7 @@ extern "C" fdcm_status fdcm_search_dense(const fdcm_dt3* m, const fdcm_templates
     CUDA_TRY(cudaSetDevice(m->device));
     cudaStream_t s;
     if (fdcm_status st = get_stream(m->device, &s)) return st;
+    if (fdcm_status st = map_wait(m, s)) return st;
     if (fdcm_status st = templates_ready(t, s)) return st;
     int smem_optin = 0;
     if (fdcm_status st = search_smem_optin(m->device, t->max_lines, &smem_optin)) return st;
@@ -2019,16 +2065,9 @@ extern "C" fdcm_status fdcm_search_dense(const fdcm_dt3* m, const fdcm_templates
     CUDA_TRY(m->s_hyp_off.reserve(hyp_off.size() * 8));
     CUDA_TRY(m->s_dense_keys.reserve((size_t)H * 8));
     CUDA_TRY(m->s_dense_rot.reserve(rot.size() * 4));
-    CUDA_TRY(cudaMemcpyAsync(m->s_hyp_off.p, hyp_off.data(), hyp_off.size() * 8, cudaMemcpyHostToDevice, s));
     CUDA_TRY(cudaMemcpyAsync(m->s_dense_rot.p, rot.data(), rot.size() * 4, cudaMemcpyHostToDevice, s));
-    const float* d_denom = nullptr;
-    if (penalty_kind != FDCM_PENALTY_NONE) {   // the search's denominators (penalty_denominator)
-        std::vector<float> den((size_t)t->n_tmpl);
-        for (int i = 0; i < t->n_tmpl; ++i) den[(size_t)i] = penalty_denominator(penalty_kind, penalty_tau, t->lengths[(size_t)i]);
-        CUDA_TRY(m->s_ref_denom.reserve(den.size() * 4));
-        CUDA_TRY(cudaMemcpyAsync(m->s_ref_denom.p, den.data(), den.size() * 4, cudaMemcpyHostToDevice, s));
-        d_denom = m->s_ref_denom.as<float>();
-    }
+    const float* d_denom = nullptr;   // the search's denominators
+    if (fdcm_status st = stage_uploads(m, t, hyp_off.data(), hyp_off.size(), penalty_kind, penalty_tau, s, &d_denom)) return st;
     DenseLaunch dl;
     dl.lines = t->lines.as<float4>();
     dl.offsets = t->offs.as<int32_t>();
@@ -2139,7 +2178,8 @@ extern "C" fdcm_status fdcm_comm_rebuild_broadcast(fdcm_comm* comm, fdcm_dt3* m,
     cudaStream_t s;
     if (fdcm_status st = get_stream(m->device, &s)) return st;
     std::lock_guard<std::mutex> lk(m->search_mutex);
-    fdcm_status st = prepare_and_upload(m, scene_xyxy, n_lines, s);
+    fdcm_status st = map_wait(m, s);
+    if (st == FDCM_OK) st = prepare_and_upload(m, scene_xyxy, n_lines, s);
     if (st == FDCM_OK && comm->rank == root) st = run_build_kernels(m, s);
     if (st == FDCM_OK && n_lines > 0) {
         const size_t bytes = (size_t)m->dm.D * m->dm.plane_elems * sizeof(float);
@@ -2147,6 +2187,7 @@ extern "C" fdcm_status fdcm_comm_rebuild_broadcast(fdcm_comm* comm, fdcm_dt3* m,
         if (r != ncclSuccess) st = fail(FDCM_ERR_CUDA, std::string("ncclBroadcast: ") + nccl_api().GetErrorString(r));
     }
     if (st == FDCM_OK) st = upload_build_scene(m, scene_xyxy, n_lines, s);
+    if (st == FDCM_OK) st = map_written(m, s);
     if (st == FDCM_OK && cudaStreamSynchronize(s) != cudaSuccess) st = fail(FDCM_ERR_CUDA, "rebuild_broadcast: stream failed");
     prof_resolve();
     if (st != FDCM_OK) {
@@ -2168,13 +2209,10 @@ struct fdcm_scene_batch {
     fdcm_dt3_params params{};
     fdcm_dt3* maps[2] = {nullptr, nullptr};
     cudaStream_t build_stream = nullptr;
-    cudaEvent_t built[2] = {nullptr, nullptr};
     ~fdcm_scene_batch() {
         cudaSetDevice(device);
-        for (int i = 0; i < 2; ++i) {
+        for (int i = 0; i < 2; ++i)
             if (maps[i]) fdcm_dt3_release(maps[i]);
-            if (built[i]) cudaEventDestroy(built[i]);
-        }
         if (build_stream) cudaStreamDestroy(build_stream);
     }
 };
@@ -2189,7 +2227,6 @@ extern "C" fdcm_status fdcm_scene_batch_create(const fdcm_dt3_params* params, in
     b->device = device;
     b->params = *params;
     cudaError_t e = cudaStreamCreateWithFlags(&b->build_stream, cudaStreamNonBlocking);
-    for (int i = 0; i < 2 && e == cudaSuccess; ++i) e = cudaEventCreateWithFlags(&b->built[i], cudaEventDisableTiming);
     for (int i = 0; i < 2 && e == cudaSuccess; ++i) {
         b->maps[i] = new (std::nothrow) fdcm_dt3();
         if (!b->maps[i]) { delete b; return fail(FDCM_ERR_NOMEM, "host allocation failed"); }
@@ -2214,9 +2251,11 @@ extern "C" fdcm_status fdcm_scene_batch_destroy(fdcm_scene_batch* b) {
 static fdcm_status batch_queue_build(fdcm_scene_batch* b, int slot, const float* scene, int32_t n_lines) {
     fdcm_dt3* m = b->maps[slot];
     std::lock_guard<std::mutex> lk(m->search_mutex);
-    fdcm_status st = prepare_and_upload(m, scene, n_lines, b->build_stream);
+    fdcm_status st = map_wait(m, b->build_stream);
+    if (st == FDCM_OK) st = prepare_and_upload(m, scene, n_lines, b->build_stream);
     if (st == FDCM_OK) st = run_build_kernels(m, b->build_stream);
     if (st == FDCM_OK) st = upload_build_scene(m, scene, n_lines, b->build_stream);
+    if (st == FDCM_OK) st = map_written(m, b->build_stream);
     if (st != FDCM_OK) {
         const std::string msg = g_last_error;
         cudaStreamSynchronize(b->build_stream);
@@ -2224,7 +2263,6 @@ static fdcm_status batch_queue_build(fdcm_scene_batch* b, int slot, const float*
         g_last_error = msg;
         return st;
     }
-    CUDA_TRY(cudaEventRecord(b->built[slot], b->build_stream));
     return FDCM_OK;
 }
 
@@ -2239,8 +2277,6 @@ static fdcm_status search_scenes_impl(fdcm_scene_batch* b, const float* scene_li
         if (scene_offsets[s + 1] < scene_offsets[s]) return fail(FDCM_ERR_INVALID, "scene offsets must be non-decreasing");
     if (scene_offsets[n_scenes] > 0 && !scene_lines) return fail(FDCM_ERR_INVALID, "scene_lines is null");
     CUDA_TRY(cudaSetDevice(b->device));
-    cudaStream_t main_s;
-    if (fdcm_status st = get_stream(b->device, &main_s)) return st;
     auto scene_ptr = [&](int s) { return scene_lines + 4 * (size_t)scene_offsets[s]; };
     auto scene_n = [&](int s) { return scene_offsets[s + 1] - scene_offsets[s]; };
     // the build stream must not overtake a search still running on the map it is about to overwrite: searches are
@@ -2250,8 +2286,7 @@ static fdcm_status search_scenes_impl(fdcm_scene_batch* b, const float* scene_li
         const int slot = s & 1;
         if (s + 1 < n_scenes)
             if (fdcm_status st = batch_queue_build(b, slot ^ 1, scene_ptr(s + 1), scene_n(s + 1))) return st;
-        CUDA_TRY(cudaStreamWaitEvent(main_s, b->built[slot], 0));
-        int64_t n = 0;
+        int64_t n = 0;   // (the search waits for the slot's build: map_wait)
         fdcm_search_params ps = *p;
         const fdcm_status st = search_impl(b->maps[slot], templates, nullptr, FDCM_SCENE_RESIDENT, &ps, out + (size_t)s * p->top_k, p->top_k, &n, nullptr,
                                            sel);
@@ -2290,6 +2325,8 @@ extern "C" fdcm_status fdcm_optimize(const fdcm_dt3* m, const float* tmpl_lines,
     CUDA_TRY(cudaSetDevice(m->device));
     cudaStream_t s;
     if (fdcm_status st = get_stream(m->device, &s)) return st;
+    std::lock_guard<std::mutex> lk(m->search_mutex);
+    if (fdcm_status st = map_wait(m, s)) return st;
     int max_lines = 1;
     for (int t = 0; t < n_tmpl; ++t) max_lines = std::max(max_lines, tmpl_offsets[t + 1] - tmpl_offsets[t]);
     int smem_optin = 0;
