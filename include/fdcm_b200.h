@@ -313,6 +313,50 @@ fdcm_status fdcm_search_dense(const fdcm_dt3* map, const fdcm_templates* templat
 fdcm_status fdcm_dense_poses(const fdcm_dense_params* dense, const float anchor[2], const float shift[2], int32_t width, int32_t height,
                              int32_t rotation, float* out, int64_t capacity, int64_t* n_out, int32_t grid_wh[2]);
 
+/* ---- match verification: oriented edge coverage (beyond the reference) ---------------------------
+ * The DT3 score of a match grows with the template's length and the scene's clutter, so one score threshold means different
+ * things for different templates.  Coverage is a support measure on a fixed scale: the fraction of the posed template's
+ * raster samples that have a scene edge pixel of similar orientation within `radius` pixels (Chebyshev).  It lies in [0, 1]
+ * and an occluded line lowers it by that line's share.  It is not a probability.
+ * Rules, in fp32 without contraction.  A match with template t = tmpl_idx - tmpl_idx_base and transform T, on a map of W x H
+ * with scene translation shift, D planes and edge masks E_q (fdcm_dt3_download_mask):
+ *   1. Lines.  Every template line (x1, y1, x2, y2) is posed as in refinement rule 4: rotated end points (T0*x + T1*y,
+ *      T3*x + T4*y), bin b = the slope-table bin of the rotated line (fdcm_dt3_classify of the rotated line), map-coordinate
+ *      end points rx + (shift_x + T2), ry + (shift_y + T5).
+ *   2. Validity.  Refinement's: no entry of T and no rotated end point is NaN, and every map-coordinate end point lies in
+ *      [0, W-1] x [0, H-1].  An invalid match, an empty template or an empty map has coverage NaN.
+ *   3. Samples.  Each posed line is rasterised with rasterizeLine (core/drawing.h:74-102, no clipping), the pixels the DT3
+ *      build draws for a scene line; duplicated pixels count every time.  n_total is the sum over the lines.
+ *   4. Covered.  Sample (x, y) of a line of bin b is covered iff some plane q with min(|q - b|, D - |q - b|) <= bin_tolerance
+ *      has an edge pixel (x', y') of E_q inside the map with |x' - x| <= radius and |y' - y| <= radius.
+ *   5. Coverage = (float)n_covered / (float)n_total.
+ *   6. Filter (fdcm_search_verify, fdcm_search_dense_verify).  With min_coverage > 0 every valid record of the search (or of
+ *      the dense grid) whose coverage is NaN or below min_coverage becomes invalid before the top-K or distinct selection;
+ *      refinement then runs on the selected records, which are not filtered again.  min_coverage == 0: no filter, the call is
+ *      byte-identical to the call without verification and runs no coverage kernel.
+ * Invalid parameters fail with FDCM_ERR_INVALID: radius outside 0..FDCM_COVERAGE_MAX_RADIUS, bin_tolerance outside 0..32,
+ * min_coverage not in [0, 1]; a tmpl_idx - tmpl_idx_base outside the template set fails with FDCM_ERR_OUT_OF_RANGE.
+ * Cost: once per (map write, radius, bin_tolerance) a dilated copy of the edge mask (the mask's size: D x H x pitch / 8
+ * bytes), then one bit gather per sample. */
+#define FDCM_COVERAGE_MAX_RADIUS 16
+typedef struct fdcm_coverage_params {    /* 12 bytes */
+    int32_t radius;             /* 0..FDCM_COVERAGE_MAX_RADIUS: Chebyshev distance to a supporting edge pixel */
+    int32_t bin_tolerance;      /* 0..32: orientation planes on either side of the line's own plane (circular) */
+    float min_coverage;         /* [0, 1]: filter threshold of the fused searches; 0: no filter */
+} fdcm_coverage_params;
+/* coverage of n host matches (any source); coverage: n floats; n == 0 is no error */
+fdcm_status fdcm_match_coverage(const fdcm_dt3* map, const fdcm_templates* templates, int32_t tmpl_idx_base,
+                                const fdcm_coverage_params* cov, const fdcm_match* in, int64_t n, float* coverage);
+/* fdcm_search_refine with select and refine each optional (NULL) and the coverage filter of rule 6; top_k > 0 */
+fdcm_status fdcm_search_verify(const fdcm_dt3* map, const fdcm_templates* templates, const float* scene_xyxy, int32_t n_scene,
+                               const fdcm_search_params* params, const fdcm_select_params* select, const fdcm_refine_params* refine,
+                               const fdcm_coverage_params* cov, fdcm_match* out, int64_t capacity, int64_t* n_out);
+/* fdcm_search_dense with the coverage filter of rule 6 */
+fdcm_status fdcm_search_dense_verify(const fdcm_dt3* map, const fdcm_templates* templates, const fdcm_dense_params* dense,
+                                     int32_t penalty_kind, float penalty_tau, int32_t top_k, int32_t tmpl_idx_base,
+                                     const fdcm_select_params* select, const fdcm_refine_params* refine,
+                                     const fdcm_coverage_params* cov, fdcm_match* out, int64_t capacity, int64_t* n_out);
+
 /* optimize(optimizer, templates, alignments, featuremap) (matching/optimizestrategy.h:62-64; BatchOptimize:
  * batchoptimize.cpp:6-123, batch_size == 0: DefaultOptimize, defaultoptimize.cpp:6-93).  The templates are used
  * as given (already aligned); alignments: n_tmpl (x,y) pairs.  Outputs per template: has_value (0 = nullopt),

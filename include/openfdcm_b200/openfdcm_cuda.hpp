@@ -360,7 +360,8 @@ struct DenseSearch {
 };
 namespace detail {
 inline std::vector<Match> search_dense(const Dt3Cuda& fm, const std::vector<LineArray>& templates, const DenseSearch& dense, int penalty_kind,
-                                       float tau, int k, const DistinctMatches* select, const PoseRefinement* refine) {
+                                       float tau, int k, const DistinctMatches* select, const PoseRefinement* refine,
+                                       const fdcm_coverage_params* cov = nullptr) {
     std::vector<float> flat;
     std::vector<int32_t> off;
     pack(templates, flat, off);
@@ -376,8 +377,12 @@ inline std::vector<Match> search_dense(const Dt3Cuda& fm, const std::vector<Line
     if (refine) r = refine_params(*refine);
     std::vector<fdcm_match> rec((size_t)std::max(k, 1));
     int64_t n = 0;
-    check(fdcm_search_dense(fm.handle(), ts, &d, penalty_kind, tau, k, 0, select ? &q : nullptr, refine ? &r : nullptr, rec.data(),
-                            (int64_t)rec.size(), &n));
+    if (cov)
+        check(fdcm_search_dense_verify(fm.handle(), ts, &d, penalty_kind, tau, k, 0, select ? &q : nullptr, refine ? &r : nullptr, cov,
+                                       rec.data(), (int64_t)rec.size(), &n));
+    else
+        check(fdcm_search_dense(fm.handle(), ts, &d, penalty_kind, tau, k, 0, select ? &q : nullptr, refine ? &r : nullptr, rec.data(),
+                                (int64_t)rec.size(), &n));
     return to_matches(rec, n);
 }
 }   // namespace detail
@@ -393,6 +398,78 @@ inline std::vector<Match> searchDense(const Dt3Cuda& fm, const std::vector<LineA
 inline std::vector<Match> searchDense(const Dt3Cuda& fm, const std::vector<LineArray>& templates, const DenseSearch& dense,
                                       const ExponentialPenalty& pen, int k, const DistinctMatches* select, const PoseRefinement* refine) {
     return detail::search_dense(fm, templates, dense, FDCM_PENALTY_EXPONENTIAL, pen.tau, k, select, refine);
+}
+
+// match verification (beyond the reference; rules of fdcm_match_coverage): the fraction of a posed template's raster
+// samples with a scene edge pixel within `radius` pixels on an orientation plane within `binTolerance` planes.  A support
+// measure for a pose in [0, 1] (NaN outside the map), not a probability; the defaults are a starting point, not tuned.
+// minCoverage > 0 filters the records of searchTopK / searchDense before their selection.
+struct EdgeCoverage {
+    int radius{2};
+    int binTolerance{1};
+    float minCoverage{0.f};
+};
+namespace detail {
+inline fdcm_coverage_params coverage_params(const EdgeCoverage& c) { return fdcm_coverage_params{c.radius, c.binTolerance, c.minCoverage}; }
+inline std::vector<Match> search_verify(const DefaultSearch& s, const BatchOptimize& o, const ExponentialPenalty& pen, const Dt3Cuda& fm,
+                                        const std::vector<LineArray>& templates, const LineArray& scene, int k, const DistinctMatches* select,
+                                        const PoseRefinement* refine, const EdgeCoverage& verify) {
+    std::vector<float> flat;
+    std::vector<int32_t> off;
+    pack(templates, flat, off);
+    fdcm_templates* ts = nullptr;
+    check(fdcm_templates_create(flat.data(), off.data(), (int32_t)templates.size(), fm.info().device, &ts));
+    const std::unique_ptr<fdcm_templates, fdcm_status (*)(fdcm_templates*)> owner(ts, fdcm_templates_release);
+    const fdcm_search_params p{(int32_t)s.max_tmpl_lines, (int32_t)s.max_scene_lines, (int32_t)o.batchSize, FDCM_PENALTY_EXPONENTIAL,
+                               pen.tau, k, 0, 0, 0.f, 0.f, 0.f, 0.f};
+    fdcm_select_params q{};
+    if (select) q = fdcm_select_params{select->maxPerTemplate, select->radius, select->maxAngle, select->acrossTemplates ? 1 : 0};
+    fdcm_refine_params r{};
+    if (refine) r = refine_params(*refine);
+    const fdcm_coverage_params c = coverage_params(verify);
+    std::vector<fdcm_match> rec((size_t)std::max(k, 1));
+    int64_t n = 0;
+    check(fdcm_search_verify(fm.handle(), ts, scene.data(), (int32_t)(scene.size() / 4), &p, select ? &q : nullptr, refine ? &r : nullptr,
+                             &c, rec.data(), (int64_t)rec.size(), &n));
+    return to_matches(rec, n);
+}
+}   // namespace detail
+// coverage of every match (tmplIdx indexes `templates`), entry i for matches[i]
+inline std::vector<float> matchCoverage(const Dt3Cuda& fm, const std::vector<LineArray>& templates, const std::vector<Match>& matches,
+                                        const EdgeCoverage& coverage = EdgeCoverage{}) {
+    std::vector<float> flat;
+    std::vector<int32_t> off;
+    detail::pack(templates, flat, off);
+    fdcm_templates* ts = nullptr;
+    check(fdcm_templates_create(flat.data(), off.data(), (int32_t)templates.size(), fm.info().device, &ts));
+    const std::unique_ptr<fdcm_templates, fdcm_status (*)(fdcm_templates*)> owner(ts, fdcm_templates_release);
+    std::vector<fdcm_match> rec(matches.size());
+    for (size_t i = 0; i < matches.size(); ++i) {
+        rec[i].tmpl_idx = matches[i].tmplIdx;
+        rec[i].score = matches[i].score;
+        for (int c = 0; c < 6; ++c) rec[i].transform[c] = matches[i].transform[(size_t)c];
+    }
+    const fdcm_coverage_params c = detail::coverage_params(coverage);
+    std::vector<float> out(matches.size());
+    check(fdcm_match_coverage(fm.handle(), ts, 0, &c, rec.data(), (int64_t)rec.size(), out.data()));
+    return out;
+}
+// fused search -> coverage filter -> top-k (or distinct top-k) [-> pose refinement] on the device
+inline std::vector<Match> searchTopK(const DefaultSearch& s, const BatchOptimize& o, const ExponentialPenalty& pen, const Dt3Cuda& fm,
+                                     const std::vector<LineArray>& templates, const LineArray& scene, int k, const EdgeCoverage& verify) {
+    return detail::search_verify(s, o, pen, fm, templates, scene, k, nullptr, nullptr, verify);
+}
+inline std::vector<Match> searchTopK(const DefaultSearch& s, const BatchOptimize& o, const ExponentialPenalty& pen, const Dt3Cuda& fm,
+                                     const std::vector<LineArray>& templates, const LineArray& scene, int k, const DistinctMatches* select,
+                                     const PoseRefinement* refine, const EdgeCoverage& verify) {
+    return detail::search_verify(s, o, pen, fm, templates, scene, k, select, refine, verify);
+}
+// dense search -> coverage filter -> top-k (or distinct top-k) [-> pose refinement] on the device
+inline std::vector<Match> searchDense(const Dt3Cuda& fm, const std::vector<LineArray>& templates, const DenseSearch& dense,
+                                      const ExponentialPenalty& pen, int k, const DistinctMatches* select, const PoseRefinement* refine,
+                                      const EdgeCoverage& verify) {
+    const fdcm_coverage_params c = detail::coverage_params(verify);
+    return detail::search_dense(fm, templates, dense, FDCM_PENALTY_EXPONENTIAL, pen.tau, k, select, refine, &c);
 }
 
 // ---- PenaltyStrategy concept, template lengths, sort ----------------------------------------------

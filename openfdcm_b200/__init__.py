@@ -22,8 +22,8 @@ from ._lib import MATCH_DTYPE, FdcmError, check, lib, ptr
 __all__ = [
     "distance", "Dt3CudaParameters", "Dt3Cuda", "build_cuda_featuremap", "ThreadPool", "DefaultSearch", "ConcentricRangeStrategy",
     "BatchOptimize", "DefaultOptimize", "DefaultMatch", "DefaultPenalty", "ExponentialPenalty", "Match",
-    "TemplateSet", "SceneBatch", "DistinctMatches", "PoseRefinement", "DenseSearch", "search", "search_topk", "search_dense",
-    "refine_matches", "penalize", "get_template_lengths",
+    "TemplateSet", "SceneBatch", "DistinctMatches", "PoseRefinement", "DenseSearch", "EdgeCoverage", "search", "search_topk",
+    "search_dense", "refine_matches", "match_coverage", "penalize", "get_template_lengths",
     "get_template_anchors", "sort_matches", "evaluate",
     "minmax_translation", "get_feature_size", "establish_search_strategy", "optimize", "read", "write", "FdcmError", "MATCH_DTYPE",
 ]
@@ -380,7 +380,27 @@ class DenseSearch:
                 f"cell={self.cell}, roi={self.roi}>")
 
 
-def _search_raw(featuremap, templates, scene, searcher, optimizer, penalty=None, top_k=0, tmpl_idx_base=0, select=None, refine=None):
+class EdgeCoverage:
+    """Match verification (beyond the reference): the coverage of a match is the fraction of its posed template's raster
+    samples that have a scene edge pixel within `radius` pixels (Chebyshev) on an orientation plane within `bin_tolerance`
+    planes of the line's own.  It lies in [0, 1] (NaN for a pose outside the map) and compares across templates; it is a
+    support measure for a pose, not a probability, and the defaults are a starting point, not tuned.  min_coverage > 0
+    filters the records of search_topk / search_dense before their selection.  Exact rules: include/fdcm_b200.h."""
+
+    def __init__(self, radius=2, bin_tolerance=1, min_coverage=0.0):
+        self.radius = int(radius)
+        self.bin_tolerance = int(bin_tolerance)
+        self.min_coverage = float(min_coverage)
+
+    def _params(self):
+        return _lib.CoverageParams(self.radius, self.bin_tolerance, self.min_coverage)
+
+    def __repr__(self):
+        return f"<EdgeCoverage: radius={self.radius}, bin_tolerance={self.bin_tolerance}, min_coverage={self.min_coverage}>"
+
+
+def _search_raw(featuremap, templates, scene, searcher, optimizer, penalty=None, top_k=0, tmpl_idx_base=0, select=None, refine=None,
+                verify=None):
     if not isinstance(featuremap, Dt3Cuda):
         raise TypeError("the CUDA search needs a Dt3Cuda feature map (build_cuda_featuremap)")
     tset = templates if isinstance(templates, TemplateSet) else TemplateSet(templates, featuremap.device)
@@ -398,7 +418,12 @@ def _search_raw(featuremap, templates, scene, searcher, optimizer, penalty=None,
     out = np.zeros(max(cap, 1), MATCH_DTYPE)
     n = C.c_int64(0)
     n_scene = _lib.FDCM_SCENE_RESIDENT if s is None else s.shape[0]
-    if refine is not None:
+    if verify is not None:
+        sp = None if select is None else C.byref(select._params())
+        rp = None if refine is None else C.byref(refine._params())
+        check(lib().fdcm_search_verify(featuremap._h, tset._h, ptr(s), n_scene, C.byref(p), sp, rp, C.byref(verify._params()), ptr(out),
+                                       out.shape[0], C.byref(n)))
+    elif refine is not None:
         sp = None if select is None else C.byref(select._params())
         check(lib().fdcm_search_refine(featuremap._h, tset._h, ptr(s), n_scene, C.byref(p), sp, C.byref(refine._params()), ptr(out),
                                        out.shape[0], C.byref(n)))
@@ -416,12 +441,14 @@ def search(matcher, searcher, optimizer, featuremap, templates, scene):
     return _to_matches(_search_raw(featuremap, templates, scene, searcher, optimizer))
 
 
-def search_topk(featuremap, templates, scene, searcher, optimizer, penalty=None, k=10, tmpl_idx_base=0, *, select=None, refine=None):
+def search_topk(featuremap, templates, scene, searcher, optimizer, penalty=None, k=10, tmpl_idx_base=0, *, select=None, refine=None,
+                verify=None):
     """Fused search -> penalize -> top-k on the device; returns a MATCH_DTYPE record array (ascending score).
     select: a DistinctMatches for the distinct top-k (the kept matches in acceptance order, also ascending score).
     refine: a PoseRefinement applied to the selected matches on the device, equal to refine_matches of the unrefined
-    result (same order: re-rank with sort_matches); it lowers the score, not the pose error (see PoseRefinement)."""
-    return _search_raw(featuremap, templates, scene, searcher, optimizer, penalty, k, tmpl_idx_base, select, refine).copy()
+    result (same order: re-rank with sort_matches); it lowers the score, not the pose error (see PoseRefinement).
+    verify: an EdgeCoverage whose min_coverage > 0 drops every match of lower (or NaN) coverage before the selection."""
+    return _search_raw(featuremap, templates, scene, searcher, optimizer, penalty, k, tmpl_idx_base, select, refine, verify).copy()
 
 
 def refine_matches(featuremap, templates, matches, refine, penalty=None, tmpl_idx_base=0):
@@ -442,10 +469,11 @@ def refine_matches(featuremap, templates, matches, refine, penalty=None, tmpl_id
     return out[: rec.shape[0]].copy()
 
 
-def search_dense(featuremap, templates, dense, penalty=None, k=10, tmpl_idx_base=0, *, select=None, refine=None):
+def search_dense(featuremap, templates, dense, penalty=None, k=10, tmpl_idx_base=0, *, select=None, refine=None, verify=None):
     """Dense pose-grid search on the device (see DenseSearch): the best pose of every (template, rotation, cell), then the
     top-k in ascending (score, record) order, or with select (a DistinctMatches) the distinct top-k, then with refine (a
-    PoseRefinement) the refinement of those, equal to refine_matches of the unrefined result.  Returns a MATCH_DTYPE array."""
+    PoseRefinement) the refinement of those, equal to refine_matches of the unrefined result.  Returns a MATCH_DTYPE array.
+    verify: an EdgeCoverage whose min_coverage > 0 drops every record of lower (or NaN) coverage before the selection."""
     if not isinstance(featuremap, Dt3Cuda):
         raise TypeError("search_dense needs a Dt3Cuda feature map (build_cuda_featuremap)")
     tset = templates if isinstance(templates, TemplateSet) else TemplateSet(templates, featuremap.device)
@@ -453,10 +481,30 @@ def search_dense(featuremap, templates, dense, penalty=None, k=10, tmpl_idx_base
     n = C.c_int64(0)
     sp = None if select is None else C.byref(select._params())
     rp = None if refine is None else C.byref(refine._params())
-    check(lib().fdcm_search_dense(featuremap._h, tset._h, C.byref(dense._params()), 0 if penalty is None else penalty.kind,
-                                  0.0 if penalty is None else float(penalty.tau), int(k), int(tmpl_idx_base), sp, rp, ptr(out), out.shape[0],
-                                  C.byref(n)))
+    pen_kind, pen_tau = (0, 0.0) if penalty is None else (penalty.kind, float(penalty.tau))
+    if verify is None:
+        check(lib().fdcm_search_dense(featuremap._h, tset._h, C.byref(dense._params()), pen_kind, pen_tau, int(k), int(tmpl_idx_base), sp, rp,
+                                      ptr(out), out.shape[0], C.byref(n)))
+    else:
+        check(lib().fdcm_search_dense_verify(featuremap._h, tset._h, C.byref(dense._params()), pen_kind, pen_tau, int(k), int(tmpl_idx_base),
+                                             sp, rp, C.byref(verify._params()), ptr(out), out.shape[0], C.byref(n)))
     return out[: n.value].copy()
+
+
+def match_coverage(featuremap, templates, matches, coverage=None, tmpl_idx_base=0):
+    """Edge coverage (see EdgeCoverage; None: the defaults) of any match list against a feature map and a template set
+    (list or TemplateSet): an (n,) float32 array, NaN where the posed template leaves the map."""
+    if not isinstance(featuremap, Dt3Cuda):
+        raise TypeError("match_coverage needs a Dt3Cuda feature map (build_cuda_featuremap)")
+    coverage = EdgeCoverage() if coverage is None else coverage
+    tset = templates if isinstance(templates, TemplateSet) else TemplateSet(templates, featuremap.device)
+    rec = _to_records(matches)
+    out = np.zeros(max(rec.shape[0], 1), np.float32)
+    st = lib().fdcm_match_coverage(featuremap._h, tset._h, int(tmpl_idx_base), C.byref(coverage._params()), ptr(rec), rec.shape[0], ptr(out))
+    if st == _lib.FDCM_ERR_OUT_OF_RANGE:
+        raise IndexError(lib().fdcm_last_error().decode())
+    check(st)
+    return out[: rec.shape[0]].copy()
 
 
 def search_all(featuremap, templates, scene, searcher, optimizer, penalty=None, tmpl_idx_base=0):

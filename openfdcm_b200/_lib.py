@@ -41,6 +41,10 @@ class DenseParams(C.Structure):
                 ("roi_on", C.c_int32), ("roi", C.c_float * 4)]
 
 
+class CoverageParams(C.Structure):
+    _fields_ = [("radius", C.c_int32), ("bin_tolerance", C.c_int32), ("min_coverage", C.c_float)]
+
+
 class Dt3Info(C.Structure):
     _fields_ = [("depth", C.c_int32), ("width", C.c_int32), ("height", C.c_int32), ("pitch", C.c_int32),
                 ("scene_translation", C.c_float * 2), ("distance", C.c_int32), ("device", C.c_int32),
@@ -90,6 +94,11 @@ SIGNATURES = {
                                     C.POINTER(RefineParams), _P, C.c_int64, C.POINTER(C.c_int64)]),
     "fdcm_dense_poses": (C.c_int, [C.POINTER(DenseParams), _P, _P, C.c_int32, C.c_int32, C.c_int32, _P, C.c_int64, C.POINTER(C.c_int64),
                                    _P]),
+    "fdcm_match_coverage": (C.c_int, [_P, _P, C.c_int32, C.POINTER(CoverageParams), _P, C.c_int64, _P]),
+    "fdcm_search_verify": (C.c_int, [_P, _P, _P, C.c_int32, C.POINTER(SearchParams), C.POINTER(SelectParams), C.POINTER(RefineParams),
+                                     C.POINTER(CoverageParams), _P, C.c_int64, C.POINTER(C.c_int64)]),
+    "fdcm_search_dense_verify": (C.c_int, [_P, _P, C.POINTER(DenseParams), C.c_int32, C.c_float, C.c_int32, C.c_int32, C.POINTER(SelectParams),
+                                           C.POINTER(RefineParams), C.POINTER(CoverageParams), _P, C.c_int64, C.POINTER(C.c_int64)]),
     "fdcm_optimize": (C.c_int, [_P, _P, _P, C.c_int32, _P, C.c_int32, _P, _P, _P]),
     "fdcm_search_host": (C.c_int, [_P, _P, _P, C.c_int32, _P, C.c_int32, C.POINTER(SearchParams), _P, C.c_int64,
                                    C.POINTER(C.c_int64)]),

@@ -60,6 +60,68 @@ __device__ __forceinline__ void rasterize_vector_dev(float vx, float vy, float& 
     oy = c ? -1.f : 1.f;
 }
 
+// relativelyEqual(x, 0.0f) (core/math.h:183-189): |x| <= eps_f + 1e-10*|x| evaluated in double
+__device__ __forceinline__ bool rel_eq_zero(float x) {
+    const double ax = (double)fabsf(x);
+    return ax <= (double)FLT_EPSILON + 1e-10 * ax;
+}
+
+// Eigen 3.4.0 LinSpaced<float>(n, lo, hi)(i) (see oracle / SURVEY App. A.7)
+struct LinSpacedDev {
+    float lo, hi, step;
+    int size1;
+    bool flip;
+    __device__ LinSpacedDev() : lo(0.f), hi(0.f), step(0.f), size1(1), flip(false) {}
+    __device__ LinSpacedDev(int n, float lo_, float hi_)
+        : lo(lo_), hi(hi_), step(n == 1 ? 0.f : (hi_ - lo_) / (float)(n - 1)), size1(n == 1 ? 1 : n - 1),
+          flip(fabsf(hi_) < fabsf(lo_)) {}
+    __device__ __forceinline__ float at(int i) const {
+        if (flip) return (i == 0) ? lo : (hi - (float)(size1 - i) * step);
+        return (i == size1) ? hi : (lo + (float)i * step);
+    }
+};
+
+// rasterizeLine (core/drawing.h:74-102) of the line (p1x, p1y) - (p2x, p2y), without clipping: n pixels, pixel i at(i)
+struct RasterLineDev {
+    int n;
+    int kind;                // 0: one pixel, 1: x fixed (steep), 2: y fixed (flat), 3: both vary
+    long long fx, fy;        // the fixed coordinate of kinds 0..2
+    LinSpacedDev lx, ly;
+    __device__ RasterLineDev(float p1x, float p1y, float p2x, float p2y) {
+        fx = round_to_ll(p1x);
+        fy = round_to_ll(p1y);
+        if (fabsf(p2x - p1x) <= 1e-5f && fabsf(p2y - p1y) <= 1e-5f) {
+            n = 1;
+            kind = 0;
+            return;
+        }
+        const float lvx = p2x - p1x, lvy = p2y - p1y;
+        float rx, ry;
+        rasterize_vector_dev(lvx, lvy, rx, ry);
+        if (rel_eq_zero(rx)) {
+            n = (int)(lvy / ry) + 1;
+            kind = 1;
+            ly = LinSpacedDev(n, p1y, p2y);
+            return;
+        }
+        if (rel_eq_zero(ry)) {
+            n = (int)(lvx / rx) + 1;
+            kind = 2;
+            lx = LinSpacedDev(n, p1x, p2x);
+            return;
+        }
+        const float a = lvx / rx, b = lvy / ry;
+        n = (int)((a < b) ? b : a) + 1;   // std::max(a, b)
+        kind = 3;
+        lx = LinSpacedDev(n, p1x, p2x);
+        ly = LinSpacedDev(n, p1y, p2y);
+    }
+    __device__ __forceinline__ void at(int i, long long& x, long long& y) const {
+        x = (kind & 2) ? round_to_ll(lx.at(i)) : fx;
+        y = (kind & 1) ? round_to_ll(ly.at(i)) : fy;
+    }
+};
+
 // orientation bin of a slope through the host-built threshold table (dt3cpu.h:93-114 semantics)
 __device__ __forceinline__ int bin_of_slope_dev(const SlopeTableDev& t, float slope) {
     if (slope != slope) return t.nan_bin;

@@ -50,26 +50,6 @@ __device__ bool clip_line_dev(float& x1, float& y1, float& x2, float& y2, float 
     return false;
 }
 
-// relativelyEqual(x, 0.0f) (core/math.h:183-189): |x| <= eps_f + 1e-10*|x| evaluated in double
-__device__ __forceinline__ bool rel_eq_zero(float x) {
-    const double ax = (double)fabsf(x);
-    return ax <= (double)FLT_EPSILON + 1e-10 * ax;
-}
-
-// Eigen 3.4.0 LinSpaced<float>(n, lo, hi)(i) (see oracle / SURVEY App. A.7)
-struct LinSpacedDev {
-    float lo, hi, step;
-    int size1;
-    bool flip;
-    __device__ LinSpacedDev(int n, float lo_, float hi_)
-        : lo(lo_), hi(hi_), step(n == 1 ? 0.f : (hi_ - lo_) / (float)(n - 1)), size1(n == 1 ? 1 : n - 1),
-          flip(fabsf(hi_) < fabsf(lo_)) {}
-    __device__ __forceinline__ float at(int i) const {
-        if (flip) return (i == 0) ? lo : (hi - (float)(size1 - i) * step);
-        return (i == size1) ? hi : (lo + (float)i * step);
-    }
-};
-
 __device__ __forceinline__ void set_edge(uint32_t* mask, const MapDims& dm, int plane, long long x, long long y) {
     if (x < 0 || y < 0 || x >= dm.W || y >= dm.H) return;   // unreachable after clipping; guards NaN input
     atomicOr(mask + ((size_t)plane * dm.H + (size_t)y) * dm.wwords + (x >> 5), 1u << (x & 31));
@@ -86,31 +66,12 @@ __global__ void __launch_bounds__(256) raster_kernel(const float4* __restrict__ 
     float p1x = l.x, p1y = l.y, p2x = l.z, p2y = l.w;
     if (!clip_line_dev(p1x, p1y, p2x, p2y, (float)(dm.W - 1), (float)(dm.H - 1))) return;   // core/drawing.h:117-118
     // rasterizeLine (core/drawing.h:74-102)
-    if (fabsf(p2x - p1x) <= 1e-5f && fabsf(p2y - p1y) <= 1e-5f) {
-        if (lane == 0) set_edge(mask, dm, plane, round_to_ll(p1x), round_to_ll(p1y));
-        return;
+    const RasterLineDev rl(p1x, p1y, p2x, p2y);
+    for (int i = lane; i < rl.n; i += 32) {
+        long long x, y;
+        rl.at(i, x, y);
+        set_edge(mask, dm, plane, x, y);
     }
-    const float lvx = p2x - p1x, lvy = p2y - p1y;
-    float rx, ry;
-    rasterize_vector_dev(lvx, lvy, rx, ry);
-    if (rel_eq_zero(rx)) {
-        const int size = (int)(lvy / ry) + 1;
-        const LinSpacedDev ly(size, p1y, p2y);
-        const long long x = round_to_ll(p1x);
-        for (int i = lane; i < size; i += 32) set_edge(mask, dm, plane, x, round_to_ll(ly.at(i)));
-        return;
-    }
-    if (rel_eq_zero(ry)) {
-        const int size = (int)(lvx / rx) + 1;
-        const LinSpacedDev lx(size, p1x, p2x);
-        const long long y = round_to_ll(p1y);
-        for (int i = lane; i < size; i += 32) set_edge(mask, dm, plane, round_to_ll(lx.at(i)), y);
-        return;
-    }
-    const float a = lvx / rx, b = lvy / ry;
-    const int size = (int)((a < b) ? b : a) + 1;   // std::max(a, b)
-    const LinSpacedDev lx(size, p1x, p2x), ly(size, p1y, p2y);
-    for (int i = lane; i < size; i += 32) set_edge(mask, dm, plane, round_to_ll(lx.at(i)), round_to_ll(ly.at(i)));
 }
 
 

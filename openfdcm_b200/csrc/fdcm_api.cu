@@ -291,6 +291,14 @@ struct fdcm_dt3 {
     mutable int denom_kind = -1;
     mutable float denom_tau = 0.f;
     mutable DevBuf s_dense_keys, s_dense_rot;   // dense pose-grid search (records: s_rec / s_valid / s_hyp_off)
+    // match verification: the dilated edge mask of (cov_radius, cov_tol) for the map write cov_gen (0: none), its scratch and
+    // the standalone call's buffers; cov_ev is recorded after the dilation, which later calls on any stream wait on
+    uint64_t write_gen = 0;         // incremented by every write of the map (map_written)
+    mutable bool mask_fresh = false;   // the edge mask belongs to the current scene (a broadcast receives planes only)
+    mutable DevBuf cov_tmp, cov_dil, cov_io, cov_out;
+    mutable uint64_t cov_gen = 0;
+    mutable int cov_radius = -1, cov_tol = -1;
+    mutable cudaEvent_t cov_ev = nullptr;
     mutable float s_scene_min[2] = {0.f, 0.f}, s_scene_max[2] = {0.f, 0.f};   // bbox of the resident search scene
     mutable std::mutex host_tset_mutex;
     mutable fdcm_templates* host_tset = nullptr;   // reusable template set of fdcm_search_host
@@ -313,12 +321,14 @@ struct fdcm_dt3 {
         for (DevBuf* b : {&planes, &mask, &stack, &lines, &bins, &band_info, &band_spill, &integ_items, &s_scene, &s_sorted_len, &s_sorted_idx, &s_hyp_off, &s_rec,
                           &s_valid, &s_hyp, &s_counters, &s_topk_score, &s_topk_idx, &s_topk_out, &s_topk_n, &s_keys, &s_keys2, &s_idx,
                           &s_perm, &s_sort_tmp, &s_sel_keys, &s_sel_keys2, &s_sel_vals, &s_sel_vals2, &s_sel_surv, &s_sel_acc,
-                          &s_sel_tmp, &s_ref_state, &s_ref_keys, &s_ref_io, &s_denom, &s_dense_keys, &s_dense_rot})
+                          &s_sel_tmp, &s_ref_state, &s_ref_keys, &s_ref_io, &s_denom, &s_dense_keys, &s_dense_rot, &cov_tmp, &cov_dil,
+                          &cov_io, &cov_out})
             b->release();
         if (h_pinned) cudaFreeHost(h_pinned);
         if (ev_fork) cudaEventDestroy(ev_fork);
         if (ev_join) cudaEventDestroy(ev_join);
         if (ev_written) cudaEventDestroy(ev_written);
+        if (cov_ev) cudaEventDestroy(cov_ev);
         if (h_scene_stage) cudaFreeHost(h_scene_stage);
         if (scene_stage_ev) cudaEventDestroy(scene_stage_ev);
         destroy_host_tset();
@@ -343,6 +353,7 @@ static fdcm_status map_wait(const fdcm_dt3* m, cudaStream_t s) {
 static fdcm_status map_written(fdcm_dt3* m, cudaStream_t s) {
     if (!m->ev_written) CUDA_TRY(cudaEventCreateWithFlags(&m->ev_written, cudaEventDisableTiming));
     CUDA_TRY(cudaEventRecord(m->ev_written, s));
+    ++m->write_gen;
     return FDCM_OK;
 }
 
@@ -501,6 +512,7 @@ static fdcm_status build_integral_plan(fdcm_dt3* m, cudaStream_t s) {
 static fdcm_status prepare_and_upload(fdcm_dt3* m, const float* scene, int32_t n_lines, cudaStream_t s) {
     m->n_lines = n_lines;
     m->scene_bins.clear();
+    m->mask_fresh = false;   // until run_build_kernels rasterises this scene
     if (n_lines == 0) {   // dt3cpu.h:180-181: empty map, translation (0,0), size (0,0)
         m->s_scene_n = 0;
         m->s_sorted_n = 0;
@@ -622,6 +634,7 @@ static fdcm_status run_build_kernels(fdcm_dt3* m, cudaStream_t s) {
         KernelScope k("raster", 0.0, s);
         launch_raster(m->lines.as<float>(), m->bins.as<int32_t>(), m->n_lines, dm, m->mask.as<uint32_t>(), s);
     }
+    m->mask_fresh = true;
     const int dist = m->params.distance;
     bool fused_propagate = false;
     if (m->band_l1) {
@@ -1706,10 +1719,81 @@ static fdcm_status run_refine(const fdcm_dt3* m, const fdcm_templates* t, int32_
     return FDCM_OK;
 }
 
-// sel: distinct top-K (fdcm_search_select); ref: pose refinement of the top-K (fdcm_search_refine); nullptr when not asked
+// parameters of the match verification (fdcm_match_coverage and the coverage filter)
+static fdcm_status check_coverage(const fdcm_coverage_params* c) {
+    if (!c) return fail(FDCM_ERR_INVALID, "cov is null");
+    if (c->radius < 0 || c->radius > FDCM_COVERAGE_MAX_RADIUS)
+        return fail(FDCM_ERR_INVALID, "edge coverage: radius must be in 0.." + std::to_string(FDCM_COVERAGE_MAX_RADIUS));
+    if (c->bin_tolerance < 0 || c->bin_tolerance > 32) return fail(FDCM_ERR_INVALID, "edge coverage: bin_tolerance must be in 0..32");
+    if (!(c->min_coverage >= 0.f && c->min_coverage <= 1.f)) return fail(FDCM_ERR_INVALID, "edge coverage: min_coverage must be in [0, 1]");
+    return FDCM_OK;
+}
+
+// The dilated edge mask of (radius, bin_tolerance) for the map's current scene, queued on `s` unless the map holds it for
+// its last write already.  A map received by broadcast has planes but no edge mask of its scene: it is rasterised first
+// (the mask bytes only: the build's work counters behind them stay).  (m->search_mutex held, map_wait done)
+static fdcm_status coverage_mask(const fdcm_dt3* m, const fdcm_coverage_params* c, cudaStream_t s) {
+    const MapDims& dm = m->dm;
+    if (m->cov_gen != m->write_gen || m->cov_radius != c->radius || m->cov_tol != c->bin_tolerance) {
+        m->cov_gen = 0;
+        const size_t mask_bytes = (size_t)dm.D * dm.H * dm.wwords * sizeof(uint32_t);
+        if (!m->mask_fresh) {
+            CUDA_TRY(cudaMemsetAsync(m->mask.p, 0, mask_bytes, s));
+            KernelScope k("coverage_raster", 0.0, s);
+            launch_raster(m->lines.as<float>(), m->bins.as<int32_t>(), m->n_lines, dm, m->mask.as<uint32_t>(), s);
+            m->mask_fresh = true;
+        }
+        CUDA_TRY(m->cov_tmp.reserve(mask_bytes));
+        CUDA_TRY(m->cov_dil.reserve(mask_bytes));
+        {
+            KernelScope k("coverage_dilate", 4.0 * (double)mask_bytes, s, 2);   // planes pass + window pass
+            launch_coverage_dilate(m->mask.as<uint32_t>(), dm, c->radius, c->bin_tolerance, m->cov_tmp.as<uint32_t>(),
+                                   m->cov_dil.as<uint32_t>(), s);
+        }
+        CUDA_TRY(cudaGetLastError());
+        if (!m->cov_ev) CUDA_TRY(cudaEventCreateWithFlags(&m->cov_ev, cudaEventDisableTiming));
+        CUDA_TRY(cudaEventRecord(m->cov_ev, s));
+        m->cov_gen = m->write_gen;
+        m->cov_radius = c->radius;
+        m->cov_tol = c->bin_tolerance;
+    }
+    CUDA_TRY(cudaStreamWaitEvent(s, m->cov_ev, 0));   // a dilation queued by an earlier call on another stream
+    return FDCM_OK;
+}
+
+// coverage of n matches at d_rec: into d_cov (standalone) or, with d_valid, the filter of rule 6 on their valid flags
+static fdcm_status run_coverage(const fdcm_dt3* m, const fdcm_templates* t, int32_t tmpl_idx_base, const fdcm_coverage_params* c,
+                                const fdcm_match* d_rec, int64_t n, float* d_cov, uint8_t* d_valid, cudaStream_t s) {
+    if (n >= ((int64_t)1 << 34)) return fail(FDCM_ERR_INVALID, "edge coverage: at most 2^34 - 1 records");   // (one warp each)
+    if (fdcm_status st = coverage_mask(m, c, s)) return st;
+    CoverageLaunch cl;
+    cl.dil = m->cov_dil.as<uint32_t>();
+    cl.dm = m->dm;
+    cl.shift_x = m->shift[0];
+    cl.shift_y = m->shift[1];
+    cl.rec = d_rec;
+    cl.n = n;
+    cl.lines = t->lines.as<float4>();
+    cl.offsets = t->offs.as<int32_t>();
+    cl.n_tmpl = t->n_tmpl;
+    cl.tmpl_idx_base = tmpl_idx_base;
+    cl.coverage = d_cov;
+    cl.valid = d_valid;
+    cl.min_coverage = c->min_coverage;
+    {
+        KernelScope k("coverage_eval", 0.0, s);
+        launch_coverage_eval(cl, m->table_dev, s);
+    }
+    CUDA_TRY(cudaGetLastError());
+    return FDCM_OK;
+}
+
+// sel: distinct top-K (fdcm_search_select); ref: pose refinement of the top-K (fdcm_search_refine); cov: the coverage filter
+// before the selection (fdcm_search_verify, min_coverage > 0); nullptr when not asked
 static fdcm_status search_impl(const fdcm_dt3* m, const fdcm_templates* tc, const float* scene, int32_t n_scene,
                                const fdcm_search_params* p, fdcm_match* out, int64_t capacity, int64_t* n_out, fdcm_comm* comm,
-                               const fdcm_select_params* sel, const fdcm_refine_params* ref = nullptr) {
+                               const fdcm_select_params* sel, const fdcm_refine_params* ref = nullptr,
+                               const fdcm_coverage_params* cov = nullptr) {
     if (!m || !tc || !p || !n_out) return fail(FDCM_ERR_INVALID, "null argument");
     *n_out = 0;
     if (sel)
@@ -1831,6 +1915,8 @@ static fdcm_status search_impl(const fdcm_dt3* m, const fdcm_templates* tc, cons
         KernelScope k("search", 0.0, s);
         CUDA_TRY(launch_search(map_view(m), m->table_dev, tv, sv, sl, so, smem_optin, s));
     }
+    if (cov)
+        if (fdcm_status st = run_coverage(m, t, p->tmpl_idx_base, cov, so.rec, H, nullptr, so.valid, s)) return st;
 
     unsigned long long counters[3] = {0, 0, 0};
     fdcm_status result = FDCM_OK;
@@ -1912,6 +1998,20 @@ extern "C" fdcm_status fdcm_search_refine(const fdcm_dt3* m, const fdcm_template
     if (p->top_k < 1 || p->top_k > kRefineMaxMatches)
         return fail(FDCM_ERR_INVALID, "pose refinement: top_k must be in 1.." + std::to_string(kRefineMaxMatches));
     return search_impl(m, tc, scene, n_scene, p, out, capacity, n_out, nullptr, select, refine);
+}
+
+extern "C" fdcm_status fdcm_search_verify(const fdcm_dt3* m, const fdcm_templates* tc, const float* scene, int32_t n_scene,
+                                          const fdcm_search_params* p, const fdcm_select_params* select, const fdcm_refine_params* refine,
+                                          const fdcm_coverage_params* cov, fdcm_match* out, int64_t capacity, int64_t* n_out) {
+    if (fdcm_status st = check_coverage(cov)) return st;
+    if (!p) return fail(FDCM_ERR_INVALID, "null argument");
+    if (p->top_k < 1) return fail(FDCM_ERR_INVALID, "verified search: top_k must be >= 1");
+    if (refine) {
+        if (fdcm_status st = check_refine(refine)) return st;
+        if (p->top_k > kRefineMaxMatches)
+            return fail(FDCM_ERR_INVALID, "pose refinement: top_k must be in 1.." + std::to_string(kRefineMaxMatches));
+    }
+    return search_impl(m, tc, scene, n_scene, p, out, capacity, n_out, nullptr, select, refine, cov->min_coverage > 0.f ? cov : nullptr);
 }
 
 extern "C" fdcm_status fdcm_refine_matches(const fdcm_dt3* m, const fdcm_templates* tc, int32_t tmpl_idx_base, int32_t penalty_kind,
@@ -2016,9 +2116,11 @@ static DenseGrid dense_grid(const fdcm_dense_params* d, const float shift[2], in
     return DenseGrid{lx, ly, ((int)hi[0] - lx) / d->stride + 1, ((int)hi[1] - ly) / d->stride + 1};
 }
 
-extern "C" fdcm_status fdcm_search_dense(const fdcm_dt3* m, const fdcm_templates* tc, const fdcm_dense_params* dense, int32_t penalty_kind,
-                                         float penalty_tau, int32_t top_k, int32_t tmpl_idx_base, const fdcm_select_params* sel,
-                                         const fdcm_refine_params* ref, fdcm_match* out, int64_t capacity, int64_t* n_out) {
+// cov: the coverage filter of the records before the selection (fdcm_search_dense_verify, min_coverage > 0), or nullptr
+static fdcm_status dense_impl(const fdcm_dt3* m, const fdcm_templates* tc, const fdcm_dense_params* dense, int32_t penalty_kind,
+                              float penalty_tau, int32_t top_k, int32_t tmpl_idx_base, const fdcm_select_params* sel,
+                              const fdcm_refine_params* ref, const fdcm_coverage_params* cov, fdcm_match* out, int64_t capacity,
+                              int64_t* n_out) {
     if (!m || !tc || !n_out) return fail(FDCM_ERR_INVALID, "null argument");
     *n_out = 0;
     if (fdcm_status st = check_dense(dense)) return st;
@@ -2102,6 +2204,8 @@ extern "C" fdcm_status fdcm_search_dense(const fdcm_dt3* m, const fdcm_templates
         KernelScope k("dense_finish", (double)H * (8 + sizeof(fdcm_match) + 1), s);
         launch_dense_finish(map_view(m), dl, s);
     }
+    if (cov)
+        if (fdcm_status st = run_coverage(m, t, tmpl_idx_base, cov, dl.rec, H, nullptr, dl.valid, s)) return st;
     const int k = top_k;
     CUDA_TRY(m->s_topk_out.reserve((size_t)k * sizeof(fdcm_match)));
     CUDA_TRY(m->s_topk_n.reserve(4));
@@ -2126,6 +2230,59 @@ extern "C" fdcm_status fdcm_search_dense(const fdcm_dt3* m, const fdcm_templates
     const fdcm_status result = finish_topk(m, nullptr, k, s, nullptr, out, capacity, n_out);
     prof_resolve();
     return result;
+}
+
+extern "C" fdcm_status fdcm_search_dense(const fdcm_dt3* m, const fdcm_templates* tc, const fdcm_dense_params* dense, int32_t penalty_kind,
+                                         float penalty_tau, int32_t top_k, int32_t tmpl_idx_base, const fdcm_select_params* sel,
+                                         const fdcm_refine_params* ref, fdcm_match* out, int64_t capacity, int64_t* n_out) {
+    return dense_impl(m, tc, dense, penalty_kind, penalty_tau, top_k, tmpl_idx_base, sel, ref, nullptr, out, capacity, n_out);
+}
+
+extern "C" fdcm_status fdcm_search_dense_verify(const fdcm_dt3* m, const fdcm_templates* tc, const fdcm_dense_params* dense,
+                                                int32_t penalty_kind, float penalty_tau, int32_t top_k, int32_t tmpl_idx_base,
+                                                const fdcm_select_params* sel, const fdcm_refine_params* ref, const fdcm_coverage_params* cov,
+                                                fdcm_match* out, int64_t capacity, int64_t* n_out) {
+    if (fdcm_status st = check_coverage(cov)) return st;
+    return dense_impl(m, tc, dense, penalty_kind, penalty_tau, top_k, tmpl_idx_base, sel, ref, cov->min_coverage > 0.f ? cov : nullptr, out,
+                      capacity, n_out);
+}
+
+// =============================================================================================
+// match verification: edge coverage of host matches (rules in include/fdcm_b200.h)
+// =============================================================================================
+extern "C" fdcm_status fdcm_match_coverage(const fdcm_dt3* m, const fdcm_templates* tc, int32_t tmpl_idx_base, const fdcm_coverage_params* cov,
+                                           const fdcm_match* in, int64_t n, float* coverage) {
+    if (fdcm_status st = check_coverage(cov)) return st;
+    if (!m || !tc || n < 0) return fail(FDCM_ERR_INVALID, "bad argument");
+    if (n == 0) return FDCM_OK;
+    if (!in || !coverage) return fail(FDCM_ERR_INVALID, "null argument");
+    if (tc->device != m->device) return fail(FDCM_ERR_INVALID, "templates and feature map live on different devices");
+    if (m->stage != 0) return fail(FDCM_ERR_INVALID, "feature map was built with a debug stage");
+    for (int64_t i = 0; i < n; ++i) {
+        const int64_t t = (int64_t)in[i].tmpl_idx - tmpl_idx_base;
+        if (t < 0 || t >= tc->n_tmpl)
+            return fail(FDCM_ERR_OUT_OF_RANGE, "match " + std::to_string(i) + ": tmpl_idx " + std::to_string(in[i].tmpl_idx) +
+                                                   " outside the template set");
+    }
+    fdcm_templates* t = const_cast<fdcm_templates*>(tc);
+    std::lock_guard<std::mutex> lk(m->search_mutex);
+    if (m->dm.D == 0 || m->dm.W == 0 || m->dm.H == 0) {   // empty map (rule 2)
+        for (int64_t i = 0; i < n; ++i) coverage[i] = NAN;
+        return FDCM_OK;
+    }
+    CUDA_TRY(cudaSetDevice(m->device));
+    cudaStream_t s;
+    if (fdcm_status st = get_stream(m->device, &s)) return st;
+    if (fdcm_status st = map_wait(m, s)) return st;
+    if (fdcm_status st = templates_ready(t, s)) return st;
+    CUDA_TRY(m->cov_io.reserve((size_t)n * sizeof(fdcm_match)));
+    CUDA_TRY(m->cov_out.reserve((size_t)n * 4));
+    CUDA_TRY(cudaMemcpyAsync(m->cov_io.p, in, (size_t)n * sizeof(fdcm_match), cudaMemcpyHostToDevice, s));
+    if (fdcm_status st = run_coverage(m, t, tmpl_idx_base, cov, m->cov_io.as<fdcm_match>(), n, m->cov_out.as<float>(), nullptr, s)) return st;
+    CUDA_TRY(cudaMemcpyAsync(coverage, m->cov_out.p, (size_t)n * 4, cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(cudaStreamSynchronize(s));
+    prof_resolve();
+    return FDCM_OK;
 }
 
 extern "C" fdcm_status fdcm_dense_poses(const fdcm_dense_params* dense, const float anchor[2], const float shift[2], int32_t width,

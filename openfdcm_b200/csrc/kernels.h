@@ -233,6 +233,26 @@ cudaError_t launch_dense_eval(const MapView& map, const SlopeTableDev& table, co
 // keys -> records and valid flags (the winning pose recomputed from its grid index, the penalty applied)
 void launch_dense_finish(const MapView& map, const DenseLaunch& p, cudaStream_t s);
 
+// ---- coverage_kernels.cu: match verification (fdcm_match_coverage / the coverage filter; rules in include/fdcm_b200.h) ----
+// the dilated edge mask of (radius, tol), the mask's layout; d_tmp: scratch of the mask's size
+void launch_coverage_dilate(const uint32_t* d_mask, const MapDims& dm, int radius, int tol, uint32_t* d_tmp, uint32_t* d_dil,
+                            cudaStream_t s);
+struct CoverageLaunch {
+    const uint32_t* dil;         // dilated mask [D][H][wwords]
+    MapDims dm;
+    float shift_x, shift_y;
+    const fdcm_match* rec;       // n matches
+    int64_t n;
+    const float4* lines;         // template set
+    const int32_t* offsets;
+    int32_t n_tmpl, tmpl_idx_base;
+    float* coverage;             // standalone: n coverages (valid == nullptr)
+    uint8_t* valid;              // filter: the records' flags, cleared below min_coverage (coverage == nullptr)
+    float min_coverage;
+};
+// one warp per match
+void launch_coverage_eval(const CoverageLaunch& p, const SlopeTableDev& table, cudaStream_t s);
+
 void launch_evaluate(const MapView& map, const SlopeTableDev& table, const float4* d_lines, const int32_t* d_toff,
                      const float2* d_transl, const int32_t* d_troff, const int32_t* d_owner, int64_t n_scores,
                      float* d_scores, cudaStream_t s);

@@ -275,20 +275,23 @@ PYBIND11_MODULE(_openfdcm_cuda, m) {
     m.def("search_topk",
           [](const Dt3Cuda& featuremap, const std::vector<LinesIn>& templates, const LinesIn& scene, const DefaultSearch& searcher,
              const BatchOptimize& optimizer, const ExponentialPenalty& penalty, int k, const std::optional<DistinctMatches>& select,
-             const std::optional<PoseRefinement>& refine) {
+             const std::optional<PoseRefinement>& refine, const std::optional<EdgeCoverage>& verify) {
               const auto t = to_templates(templates);
               const auto s = to_lines(scene);
               py::gil_scoped_release release;
+              if (verify)
+                  return searchTopK(searcher, optimizer, penalty, featuremap, t, s, k, select ? &*select : nullptr, refine ? &*refine : nullptr,
+                                    *verify);
               if (refine && select) return searchTopK(searcher, optimizer, penalty, featuremap, t, s, k, *select, *refine);
               if (refine) return searchTopK(searcher, optimizer, penalty, featuremap, t, s, k, *refine);
               if (select) return searchTopK(searcher, optimizer, penalty, featuremap, t, s, k, *select);
               return searchTopK(searcher, optimizer, penalty, featuremap, t, s, k);
           },
           "featuremap"_a, "templates"_a, "scene"_a, "searcher"_a, "optimizer"_a, "penalty"_a, "k"_a = 10, py::kw_only(), "select"_a = py::none(),
-          "refine"_a = py::none(),
+          "refine"_a = py::none(), "verify"_a = py::none(),
           "Fused search -> penalize -> top-k on the device (ascending score); select: DistinctMatches for the distinct top-k; "
           "refine: PoseRefinement of the selected matches (not re-sorted; it minimises the score, which was measured to increase the "
-          "error against known poses)");
+          "error against known poses); verify: EdgeCoverage whose min_coverage > 0 drops matches of lower coverage before the selection");
 
     m.def("refine_matches",
           [](const Dt3Cuda& featuremap, const std::vector<LinesIn>& templates, const std::vector<Match>& matches, const PoseRefinement& refine,
@@ -327,14 +330,40 @@ PYBIND11_MODULE(_openfdcm_cuda, m) {
 
     m.def("search_dense",
           [](const Dt3Cuda& featuremap, const std::vector<LinesIn>& templates, const DenseSearch& dense, const ExponentialPenalty& penalty, int k,
-             const std::optional<DistinctMatches>& select, const std::optional<PoseRefinement>& refine) {
+             const std::optional<DistinctMatches>& select, const std::optional<PoseRefinement>& refine,
+             const std::optional<EdgeCoverage>& verify) {
               const auto t = to_templates(templates);
               py::gil_scoped_release release;
+              if (verify) return searchDense(featuremap, t, dense, penalty, k, select ? &*select : nullptr, refine ? &*refine : nullptr, *verify);
               return searchDense(featuremap, t, dense, penalty, k, select ? &*select : nullptr, refine ? &*refine : nullptr);
           },
           "featuremap"_a, "templates"_a, "dense"_a, "penalty"_a, "k"_a = 10, py::kw_only(), "select"_a = py::none(), "refine"_a = py::none(),
+          "verify"_a = py::none(),
           "Dense pose-grid search on the device: the best pose of every (template, rotation, cell), then the top-k (ascending score) "
-          "or with select the distinct top-k, then with refine the pose refinement of those");
+          "or with select the distinct top-k, then with refine the pose refinement of those; verify: EdgeCoverage whose "
+          "min_coverage > 0 drops records of lower coverage before the selection");
+
+    py::class_<EdgeCoverage>(m, "EdgeCoverage")
+        .def(py::init([](int radius, int bin_tolerance, float min_coverage) { return EdgeCoverage{radius, bin_tolerance, min_coverage}; }),
+             "radius"_a = 2, "bin_tolerance"_a = 1, "min_coverage"_a = 0.f)
+        .def_readwrite("radius", &EdgeCoverage::radius)
+        .def_readwrite("bin_tolerance", &EdgeCoverage::binTolerance)
+        .def_readwrite("min_coverage", &EdgeCoverage::minCoverage)
+        .def("__repr__", [](const EdgeCoverage& a) {
+            return "<EdgeCoverage: radius=" + std::to_string(a.radius) + ", bin_tolerance=" + std::to_string(a.binTolerance) +
+                   ", min_coverage=" + std::to_string(a.minCoverage) + ">";
+        });
+
+    m.def("match_coverage",
+          [](const Dt3Cuda& featuremap, const std::vector<LinesIn>& templates, const std::vector<Match>& matches,
+             const std::optional<EdgeCoverage>& coverage) {
+              const auto t = to_templates(templates);
+              py::gil_scoped_release release;
+              return matchCoverage(featuremap, t, matches, coverage ? *coverage : EdgeCoverage{});
+          },
+          "featuremap"_a, "templates"_a, "matches"_a, "coverage"_a = py::none(),
+          "Edge coverage of every match (entry i for matches[i]): the fraction of the posed template's raster samples with a scene "
+          "edge pixel of similar orientation nearby; NaN where the posed template leaves the map");
 
     m.def("penalize",
           [](const PenaltyStrategy& penalty, const std::vector<Match>& matches, const std::vector<float>& templatelengths) {
