@@ -357,6 +357,76 @@ fdcm_status fdcm_search_dense_verify(const fdcm_dt3* map, const fdcm_templates* 
                                      const fdcm_select_params* select, const fdcm_refine_params* refine,
                                      const fdcm_coverage_params* cov, fdcm_match* out, int64_t capacity, int64_t* n_out);
 
+/* ---- pose fit: point-to-line least squares against the scene lines (beyond the reference) --------------------------
+ * A search match puts one template line on one scene line, the dense grid is off by up to stride / 2 px and rot_step / 2
+ * rad, and refinement minimises the DT3 score, an integer-pixel, binned-orientation cost that has no minimum at the true
+ * pose below a pixel.  The fit moves each match to the pose that best explains the scene's line segments: a few
+ * Gauss-Newton iterations of oriented point-to-line least squares against the build scene's lines, which keep their
+ * sub-pixel end points.  It needs scene lines within max_distance of the posed template, uses no robust loss beyond that
+ * gate, and does not re-rank or re-select: two matches may converge on one instance.
+ * Rules, in IEEE double without contraction (no transcendental function: a float64 model reproduces every bit).  A match
+ * with template t = tmpl_idx - tmpl_idx_base and float32 transform T, on a map of W x H with scene translation shift, D
+ * planes, and scene lines S_j = (A_j, B_j) (the build scene plus shift, float32, as the build stores them) with bins b_j
+ * (fdcm_dt3_scene_bins):
+ *   1. Pose state.  M = (m0 m1; m3 m4) = (T0 T1; T3 T4) and e = ((double)T2 + shift_x, (double)T5 + shift_y).  Its float32
+ *      rounding is F = ((float)m0, (float)m1, (float)(ex - shift_x), (float)m3, (float)m4, (float)(ey - shift_y)); before the
+ *      first accepted update F is T itself.  Rotation centre c = M a + e: cx = (m0*ax + m1*ay) + ex, cy likewise, with the
+ *      anchor a of t (fdcm_template_anchors).
+ *   2. Samples, in the template frame (fdcm_fit_samples): a line (x1, y1, x2, y2) of len = sqrtf(dx*dx + dy*dy) > 0 (float32)
+ *      has n = max(2, (int)ceilf(len / sample_step) + 1) samples s_i = x1 + (x2 - x1) * ((double)i / (n - 1)) (y likewise),
+ *      i = 0..n-1; a line of length 0 (or NaN) has none.  rho = sqrt of the largest (sx - ax)^2 + (sy - ay)^2.
+ *   3. Correspondence of a sample of line q at the pose: p = M s + e (px = (m0*sx + m1*sy) + ex).  b = the slope-table bin of
+ *      line q posed by F (refinement rule 4, float32).  Candidates: the scene lines with min(|b_j - b|, D - |b_j - b|) <=
+ *      bin_tolerance and |B - A|^2 > 0.  For each, u = clamp(((px - Ax)*dx + (py - Ay)*dy) / (dx*dx + dy*dy), 0, 1) with
+ *      (dx, dy) = B - A, q = A + u (dx, dy), d2 = ex*ex + ey*ey for (ex, ey) = p - q; taken iff d2 <= max_distance^2 (double).
+ *      The least (d2, j) wins.  Residual r = nx*(px - Ax) + ny*(py - Ay), n = (-dy / l, dx / l), l = sqrt(dx*dx + dy*dy).
+ *   4. Normal equations.  J = (nx, ny, jt), jt = ny*(px - cx) - nx*(py - cy).  Sums, in this order per sample: A00 = nx*nx,
+ *      A01 = nx*ny, A02 = nx*jt, A11 = ny*ny, A12 = ny*jt, A22 = jt*jt, g0 = nx*r, g1 = ny*r, g2 = jt*r, rr = r*r.  Order: lane
+ *      i mod 32 takes sample i of a line, lines in order; each lane adds its terms in that order to sums starting at 0.0, then
+ *      v = v + v[lane ^ o] for o = 16, 8, 4, 2, 1 (every lane ends with the same values).  Solve (A + lambda I) delta = -g,
+ *      lambda = 1e-9 * ((A00 + A11) + A22), by Cholesky: l00 = sqrt(B00), l10 = A01 / l00, l20 = A02 / l00,
+ *      l11 = sqrt(B11 - l10*l10), l21 = (A12 - l20*l10) / l11, l22 = sqrt((B22 - l20*l20) - l21*l21), where B = A + lambda I;
+ *      it fails when a radicand is not > 0.  y0 = -g0 / l00, y1 = (-g1 - l10*y0) / l11, y2 = ((-g2 - l20*y0) - l21*y1) / l22;
+ *      delta = (dx, dy, dth): dth = y2 / l22, dy = (y1 - l21*dth) / l11, dx = ((y0 - l10*dy) - l20*dth) / l00.
+ *   5. Update (half-angle form, no cos / sin).  tau = dth * 0.5, k = 1 + tau*tau, cr = (1 - tau*tau) / k, sr = (2*tau) / k;
+ *      M' = (cr*m0 - sr*m3, cr*m1 - sr*m4; sr*m0 + cr*m3, sr*m1 + cr*m4), ux = ex - cx, uy = ey - cy,
+ *      e' = (((cr*ux - sr*uy) + cx) + dx, ((sr*ux + cr*uy) + cy) + dy).  Iteration k = 1..iterations: correspondences at the
+ *      pose; stop if fewer than min_inliers; solve, stop if it fails; stop (keeping the pose) if F of the update is invalid
+ *      (refinement rule 4: a NaN, or a posed end point outside [0, W-1] x [0, H-1]); accept it; stop if
+ *      max(|dx|, |dy|, |dth| * rho) <= tolerance.
+ *   6. Result.  tmpl_idx unchanged; transform F of the final pose; score evaluate<Dt3Cpu> at F (refinement rule 4), divided
+ *      by the search's penalty denominator of t when a penalty is given.  Stats: n_samples (rule 2), n_inliers and
+ *      rms = (float)sqrt(rr / n_inliers) of the correspondences at F (NaN without inliers), iterations = accepted updates.
+ *      An invalid input (an empty template, T invalid under refinement rule 4, an empty map) comes back with its transform,
+ *      score NaN and stats {0, 0, 0, NaN}.  A fit never makes a valid match invalid.  Output i is the fit of input i.
+ * Invalid parameters fail with FDCM_ERR_INVALID before any device work: iterations outside 1..100, max_distance outside
+ * (0, FDCM_FIT_MAX_DISTANCE], sample_step not finite or < 0.5, bin_tolerance outside 0..32, tolerance not finite or < 0,
+ * min_inliers < 3; a tmpl_idx - tmpl_idx_base outside the template set fails with FDCM_ERR_OUT_OF_RANGE.
+ * Cost: once per (map write, max_distance) a grid of 16-px cells listing the scene lines in reach of each cell; per match
+ * and iteration, every sample scans the lines of its cell.  The defaults are a starting point, not tuned values. */
+#define FDCM_FIT_MAX_DISTANCE 16
+typedef struct fdcm_fit_params {         /* 24 bytes */
+    int32_t iterations;         /* 1..100: Gauss-Newton iterations at most (default 10) */
+    float max_distance;         /* (0, FDCM_FIT_MAX_DISTANCE]: correspondence gate in pixels (default 3) */
+    float sample_step;          /* >= 0.5: template-frame pixels between samples of a line (default 2) */
+    int32_t bin_tolerance;      /* 0..32: orientation planes on either side of the posed line's (circular; default 1) */
+    float tolerance;            /* >= 0: stop when the step moves no sample more than this, in pixels (default 1e-3) */
+    int32_t min_inliers;        /* >= 3: stop with fewer correspondences (default 6) */
+} fdcm_fit_params;
+typedef struct fdcm_fit_stats {          /* 16 bytes */
+    int32_t n_samples;
+    int32_t n_inliers;          /* correspondences at the returned pose */
+    int32_t iterations;         /* accepted updates */
+    float rms;                  /* root mean square residual of those correspondences, pixels */
+} fdcm_fit_stats;
+/* fit n host matches (any source); out: n records (may be in); stats: n entries or NULL; n == 0 is no error */
+fdcm_status fdcm_fit_matches(const fdcm_dt3* map, const fdcm_templates* templates, int32_t tmpl_idx_base, int32_t penalty_kind,
+                             float penalty_tau, const fdcm_fit_params* fit, const fdcm_match* in, int64_t n, fdcm_match* out,
+                             fdcm_fit_stats* stats);
+/* the samples of rule 2 of n_lines template lines, (x, y) pairs in line order; *n_out = the number of samples
+ * (FDCM_ERR_CAPACITY when it exceeds capacity); host-only parity hook */
+fdcm_status fdcm_fit_samples(const float* tmpl_xyxy, int32_t n_lines, float sample_step, double* out_xy, int64_t capacity, int64_t* n_out);
+
 /* optimize(optimizer, templates, alignments, featuremap) (matching/optimizestrategy.h:62-64; BatchOptimize:
  * batchoptimize.cpp:6-123, batch_size == 0: DefaultOptimize, defaultoptimize.cpp:6-93).  The templates are used
  * as given (already aligned); alignments: n_tmpl (x,y) pairs.  Outputs per template: has_value (0 = nullopt),

@@ -472,6 +472,62 @@ inline std::vector<Match> searchDense(const Dt3Cuda& fm, const std::vector<LineA
     return detail::search_dense(fm, templates, dense, FDCM_PENALTY_EXPONENTIAL, pen.tau, k, select, refine, &c);
 }
 
+// pose fit (beyond the reference; rules of fdcm_fit_matches): per match, up to `iterations` Gauss-Newton steps of oriented
+// point-to-line least squares of the template's samples against the build scene's line segments (nearest scene line within
+// maxDistance pixels on an orientation plane within binTolerance planes).  It needs scene lines near the pose, uses no
+// robust loss beyond that gate and does not re-rank; the defaults are a starting point, not tuned.
+struct PoseFit {
+    int iterations{10};
+    float maxDistance{3.f};
+    float sampleStep{2.f};
+    int binTolerance{1};
+    float tolerance{1e-3f};
+    int minInliers{6};
+};
+struct FitStats {
+    int nSamples;
+    int nInliers;     // correspondences at the returned pose
+    int iterations;   // accepted updates
+    float rms;        // root mean square residual of those correspondences (NaN without any)
+};
+namespace detail {
+inline std::vector<Match> fit_matches(const Dt3Cuda& fm, const std::vector<LineArray>& templates, const std::vector<Match>& matches,
+                                      const PoseFit& fit, int penalty_kind, float tau, std::vector<FitStats>* stats) {
+    std::vector<float> flat;
+    std::vector<int32_t> off;
+    pack(templates, flat, off);
+    fdcm_templates* ts = nullptr;
+    check(fdcm_templates_create(flat.data(), off.data(), (int32_t)templates.size(), fm.info().device, &ts));
+    const std::unique_ptr<fdcm_templates, fdcm_status (*)(fdcm_templates*)> owner(ts, fdcm_templates_release);
+    std::vector<fdcm_match> rec(matches.size());
+    for (size_t i = 0; i < matches.size(); ++i) {
+        rec[i].tmpl_idx = matches[i].tmplIdx;
+        rec[i].score = matches[i].score;
+        for (int c = 0; c < 6; ++c) rec[i].transform[c] = matches[i].transform[(size_t)c];
+    }
+    const fdcm_fit_params p{fit.iterations, fit.maxDistance, fit.sampleStep, fit.binTolerance, fit.tolerance, fit.minInliers};
+    std::vector<fdcm_match> out(matches.size());
+    std::vector<fdcm_fit_stats> st(stats ? matches.size() : 0);
+    check(fdcm_fit_matches(fm.handle(), ts, 0, penalty_kind, tau, &p, rec.data(), (int64_t)rec.size(), out.data(), stats ? st.data() : nullptr));
+    if (stats) {
+        stats->resize(matches.size());
+        for (size_t i = 0; i < st.size(); ++i) (*stats)[i] = FitStats{st[i].n_samples, st[i].n_inliers, st[i].iterations, st[i].rms};
+    }
+    return to_matches(out, (int64_t)out.size());
+}
+}   // namespace detail
+// fit of every match (tmplIdx indexes `templates`), entry i for matches[i], raw evaluate<Dt3Cpu> score at the fitted pose;
+// stats (optional): one FitStats per match
+inline std::vector<Match> fitMatches(const Dt3Cuda& fm, const std::vector<LineArray>& templates, const std::vector<Match>& matches,
+                                     const PoseFit& fit = PoseFit{}, std::vector<FitStats>* stats = nullptr) {
+    return detail::fit_matches(fm, templates, matches, fit, FDCM_PENALTY_NONE, 0.f, stats);
+}
+// the same, scored with the search's exponential penalty
+inline std::vector<Match> fitMatches(const Dt3Cuda& fm, const std::vector<LineArray>& templates, const std::vector<Match>& matches,
+                                     const ExponentialPenalty& pen, const PoseFit& fit = PoseFit{}, std::vector<FitStats>* stats = nullptr) {
+    return detail::fit_matches(fm, templates, matches, fit, FDCM_PENALTY_EXPONENTIAL, pen.tau, stats);
+}
+
 // ---- PenaltyStrategy concept, template lengths, sort ----------------------------------------------
 inline std::vector<float> getTemplateLengths(const std::vector<LineArray>& templates) {   // core/math.h:319-324
     std::vector<float> flat, len(templates.size());

@@ -17,15 +17,16 @@ import numpy as np
 
 from . import _lib
 from .io import read, write
-from ._lib import MATCH_DTYPE, FdcmError, check, lib, ptr
+from ._lib import FIT_STATS_DTYPE, MATCH_DTYPE, FdcmError, check, lib, ptr
 
 __all__ = [
     "distance", "Dt3CudaParameters", "Dt3Cuda", "build_cuda_featuremap", "ThreadPool", "DefaultSearch", "ConcentricRangeStrategy",
     "BatchOptimize", "DefaultOptimize", "DefaultMatch", "DefaultPenalty", "ExponentialPenalty", "Match",
-    "TemplateSet", "SceneBatch", "DistinctMatches", "PoseRefinement", "DenseSearch", "EdgeCoverage", "search", "search_topk",
-    "search_dense", "refine_matches", "match_coverage", "penalize", "get_template_lengths",
+    "TemplateSet", "SceneBatch", "DistinctMatches", "PoseRefinement", "DenseSearch", "EdgeCoverage", "PoseFit", "search", "search_topk",
+    "search_dense", "refine_matches", "match_coverage", "fit_matches", "penalize", "get_template_lengths",
     "get_template_anchors", "sort_matches", "evaluate",
     "minmax_translation", "get_feature_size", "establish_search_strategy", "optimize", "read", "write", "FdcmError", "MATCH_DTYPE",
+    "FIT_STATS_DTYPE",
 ]
 
 
@@ -399,6 +400,31 @@ class EdgeCoverage:
         return f"<EdgeCoverage: radius={self.radius}, bin_tolerance={self.bin_tolerance}, min_coverage={self.min_coverage}>"
 
 
+class PoseFit:
+    """Pose fit (beyond the reference): per match, up to `iterations` Gauss-Newton steps of oriented point-to-line least
+    squares of the template's samples (every `sample_step` template pixels) against the build scene's line segments, each
+    sample taking the nearest scene line within `max_distance` pixels whose orientation plane is within `bin_tolerance`
+    planes of the posed line's; stops when a step moves no sample more than `tolerance` pixels, with fewer than
+    `min_inliers` correspondences, or when the next pose would leave the map.  It needs scene lines near the pose, uses no
+    robust loss beyond that gate and does not re-rank.  The defaults are a starting point, not tuned.  Exact rules:
+    include/fdcm_b200.h."""
+
+    def __init__(self, iterations=10, max_distance=3.0, sample_step=2.0, bin_tolerance=1, tolerance=1e-3, min_inliers=6):
+        self.iterations = int(iterations)
+        self.max_distance = float(max_distance)
+        self.sample_step = float(sample_step)
+        self.bin_tolerance = int(bin_tolerance)
+        self.tolerance = float(tolerance)
+        self.min_inliers = int(min_inliers)
+
+    def _params(self):
+        return _lib.FitParams(self.iterations, self.max_distance, self.sample_step, self.bin_tolerance, self.tolerance, self.min_inliers)
+
+    def __repr__(self):
+        return (f"<PoseFit: iterations={self.iterations}, max_distance={self.max_distance}, sample_step={self.sample_step}, "
+                f"bin_tolerance={self.bin_tolerance}, tolerance={self.tolerance}, min_inliers={self.min_inliers}>")
+
+
 def _search_raw(featuremap, templates, scene, searcher, optimizer, penalty=None, top_k=0, tmpl_idx_base=0, select=None, refine=None,
                 verify=None):
     if not isinstance(featuremap, Dt3Cuda):
@@ -442,13 +468,18 @@ def search(matcher, searcher, optimizer, featuremap, templates, scene):
 
 
 def search_topk(featuremap, templates, scene, searcher, optimizer, penalty=None, k=10, tmpl_idx_base=0, *, select=None, refine=None,
-                verify=None):
+                verify=None, fit=None):
     """Fused search -> penalize -> top-k on the device; returns a MATCH_DTYPE record array (ascending score).
     select: a DistinctMatches for the distinct top-k (the kept matches in acceptance order, also ascending score).
     refine: a PoseRefinement applied to the selected matches on the device, equal to refine_matches of the unrefined
     result (same order: re-rank with sort_matches); it lowers the score, not the pose error (see PoseRefinement).
-    verify: an EdgeCoverage whose min_coverage > 0 drops every match of lower (or NaN) coverage before the selection."""
-    return _search_raw(featuremap, templates, scene, searcher, optimizer, penalty, k, tmpl_idx_base, select, refine, verify).copy()
+    verify: an EdgeCoverage whose min_coverage > 0 drops every match of lower (or NaN) coverage before the selection.
+    fit: a PoseFit applied last (after select / refine / verify), equal to fit_matches of the unfitted result; the fitted
+    list is not re-selected or re-sorted, so two distinct matches may converge on one instance."""
+    if fit is not None and not isinstance(templates, TemplateSet) and isinstance(featuremap, Dt3Cuda):
+        templates = TemplateSet(templates, featuremap.device)
+    out = _search_raw(featuremap, templates, scene, searcher, optimizer, penalty, k, tmpl_idx_base, select, refine, verify).copy()
+    return out if fit is None else fit_matches(featuremap, templates, out, fit, penalty, tmpl_idx_base)
 
 
 def refine_matches(featuremap, templates, matches, refine, penalty=None, tmpl_idx_base=0):
@@ -469,11 +500,13 @@ def refine_matches(featuremap, templates, matches, refine, penalty=None, tmpl_id
     return out[: rec.shape[0]].copy()
 
 
-def search_dense(featuremap, templates, dense, penalty=None, k=10, tmpl_idx_base=0, *, select=None, refine=None, verify=None):
+def search_dense(featuremap, templates, dense, penalty=None, k=10, tmpl_idx_base=0, *, select=None, refine=None, verify=None, fit=None):
     """Dense pose-grid search on the device (see DenseSearch): the best pose of every (template, rotation, cell), then the
     top-k in ascending (score, record) order, or with select (a DistinctMatches) the distinct top-k, then with refine (a
     PoseRefinement) the refinement of those, equal to refine_matches of the unrefined result.  Returns a MATCH_DTYPE array.
-    verify: an EdgeCoverage whose min_coverage > 0 drops every record of lower (or NaN) coverage before the selection."""
+    verify: an EdgeCoverage whose min_coverage > 0 drops every record of lower (or NaN) coverage before the selection.
+    fit: a PoseFit applied last, equal to fit_matches of the unfitted result; the fitted list is not re-selected or
+    re-sorted, so two distinct matches may converge on one instance."""
     if not isinstance(featuremap, Dt3Cuda):
         raise TypeError("search_dense needs a Dt3Cuda feature map (build_cuda_featuremap)")
     tset = templates if isinstance(templates, TemplateSet) else TemplateSet(templates, featuremap.device)
@@ -488,7 +521,8 @@ def search_dense(featuremap, templates, dense, penalty=None, k=10, tmpl_idx_base
     else:
         check(lib().fdcm_search_dense_verify(featuremap._h, tset._h, C.byref(dense._params()), pen_kind, pen_tau, int(k), int(tmpl_idx_base),
                                              sp, rp, C.byref(verify._params()), ptr(out), out.shape[0], C.byref(n)))
-    return out[: n.value].copy()
+    out = out[: n.value].copy()
+    return out if fit is None else fit_matches(featuremap, tset, out, fit, penalty, tmpl_idx_base)
 
 
 def match_coverage(featuremap, templates, matches, coverage=None, tmpl_idx_base=0):
@@ -505,6 +539,28 @@ def match_coverage(featuremap, templates, matches, coverage=None, tmpl_idx_base=
         raise IndexError(lib().fdcm_last_error().decode())
     check(st)
     return out[: rec.shape[0]].copy()
+
+
+def fit_matches(featuremap, templates, matches, fit=None, penalty=None, tmpl_idx_base=0, return_stats=False):
+    """Pose fit (see PoseFit; None: the defaults) of any match list against a feature map and a template set (list or
+    TemplateSet): a MATCH_DTYPE array, entry i fitting matches[i], scored like search_topk with the same penalty; a match
+    whose pose is invalid comes back unchanged with score NaN.  The list is not re-sorted or re-selected: two matches may
+    converge on one instance.  return_stats: also a FIT_STATS_DTYPE array (n_samples, n_inliers, iterations, rms)."""
+    if not isinstance(featuremap, Dt3Cuda):
+        raise TypeError("fit_matches needs a Dt3Cuda feature map (build_cuda_featuremap)")
+    fit = PoseFit() if fit is None else fit
+    tset = templates if isinstance(templates, TemplateSet) else TemplateSet(templates, featuremap.device)
+    rec = _to_records(matches)
+    out = np.zeros(max(rec.shape[0], 1), MATCH_DTYPE)
+    stats = np.zeros(max(rec.shape[0], 1), FIT_STATS_DTYPE) if return_stats else None
+    st = lib().fdcm_fit_matches(featuremap._h, tset._h, int(tmpl_idx_base), 0 if penalty is None else penalty.kind,
+                                0.0 if penalty is None else float(penalty.tau), C.byref(fit._params()), ptr(rec), rec.shape[0], ptr(out),
+                                ptr(stats))
+    if st == _lib.FDCM_ERR_OUT_OF_RANGE:
+        raise IndexError(lib().fdcm_last_error().decode())
+    check(st)
+    out = out[: rec.shape[0]].copy()
+    return (out, stats[: rec.shape[0]].copy()) if return_stats else out
 
 
 def search_all(featuremap, templates, scene, searcher, optimizer, penalty=None, tmpl_idx_base=0):

@@ -45,6 +45,15 @@ class CoverageParams(C.Structure):
     _fields_ = [("radius", C.c_int32), ("bin_tolerance", C.c_int32), ("min_coverage", C.c_float)]
 
 
+class FitParams(C.Structure):
+    _fields_ = [("iterations", C.c_int32), ("max_distance", C.c_float), ("sample_step", C.c_float), ("bin_tolerance", C.c_int32),
+                ("tolerance", C.c_float), ("min_inliers", C.c_int32)]
+
+
+FIT_STATS_DTYPE = np.dtype([("n_samples", "<i4"), ("n_inliers", "<i4"), ("iterations", "<i4"), ("rms", "<f4")])
+assert FIT_STATS_DTYPE.itemsize == 16
+
+
 class Dt3Info(C.Structure):
     _fields_ = [("depth", C.c_int32), ("width", C.c_int32), ("height", C.c_int32), ("pitch", C.c_int32),
                 ("scene_translation", C.c_float * 2), ("distance", C.c_int32), ("device", C.c_int32),
@@ -99,6 +108,8 @@ SIGNATURES = {
                                      C.POINTER(CoverageParams), _P, C.c_int64, C.POINTER(C.c_int64)]),
     "fdcm_search_dense_verify": (C.c_int, [_P, _P, C.POINTER(DenseParams), C.c_int32, C.c_float, C.c_int32, C.c_int32, C.POINTER(SelectParams),
                                            C.POINTER(RefineParams), C.POINTER(CoverageParams), _P, C.c_int64, C.POINTER(C.c_int64)]),
+    "fdcm_fit_matches": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_float, C.POINTER(FitParams), _P, C.c_int64, _P, _P]),
+    "fdcm_fit_samples": (C.c_int, [_P, C.c_int32, C.c_float, _P, C.c_int64, C.POINTER(C.c_int64)]),
     "fdcm_optimize": (C.c_int, [_P, _P, _P, C.c_int32, _P, C.c_int32, _P, _P, _P]),
     "fdcm_search_host": (C.c_int, [_P, _P, _P, C.c_int32, _P, C.c_int32, C.POINTER(SearchParams), _P, C.c_int64,
                                    C.POINTER(C.c_int64)]),

@@ -133,4 +133,55 @@ __device__ __forceinline__ int bin_of_slope_dev(const SlopeTableDev& t, float sl
     return t.piece_bin[lo];
 }
 
+// Eigen 3.4.0 VectorXf::sum() order (Redux.h, SSE2 packet 4, 2x unrolled) over lazily produced terms
+template <class CostFn>
+__device__ __forceinline__ float eigen_sum_lazy(int n, CostFn c) {
+    if (n < 4) {
+        if (n == 0) return 0.f;
+        float r = c(0);
+        for (int i = 1; i < n; ++i) r = r + c(i);
+        return r;
+    }
+    const int n4 = n & ~3, n8 = n & ~7;
+    float A0 = c(0), A1 = c(1), A2 = c(2), A3 = c(3);
+    if (n4 > 4) {
+        float B0 = c(4), B1 = c(5), B2 = c(6), B3 = c(7);
+        for (int i = 8; i < n8; i += 8) {
+            const float c0 = c(i), c1 = c(i + 1), c2 = c(i + 2), c3 = c(i + 3);
+            const float c4 = c(i + 4), c5 = c(i + 5), c6 = c(i + 6), c7 = c(i + 7);
+            A0 = A0 + c0; A1 = A1 + c1; A2 = A2 + c2; A3 = A3 + c3;
+            B0 = B0 + c4; B1 = B1 + c5; B2 = B2 + c6; B3 = B3 + c7;
+        }
+        A0 = A0 + B0; A1 = A1 + B1; A2 = A2 + B2; A3 = A3 + B3;
+        if (n4 > n8) {
+            const float c0 = c(n8), c1 = c(n8 + 1), c2 = c(n8 + 2), c3 = c(n8 + 3);
+            A0 = A0 + c0; A1 = A1 + c1; A2 = A2 + c2; A3 = A3 + c3;
+        }
+    }
+    float r = (A0 + A2) + (A1 + A3);
+    for (int i = n4; i < n; ++i) r = r + c(i);
+    return r;
+}
+
+// line q of the template posed by T (refinement rule 4): map-coordinate end points and the orientation bin
+struct PosedLine { float x1, y1, x2, y2; int bin; };
+__device__ __forceinline__ PosedLine pose_line(const float4 v, const float* T, float offx, float offy, const SlopeTableDev& table) {
+    const float x1 = T[0] * v.x + T[1] * v.y, y1 = T[3] * v.x + T[4] * v.y;
+    const float x2 = T[0] * v.z + T[1] * v.w, y2 = T[3] * v.z + T[4] * v.w;
+    PosedLine p;
+    p.bin = bin_of_slope_dev(table, (y2 - y1) / (x2 - x1));
+    p.x1 = x1 + offx; p.y1 = y1 + offy;
+    p.x2 = x2 + offx; p.y2 = y2 + offy;
+    return p;
+}
+
+// the evaluate<Dt3Cpu> term of one posed line (dt3cpu.cpp:126-179): |plane(x1, y1) - plane(x2, y2)| of its plane at the
+// truncated map-coordinate end points, which the caller has checked to lie inside the map
+__device__ __forceinline__ float line_cost(const float* planes, size_t pitch, size_t plane_elems, int bin, float x1, float y1, float x2,
+                                           float y2) {
+    const int ix1 = (int)x1, iy1 = (int)y1, ix2 = (int)x2, iy2 = (int)y2;
+    const float* P = planes + (size_t)bin * plane_elems;
+    return fabsf(__ldg(P + (size_t)iy1 * pitch + ix1) - __ldg(P + (size_t)iy2 * pitch + ix2));
+}
+
 }   // namespace fdcm

@@ -66,18 +66,6 @@ void launch_coverage_dilate(const uint32_t* d_mask, const MapDims& dm, int radiu
     coverage_window_kernel<<<blocks, 256, 0, s>>>(d_tmp, dm, radius, d_dil);
 }
 
-// line q of the template posed by T (refinement rule 4): map-coordinate end points and the orientation bin
-struct PosedLine { float x1, y1, x2, y2; int bin; };
-__device__ __forceinline__ PosedLine pose_line(const float4 v, const float* T, float offx, float offy, const SlopeTableDev& table) {
-    const float x1 = T[0] * v.x + T[1] * v.y, y1 = T[3] * v.x + T[4] * v.y;
-    const float x2 = T[0] * v.z + T[1] * v.w, y2 = T[3] * v.z + T[4] * v.w;
-    PosedLine p;
-    p.bin = bin_of_slope_dev(table, (y2 - y1) / (x2 - x1));
-    p.x1 = x1 + offx; p.y1 = y1 + offy;
-    p.x2 = x2 + offx; p.y2 = y2 + offy;
-    return p;
-}
-
 constexpr int kCoverageThreads = 256;
 
 __global__ void __launch_bounds__(kCoverageThreads) coverage_eval_kernel(const __grid_constant__ CoverageLaunch p,

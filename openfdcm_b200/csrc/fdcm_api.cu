@@ -299,6 +299,12 @@ struct fdcm_dt3 {
     mutable uint64_t cov_gen = 0;
     mutable int cov_radius = -1, cov_tol = -1;
     mutable cudaEvent_t cov_ev = nullptr;
+    // pose fit: the scene-line grid of fit_md for the map write fit_gen (0: none) and the call's buffers; fit_ev is recorded
+    // after the grid build, which later calls on any stream wait on
+    mutable DevBuf fit_cnt, fit_off, fit_items, fit_tmp, fit_in, fit_out, fit_st;
+    mutable uint64_t fit_gen = 0;
+    mutable float fit_md = 0.f;
+    mutable cudaEvent_t fit_ev = nullptr;
     mutable float s_scene_min[2] = {0.f, 0.f}, s_scene_max[2] = {0.f, 0.f};   // bbox of the resident search scene
     mutable std::mutex host_tset_mutex;
     mutable fdcm_templates* host_tset = nullptr;   // reusable template set of fdcm_search_host
@@ -322,13 +328,14 @@ struct fdcm_dt3 {
                           &s_valid, &s_hyp, &s_counters, &s_topk_score, &s_topk_idx, &s_topk_out, &s_topk_n, &s_keys, &s_keys2, &s_idx,
                           &s_perm, &s_sort_tmp, &s_sel_keys, &s_sel_keys2, &s_sel_vals, &s_sel_vals2, &s_sel_surv, &s_sel_acc,
                           &s_sel_tmp, &s_ref_state, &s_ref_keys, &s_ref_io, &s_denom, &s_dense_keys, &s_dense_rot, &cov_tmp, &cov_dil,
-                          &cov_io, &cov_out})
+                          &cov_io, &cov_out, &fit_cnt, &fit_off, &fit_items, &fit_tmp, &fit_in, &fit_out, &fit_st})
             b->release();
         if (h_pinned) cudaFreeHost(h_pinned);
         if (ev_fork) cudaEventDestroy(ev_fork);
         if (ev_join) cudaEventDestroy(ev_join);
         if (ev_written) cudaEventDestroy(ev_written);
         if (cov_ev) cudaEventDestroy(cov_ev);
+        if (fit_ev) cudaEventDestroy(fit_ev);
         if (h_scene_stage) cudaFreeHost(h_scene_stage);
         if (scene_stage_ev) cudaEventDestroy(scene_stage_ev);
         destroy_host_tset();
@@ -2282,6 +2289,140 @@ extern "C" fdcm_status fdcm_match_coverage(const fdcm_dt3* m, const fdcm_templat
     CUDA_TRY(cudaMemcpyAsync(coverage, m->cov_out.p, (size_t)n * 4, cudaMemcpyDeviceToHost, s));
     CUDA_TRY(cudaStreamSynchronize(s));
     prof_resolve();
+    return FDCM_OK;
+}
+
+// =============================================================================================
+// pose fit of host matches (rules in include/fdcm_b200.h)
+// =============================================================================================
+static fdcm_status check_fit(const fdcm_fit_params* f) {
+    if (!f) return fail(FDCM_ERR_INVALID, "fit is null");
+    if (f->iterations < 1 || f->iterations > 100) return fail(FDCM_ERR_INVALID, "pose fit: iterations must be in 1..100");
+    if (!(f->max_distance > 0.f && f->max_distance <= (float)FDCM_FIT_MAX_DISTANCE))
+        return fail(FDCM_ERR_INVALID, "pose fit: max_distance must be in (0, " + std::to_string(FDCM_FIT_MAX_DISTANCE) + "]");
+    if (!(f->sample_step >= 0.5f) || !std::isfinite(f->sample_step)) return fail(FDCM_ERR_INVALID, "pose fit: sample_step must be finite and >= 0.5");
+    if (f->bin_tolerance < 0 || f->bin_tolerance > 32) return fail(FDCM_ERR_INVALID, "pose fit: bin_tolerance must be in 0..32");
+    if (!(f->tolerance >= 0.f) || !std::isfinite(f->tolerance)) return fail(FDCM_ERR_INVALID, "pose fit: tolerance must be finite and >= 0");
+    if (f->min_inliers < 3) return fail(FDCM_ERR_INVALID, "pose fit: min_inliers must be >= 3");
+    return FDCM_OK;
+}
+
+// The scene-line grid of max_distance for the map's current scene, queued on `s` unless the map holds it for its last write
+// already.  (m->search_mutex held, map_wait done)
+static fdcm_status fit_grid(const fdcm_dt3* m, float max_distance, cudaStream_t s) {
+    const int gx = (m->dm.W + kFitCell - 1) / kFitCell, gy = (m->dm.H + kFitCell - 1) / kFitCell;
+    if (m->fit_gen != m->write_gen || m->fit_md != max_distance) {
+        m->fit_gen = 0;
+        const size_t cells = (size_t)gx * gy;
+        const size_t tmp = fit_grid_scan_bytes((int)cells);
+        CUDA_TRY(m->fit_cnt.reserve((cells + 1) * 8));
+        CUDA_TRY(m->fit_off.reserve((cells + 1) * 8));
+        CUDA_TRY(m->fit_tmp.reserve(std::max<size_t>(tmp, 16)));
+        unsigned long long total = 0;
+        {
+            KernelScope k("fit_grid", 0.0, s, 2);   // count + fill; the CUB scan between them is library code
+            CUDA_TRY(cudaMemsetAsync(m->fit_cnt.p, 0, (cells + 1) * 8, s));
+            launch_fit_grid_count(m->lines.as<float4>(), m->n_lines, max_distance, gx, gy, m->fit_cnt.as<unsigned long long>(),
+                                  m->fit_off.as<unsigned long long>(), m->fit_tmp.p, tmp, s);
+            CUDA_TRY(cudaMemcpyAsync(&total, m->fit_off.as<unsigned long long>() + cells, 8, cudaMemcpyDeviceToHost, s));
+            CUDA_TRY(cudaStreamSynchronize(s));
+            CUDA_TRY(m->fit_items.reserve(std::max<size_t>((size_t)total * 4, 16)));
+            CUDA_TRY(cudaMemsetAsync(m->fit_cnt.p, 0, cells * 8, s));
+            launch_fit_grid_fill(m->lines.as<float4>(), m->n_lines, max_distance, gx, gy, m->fit_off.as<unsigned long long>(),
+                                 m->fit_cnt.as<unsigned long long>(), m->fit_items.as<int32_t>(), s);
+        }
+        CUDA_TRY(cudaGetLastError());
+        if (!m->fit_ev) CUDA_TRY(cudaEventCreateWithFlags(&m->fit_ev, cudaEventDisableTiming));
+        CUDA_TRY(cudaEventRecord(m->fit_ev, s));
+        m->fit_gen = m->write_gen;
+        m->fit_md = max_distance;
+    }
+    CUDA_TRY(cudaStreamWaitEvent(s, m->fit_ev, 0));   // a grid queued by an earlier call on another stream
+    return FDCM_OK;
+}
+
+extern "C" fdcm_status fdcm_fit_matches(const fdcm_dt3* m, const fdcm_templates* tc, int32_t tmpl_idx_base, int32_t penalty_kind,
+                                        float penalty_tau, const fdcm_fit_params* fit, const fdcm_match* in, int64_t n, fdcm_match* out,
+                                        fdcm_fit_stats* stats) {
+    if (fdcm_status st = check_fit(fit)) return st;
+    if (!m || !tc || n < 0) return fail(FDCM_ERR_INVALID, "bad argument");
+    if (penalty_kind < 0 || penalty_kind > 2) return fail(FDCM_ERR_INVALID, "bad penalty kind");
+    if (n == 0) return FDCM_OK;
+    if (!in || !out) return fail(FDCM_ERR_INVALID, "null argument");
+    if (n >= ((int64_t)1 << 34)) return fail(FDCM_ERR_INVALID, "pose fit: at most 2^34 - 1 matches per call");   // (one warp each)
+    if (tc->device != m->device) return fail(FDCM_ERR_INVALID, "templates and feature map live on different devices");
+    if (m->stage != 0) return fail(FDCM_ERR_INVALID, "feature map was built with a debug stage");
+    for (int64_t i = 0; i < n; ++i) {
+        const int64_t t = (int64_t)in[i].tmpl_idx - tmpl_idx_base;
+        if (t < 0 || t >= tc->n_tmpl)
+            return fail(FDCM_ERR_OUT_OF_RANGE, "match " + std::to_string(i) + ": tmpl_idx " + std::to_string(in[i].tmpl_idx) +
+                                                   " outside the template set");
+    }
+    fdcm_templates* t = const_cast<fdcm_templates*>(tc);
+    std::lock_guard<std::mutex> lk(m->search_mutex);
+    if (m->dm.D == 0 || m->dm.W == 0 || m->dm.H == 0) {   // empty map: every input is invalid (rule 6)
+        for (int64_t i = 0; i < n; ++i) {
+            out[i] = in[i];
+            out[i].score = NAN;
+            if (stats) stats[i] = fdcm_fit_stats{0, 0, 0, NAN};
+        }
+        return FDCM_OK;
+    }
+    CUDA_TRY(cudaSetDevice(m->device));
+    cudaStream_t s;
+    if (fdcm_status st = get_stream(m->device, &s)) return st;
+    if (fdcm_status st = map_wait(m, s)) return st;
+    if (fdcm_status st = templates_ready(t, s)) return st;
+    CUDA_TRY(m->fit_in.reserve((size_t)n * sizeof(fdcm_match)));
+    CUDA_TRY(m->fit_out.reserve((size_t)n * sizeof(fdcm_match)));
+    if (stats) CUDA_TRY(m->fit_st.reserve((size_t)n * sizeof(fdcm_fit_stats)));
+    CUDA_TRY(cudaMemcpyAsync(m->fit_in.p, in, (size_t)n * sizeof(fdcm_match), cudaMemcpyHostToDevice, s));
+    const float* d_denom = nullptr;   // the search's denominators
+    if (fdcm_status st = stage_uploads(m, t, nullptr, 0, penalty_kind, penalty_tau, s, &d_denom)) return st;
+    if (fdcm_status st = fit_grid(m, fit->max_distance, s)) return st;
+    FitLaunch fl;
+    fl.map = map_view(m);
+    fl.scene = m->lines.as<float4>();
+    fl.scene_bins = m->bins.as<int32_t>();
+    fl.cell_off = m->fit_off.as<unsigned long long>();
+    fl.cell_items = m->fit_items.as<int32_t>();
+    fl.gx = (m->dm.W + kFitCell - 1) / kFitCell;
+    fl.gy = (m->dm.H + kFitCell - 1) / kFitCell;
+    fl.in = m->fit_in.as<fdcm_match>();
+    fl.n = n;
+    fl.lines = t->lines.as<float4>();
+    fl.offsets = t->offs.as<int32_t>();
+    fl.anchors = t->anchors.as<float2>();
+    fl.denom = d_denom;
+    fl.tmpl_idx_base = tmpl_idx_base;
+    fl.prm = *fit;
+    fl.out = m->fit_out.as<fdcm_match>();
+    fl.stats = stats ? m->fit_st.as<fdcm_fit_stats>() : nullptr;
+    {
+        KernelScope k("fit_eval", 0.0, s);
+        launch_fit_eval(fl, m->table_dev, s);
+    }
+    CUDA_TRY(cudaGetLastError());
+    CUDA_TRY(cudaMemcpyAsync(out, m->fit_out.p, (size_t)n * sizeof(fdcm_match), cudaMemcpyDeviceToHost, s));
+    if (stats) CUDA_TRY(cudaMemcpyAsync(stats, m->fit_st.p, (size_t)n * sizeof(fdcm_fit_stats), cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(cudaStreamSynchronize(s));
+    prof_resolve();
+    return FDCM_OK;
+}
+
+extern "C" fdcm_status fdcm_fit_samples(const float* tl, int32_t n_lines, float sample_step, double* out_xy, int64_t capacity, int64_t* n_out) {
+    if (n_lines < 0 || (n_lines > 0 && !tl) || !n_out) return fail(FDCM_ERR_INVALID, "null argument");
+    if (!(sample_step >= 0.5f) || !std::isfinite(sample_step)) return fail(FDCM_ERR_INVALID, "pose fit: sample_step must be finite and >= 0.5");
+    int64_t total = 0;
+    for (int q = 0; q < n_lines; ++q) total += fit_line_samples(tl[4 * q], tl[4 * q + 1], tl[4 * q + 2], tl[4 * q + 3], sample_step);
+    *n_out = total;
+    if (total > capacity || (total > 0 && !out_xy)) return fail(FDCM_ERR_CAPACITY, "output buffer too small");
+    int64_t k = 0;
+    for (int q = 0; q < n_lines; ++q) {
+        const float* l = tl + 4 * (size_t)q;
+        const int n = fit_line_samples(l[0], l[1], l[2], l[3], sample_step);
+        for (int i = 0; i < n; ++i, ++k) fit_sample(l[0], l[1], l[2], l[3], i, n, out_xy[2 * k], out_xy[2 * k + 1]);
+    }
     return FDCM_OK;
 }
 

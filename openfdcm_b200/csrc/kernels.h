@@ -253,6 +253,50 @@ struct CoverageLaunch {
 // one warp per match
 void launch_coverage_eval(const CoverageLaunch& p, const SlopeTableDev& table, cudaStream_t s);
 
+// ---- fit_kernels.cu: pose fit (fdcm_fit_matches; rules in include/fdcm_b200.h) ----
+constexpr int kFitCell = 16;     // side of a cell of the scene-line grid, in map pixels
+// samples of a template line (rule 2): the same arithmetic on the host (fdcm_fit_samples) and the device
+__host__ __device__ inline int fit_line_samples(float x1, float y1, float x2, float y2, float step) {
+    const float dx = x2 - x1, dy = y2 - y1;
+    const float len = sqrtf(dx * dx + dy * dy);
+    if (!(len > 0.f)) return 0;
+    const int n = (int)ceilf(len / step) + 1;
+    return n < 2 ? 2 : n;
+}
+__host__ __device__ inline void fit_sample(float x1, float y1, float x2, float y2, int i, int n, double& sx, double& sy) {
+    const double f = (double)i / (double)(n - 1);
+    sx = (double)x1 + ((double)x2 - (double)x1) * f;
+    sy = (double)y1 + ((double)y2 - (double)y1) * f;
+}
+// the scene-line grid of (map, max_distance): cells gx x gy; the lines of cell c are items[off[c] .. off[c + 1])
+size_t fit_grid_scan_bytes(int n_cells);
+// pass 0: per-cell counts into cnt (zeroed, n_cells + 1 entries); then an exclusive scan of cnt into off
+void launch_fit_grid_count(const float4* d_lines, int n_lines, float max_distance, int gx, int gy, unsigned long long* d_cnt,
+                           unsigned long long* d_off, void* d_temp, size_t temp_bytes, cudaStream_t s);
+// pass 1: the line indices into items; d_cursor: n_cells zeroed counters
+void launch_fit_grid_fill(const float4* d_lines, int n_lines, float max_distance, int gx, int gy, const unsigned long long* d_off,
+                          unsigned long long* d_cursor, int32_t* d_items, cudaStream_t s);
+struct FitLaunch {
+    MapView map;
+    const float4* scene;         // the build scene's lines in map coordinates, and their bins
+    const int32_t* scene_bins;
+    const unsigned long long* cell_off;   // gx * gy + 1
+    const int32_t* cell_items;
+    int32_t gx, gy;
+    const fdcm_match* in;        // n matches
+    int64_t n;
+    const float4* lines;         // template set
+    const int32_t* offsets;
+    const float2* anchors;
+    const float* denom;          // per template penalty denominator, or nullptr
+    int32_t tmpl_idx_base;
+    fdcm_fit_params prm;
+    fdcm_match* out;             // n records
+    fdcm_fit_stats* stats;       // n entries
+};
+// one warp per match
+void launch_fit_eval(const FitLaunch& p, const SlopeTableDev& table, cudaStream_t s);
+
 void launch_evaluate(const MapView& map, const SlopeTableDev& table, const float4* d_lines, const int32_t* d_toff,
                      const float2* d_transl, const int32_t* d_troff, const int32_t* d_owner, int64_t n_scores,
                      float* d_scores, cudaStream_t s);

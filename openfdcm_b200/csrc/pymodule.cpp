@@ -365,6 +365,36 @@ PYBIND11_MODULE(_openfdcm_cuda, m) {
           "Edge coverage of every match (entry i for matches[i]): the fraction of the posed template's raster samples with a scene "
           "edge pixel of similar orientation nearby; NaN where the posed template leaves the map");
 
+    py::class_<PoseFit>(m, "PoseFit")
+        .def(py::init([](int iterations, float max_distance, float sample_step, int bin_tolerance, float tolerance, int min_inliers) {
+                 return PoseFit{iterations, max_distance, sample_step, bin_tolerance, tolerance, min_inliers};
+             }),
+             "iterations"_a = 10, "max_distance"_a = 3.f, "sample_step"_a = 2.f, "bin_tolerance"_a = 1, "tolerance"_a = 1e-3f,
+             "min_inliers"_a = 6)
+        .def_readwrite("iterations", &PoseFit::iterations)
+        .def_readwrite("max_distance", &PoseFit::maxDistance)
+        .def_readwrite("sample_step", &PoseFit::sampleStep)
+        .def_readwrite("bin_tolerance", &PoseFit::binTolerance)
+        .def_readwrite("tolerance", &PoseFit::tolerance)
+        .def_readwrite("min_inliers", &PoseFit::minInliers)
+        .def("__repr__", [](const PoseFit& f) {
+            return "<PoseFit: iterations=" + std::to_string(f.iterations) + ", max_distance=" + std::to_string(f.maxDistance) +
+                   ", sample_step=" + std::to_string(f.sampleStep) + ", bin_tolerance=" + std::to_string(f.binTolerance) +
+                   ", tolerance=" + std::to_string(f.tolerance) + ", min_inliers=" + std::to_string(f.minInliers) + ">";
+        });
+
+    m.def("fit_matches",
+          [](const Dt3Cuda& featuremap, const std::vector<LinesIn>& templates, const std::vector<Match>& matches,
+             const std::optional<PoseFit>& fit, const std::optional<ExponentialPenalty>& penalty) {
+              const auto t = to_templates(templates);
+              py::gil_scoped_release release;
+              return penalty ? fitMatches(featuremap, t, matches, *penalty, fit ? *fit : PoseFit{})
+                             : fitMatches(featuremap, t, matches, fit ? *fit : PoseFit{});
+          },
+          "featuremap"_a, "templates"_a, "matches"_a, "fit"_a = py::none(), "penalty"_a = py::none(),
+          "Pose fit of every match (entry i for matches[i]): point-to-line least squares of the template's samples against the "
+          "scene lines; scored like search_topk with the same penalty; a match whose pose is invalid comes back with score NaN");
+
     m.def("penalize",
           [](const PenaltyStrategy& penalty, const std::vector<Match>& matches, const std::vector<float>& templatelengths) {
               return penalize(penalty, matches, templatelengths);

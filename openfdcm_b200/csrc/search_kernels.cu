@@ -58,36 +58,6 @@ __device__ __forceinline__ Rigid align_dev(const float4 tl, const float4 sl, int
     return Rigid{r00, r01, cx - mx, r10, r11, cy - my};
 }
 
-// Eigen 3.4.0 VectorXf::sum() order (Redux.h, SSE2 packet 4, 2x unrolled) over lazily produced terms
-template <class CostFn>
-__device__ __forceinline__ float eigen_sum_lazy(int n, CostFn c) {
-    if (n < 4) {
-        if (n == 0) return 0.f;
-        float r = c(0);
-        for (int i = 1; i < n; ++i) r = r + c(i);
-        return r;
-    }
-    const int n4 = n & ~3, n8 = n & ~7;
-    float A0 = c(0), A1 = c(1), A2 = c(2), A3 = c(3);
-    if (n4 > 4) {
-        float B0 = c(4), B1 = c(5), B2 = c(6), B3 = c(7);
-        for (int i = 8; i < n8; i += 8) {
-            const float c0 = c(i), c1 = c(i + 1), c2 = c(i + 2), c3 = c(i + 3);
-            const float c4 = c(i + 4), c5 = c(i + 5), c6 = c(i + 6), c7 = c(i + 7);
-            A0 = A0 + c0; A1 = A1 + c1; A2 = A2 + c2; A3 = A3 + c3;
-            B0 = B0 + c4; B1 = B1 + c5; B2 = B2 + c6; B3 = B3 + c7;
-        }
-        A0 = A0 + B0; A1 = A1 + B1; A2 = A2 + B2; A3 = A3 + B3;
-        if (n4 > n8) {
-            const float c0 = c(n8), c1 = c(n8 + 1), c2 = c(n8 + 2), c3 = c(n8 + 3);
-            A0 = A0 + c0; A1 = A1 + c1; A2 = A2 + c2; A3 = A3 + c3;
-        }
-    }
-    float r = (A0 + A2) + (A1 + A3);
-    for (int i = n4; i < n; ++i) r = r + c(i);
-    return r;
-}
-
 // minmaxTranslation (dt3cpu.cpp:30-75) given the bbox of the aligned template already shifted by the
 // scene translation
 __device__ void minmax_dev(float mnx, float mny, float mxx, float mxy, float sizex, float sizey, float vx, float vy,
@@ -835,9 +805,7 @@ __device__ __forceinline__ float staged_score(const MapView& map, const float4* 
     const size_t pitch = (size_t)map.dm.pitch, pe = map.dm.plane_elems;
     return eigen_sum_lazy(L, [&](int q) {
         const float4 e = apts[q];
-        const int x1 = (int)(e.x + offx), y1 = (int)(e.y + offy), x2 = (int)(e.z + offx), y2 = (int)(e.w + offy);
-        const float* P = planes + (size_t)bins[q] * pe;
-        return fabsf(__ldg(P + (size_t)y1 * pitch + x1) - __ldg(P + (size_t)y2 * pitch + x2));
+        return line_cost(planes, pitch, pe, bins[q], e.x + offx, e.y + offy, e.z + offx, e.w + offy);
     });
 }
 
