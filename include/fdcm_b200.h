@@ -357,6 +357,45 @@ fdcm_status fdcm_search_dense_verify(const fdcm_dt3* map, const fdcm_templates* 
                                      const fdcm_select_params* select, const fdcm_refine_params* refine,
                                      const fdcm_coverage_params* cov, fdcm_match* out, int64_t capacity, int64_t* n_out);
 
+/* ---- scale as a pose dimension of the dense search (beyond the reference) ----------------------------------------
+ * Templates rendered at one camera distance appear larger or smaller when the object is nearer or farther.  The scaled
+ * dense search scores every template at a geometric grid of scales as well as rotations and translations.  Rules, in the
+ * dense section's terms (fp32 without contraction):
+ *   1. Scales k = 0..scales-1: s_k = (float)((double)scale_start * pow((double)scale_ratio, k)) (host C library).  Pose
+ *      matrix of (k, r): a_kr = (float)((double)s_k * cos(theta_r)), b_kr = (float)((double)s_k * sin(theta_r)); dense
+ *      rule 3 with (a, b) in place of (c, s): P = (a, -b, qx - (a*ax - b*ay), b, a, qy - (b*ax + a*ay)); the end points are
+ *      used as given iff a == 1 && b == 0.  With s_k == 1.0f, (a, b) is (c_r, s_r) bit for bit.
+ *   2. Records: h = ((((t * scales + k) * rotations + r) * cells_y + cv) * cells_x + cu); the record limit of 2^31 - 1
+ *      counts the scales (T * scales * rotations * cells_y * cells_x).
+ *   3. Penalty: the score of a record of (t, k) is its raw score divided by the penalty denominator of the length
+ *      len_t * s_k (one fp32 multiply; host powf like the search).  The raw score is a sum along the posed lines, so
+ *      WITHOUT a penalty a smaller scale scores lower for no other reason: the raw search favours small scales.
+ *   4. Selection: fdcm_search_select's walk, with the angle test of near(a, b) replaced by
+ *      Ta0*Tb0 + Ta3*Tb3 >= cos_thr * (s_a * s_b), s_a and s_b the grid scales of the two records (with every s == 1.0f
+ *      this is the unscaled test); max_per_template counts a template over all its scales.
+ *   5. Refinement and the coverage filter run on the scaled records unchanged: their rules take any 2x3 transform, and
+ *      refinement rotates the pose, so it keeps each record's scale.  Refinement scores with the search's denominator of
+ *      t (the unscaled length), so the refined list equals fdcm_refine_matches of the unrefined output.
+ * scales == 1 with scale_start == 1 gives output byte-identical to fdcm_search_dense (cov NULL or min_coverage == 0) or
+ * fdcm_search_dense_verify.  Invalid parameters fail with FDCM_ERR_INVALID: scales outside 1..FDCM_DENSE_MAX_SCALES,
+ * scale_start or scale_ratio not finite or not > 0, an s_k that is not finite or not > 0 after rounding, and everything
+ * fdcm_search_dense(_verify) rejects.  Cost: scales times that of the unscaled call. */
+#define FDCM_DENSE_MAX_SCALES 64
+typedef struct fdcm_scale_grid {         /* 12 bytes */
+    int32_t scales;             /* 1..FDCM_DENSE_MAX_SCALES */
+    float scale_start;          /* > 0 */
+    float scale_ratio;          /* > 0: s_k = scale_start * scale_ratio^k */
+} fdcm_scale_grid;
+/* fdcm_search_dense_verify over the scale grid; cov NULL: no coverage filter */
+fdcm_status fdcm_search_dense_scales(const fdcm_dt3* map, const fdcm_templates* templates, const fdcm_dense_params* dense,
+                                     const fdcm_scale_grid* scales, int32_t penalty_kind, float penalty_tau, int32_t top_k,
+                                     int32_t tmpl_idx_base, const fdcm_select_params* select, const fdcm_refine_params* refine,
+                                     const fdcm_coverage_params* cov, fdcm_match* out, int64_t capacity, int64_t* n_out);
+/* fdcm_dense_poses of scale index `scale` and rotation `rotation`; host-only parity hook */
+fdcm_status fdcm_dense_scaled_poses(const fdcm_dense_params* dense, const fdcm_scale_grid* scales, const float anchor[2],
+                                    const float shift[2], int32_t width, int32_t height, int32_t scale, int32_t rotation, float* out,
+                                    int64_t capacity, int64_t* n_out, int32_t grid_wh[2]);
+
 /* ---- pose fit: point-to-line least squares against the scene lines (beyond the reference) --------------------------
  * A search match puts one template line on one scene line, the dense grid is off by up to stride / 2 px and rot_step / 2
  * rad, and refinement minimises the DT3 score, an integer-pixel, binned-orientation cost that has no minimum at the true
@@ -426,6 +465,37 @@ fdcm_status fdcm_fit_matches(const fdcm_dt3* map, const fdcm_templates* template
 /* the samples of rule 2 of n_lines template lines, (x, y) pairs in line order; *n_out = the number of samples
  * (FDCM_ERR_CAPACITY when it exceeds capacity); host-only parity hook */
 fdcm_status fdcm_fit_samples(const float* tmpl_xyxy, int32_t n_lines, float sample_step, double* out_xy, int64_t capacity, int64_t* n_out);
+
+/* ---- scaled pose fit (beyond the reference) -------------------------------------------------------------------------
+ * Rules 1-6 of the pose fit with a fourth parameter, a scale step about the rotation centre c (IEEE double, no
+ * transcendental function).  Where a rule is not restated here it holds as written above.
+ *   4'. J = (nx, ny, jt, js), js = nx*(px - cx) + ny*(py - cy).  Fifteen sums, per sample in this order: A00 = nx*nx,
+ *       A01 = nx*ny, A02 = nx*jt, A03 = nx*js, A11 = ny*ny, A12 = ny*jt, A13 = ny*js, A22 = jt*jt, A23 = jt*js, A33 = js*js,
+ *       g0 = nx*r, g1 = ny*r, g2 = jt*r, g3 = js*r, rr = r*r; lanes and butterfly as in rule 4.  B = A + lambda I with
+ *       lambda = 1e-9 * (((A00 + A11) + A22) + A33).  Cholesky, failing when a radicand is not > 0:
+ *       l00 = sqrt(B00), l10 = A01 / l00, l20 = A02 / l00, l30 = A03 / l00,
+ *       l11 = sqrt(B11 - l10*l10), l21 = (A12 - l20*l10) / l11, l31 = (A13 - l30*l10) / l11,
+ *       l22 = sqrt((B22 - l20*l20) - l21*l21), l32 = ((A23 - l30*l20) - l31*l21) / l22,
+ *       l33 = sqrt(((B33 - l30*l30) - l31*l31) - l32*l32);
+ *       y0 = -g0 / l00, y1 = (-g1 - l10*y0) / l11, y2 = ((-g2 - l20*y0) - l21*y1) / l22,
+ *       y3 = (((-g3 - l30*y0) - l31*y1) - l32*y2) / l33;
+ *       delta = (dx, dy, dth, ds): ds = y3 / l33, dth = (y2 - l32*ds) / l22, dy = ((y1 - l21*dth) - l31*ds) / l11,
+ *       dx = (((y0 - l10*dy) - l20*dth) - l30*ds) / l00.
+ *   5'. Update: cr and sr of rule 5, f = 1 + ds, cr' = f*cr, sr' = f*sr; M' and e' of rule 5 with cr', sr'.  The scale of a
+ *       pose is sigma = sqrt(m0*m4 - m1*m3).  After the solve the iteration stops, keeping the pose, when sigma' of the
+ *       update is NaN or outside [min_scale, max_scale] (then, as in rule 5, when F of the update is invalid).  After an
+ *       accepted update it stops when max(|dx|, |dy|, (|dth| * sigma) * rho, (|ds| * sigma) * rho) <= tolerance, sigma the
+ *       scale of the pose before the update.
+ * Stats, invalid inputs and the score (the search's penalty denominator of t) are those of rule 6.  Invalid parameters:
+ * those of fdcm_fit_matches, and min_scale or max_scale not finite, min_scale not > 0 or min_scale > max_scale.  The scale
+ * bounds are the only guard against a runaway scale; a direction the samples do not observe (along the lines of a template
+ * of parallel lines) is held where it is by the damping, as in the rigid fit. */
+typedef struct fdcm_fit_scale {          /* 8 bytes */
+    float min_scale, max_scale; /* 0 < min_scale <= max_scale, finite */
+} fdcm_fit_scale;
+fdcm_status fdcm_fit_matches_scaled(const fdcm_dt3* map, const fdcm_templates* templates, int32_t tmpl_idx_base, int32_t penalty_kind,
+                                    float penalty_tau, const fdcm_fit_params* fit, const fdcm_fit_scale* scale, const fdcm_match* in,
+                                    int64_t n, fdcm_match* out, fdcm_fit_stats* stats);
 
 /* optimize(optimizer, templates, alignments, featuremap) (matching/optimizestrategy.h:62-64; BatchOptimize:
  * batchoptimize.cpp:6-123, batch_size == 0: DefaultOptimize, defaultoptimize.cpp:6-93).  The templates are used

@@ -18,6 +18,7 @@
 #include <optional>
 #include <stdexcept>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "../fdcm_b200.h"
@@ -358,10 +359,17 @@ struct DenseSearch {
     bool hasRoi{false};
     std::array<float, 4> roi{{0.f, 0.f, 0.f, 0.f}};
 };
+// scale grid of the dense search (rules of fdcm_search_dense_scales): scales start * ratio^k, k = 0..scales-1.  The cost
+// grows linearly with the number of scales; without a penalty the raw score favours small scales.
+struct ScaleGrid {
+    int scales{1};
+    float start{1.f};
+    float ratio{1.f};
+};
 namespace detail {
 inline std::vector<Match> search_dense(const Dt3Cuda& fm, const std::vector<LineArray>& templates, const DenseSearch& dense, int penalty_kind,
                                        float tau, int k, const DistinctMatches* select, const PoseRefinement* refine,
-                                       const fdcm_coverage_params* cov = nullptr) {
+                                       const fdcm_coverage_params* cov = nullptr, const ScaleGrid* scales = nullptr) {
     std::vector<float> flat;
     std::vector<int32_t> off;
     pack(templates, flat, off);
@@ -377,7 +385,11 @@ inline std::vector<Match> search_dense(const Dt3Cuda& fm, const std::vector<Line
     if (refine) r = refine_params(*refine);
     std::vector<fdcm_match> rec((size_t)std::max(k, 1));
     int64_t n = 0;
-    if (cov)
+    if (scales) {
+        const fdcm_scale_grid g{scales->scales, scales->start, scales->ratio};
+        check(fdcm_search_dense_scales(fm.handle(), ts, &d, &g, penalty_kind, tau, k, 0, select ? &q : nullptr, refine ? &r : nullptr, cov,
+                                       rec.data(), (int64_t)rec.size(), &n));
+    } else if (cov)
         check(fdcm_search_dense_verify(fm.handle(), ts, &d, penalty_kind, tau, k, 0, select ? &q : nullptr, refine ? &r : nullptr, cov,
                                        rec.data(), (int64_t)rec.size(), &n));
     else
@@ -471,11 +483,24 @@ inline std::vector<Match> searchDense(const Dt3Cuda& fm, const std::vector<LineA
     const fdcm_coverage_params c = detail::coverage_params(verify);
     return detail::search_dense(fm, templates, dense, FDCM_PENALTY_EXPONENTIAL, pen.tau, k, select, refine, &c);
 }
+// dense search over a scale grid [-> coverage filter] -> top-k (or distinct top-k) [-> pose refinement] on the device
+inline std::vector<Match> searchDense(const Dt3Cuda& fm, const std::vector<LineArray>& templates, const DenseSearch& dense,
+                                      const ScaleGrid& scales, const ExponentialPenalty& pen, int k, const DistinctMatches* select = nullptr,
+                                      const PoseRefinement* refine = nullptr) {
+    return detail::search_dense(fm, templates, dense, FDCM_PENALTY_EXPONENTIAL, pen.tau, k, select, refine, nullptr, &scales);
+}
+inline std::vector<Match> searchDense(const Dt3Cuda& fm, const std::vector<LineArray>& templates, const DenseSearch& dense,
+                                      const ScaleGrid& scales, const ExponentialPenalty& pen, int k, const DistinctMatches* select,
+                                      const PoseRefinement* refine, const EdgeCoverage& verify) {
+    const fdcm_coverage_params c = detail::coverage_params(verify);
+    return detail::search_dense(fm, templates, dense, FDCM_PENALTY_EXPONENTIAL, pen.tau, k, select, refine, &c, &scales);
+}
 
 // pose fit (beyond the reference; rules of fdcm_fit_matches): per match, up to `iterations` Gauss-Newton steps of oriented
 // point-to-line least squares of the template's samples against the build scene's line segments (nearest scene line within
 // maxDistance pixels on an orientation plane within binTolerance planes).  It needs scene lines near the pose, uses no
-// robust loss beyond that gate and does not re-rank; the defaults are a starting point, not tuned.
+// robust loss beyond that gate and does not re-rank; the defaults are a starting point, not tuned.  scaleRange {lo, hi}: the
+// scaled fit (fdcm_fit_matches_scaled), which also fits the scale within [lo, hi]; empty: the rigid fit.
 struct PoseFit {
     int iterations{10};
     float maxDistance{3.f};
@@ -483,6 +508,7 @@ struct PoseFit {
     int binTolerance{1};
     float tolerance{1e-3f};
     int minInliers{6};
+    std::optional<std::pair<float, float>> scaleRange{};
 };
 struct FitStats {
     int nSamples;
@@ -508,7 +534,13 @@ inline std::vector<Match> fit_matches(const Dt3Cuda& fm, const std::vector<LineA
     const fdcm_fit_params p{fit.iterations, fit.maxDistance, fit.sampleStep, fit.binTolerance, fit.tolerance, fit.minInliers};
     std::vector<fdcm_match> out(matches.size());
     std::vector<fdcm_fit_stats> st(stats ? matches.size() : 0);
-    check(fdcm_fit_matches(fm.handle(), ts, 0, penalty_kind, tau, &p, rec.data(), (int64_t)rec.size(), out.data(), stats ? st.data() : nullptr));
+    if (fit.scaleRange) {
+        const fdcm_fit_scale sc{fit.scaleRange->first, fit.scaleRange->second};
+        check(fdcm_fit_matches_scaled(fm.handle(), ts, 0, penalty_kind, tau, &p, &sc, rec.data(), (int64_t)rec.size(), out.data(),
+                                      stats ? st.data() : nullptr));
+    } else {
+        check(fdcm_fit_matches(fm.handle(), ts, 0, penalty_kind, tau, &p, rec.data(), (int64_t)rec.size(), out.data(), stats ? st.data() : nullptr));
+    }
     if (stats) {
         stats->resize(matches.size());
         for (size_t i = 0; i < st.size(); ++i) (*stats)[i] = FitStats{st[i].n_samples, st[i].n_inliers, st[i].iterations, st[i].rms};

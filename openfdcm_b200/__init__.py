@@ -22,7 +22,8 @@ from ._lib import FIT_STATS_DTYPE, MATCH_DTYPE, FdcmError, check, lib, ptr
 __all__ = [
     "distance", "Dt3CudaParameters", "Dt3Cuda", "build_cuda_featuremap", "ThreadPool", "DefaultSearch", "ConcentricRangeStrategy",
     "BatchOptimize", "DefaultOptimize", "DefaultMatch", "DefaultPenalty", "ExponentialPenalty", "Match",
-    "TemplateSet", "SceneBatch", "DistinctMatches", "PoseRefinement", "DenseSearch", "EdgeCoverage", "PoseFit", "search", "search_topk",
+    "TemplateSet", "SceneBatch", "DistinctMatches", "PoseRefinement", "DenseSearch", "ScaleGrid", "EdgeCoverage", "PoseFit", "search",
+    "search_topk",
     "search_dense", "refine_matches", "match_coverage", "fit_matches", "penalize", "get_template_lengths",
     "get_template_anchors", "sort_matches", "evaluate",
     "minmax_translation", "get_feature_size", "establish_search_strategy", "optimize", "read", "write", "FdcmError", "MATCH_DTYPE",
@@ -381,6 +382,24 @@ class DenseSearch:
                 f"cell={self.cell}, roi={self.roi}>")
 
 
+class ScaleGrid:
+    """Scale grid of the dense search (beyond the reference): `scales` template scales start * ratio^k, k = 0..scales-1,
+    searched like the rotations.  The cost grows linearly with the number of scales.  The raw score is a sum along the posed
+    lines, so without a penalty small scales score lower: search scales with a penalty (DefaultPenalty divides by the
+    scaled length).  Exact rules: include/fdcm_b200.h."""
+
+    def __init__(self, scales=1, start=1.0, ratio=1.0):
+        self.scales = int(scales)
+        self.start = float(start)
+        self.ratio = float(ratio)
+
+    def _params(self):
+        return _lib.ScaleGridParams(self.scales, self.start, self.ratio)
+
+    def __repr__(self):
+        return f"<ScaleGrid: scales={self.scales}, start={self.start}, ratio={self.ratio}>"
+
+
 class EdgeCoverage:
     """Match verification (beyond the reference): the coverage of a match is the fraction of its posed template's raster
     samples that have a scene edge pixel within `radius` pixels (Chebyshev) on an orientation plane within `bin_tolerance`
@@ -406,23 +425,28 @@ class PoseFit:
     sample taking the nearest scene line within `max_distance` pixels whose orientation plane is within `bin_tolerance`
     planes of the posed line's; stops when a step moves no sample more than `tolerance` pixels, with fewer than
     `min_inliers` correspondences, or when the next pose would leave the map.  It needs scene lines near the pose, uses no
-    robust loss beyond that gate and does not re-rank.  The defaults are a starting point, not tuned.  Exact rules:
-    include/fdcm_b200.h."""
+    robust loss beyond that gate and does not re-rank.  The defaults are a starting point, not tuned.  scale_range (lo, hi):
+    the scaled fit, which also fits the pose's scale about the template anchor and stops before a scale outside [lo, hi];
+    None: the rigid fit, which keeps the scale.  Exact rules: include/fdcm_b200.h."""
 
-    def __init__(self, iterations=10, max_distance=3.0, sample_step=2.0, bin_tolerance=1, tolerance=1e-3, min_inliers=6):
+    def __init__(self, iterations=10, max_distance=3.0, sample_step=2.0, bin_tolerance=1, tolerance=1e-3, min_inliers=6, scale_range=None):
         self.iterations = int(iterations)
         self.max_distance = float(max_distance)
         self.sample_step = float(sample_step)
         self.bin_tolerance = int(bin_tolerance)
         self.tolerance = float(tolerance)
         self.min_inliers = int(min_inliers)
+        self.scale_range = None if scale_range is None else tuple(float(v) for v in scale_range)
+        if self.scale_range is not None and len(self.scale_range) != 2:
+            raise ValueError("scale_range must be (min_scale, max_scale)")
 
     def _params(self):
         return _lib.FitParams(self.iterations, self.max_distance, self.sample_step, self.bin_tolerance, self.tolerance, self.min_inliers)
 
     def __repr__(self):
         return (f"<PoseFit: iterations={self.iterations}, max_distance={self.max_distance}, sample_step={self.sample_step}, "
-                f"bin_tolerance={self.bin_tolerance}, tolerance={self.tolerance}, min_inliers={self.min_inliers}>")
+                f"bin_tolerance={self.bin_tolerance}, tolerance={self.tolerance}, min_inliers={self.min_inliers}, "
+                f"scale_range={self.scale_range}>")
 
 
 def _search_raw(featuremap, templates, scene, searcher, optimizer, penalty=None, top_k=0, tmpl_idx_base=0, select=None, refine=None,
@@ -500,13 +524,16 @@ def refine_matches(featuremap, templates, matches, refine, penalty=None, tmpl_id
     return out[: rec.shape[0]].copy()
 
 
-def search_dense(featuremap, templates, dense, penalty=None, k=10, tmpl_idx_base=0, *, select=None, refine=None, verify=None, fit=None):
+def search_dense(featuremap, templates, dense, penalty=None, k=10, tmpl_idx_base=0, *, select=None, refine=None, verify=None, fit=None,
+                 scales=None):
     """Dense pose-grid search on the device (see DenseSearch): the best pose of every (template, rotation, cell), then the
     top-k in ascending (score, record) order, or with select (a DistinctMatches) the distinct top-k, then with refine (a
     PoseRefinement) the refinement of those, equal to refine_matches of the unrefined result.  Returns a MATCH_DTYPE array.
     verify: an EdgeCoverage whose min_coverage > 0 drops every record of lower (or NaN) coverage before the selection.
     fit: a PoseFit applied last, equal to fit_matches of the unfitted result; the fitted list is not re-selected or
-    re-sorted, so two distinct matches may converge on one instance."""
+    re-sorted, so two distinct matches may converge on one instance.
+    scales: a ScaleGrid searched as a further pose dimension (a penalty then divides by the scaled length; max_per_template
+    counts a template over all its scales); None: the unscaled search."""
     if not isinstance(featuremap, Dt3Cuda):
         raise TypeError("search_dense needs a Dt3Cuda feature map (build_cuda_featuremap)")
     tset = templates if isinstance(templates, TemplateSet) else TemplateSet(templates, featuremap.device)
@@ -515,7 +542,11 @@ def search_dense(featuremap, templates, dense, penalty=None, k=10, tmpl_idx_base
     sp = None if select is None else C.byref(select._params())
     rp = None if refine is None else C.byref(refine._params())
     pen_kind, pen_tau = (0, 0.0) if penalty is None else (penalty.kind, float(penalty.tau))
-    if verify is None:
+    if scales is not None:
+        vp = None if verify is None else C.byref(verify._params())
+        check(lib().fdcm_search_dense_scales(featuremap._h, tset._h, C.byref(dense._params()), C.byref(scales._params()), pen_kind, pen_tau,
+                                             int(k), int(tmpl_idx_base), sp, rp, vp, ptr(out), out.shape[0], C.byref(n)))
+    elif verify is None:
         check(lib().fdcm_search_dense(featuremap._h, tset._h, C.byref(dense._params()), pen_kind, pen_tau, int(k), int(tmpl_idx_base), sp, rp,
                                       ptr(out), out.shape[0], C.byref(n)))
     else:
@@ -545,7 +576,7 @@ def fit_matches(featuremap, templates, matches, fit=None, penalty=None, tmpl_idx
     """Pose fit (see PoseFit; None: the defaults) of any match list against a feature map and a template set (list or
     TemplateSet): a MATCH_DTYPE array, entry i fitting matches[i], scored like search_topk with the same penalty; a match
     whose pose is invalid comes back unchanged with score NaN.  The list is not re-sorted or re-selected: two matches may
-    converge on one instance.  return_stats: also a FIT_STATS_DTYPE array (n_samples, n_inliers, iterations, rms)."""
+    converge on one instance.  A fit with scale_range also fits the scale (fdcm_fit_matches_scaled).  return_stats: also a FIT_STATS_DTYPE array (n_samples, n_inliers, iterations, rms)."""
     if not isinstance(featuremap, Dt3Cuda):
         raise TypeError("fit_matches needs a Dt3Cuda feature map (build_cuda_featuremap)")
     fit = PoseFit() if fit is None else fit
@@ -553,9 +584,14 @@ def fit_matches(featuremap, templates, matches, fit=None, penalty=None, tmpl_idx
     rec = _to_records(matches)
     out = np.zeros(max(rec.shape[0], 1), MATCH_DTYPE)
     stats = np.zeros(max(rec.shape[0], 1), FIT_STATS_DTYPE) if return_stats else None
-    st = lib().fdcm_fit_matches(featuremap._h, tset._h, int(tmpl_idx_base), 0 if penalty is None else penalty.kind,
-                                0.0 if penalty is None else float(penalty.tau), C.byref(fit._params()), ptr(rec), rec.shape[0], ptr(out),
-                                ptr(stats))
+    pen_kind, pen_tau = (0, 0.0) if penalty is None else (penalty.kind, float(penalty.tau))
+    if fit.scale_range is None:
+        st = lib().fdcm_fit_matches(featuremap._h, tset._h, int(tmpl_idx_base), pen_kind, pen_tau, C.byref(fit._params()), ptr(rec),
+                                    rec.shape[0], ptr(out), ptr(stats))
+    else:
+        sc = _lib.FitScaleParams(*fit.scale_range)
+        st = lib().fdcm_fit_matches_scaled(featuremap._h, tset._h, int(tmpl_idx_base), pen_kind, pen_tau, C.byref(fit._params()), C.byref(sc),
+                                           ptr(rec), rec.shape[0], ptr(out), ptr(stats))
     if st == _lib.FDCM_ERR_OUT_OF_RANGE:
         raise IndexError(lib().fdcm_last_error().decode())
     check(st)

@@ -50,6 +50,14 @@ class FitParams(C.Structure):
                 ("tolerance", C.c_float), ("min_inliers", C.c_int32)]
 
 
+class ScaleGridParams(C.Structure):
+    _fields_ = [("scales", C.c_int32), ("scale_start", C.c_float), ("scale_ratio", C.c_float)]
+
+
+class FitScaleParams(C.Structure):
+    _fields_ = [("min_scale", C.c_float), ("max_scale", C.c_float)]
+
+
 FIT_STATS_DTYPE = np.dtype([("n_samples", "<i4"), ("n_inliers", "<i4"), ("iterations", "<i4"), ("rms", "<f4")])
 assert FIT_STATS_DTYPE.itemsize == 16
 
@@ -109,6 +117,13 @@ SIGNATURES = {
     "fdcm_search_dense_verify": (C.c_int, [_P, _P, C.POINTER(DenseParams), C.c_int32, C.c_float, C.c_int32, C.c_int32, C.POINTER(SelectParams),
                                            C.POINTER(RefineParams), C.POINTER(CoverageParams), _P, C.c_int64, C.POINTER(C.c_int64)]),
     "fdcm_fit_matches": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_float, C.POINTER(FitParams), _P, C.c_int64, _P, _P]),
+    "fdcm_search_dense_scales": (C.c_int, [_P, _P, C.POINTER(DenseParams), C.POINTER(ScaleGridParams), C.c_int32, C.c_float, C.c_int32,
+                                           C.c_int32, C.POINTER(SelectParams), C.POINTER(RefineParams), C.POINTER(CoverageParams), _P,
+                                           C.c_int64, C.POINTER(C.c_int64)]),
+    "fdcm_dense_scaled_poses": (C.c_int, [C.POINTER(DenseParams), C.POINTER(ScaleGridParams), _P, _P, C.c_int32, C.c_int32, C.c_int32,
+                                          C.c_int32, _P, C.c_int64, C.POINTER(C.c_int64), _P]),
+    "fdcm_fit_matches_scaled": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_float, C.POINTER(FitParams), C.POINTER(FitScaleParams), _P,
+                                          C.c_int64, _P, _P]),
     "fdcm_fit_samples": (C.c_int, [_P, C.c_int32, C.c_float, _P, C.c_int64, C.POINTER(C.c_int64)]),
     "fdcm_optimize": (C.c_int, [_P, _P, _P, C.c_int32, _P, C.c_int32, _P, _P, _P]),
     "fdcm_search_host": (C.c_int, [_P, _P, _P, C.c_int32, _P, C.c_int32, C.POINTER(SearchParams), _P, C.c_int64,

@@ -290,7 +290,11 @@ struct fdcm_dt3 {
     mutable uint64_t denom_set = 0;
     mutable int denom_kind = -1;
     mutable float denom_tau = 0.f;
+    // the scales of the scaled dense search the buffer also holds denominators of (T per-template ones, then T x S of
+    // (t, k) at t * S + k); empty: the T per-template ones only
+    mutable std::vector<float> denom_scales;
     mutable DevBuf s_dense_keys, s_dense_rot;   // dense pose-grid search (records: s_rec / s_valid / s_hyp_off)
+    mutable DevBuf s_dense_rs;                  // scaled dense search: the grid scale of every record
     // match verification: the dilated edge mask of (cov_radius, cov_tol) for the map write cov_gen (0: none), its scratch and
     // the standalone call's buffers; cov_ev is recorded after the dilation, which later calls on any stream wait on
     uint64_t write_gen = 0;         // incremented by every write of the map (map_written)
@@ -327,7 +331,7 @@ struct fdcm_dt3 {
         for (DevBuf* b : {&planes, &mask, &stack, &lines, &bins, &band_info, &band_spill, &integ_items, &s_scene, &s_sorted_len, &s_sorted_idx, &s_hyp_off, &s_rec,
                           &s_valid, &s_hyp, &s_counters, &s_topk_score, &s_topk_idx, &s_topk_out, &s_topk_n, &s_keys, &s_keys2, &s_idx,
                           &s_perm, &s_sort_tmp, &s_sel_keys, &s_sel_keys2, &s_sel_vals, &s_sel_vals2, &s_sel_surv, &s_sel_acc,
-                          &s_sel_tmp, &s_ref_state, &s_ref_keys, &s_ref_io, &s_denom, &s_dense_keys, &s_dense_rot, &cov_tmp, &cov_dil,
+                          &s_sel_tmp, &s_ref_state, &s_ref_keys, &s_ref_io, &s_denom, &s_dense_keys, &s_dense_rot, &s_dense_rs, &cov_tmp, &cov_dil,
                           &cov_io, &cov_out, &fit_cnt, &fit_off, &fit_items, &fit_tmp, &fit_in, &fit_out, &fit_st})
             b->release();
         if (h_pinned) cudaFreeHost(h_pinned);
@@ -1545,18 +1549,27 @@ static fdcm_status exchange_empty(const fdcm_dt3* m, fdcm_comm* comm, int k, fdc
 // Penalty denominators of set t for (kind, tau) (host powf like the reference) in the map's buffer: written through the
 // pinned staging `stage` on the copy stream `cs` unless the map holds them already.  Nothing else reads that buffer: every
 // earlier use of the map has synchronised (m->search_mutex held), and other maps sharing the set have their own.
-static fdcm_status map_denominators(const fdcm_dt3* m, const fdcm_templates* t, int kind, float tau, float* stage, cudaStream_t cs,
-                                    const float** d_denom) {
+// With `scales` (the scaled dense search) the T per-template denominators are followed by the T x S ones of the lengths
+// len_t * s_k, at T + t * S + k; the cache key holds the scales, so a cache of T entries is never read as one of T x S.
+static fdcm_status map_denominators(const fdcm_dt3* m, const fdcm_templates* t, int kind, float tau, const std::vector<float>& scales,
+                                    float* stage, cudaStream_t cs, const float** d_denom) {
     *d_denom = nullptr;
     if (kind == FDCM_PENALTY_NONE) return FDCM_OK;
-    if (m->denom_set != t->load_id || m->denom_kind != kind || m->denom_tau != tau) {
+    if (m->denom_set != t->load_id || m->denom_kind != kind || m->denom_tau != tau || m->denom_scales != scales) {
         m->denom_set = 0;
-        CUDA_TRY(m->s_denom.reserve(std::max<size_t>(4, (size_t)t->n_tmpl * 4)));
+        const size_t S = scales.size(), n = (size_t)t->n_tmpl * (1 + S);
+        CUDA_TRY(m->s_denom.reserve(std::max<size_t>(4, n * 4)));
         for (int i = 0; i < t->n_tmpl; ++i) stage[i] = penalty_denominator(kind, tau, t->lengths[(size_t)i]);
-        CUDA_TRY(cudaMemcpyAsync(m->s_denom.p, stage, (size_t)t->n_tmpl * 4, cudaMemcpyHostToDevice, cs));
+        for (int i = 0; i < t->n_tmpl; ++i)
+            for (size_t k = 0; k < S; ++k) {
+                const float len = t->lengths[(size_t)i] * scales[k];   // one fp32 multiply
+                stage[(size_t)t->n_tmpl + (size_t)i * S + k] = penalty_denominator(kind, tau, len);
+            }
+        CUDA_TRY(cudaMemcpyAsync(m->s_denom.p, stage, n * 4, cudaMemcpyHostToDevice, cs));
         m->denom_set = t->load_id;
         m->denom_kind = kind;
         m->denom_tau = tau;
+        m->denom_scales = scales;
     }
     *d_denom = m->s_denom.as<float>();
     return FDCM_OK;
@@ -1566,20 +1579,20 @@ static fdcm_status map_denominators(const fdcm_dt3* m, const fdcm_templates* t, 
 // staging on the copy stream, and `s` waits for them: a pageable copy on `s` would first wait for everything queued there,
 // e.g. a map build in flight.  (m->search_mutex held)
 static fdcm_status stage_uploads(const fdcm_dt3* m, fdcm_templates* t, const int64_t* hyp_off, size_t n_off, int kind, float tau,
-                                 cudaStream_t s, const float** d_denom) {
+                                 cudaStream_t s, const float** d_denom, const std::vector<float>& scales = {}) {
     std::lock_guard<std::mutex> lk(t->mu);
     cudaStream_t cs;
     if (fdcm_status st = get_copy_stream(m->device, &cs)) return st;
     if (!t->ready) CUDA_TRY(cudaEventCreateWithFlags(&t->ready, cudaEventDisableTiming));
     else CUDA_TRY(cudaEventSynchronize(t->ready));   // the staging buffer may still feed an earlier upload (other threads)
-    const size_t off_bytes = n_off * 8, den_bytes = (size_t)t->n_tmpl * 4;
+    const size_t off_bytes = n_off * 8, den_bytes = (size_t)t->n_tmpl * (1 + scales.size()) * 4;
     CUDA_TRY(t->stage_reserve(std::max<size_t>(16, off_bytes + den_bytes)));
     unsigned char* stage = static_cast<unsigned char*>(t->h_stage);
     if (off_bytes) {
         std::memcpy(stage, hyp_off, off_bytes);
         CUDA_TRY(cudaMemcpyAsync(m->s_hyp_off.p, stage, off_bytes, cudaMemcpyHostToDevice, cs));
     }
-    if (fdcm_status st = map_denominators(m, t, kind, tau, reinterpret_cast<float*>(stage + off_bytes), cs, d_denom)) return st;
+    if (fdcm_status st = map_denominators(m, t, kind, tau, scales, reinterpret_cast<float*>(stage + off_bytes), cs, d_denom)) return st;
     CUDA_TRY(cudaEventRecord(t->ready, cs));
     CUDA_TRY(cudaStreamWaitEvent(s, t->ready, 0));
     t->upload_pending = false;   // (this event is recorded after any template upload on the same copy stream)
@@ -1612,8 +1625,9 @@ static fdcm_status check_select(const fdcm_select_params* q, int32_t top_k, bool
 }
 
 // Distinct top-K over the records the search kernel just queued on `s`: writes s_topk_out / s_topk_n like the top-K kernels
+// rec_scale: the grid scale of every record (the scaled dense search), or nullptr
 static fdcm_status run_select(const fdcm_dt3* m, const fdcm_templates* t, const fdcm_search_params* p, const fdcm_select_params* q,
-                              int64_t H, cudaStream_t s) {
+                              int64_t H, cudaStream_t s, const float* rec_scale = nullptr) {
     if (H >= ((int64_t)1 << 31)) return fail(FDCM_ERR_INVALID, "distinct top-K: more than 2^31 - 1 hypotheses");
     SelectLaunch sp;
     sp.rec = m->s_rec.as<fdcm_match>();
@@ -1629,6 +1643,7 @@ static fdcm_status run_select(const fdcm_dt3* m, const fdcm_templates* t, const 
     sp.r2 = q->radius * q->radius;
     sp.any_angle = q->max_angle >= 3.14159274f;
     sp.cos_thr = (float)std::cos((double)q->max_angle);
+    sp.rec_scale = rec_scale;
     const bool within = q->across_templates == 0;
     const size_t tmp = select_temp_bytes(H);
     CUDA_TRY(m->s_sel_keys.reserve((size_t)H * 8));
@@ -1648,7 +1663,7 @@ static fdcm_status run_select(const fdcm_dt3* m, const fdcm_templates* t, const 
     int* d_n = m->s_topk_n.as<int>();
     if (within) {
         CUDA_TRY(m->s_sel_surv.reserve((size_t)H * 4));
-        if (sp.radius_on) CUDA_TRY(m->s_sel_acc.reserve((size_t)H * 16));
+        if (sp.radius_on) CUDA_TRY(m->s_sel_acc.reserve((size_t)H * (rec_scale ? 20 : 16)));
         {
             KernelScope k("select_greedy", 0.0, s);
             launch_select_greedy(sp, sorted_keys, sorted_h, m->s_sel_surv.as<uint32_t>(), m->s_sel_acc.as<float4>(), s);
@@ -2109,6 +2124,30 @@ static void dense_rotation(const fdcm_dense_params* d, int r, float* c, float* s
     *s = (float)std::sin(th);
 }
 
+// scaled dense search, rule 1: the scales s_k of a grid, or FDCM_ERR_INVALID
+static fdcm_status dense_scales(const fdcm_scale_grid* g, std::vector<float>* out) {
+    if (!g) return fail(FDCM_ERR_INVALID, "scales is null");
+    if (g->scales < 1 || g->scales > FDCM_DENSE_MAX_SCALES)
+        return fail(FDCM_ERR_INVALID, "scaled dense search: scales must be in 1.." + std::to_string(FDCM_DENSE_MAX_SCALES));
+    if (!(g->scale_start > 0.f) || !std::isfinite(g->scale_start) || !(g->scale_ratio > 0.f) || !std::isfinite(g->scale_ratio))
+        return fail(FDCM_ERR_INVALID, "scaled dense search: scale_start and scale_ratio must be finite and > 0");
+    out->resize((size_t)g->scales);
+    for (int k = 0; k < g->scales; ++k) {
+        const float sk = (float)((double)g->scale_start * std::pow((double)g->scale_ratio, (double)k));
+        if (!(sk > 0.f) || !std::isfinite(sk))
+            return fail(FDCM_ERR_INVALID, "scaled dense search: scale " + std::to_string(k) + " is not a finite number > 0 in float32");
+        (*out)[(size_t)k] = sk;
+    }
+    return FDCM_OK;
+}
+
+// scaled dense search, rule 1: the pose matrix entries (a, b) of scale s_k and rotation r
+static void dense_scaled_rotation(const fdcm_dense_params* d, float sk, int r, float* a, float* b) {
+    const double th = (double)d->rot_start + (double)r * (double)d->rot_step;
+    *a = (float)((double)sk * std::cos(th));
+    *b = (float)((double)sk * std::sin(th));
+}
+
 // rule 2: the grid points of a W x H map with scene translation shift (nx = ny = 0: none)
 struct DenseGrid { int lo_x, lo_y, nx, ny; };
 static DenseGrid dense_grid(const fdcm_dense_params* d, const float shift[2], int W, int H) {
@@ -2123,14 +2162,19 @@ static DenseGrid dense_grid(const fdcm_dense_params* d, const float shift[2], in
     return DenseGrid{lx, ly, ((int)hi[0] - lx) / d->stride + 1, ((int)hi[1] - ly) / d->stride + 1};
 }
 
-// cov: the coverage filter of the records before the selection (fdcm_search_dense_verify, min_coverage > 0), or nullptr
+// cov: the coverage filter of the records before the selection (fdcm_search_dense_verify, min_coverage > 0), or nullptr;
+// grid: the scale grid of fdcm_search_dense_scales, or nullptr
 static fdcm_status dense_impl(const fdcm_dt3* m, const fdcm_templates* tc, const fdcm_dense_params* dense, int32_t penalty_kind,
                               float penalty_tau, int32_t top_k, int32_t tmpl_idx_base, const fdcm_select_params* sel,
                               const fdcm_refine_params* ref, const fdcm_coverage_params* cov, fdcm_match* out, int64_t capacity,
-                              int64_t* n_out) {
+                              int64_t* n_out, const fdcm_scale_grid* grid = nullptr) {
     if (!m || !tc || !n_out) return fail(FDCM_ERR_INVALID, "null argument");
     *n_out = 0;
     if (fdcm_status st = check_dense(dense)) return st;
+    std::vector<float> scales;   // empty: the unscaled search
+    if (grid)
+        if (fdcm_status st = dense_scales(grid, &scales)) return st;
+    const int S = grid ? (int)scales.size() : 1;
     if (penalty_kind < 0 || penalty_kind > 2) return fail(FDCM_ERR_INVALID, "bad penalty kind");
     if (top_k < 1) return fail(FDCM_ERR_INVALID, "dense search: top_k must be >= 1");
     if (sel)
@@ -2158,34 +2202,46 @@ static fdcm_status dense_impl(const fdcm_dt3* m, const fdcm_templates* tc, const
     if (g.nx == 0 || g.ny == 0) return FDCM_OK;
     const int cell = std::min(dense->cell, std::max(g.nx, g.ny));   // (a larger cell holds the same points)
     const int cells_x = (g.nx + cell - 1) / cell, cells_y = (g.ny + cell - 1) / cell;
-    const int64_t per_tmpl = (int64_t)dense->rotations * cells_y * cells_x;
+    const int64_t per_tmpl = (int64_t)S * dense->rotations * cells_y * cells_x;
     const int64_t limit = ((int64_t)1 << 31) - 1;
     if (per_tmpl > limit || per_tmpl * t->n_tmpl > limit)
         return fail(FDCM_ERR_INVALID, "dense search: " + std::to_string(per_tmpl) + " records per template x " + std::to_string(t->n_tmpl) +
-                                          " templates; at most 2^31 - 1 records (use fewer rotations or templates, a larger cell or stride, or a region)");
+                                          " templates; at most 2^31 - 1 records (use fewer scales, rotations or templates, a larger cell or stride, or a region)");
     const int64_t H = per_tmpl * t->n_tmpl;
 
     std::vector<int64_t> hyp_off((size_t)t->n_tmpl + 1);
     for (int i = 0; i <= t->n_tmpl; ++i) hyp_off[(size_t)i] = (int64_t)i * per_tmpl;
-    std::vector<float> rot(2 * (size_t)dense->rotations);
-    for (int r = 0; r < dense->rotations; ++r) dense_rotation(dense, r, &rot[2 * (size_t)r], &rot[2 * (size_t)r + 1]);
+    // (c_r, s_r) of every rotation; scaled: (a_kr, b_kr) at k * rotations + r, then the S scales
+    const size_t SR = (size_t)S * dense->rotations;
+    std::vector<float> rot(2 * SR + scales.size());
+    for (int k = 0; k < S; ++k)
+        for (int r = 0; r < dense->rotations; ++r) {
+            float* cs = &rot[2 * ((size_t)k * dense->rotations + r)];
+            if (grid) dense_scaled_rotation(dense, scales[(size_t)k], r, cs, cs + 1);
+            else dense_rotation(dense, r, cs, cs + 1);
+        }
+    std::copy(scales.begin(), scales.end(), rot.begin() + 2 * SR);
+    if (grid) CUDA_TRY(m->s_dense_rs.reserve((size_t)H * 4));
     CUDA_TRY(m->s_rec.reserve((size_t)H * sizeof(fdcm_match)));
     CUDA_TRY(m->s_valid.reserve((size_t)H));
     CUDA_TRY(m->s_hyp_off.reserve(hyp_off.size() * 8));
     CUDA_TRY(m->s_dense_keys.reserve((size_t)H * 8));
     CUDA_TRY(m->s_dense_rot.reserve(rot.size() * 4));
     CUDA_TRY(cudaMemcpyAsync(m->s_dense_rot.p, rot.data(), rot.size() * 4, cudaMemcpyHostToDevice, s));
-    const float* d_denom = nullptr;   // the search's denominators
-    if (fdcm_status st = stage_uploads(m, t, hyp_off.data(), hyp_off.size(), penalty_kind, penalty_tau, s, &d_denom)) return st;
+    const float* d_denom = nullptr;   // the search's denominators (scaled: then those of (t, k))
+    if (fdcm_status st = stage_uploads(m, t, hyp_off.data(), hyp_off.size(), penalty_kind, penalty_tau, s, &d_denom, scales)) return st;
     DenseLaunch dl;
     dl.lines = t->lines.as<float4>();
     dl.offsets = t->offs.as<int32_t>();
     dl.anchors = t->anchors.as<float2>();
     dl.rot = m->s_dense_rot.as<float2>();
-    dl.denom = d_denom;
+    dl.denom = d_denom && grid ? d_denom + t->n_tmpl : d_denom;
     dl.n_tmpl = t->n_tmpl;
     dl.rotations = dense->rotations;
     dl.tmpl_idx_base = tmpl_idx_base;
+    dl.scales = S;
+    dl.scale = grid ? m->s_dense_rot.as<float>() + 2 * SR : nullptr;
+    dl.rec_scale = grid ? m->s_dense_rs.as<float>() : nullptr;
     dl.lo_x = g.lo_x;
     dl.lo_y = g.lo_y;
     dl.stride = dense->stride;
@@ -2220,7 +2276,7 @@ static fdcm_status dense_impl(const fdcm_dt3* m, const fdcm_templates* tc, const
         fdcm_search_params sp{};
         sp.top_k = k;
         sp.tmpl_idx_base = tmpl_idx_base;
-        if (fdcm_status st = run_select(m, t, &sp, sel, H, s)) return st;
+        if (fdcm_status st = run_select(m, t, &sp, sel, H, s, dl.rec_scale)) return st;
     } else {
         const int blocks = topk_ws_blocks(H);
         CUDA_TRY(m->s_topk_score.reserve((size_t)blocks * k * 4));
@@ -2252,6 +2308,17 @@ extern "C" fdcm_status fdcm_search_dense_verify(const fdcm_dt3* m, const fdcm_te
     if (fdcm_status st = check_coverage(cov)) return st;
     return dense_impl(m, tc, dense, penalty_kind, penalty_tau, top_k, tmpl_idx_base, sel, ref, cov->min_coverage > 0.f ? cov : nullptr, out,
                       capacity, n_out);
+}
+
+extern "C" fdcm_status fdcm_search_dense_scales(const fdcm_dt3* m, const fdcm_templates* tc, const fdcm_dense_params* dense,
+                                                const fdcm_scale_grid* scales, int32_t penalty_kind, float penalty_tau, int32_t top_k,
+                                                int32_t tmpl_idx_base, const fdcm_select_params* sel, const fdcm_refine_params* ref,
+                                                const fdcm_coverage_params* cov, fdcm_match* out, int64_t capacity, int64_t* n_out) {
+    if (!scales) return fail(FDCM_ERR_INVALID, "scales is null");
+    if (cov)
+        if (fdcm_status st = check_coverage(cov)) return st;
+    return dense_impl(m, tc, dense, penalty_kind, penalty_tau, top_k, tmpl_idx_base, sel, ref, cov && cov->min_coverage > 0.f ? cov : nullptr,
+                      out, capacity, n_out, scales);
 }
 
 // =============================================================================================
@@ -2341,9 +2408,10 @@ static fdcm_status fit_grid(const fdcm_dt3* m, float max_distance, cudaStream_t 
     return FDCM_OK;
 }
 
-extern "C" fdcm_status fdcm_fit_matches(const fdcm_dt3* m, const fdcm_templates* tc, int32_t tmpl_idx_base, int32_t penalty_kind,
-                                        float penalty_tau, const fdcm_fit_params* fit, const fdcm_match* in, int64_t n, fdcm_match* out,
-                                        fdcm_fit_stats* stats) {
+// scale: the scale range of fdcm_fit_matches_scaled, or nullptr (the rigid fit)
+static fdcm_status fit_impl(const fdcm_dt3* m, const fdcm_templates* tc, int32_t tmpl_idx_base, int32_t penalty_kind, float penalty_tau,
+                            const fdcm_fit_params* fit, const fdcm_fit_scale* scale, const fdcm_match* in, int64_t n, fdcm_match* out,
+                            fdcm_fit_stats* stats) {
     if (fdcm_status st = check_fit(fit)) return st;
     if (!m || !tc || n < 0) return fail(FDCM_ERR_INVALID, "bad argument");
     if (penalty_kind < 0 || penalty_kind > 2) return fail(FDCM_ERR_INVALID, "bad penalty kind");
@@ -2398,8 +2466,11 @@ extern "C" fdcm_status fdcm_fit_matches(const fdcm_dt3* m, const fdcm_templates*
     fl.prm = *fit;
     fl.out = m->fit_out.as<fdcm_match>();
     fl.stats = stats ? m->fit_st.as<fdcm_fit_stats>() : nullptr;
+    fl.scaled = scale ? 1 : 0;
+    fl.min_scale = scale ? scale->min_scale : 0.f;
+    fl.max_scale = scale ? scale->max_scale : 0.f;
     {
-        KernelScope k("fit_eval", 0.0, s);
+        KernelScope k(scale ? "fit_eval_scaled" : "fit_eval", 0.0, s);
         launch_fit_eval(fl, m->table_dev, s);
     }
     CUDA_TRY(cudaGetLastError());
@@ -2408,6 +2479,22 @@ extern "C" fdcm_status fdcm_fit_matches(const fdcm_dt3* m, const fdcm_templates*
     CUDA_TRY(cudaStreamSynchronize(s));
     prof_resolve();
     return FDCM_OK;
+}
+
+extern "C" fdcm_status fdcm_fit_matches(const fdcm_dt3* m, const fdcm_templates* tc, int32_t tmpl_idx_base, int32_t penalty_kind,
+                                        float penalty_tau, const fdcm_fit_params* fit, const fdcm_match* in, int64_t n, fdcm_match* out,
+                                        fdcm_fit_stats* stats) {
+    return fit_impl(m, tc, tmpl_idx_base, penalty_kind, penalty_tau, fit, nullptr, in, n, out, stats);
+}
+
+extern "C" fdcm_status fdcm_fit_matches_scaled(const fdcm_dt3* m, const fdcm_templates* tc, int32_t tmpl_idx_base, int32_t penalty_kind,
+                                               float penalty_tau, const fdcm_fit_params* fit, const fdcm_fit_scale* scale, const fdcm_match* in,
+                                               int64_t n, fdcm_match* out, fdcm_fit_stats* stats) {
+    if (!scale) return fail(FDCM_ERR_INVALID, "scale is null");
+    if (!std::isfinite(scale->min_scale) || !std::isfinite(scale->max_scale) || !(scale->min_scale > 0.f) ||
+        !(scale->min_scale <= scale->max_scale))
+        return fail(FDCM_ERR_INVALID, "scaled pose fit: min_scale and max_scale must be finite with 0 < min_scale <= max_scale");
+    return fit_impl(m, tc, tmpl_idx_base, penalty_kind, penalty_tau, fit, scale, in, n, out, stats);
 }
 
 extern "C" fdcm_status fdcm_fit_samples(const float* tl, int32_t n_lines, float sample_step, double* out_xy, int64_t capacity, int64_t* n_out) {
@@ -2443,6 +2530,31 @@ extern "C" fdcm_status fdcm_dense_poses(const fdcm_dense_params* dense, const fl
     for (int v = 0; v < g.ny; ++v)
         for (int u = 0; u < g.nx; ++u)
             dense_pose(c, s, anchor[0], anchor[1], g.lo_x + u * dense->stride, g.lo_y + v * dense->stride, shift[0], shift[1],
+                       out + 6 * ((size_t)v * g.nx + u));
+    return FDCM_OK;
+}
+
+extern "C" fdcm_status fdcm_dense_scaled_poses(const fdcm_dense_params* dense, const fdcm_scale_grid* grid, const float anchor[2],
+                                               const float shift[2], int32_t width, int32_t height, int32_t scale, int32_t rotation,
+                                               float* out, int64_t capacity, int64_t* n_out, int32_t grid_wh[2]) {
+    if (fdcm_status st = check_dense(dense)) return st;
+    std::vector<float> scales;
+    if (fdcm_status st = dense_scales(grid, &scales)) return st;
+    if (!anchor || !shift || !n_out || !grid_wh) return fail(FDCM_ERR_INVALID, "null argument");
+    if (width < 0 || height < 0) return fail(FDCM_ERR_INVALID, "width and height must be >= 0");
+    if (scale < 0 || scale >= grid->scales) return fail(FDCM_ERR_INVALID, "scale must be in 0..scales - 1");
+    if (rotation < 0 || rotation >= dense->rotations) return fail(FDCM_ERR_INVALID, "rotation must be in 0..rotations - 1");
+    const DenseGrid g = dense_grid(dense, shift, width, height);
+    grid_wh[0] = g.nx;
+    grid_wh[1] = g.ny;
+    const int64_t n = (int64_t)g.nx * g.ny;
+    *n_out = n;
+    if (n > capacity || (n > 0 && !out)) return fail(FDCM_ERR_CAPACITY, "output buffer too small");
+    float a, b;
+    dense_scaled_rotation(dense, scales[(size_t)scale], rotation, &a, &b);
+    for (int v = 0; v < g.ny; ++v)
+        for (int u = 0; u < g.nx; ++u)
+            dense_pose(a, b, anchor[0], anchor[1], g.lo_x + u * dense->stride, g.lo_y + v * dense->stride, shift[0], shift[1],
                        out + 6 * ((size_t)v * g.nx + u));
     return FDCM_OK;
 }

@@ -5,9 +5,9 @@
 //                                                            within max_distance of a point of the cell.  A superset: rule 3
 //                                                            takes the least (d2, j), so extra entries change no result and
 //                                                            the fill may use atomic cursors
-//   fit_eval_kernel                                         one warp per match: per iteration the correspondences of every
+//   fit_eval_kernel<kScaled>                                one warp per match: per iteration the correspondences of every
 //                                                            sample (lane i mod 32 takes sample i of a line), a butterfly
-//                                                            reduction of the normal equations, the 3x3 solve and the update
+//                                                            reduction of the normal equations, the 3x3 (scaled: 4x4) solve and the update
 //                                                            on every lane (the same values everywhere); then the stats pass
 //                                                            and the evaluate<Dt3Cpu> score of the final pose
 // Built with -fmad=false like every kernel of the library: the double arithmetic is the rules', operation by operation.
@@ -102,17 +102,20 @@ __device__ bool fit_valid(const float4* __restrict__ tl, int L, const float* F, 
     return !__any_sync(0xffffffffu, bad);
 }
 
-// sums of rule 4: A00 A01 A02 A11 A12 A22 g0 g1 g2 rr
-constexpr int kFitSums = 10;
+// sums of rule 4: A00 A01 A02 A11 A12 A22 g0 g1 g2 rr; of rule 4' (scaled): A00 A01 A02 A03 A11 A12 A13 A22 A23 A33 g0 g1 g2
+// g3 rr
+template <bool kScaled>
+constexpr int kFitSums = kScaled ? 15 : 10;
 
 // rule 3 + 4 at pose P (float rounding F, centre c): every lane's sums, then the butterfly; also rho^2 (rule 2)
+template <bool kScaled>
 __device__ void fit_pass(const FitLaunch& p, const SlopeTableDev& table, const float4* __restrict__ tl, int L, const FitPose& P,
                          const float* F, double cx, double cy, double ax, double ay, int lane, double* acc, int& n_in, double& rho2) {
     const float offx = p.map.shift_x + F[2], offy = p.map.shift_y + F[5];
     const int D = p.map.dm.D, tol = p.prm.bin_tolerance;
     const double md2 = (double)p.prm.max_distance * (double)p.prm.max_distance;
 #pragma unroll
-    for (int k = 0; k < kFitSums; ++k) acc[k] = 0.0;
+    for (int k = 0; k < kFitSums<kScaled>; ++k) acc[k] = 0.0;
     n_in = 0;
     rho2 = 0.0;
     for (int q = 0; q < L; ++q) {
@@ -157,17 +160,26 @@ __device__ void fit_pass(const FitLaunch& p, const SlopeTableDev& table, const f
             const double nx = -dy / l, ny = dx / l;
             const double r = nx * (px - Ax) + ny * (py - Ay);
             const double jt = ny * (px - cx) - nx * (py - cy);
-            acc[0] = acc[0] + nx * nx; acc[1] = acc[1] + nx * ny; acc[2] = acc[2] + nx * jt;
-            acc[3] = acc[3] + ny * ny; acc[4] = acc[4] + ny * jt; acc[5] = acc[5] + jt * jt;
-            acc[6] = acc[6] + nx * r;  acc[7] = acc[7] + ny * r;  acc[8] = acc[8] + jt * r;
-            acc[9] = acc[9] + r * r;
+            if constexpr (kScaled) {
+                const double js = nx * (px - cx) + ny * (py - cy);
+                acc[0] = acc[0] + nx * nx;  acc[1] = acc[1] + nx * ny;  acc[2] = acc[2] + nx * jt;  acc[3] = acc[3] + nx * js;
+                acc[4] = acc[4] + ny * ny;  acc[5] = acc[5] + ny * jt;  acc[6] = acc[6] + ny * js;
+                acc[7] = acc[7] + jt * jt;  acc[8] = acc[8] + jt * js;  acc[9] = acc[9] + js * js;
+                acc[10] = acc[10] + nx * r; acc[11] = acc[11] + ny * r; acc[12] = acc[12] + jt * r; acc[13] = acc[13] + js * r;
+                acc[14] = acc[14] + r * r;
+            } else {
+                acc[0] = acc[0] + nx * nx; acc[1] = acc[1] + nx * ny; acc[2] = acc[2] + nx * jt;
+                acc[3] = acc[3] + ny * ny; acc[4] = acc[4] + ny * jt; acc[5] = acc[5] + jt * jt;
+                acc[6] = acc[6] + nx * r;  acc[7] = acc[7] + ny * r;  acc[8] = acc[8] + jt * r;
+                acc[9] = acc[9] + r * r;
+            }
             ++n_in;
         }
     }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
 #pragma unroll
-        for (int k = 0; k < kFitSums; ++k) acc[k] = acc[k] + __shfl_xor_sync(0xffffffffu, acc[k], o);
+        for (int k = 0; k < kFitSums<kScaled>; ++k) acc[k] = acc[k] + __shfl_xor_sync(0xffffffffu, acc[k], o);
         n_in += __shfl_xor_sync(0xffffffffu, n_in, o);
         const double o2 = __shfl_xor_sync(0xffffffffu, rho2, o);
         rho2 = o2 > rho2 ? o2 : rho2;
@@ -193,8 +205,33 @@ __device__ __forceinline__ bool fit_solve(const double* a, double* d) {
     return true;
 }
 
+// rule 4': the damped 4x4 Cholesky solve in the header's order; false when a radicand is not > 0.  d = (dx, dy, dth, ds)
+__device__ __forceinline__ bool fit_solve_scaled(const double* a, double* d) {
+    const double lam = 1e-9 * (((a[0] + a[4]) + a[7]) + a[9]);
+    const double b00 = a[0] + lam, b11 = a[4] + lam, b22 = a[7] + lam, b33 = a[9] + lam;
+    if (!(b00 > 0.0)) return false;
+    const double l00 = sqrt(b00), l10 = a[1] / l00, l20 = a[2] / l00, l30 = a[3] / l00;
+    const double r1 = b11 - l10 * l10;
+    if (!(r1 > 0.0)) return false;
+    const double l11 = sqrt(r1), l21 = (a[5] - l20 * l10) / l11, l31 = (a[6] - l30 * l10) / l11;
+    const double r2 = (b22 - l20 * l20) - l21 * l21;
+    if (!(r2 > 0.0)) return false;
+    const double l22 = sqrt(r2), l32 = ((a[8] - l30 * l20) - l31 * l21) / l22;
+    const double r3 = ((b33 - l30 * l30) - l31 * l31) - l32 * l32;
+    if (!(r3 > 0.0)) return false;
+    const double l33 = sqrt(r3);
+    const double y0 = -a[10] / l00, y1 = (-a[11] - l10 * y0) / l11, y2 = ((-a[12] - l20 * y0) - l21 * y1) / l22;
+    const double y3 = (((-a[13] - l30 * y0) - l31 * y1) - l32 * y2) / l33;
+    d[3] = y3 / l33;
+    d[2] = (y2 - l32 * d[3]) / l22;
+    d[1] = ((y1 - l21 * d[2]) - l31 * d[3]) / l11;
+    d[0] = (((y0 - l10 * d[1]) - l20 * d[2]) - l30 * d[3]) / l00;
+    return true;
+}
+
 constexpr int kFitThreads = 128;
 
+template <bool kScaled>
 __global__ void __launch_bounds__(kFitThreads) fit_eval_kernel(const __grid_constant__ FitLaunch p,
                                                                const __grid_constant__ SlopeTableDev table) {
     const long long h = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -228,22 +265,37 @@ __global__ void __launch_bounds__(kFitThreads) fit_eval_kernel(const __grid_cons
               (double)m.transform[2] + (double)shx, (double)m.transform[5] + (double)shy};
     float F[6];
     for (int k = 0; k < 6; ++k) F[k] = m.transform[k];
-    double acc[kFitSums], rho2 = 0.0;
+    double acc[kFitSums<kScaled>], rho2 = 0.0;
     int n_in = 0, iters = 0;
     bool at_pose = false;   // acc / n_in hold the correspondences of the current pose
     for (int it = 0; it < p.prm.iterations; ++it) {
         const double cx = (P.m0 * ax + P.m1 * ay) + P.ex, cy = (P.m3 * ax + P.m4 * ay) + P.ey;
-        fit_pass(p, table, tl, L, P, F, cx, cy, ax, ay, lane, acc, n_in, rho2);
+        fit_pass<kScaled>(p, table, tl, L, P, F, cx, cy, ax, ay, lane, acc, n_in, rho2);
         at_pose = true;
         if (n_in < p.prm.min_inliers) break;
-        double d[3];
-        if (!fit_solve(acc, d)) break;
+        double d[kScaled ? 4 : 3];
+        if constexpr (kScaled) {
+            if (!fit_solve_scaled(acc, d)) break;
+        } else {
+            if (!fit_solve(acc, d)) break;
+        }
         // rule 5: the half-angle rotation about c, then the translation
         const double tau = d[2] * 0.5, k = 1.0 + tau * tau;
-        const double cr = (1.0 - tau * tau) / k, sr = (2.0 * tau) / k;
+        double cr = (1.0 - tau * tau) / k, sr = (2.0 * tau) / k;
+        if constexpr (kScaled) {   // rule 5': the scale step about c
+            const double f = 1.0 + d[3];
+            cr = f * cr;
+            sr = f * sr;
+        }
         const double ux = P.ex - cx, uy = P.ey - cy;
         const FitPose N{cr * P.m0 - sr * P.m3, cr * P.m1 - sr * P.m4, sr * P.m0 + cr * P.m3, sr * P.m1 + cr * P.m4,
                         ((cr * ux - sr * uy) + cx) + d[0], ((sr * ux + cr * uy) + cy) + d[1]};
+        double sigma = 0.0;   // the scale of the pose before the update
+        if constexpr (kScaled) {
+            const double sig_n = sqrt(N.m0 * N.m4 - N.m1 * N.m3);
+            if (!(sig_n >= (double)p.min_scale && sig_n <= (double)p.max_scale)) break;   // (NaN fails too)
+            sigma = sqrt(P.m0 * P.m4 - P.m1 * P.m3);
+        }
         float FN[6];
         fit_round(N, shx, shy, FN);
         if (!fit_valid(tl, L, FN, p.map, table, lane)) break;
@@ -251,13 +303,21 @@ __global__ void __launch_bounds__(kFitThreads) fit_eval_kernel(const __grid_cons
         for (int q = 0; q < 6; ++q) F[q] = FN[q];
         ++iters;
         at_pose = false;
-        const double ad0 = fabs(d[0]), ad1 = fabs(d[1]), adt = fabs(d[2]) * sqrt(rho2);
-        const double step = ad0 > ad1 ? (ad0 > adt ? ad0 : adt) : (ad1 > adt ? ad1 : adt);
-        if (step <= (double)p.prm.tolerance) break;
+        if constexpr (kScaled) {
+            const double rho = sqrt(rho2);
+            const double ad0 = fabs(d[0]), ad1 = fabs(d[1]), adt = (fabs(d[2]) * sigma) * rho, ads = (fabs(d[3]) * sigma) * rho;
+            const double s01 = ad0 > ad1 ? ad0 : ad1, sts = adt > ads ? adt : ads;
+            const double step = s01 > sts ? s01 : sts;
+            if (step <= (double)p.prm.tolerance) break;
+        } else {
+            const double ad0 = fabs(d[0]), ad1 = fabs(d[1]), adt = fabs(d[2]) * sqrt(rho2);
+            const double step = ad0 > ad1 ? (ad0 > adt ? ad0 : adt) : (ad1 > adt ? ad1 : adt);
+            if (step <= (double)p.prm.tolerance) break;
+        }
     }
     if (!at_pose) {
         const double cx = (P.m0 * ax + P.m1 * ay) + P.ex, cy = (P.m3 * ax + P.m4 * ay) + P.ey;
-        fit_pass(p, table, tl, L, P, F, cx, cy, ax, ay, lane, acc, n_in, rho2);
+        fit_pass<kScaled>(p, table, tl, L, P, F, cx, cy, ax, ay, lane, acc, n_in, rho2);
     }
     if (lane != 0) return;
     // rule 6: the score of F, evaluate<Dt3Cpu> in Eigen's order (refinement's scoring terms)
@@ -273,7 +333,7 @@ __global__ void __launch_bounds__(kFitThreads) fit_eval_kernel(const __grid_cons
         st.n_samples = n_samples;
         st.n_inliers = n_in;
         st.iterations = iters;
-        st.rms = n_in > 0 ? (float)sqrt(acc[9] / (double)n_in) : NAN;
+        st.rms = n_in > 0 ? (float)sqrt(acc[kFitSums<kScaled> - 1] / (double)n_in) : NAN;
         p.stats[h] = st;
     }
 }
@@ -281,7 +341,8 @@ __global__ void __launch_bounds__(kFitThreads) fit_eval_kernel(const __grid_cons
 void launch_fit_eval(const FitLaunch& p, const SlopeTableDev& table, cudaStream_t s) {
     if (p.n <= 0) return;
     const long long blocks = (p.n + kFitThreads / 32 - 1) / (kFitThreads / 32);
-    fit_eval_kernel<<<(unsigned)blocks, kFitThreads, 0, s>>>(p, table);
+    if (p.scaled) fit_eval_kernel<true><<<(unsigned)blocks, kFitThreads, 0, s>>>(p, table);
+    else fit_eval_kernel<false><<<(unsigned)blocks, kFitThreads, 0, s>>>(p, table);
 }
 
 }   // namespace fdcm

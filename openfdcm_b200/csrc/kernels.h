@@ -140,6 +140,7 @@ struct SelectLaunch {
     int32_t cap;                 // max_per_template (0: none)
     int32_t radius_on, any_angle;
     float r2, cos_thr;           // radius * radius, (float)cos((double)max_angle)
+    const float* rec_scale;      // n_hyp grid scales of the scaled dense search (angle test cos_thr * (s_a * s_b)), or nullptr
 };
 constexpr int kSelectMaxAcross = FDCM_SELECT_MAX_ACROSS;   // accepted list of the across-template walk (shared memory)
 // bytes of CUB scratch the select sorts need for n_hyp (< 2^31) hypotheses
@@ -203,15 +204,18 @@ struct DenseLaunch {
     const float4* lines;         // template set
     const int32_t* offsets;
     const float2* anchors;
-    const float2* rot;           // (c_r, s_r) of every rotation
-    const float* denom;          // per template penalty denominator, or nullptr
+    const float2* rot;           // (c_r, s_r) of every rotation; scaled: (a_kr, b_kr) at k * rotations + r
+    const float* denom;          // per template penalty denominator, or nullptr; scaled: per (t, k) at t * scales + k
     int32_t n_tmpl, rotations, tmpl_idx_base;
+    int32_t scales;              // 1 for the unscaled search
+    const float* scale;          // scaled: the s_k, or nullptr
+    float* rec_scale;            // scaled: n_rec grid scales of the records, written for the valid ones (or nullptr)
     int32_t lo_x, lo_y, stride;  // grid point (u, v) is the map pixel (lo_x + u stride, lo_y + v stride)
     int32_t nx, ny;              // grid points per row / column
     int32_t cell, cells_x, cells_y;
     int32_t band;                // cell rows per block of the evaluation kernel
     int32_t n_bands;             // ceil(cells_y / band)
-    int64_t n_rec;               // n_tmpl * rotations * cells_y * cells_x
+    int64_t n_rec;               // n_tmpl * scales * rotations * cells_y * cells_x
     unsigned long long* keys;    // n_rec: (score bits << 32 | grid index << 1 | score is NaN) of the cell's best, ~0 when none
     fdcm_match* rec;             // n_rec records and valid flags (the search's record buffers)
     uint8_t* valid;
@@ -227,7 +231,7 @@ __host__ __device__ inline void dense_pose(float c, float s, float ax, float ay,
     P[0] = c; P[1] = -s; P[2] = dense_tx(c, s, ax, ay, gx, shift_x);
     P[3] = s; P[4] = c;  P[5] = dense_ty(c, s, ax, ay, gy, shift_y);
 }
-// one block per (template, rotation, band of cell rows); atomicMin of the key per record.  keys must hold ~0 on entry.
+// one block per (template, scale, rotation, band of cell rows); atomicMin of the key per record.  keys must hold ~0 on entry.
 cudaError_t launch_dense_eval(const MapView& map, const SlopeTableDev& table, const DenseLaunch& p, int max_lines, int smem_optin,
                               cudaStream_t s);
 // keys -> records and valid flags (the winning pose recomputed from its grid index, the penalty applied)
@@ -293,8 +297,10 @@ struct FitLaunch {
     fdcm_fit_params prm;
     fdcm_match* out;             // n records
     fdcm_fit_stats* stats;       // n entries
+    int32_t scaled;              // 0: the rigid fit; 1: the scaled fit within [min_scale, max_scale]
+    float min_scale, max_scale;
 };
-// one warp per match
+// one warp per match; the rigid and the scaled fit are two instantiations of one kernel
 void launch_fit_eval(const FitLaunch& p, const SlopeTableDev& table, cudaStream_t s);
 
 void launch_evaluate(const MapView& map, const SlopeTableDev& table, const float4* d_lines, const int32_t* d_toff,

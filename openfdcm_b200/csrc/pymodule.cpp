@@ -328,20 +328,36 @@ PYBIND11_MODULE(_openfdcm_cuda, m) {
                    std::to_string(a.rotStep) + ", stride=" + std::to_string(a.stride) + ", cell=" + std::to_string(a.cell) + ">";
         });
 
+    py::class_<ScaleGrid>(m, "ScaleGrid")
+        .def(py::init([](int scales, float start, float ratio) { return ScaleGrid{scales, start, ratio}; }), "scales"_a = 1, "start"_a = 1.f,
+             "ratio"_a = 1.f)
+        .def_readwrite("scales", &ScaleGrid::scales)
+        .def_readwrite("start", &ScaleGrid::start)
+        .def_readwrite("ratio", &ScaleGrid::ratio)
+        .def("__repr__", [](const ScaleGrid& g) {
+            return "<ScaleGrid: scales=" + std::to_string(g.scales) + ", start=" + std::to_string(g.start) + ", ratio=" + std::to_string(g.ratio) +
+                   ">";
+        });
+
     m.def("search_dense",
           [](const Dt3Cuda& featuremap, const std::vector<LinesIn>& templates, const DenseSearch& dense, const ExponentialPenalty& penalty, int k,
              const std::optional<DistinctMatches>& select, const std::optional<PoseRefinement>& refine,
-             const std::optional<EdgeCoverage>& verify) {
+             const std::optional<EdgeCoverage>& verify, const std::optional<ScaleGrid>& scales) {
               const auto t = to_templates(templates);
               py::gil_scoped_release release;
-              if (verify) return searchDense(featuremap, t, dense, penalty, k, select ? &*select : nullptr, refine ? &*refine : nullptr, *verify);
-              return searchDense(featuremap, t, dense, penalty, k, select ? &*select : nullptr, refine ? &*refine : nullptr);
+              const DistinctMatches* sp = select ? &*select : nullptr;
+              const PoseRefinement* rp = refine ? &*refine : nullptr;
+              if (scales) return verify ? searchDense(featuremap, t, dense, *scales, penalty, k, sp, rp, *verify)
+                                        : searchDense(featuremap, t, dense, *scales, penalty, k, sp, rp);
+              if (verify) return searchDense(featuremap, t, dense, penalty, k, sp, rp, *verify);
+              return searchDense(featuremap, t, dense, penalty, k, sp, rp);
           },
           "featuremap"_a, "templates"_a, "dense"_a, "penalty"_a, "k"_a = 10, py::kw_only(), "select"_a = py::none(), "refine"_a = py::none(),
-          "verify"_a = py::none(),
+          "verify"_a = py::none(), "scales"_a = py::none(),
           "Dense pose-grid search on the device: the best pose of every (template, rotation, cell), then the top-k (ascending score) "
           "or with select the distinct top-k, then with refine the pose refinement of those; verify: EdgeCoverage whose "
-          "min_coverage > 0 drops records of lower coverage before the selection");
+          "min_coverage > 0 drops records of lower coverage before the selection; scales: a ScaleGrid searched as a further pose "
+          "dimension");
 
     py::class_<EdgeCoverage>(m, "EdgeCoverage")
         .def(py::init([](int radius, int bin_tolerance, float min_coverage) { return EdgeCoverage{radius, bin_tolerance, min_coverage}; }),
@@ -366,17 +382,19 @@ PYBIND11_MODULE(_openfdcm_cuda, m) {
           "edge pixel of similar orientation nearby; NaN where the posed template leaves the map");
 
     py::class_<PoseFit>(m, "PoseFit")
-        .def(py::init([](int iterations, float max_distance, float sample_step, int bin_tolerance, float tolerance, int min_inliers) {
-                 return PoseFit{iterations, max_distance, sample_step, bin_tolerance, tolerance, min_inliers};
+        .def(py::init([](int iterations, float max_distance, float sample_step, int bin_tolerance, float tolerance, int min_inliers,
+                         std::optional<std::pair<float, float>> scale_range) {
+                 return PoseFit{iterations, max_distance, sample_step, bin_tolerance, tolerance, min_inliers, scale_range};
              }),
              "iterations"_a = 10, "max_distance"_a = 3.f, "sample_step"_a = 2.f, "bin_tolerance"_a = 1, "tolerance"_a = 1e-3f,
-             "min_inliers"_a = 6)
+             "min_inliers"_a = 6, "scale_range"_a = py::none())
         .def_readwrite("iterations", &PoseFit::iterations)
         .def_readwrite("max_distance", &PoseFit::maxDistance)
         .def_readwrite("sample_step", &PoseFit::sampleStep)
         .def_readwrite("bin_tolerance", &PoseFit::binTolerance)
         .def_readwrite("tolerance", &PoseFit::tolerance)
         .def_readwrite("min_inliers", &PoseFit::minInliers)
+        .def_readwrite("scale_range", &PoseFit::scaleRange)
         .def("__repr__", [](const PoseFit& f) {
             return "<PoseFit: iterations=" + std::to_string(f.iterations) + ", max_distance=" + std::to_string(f.maxDistance) +
                    ", sample_step=" + std::to_string(f.sampleStep) + ", bin_tolerance=" + std::to_string(f.binTolerance) +

@@ -566,6 +566,14 @@ __device__ __forceinline__ bool anchors_near(const float4 a, const float4 b, con
     if (!(dx * dx + dy * dy <= p.r2)) return false;
     return p.any_angle || a.z * b.z + a.w * b.w >= p.cos_thr;
 }
+// near(a, b) of the scaled dense search: the angle test against cos_thr * (s_a * s_b), s_a and s_b the grid scales
+template <bool kScaled>
+__device__ __forceinline__ bool anchors_near(const float4 a, float sa, const float4 b, float sb, const SelectLaunch& p) {
+    if constexpr (!kScaled) return anchors_near(a, b, p);
+    const float dx = a.x - b.x, dy = a.y - b.y;
+    if (!(dx * dx + dy * dy <= p.r2)) return false;
+    return p.any_angle || a.z * b.z + a.w * b.w >= p.cos_thr * (sa * sb);
+}
 
 __device__ __forceinline__ void write_invalid(fdcm_match* out) {
     fdcm_match m;
@@ -617,9 +625,12 @@ void launch_select_sort(const SelectLaunch& p, bool by_template, uint64_t* keys_
 // exactly the walk over the global order.  The warp takes its sorted range 32 candidates at a time: each lane tests its
 // candidate against the template's accepted anchors, then the chunk is settled in order (the first live lane is accepted
 // and removes the live lanes near it).  The walk ends at min(cap, top_k) accepted or at the first invalid key.
+// kScaled: the grid scales of the accepted anchors follow the n_hyp anchors of acc
+template <bool kScaled>
 __global__ void __launch_bounds__(128) select_greedy_kernel(const __grid_constant__ SelectLaunch p, const uint64_t* __restrict__ skeys,
                                                             const int32_t* __restrict__ sh, uint32_t* __restrict__ surv_keys,
                                                             float4* __restrict__ acc) {
+    float* __restrict__ acc_s = reinterpret_cast<float*>(acc + p.n_hyp);
     const int lane = threadIdx.x & 31;
     const int t = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     if (t >= p.n_tmpl) return;   // whole warp
@@ -634,9 +645,11 @@ __global__ void __launch_bounds__(128) select_greedy_kernel(const __grid_constan
         const bool last_chunk = __ballot_sync(0xffffffffu, i < e && !live) != 0u;
         const int h = live ? sh[i] : 0;
         float4 me = make_float4(0.f, 0.f, 0.f, 0.f);
+        float me_s = 1.f;
         if (live && p.radius_on) {
             me = match_anchor(p.rec[h], anchor);
-            for (int j = 0; j < n_acc && live; ++j) live = !anchors_near(acc[b + j], me, p);
+            if constexpr (kScaled) me_s = p.rec_scale[h];
+            for (int j = 0; j < n_acc && live; ++j) live = !anchors_near<kScaled>(acc[b + j], kScaled ? acc_s[b + j] : 1.f, me, me_s, p);
         }
         for (;;) {
             const unsigned alive = __ballot_sync(0xffffffffu, live);
@@ -644,11 +657,15 @@ __global__ void __launch_bounds__(128) select_greedy_kernel(const __grid_constan
             const int ld = __ffs(alive) - 1;
             const float4 a = make_float4(__shfl_sync(0xffffffffu, me.x, ld), __shfl_sync(0xffffffffu, me.y, ld),
                                          __shfl_sync(0xffffffffu, me.z, ld), __shfl_sync(0xffffffffu, me.w, ld));
+            const float a_s = kScaled ? __shfl_sync(0xffffffffu, me_s, ld) : 1.f;
             if (lane == ld) {
                 surv_keys[h] = key;
-                if (p.radius_on) acc[b + n_acc] = me;
+                if (p.radius_on) {
+                    acc[b + n_acc] = me;
+                    if constexpr (kScaled) acc_s[b + n_acc] = me_s;
+                }
                 live = false;
-            } else if (live && p.radius_on && anchors_near(a, me, p)) {
+            } else if (live && p.radius_on && anchors_near<kScaled>(a, a_s, me, me_s, p)) {
                 live = false;
             }
             ++n_acc;
@@ -661,7 +678,8 @@ __global__ void __launch_bounds__(128) select_greedy_kernel(const __grid_constan
 void launch_select_greedy(const SelectLaunch& p, const uint64_t* sorted_keys, const int32_t* sorted_h, uint32_t* surv_keys, float4* acc,
                           cudaStream_t s) {
     cudaMemsetAsync(surv_keys, 0xFF, (size_t)p.n_hyp * 4, s);
-    select_greedy_kernel<<<(unsigned)((p.n_tmpl + 3) / 4), 128, 0, s>>>(p, sorted_keys, sorted_h, surv_keys, acc);
+    if (p.rec_scale) select_greedy_kernel<true><<<(unsigned)((p.n_tmpl + 3) / 4), 128, 0, s>>>(p, sorted_keys, sorted_h, surv_keys, acc);
+    else select_greedy_kernel<false><<<(unsigned)((p.n_tmpl + 3) / 4), 128, 0, s>>>(p, sorted_keys, sorted_h, surv_keys, acc);
 }
 
 __global__ void select_gather_kernel(const uint32_t* __restrict__ skeys, const int32_t* __restrict__ sh, long long n,
@@ -692,10 +710,12 @@ void launch_select_topk(const SelectLaunch& p, const uint32_t* surv_keys, uint32
 // across_templates != 0: one block walks the global (score, h) order blockDim candidates at a time.  Every thread tests its
 // candidate against the accepted list in shared memory (anchor, rotation, template: the per-template count for the cap is
 // taken in the same pass), then the chunk is settled in order like the warp version above.  Worst case H x top_k tests.
+template <bool kScaled>
 __global__ void __launch_bounds__(1024) select_walk_kernel(const __grid_constant__ SelectLaunch p, const uint64_t* __restrict__ skeys,
                                                            const int32_t* __restrict__ sh, fdcm_match* __restrict__ out,
                                                            int* __restrict__ n_out) {
     __shared__ float4 s_acc[kSelectMaxAcross];
+    __shared__ float s_acc_s[kScaled ? kSelectMaxAcross : 1];   // grid scales of the accepted records
     __shared__ int s_tmpl[kSelectMaxAcross];
     __shared__ unsigned s_live[32];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, n_warps = blockDim.x >> 5;
@@ -707,14 +727,16 @@ __global__ void __launch_bounds__(1024) select_walk_kernel(const __grid_constant
         const bool last_chunk = __syncthreads_or(!live) != 0;
         int h = 0, t = -1, same = 0;
         float4 me = make_float4(0.f, 0.f, 0.f, 0.f);
+        float me_s = 1.f;
         if (live) {
             h = sh[i];
             const fdcm_match m = p.rec[h];
             t = m.tmpl_idx - p.tmpl_idx_base;
             me = match_anchor(m, p.anchors[t]);
+            if constexpr (kScaled) me_s = p.rec_scale[h];
             for (int j = 0; j < n_acc && live; ++j) {
                 same += s_tmpl[j] == t;
-                live = !(p.radius_on && anchors_near(s_acc[j], me, p));
+                live = !(p.radius_on && anchors_near<kScaled>(s_acc[j], kScaled ? s_acc_s[j] : 1.f, me, me_s, p));
             }
             if (p.cap > 0 && same >= p.cap) live = false;
         }
@@ -728,18 +750,20 @@ __global__ void __launch_bounds__(1024) select_walk_kernel(const __grid_constant
             if (ld < 0) break;   // uniform
             if (tid == ld) {
                 s_acc[n_acc] = me;
+                if constexpr (kScaled) s_acc_s[n_acc] = me_s;
                 s_tmpl[n_acc] = t;
                 out[n_acc] = p.rec[h];
                 live = false;
             }
             __syncthreads();
             const float4 a = s_acc[n_acc];
+            const float a_s = kScaled ? s_acc_s[n_acc] : 1.f;
             const int at = s_tmpl[n_acc];
             ++n_acc;
             if (n_acc == p.top_k) break;   // uniform
             if (live) {
                 same += at == t;
-                if ((p.cap > 0 && same >= p.cap) || (p.radius_on && anchors_near(a, me, p))) live = false;
+                if ((p.cap > 0 && same >= p.cap) || (p.radius_on && anchors_near<kScaled>(a, a_s, me, me_s, p))) live = false;
             }
         }
         __syncthreads();   // s_live is rewritten by the next chunk
@@ -751,7 +775,8 @@ __global__ void __launch_bounds__(1024) select_walk_kernel(const __grid_constant
 
 void launch_select_walk(const SelectLaunch& p, const uint64_t* sorted_keys, const int32_t* sorted_h, fdcm_match* d_out, int* d_n_out,
                         cudaStream_t s) {
-    select_walk_kernel<<<1, 1024, 0, s>>>(p, sorted_keys, sorted_h, d_out, d_n_out);
+    if (p.rec_scale) select_walk_kernel<true><<<1, 1024, 0, s>>>(p, sorted_keys, sorted_h, d_out, d_n_out);
+    else select_walk_kernel<false><<<1, 1024, 0, s>>>(p, sorted_keys, sorted_h, d_out, d_n_out);
 }
 
 // =============================================================================================
@@ -949,12 +974,13 @@ __global__ void __launch_bounds__(kDenseThreads) dense_eval_kernel(const __grid_
                                                                    const __grid_constant__ SlopeTableDev table,
                                                                    const __grid_constant__ DenseLaunch p) {
     extern __shared__ __align__(16) uint8_t s_raw[];   // rotated end points float4[L], planes u8[L], as refinement
-    const long long tr = blockIdx.x / p.n_bands;
+    const long long tr = blockIdx.x / p.n_bands;   // (t * scales + k) * rotations + r
     const int band = (int)(blockIdx.x - tr * p.n_bands);
-    const int r = (int)(tr % p.rotations), t = (int)(tr / p.rotations);
+    const int per_t = p.scales * p.rotations;
+    const int kr = (int)(tr % per_t), t = (int)(tr / per_t);   // kr = k * rotations + r
     const int l0 = p.offsets[t], L = p.offsets[t + 1] - l0;
     if (L == 0) return;   // whole block: an empty template has no records
-    const float2 cs = p.rot[r], a = p.anchors[t];
+    const float2 cs = p.rot[kr], a = p.anchors[t];
     const float c = cs.x, s = cs.y;
     float4* apts = reinterpret_cast<float4*>(s_raw);
     uint8_t* bins = reinterpret_cast<uint8_t*>(apts + L);
@@ -975,7 +1001,7 @@ __global__ void __launch_bounds__(kDenseThreads) dense_eval_kernel(const __grid_
     if (ulo > uhi || vlo > vhi) return;   // uniform
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, n_warps = blockDim.x >> 5;
     const int n_chunks = (uhi - ulo + 32) / 32;
-    const long long rec0 = ((long long)t * p.rotations + r) * p.cells_y;
+    const long long rec0 = tr * p.cells_y;
     const int cv1 = min(p.cells_y, (band + 1) * p.band);
     for (int cv = band * p.band; cv < cv1; ++cv) {
         const int ra = max(cv * p.cell, vlo), rb = min(cv * p.cell + (p.cell - 1), vhi);
@@ -1019,7 +1045,7 @@ cudaError_t launch_dense_eval(const MapView& map, const SlopeTableDev& table, co
         const cudaError_t e = cudaFuncSetAttribute(dense_eval_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
     }
-    const long long blocks = (long long)p.n_tmpl * p.rotations * p.n_bands;   // <= n_rec < 2^31
+    const long long blocks = (long long)p.n_tmpl * p.scales * p.rotations * p.n_bands;   // <= n_rec < 2^31
     dense_eval_kernel<<<(unsigned)blocks, kDenseThreads, smem, s>>>(map, table, p);
     return cudaGetLastError();
 }
@@ -1032,15 +1058,16 @@ __global__ void dense_finish_kernel(const __grid_constant__ MapView map, const _
         p.valid[h] = 0;
         return;
     }
-    const long long tr = h / ((long long)p.cells_y * p.cells_x);
-    const int r = (int)(tr % p.rotations), t = (int)(tr / p.rotations);
+    const long long tr = h / ((long long)p.cells_y * p.cells_x);   // (t * scales + k) * rotations + r
+    const int r = (int)(tr % p.rotations), tk = (int)(tr / p.rotations), t = tk / p.scales, k = tk - t * p.scales;
     const unsigned g = (unsigned)key >> 1;
     const int u = (int)(g % (unsigned)p.nx), v = (int)(g / (unsigned)p.nx);
-    const float2 cs = p.rot[r], a = p.anchors[t];
+    const float2 cs = p.rot[k * p.rotations + r], a = p.anchors[t];
     fdcm_match m;
     m.tmpl_idx = t + p.tmpl_idx_base;
     const float raw = (key & 1ull) ? NAN : __uint_as_float((unsigned)(key >> 32));
-    m.score = p.denom ? raw / p.denom[t] : raw;
+    m.score = p.denom ? raw / p.denom[tk] : raw;
+    if (p.rec_scale) p.rec_scale[h] = p.scale[k];
     // the pose dense_eval_kernel scored, recomputed from its grid index
     dense_pose(cs.x, cs.y, a.x, a.y, p.lo_x + u * p.stride, p.lo_y + v * p.stride, map.shift_x, map.shift_y, m.transform);
     p.rec[h] = m;
