@@ -221,26 +221,58 @@ extern "C" fdcm_status fdcm_profile_get(int32_t index, char* name, int32_t name_
 extern "C" int64_t fdcm_kernel_launch_count(void) { return g_launches.load(); }
 
 // =============================================================================================
-// device buffer with grow-only capacity
+// owning buffers and events
 // =============================================================================================
-struct DevBuf {
+// grow-only buffer of exactly the bytes last asked for beyond its capacity, freed with its owner (the owner's device must
+// be current then): device memory, or page-locked host memory for truly asynchronous copies
+template <bool Pinned>
+struct Buf {
     void* p = nullptr;
     size_t cap = 0;
+    Buf() = default;
+    Buf(const Buf&) = delete;
+    Buf& operator=(const Buf&) = delete;
+    ~Buf() { free(); }
     cudaError_t reserve(size_t bytes) {
         if (bytes <= cap) return cudaSuccess;
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
-        cudaError_t e = cudaMalloc(&p, bytes);
+        free();
+        cudaError_t e = Pinned ? cudaMallocHost(&p, bytes) : cudaMalloc(&p, bytes);
         if (e == cudaSuccess) cap = bytes;
+        else p = nullptr;
         return e;
     }
-    void release() {
-        if (p) cudaFree(p);
+    template <class T> T* as() const { return reinterpret_cast<T*>(p); }
+
+private:
+    void free() {
+        if (p && Pinned) cudaFreeHost(p);
+        else if (p) cudaFree(p);
         p = nullptr;
         cap = 0;
     }
-    template <class T> T* as() const { return reinterpret_cast<T*>(p); }
+};
+using DevBuf = Buf<false>;
+using PinnedBuf = Buf<true>;
+
+// event without timing, created by its first record and destroyed with its owner
+struct LazyEvent {
+    cudaEvent_t e = nullptr;
+    LazyEvent() = default;
+    LazyEvent(const LazyEvent&) = delete;
+    LazyEvent& operator=(const LazyEvent&) = delete;
+    ~LazyEvent() {
+        if (e) cudaEventDestroy(e);
+    }
+    cudaError_t record(cudaStream_t s) {
+        if (!e) {
+            cudaError_t r = cudaEventCreateWithFlags(&e, cudaEventDisableTiming);
+            if (r != cudaSuccess) {
+                e = nullptr;
+                return r;
+            }
+        }
+        return cudaEventRecord(e, s);
+    }
 };
 
 // =============================================================================================
@@ -272,10 +304,10 @@ struct fdcm_dt3 {
     const void* plan_planes = nullptr;
     int plan_tables_depth = -1;
     int n_sms = 148;
-    cudaEvent_t ev_fork = nullptr, ev_join = nullptr;   // fork / join of the second stream inside a build
+    LazyEvent ev_fork, ev_join;   // fork / join of the second stream inside a build
     // recorded after everything that writes the map (build, rebuild, rerun, SceneBatch slot build, broadcast); every call that
     // reads or writes the map makes its stream wait on it, so work queued on another stream stays ordered before it
-    cudaEvent_t ev_written = nullptr;
+    LazyEvent ev_written;
     bool band_path = false, band_l1 = false;   // which distance-transform formulation this map uses (set by prepare)
     // search workspace (mutable state of the last search on this map)
     mutable std::mutex search_mutex;
@@ -302,13 +334,13 @@ struct fdcm_dt3 {
     mutable DevBuf cov_tmp, cov_dil, cov_io, cov_out;
     mutable uint64_t cov_gen = 0;
     mutable int cov_radius = -1, cov_tol = -1;
-    mutable cudaEvent_t cov_ev = nullptr;
+    mutable LazyEvent cov_ev;
     // pose fit: the scene-line grid of fit_md for the map write fit_gen (0: none) and the call's buffers; fit_ev is recorded
     // after the grid build, which later calls on any stream wait on
     mutable DevBuf fit_cnt, fit_off, fit_items, fit_tmp, fit_in, fit_out, fit_st;
     mutable uint64_t fit_gen = 0;
     mutable float fit_md = 0.f;
-    mutable cudaEvent_t fit_ev = nullptr;
+    mutable LazyEvent fit_ev;
     mutable float s_scene_min[2] = {0.f, 0.f}, s_scene_max[2] = {0.f, 0.f};   // bbox of the resident search scene
     mutable std::mutex host_tset_mutex;
     mutable fdcm_templates* host_tset = nullptr;   // reusable template set of fdcm_search_host
@@ -320,28 +352,12 @@ struct fdcm_dt3 {
     std::vector<float> h_build_scene;   // host copy of the build scene (for scene == NULL searches with a new filter)
     mutable int64_t last_n_hyp = 0;
     mutable fdcm_search_stats last_stats{};
-    mutable void* h_scene_stage = nullptr;   // pinned staging for the search-scene upload (truly asynchronous copies)
-    mutable size_t h_scene_stage_cap = 0;
-    mutable cudaEvent_t scene_stage_ev = nullptr;
-    mutable void* h_pinned = nullptr;   // pinned staging for match download
-    mutable size_t h_pinned_cap = 0;
+    mutable PinnedBuf h_scene_stage;   // staging for the search-scene upload (truly asynchronous copies)
+    mutable LazyEvent scene_stage_ev;
+    mutable PinnedBuf h_pinned;        // staging for match download
 
     ~fdcm_dt3() {
-        cudaSetDevice(device);
-        for (DevBuf* b : {&planes, &mask, &stack, &lines, &bins, &band_info, &band_spill, &integ_items, &s_scene, &s_sorted_len, &s_sorted_idx, &s_hyp_off, &s_rec,
-                          &s_valid, &s_hyp, &s_counters, &s_topk_score, &s_topk_idx, &s_topk_out, &s_topk_n, &s_keys, &s_keys2, &s_idx,
-                          &s_perm, &s_sort_tmp, &s_sel_keys, &s_sel_keys2, &s_sel_vals, &s_sel_vals2, &s_sel_surv, &s_sel_acc,
-                          &s_sel_tmp, &s_ref_state, &s_ref_keys, &s_ref_io, &s_denom, &s_dense_keys, &s_dense_rot, &s_dense_rs, &cov_tmp, &cov_dil,
-                          &cov_io, &cov_out, &fit_cnt, &fit_off, &fit_items, &fit_tmp, &fit_in, &fit_out, &fit_st})
-            b->release();
-        if (h_pinned) cudaFreeHost(h_pinned);
-        if (ev_fork) cudaEventDestroy(ev_fork);
-        if (ev_join) cudaEventDestroy(ev_join);
-        if (ev_written) cudaEventDestroy(ev_written);
-        if (cov_ev) cudaEventDestroy(cov_ev);
-        if (fit_ev) cudaEventDestroy(fit_ev);
-        if (h_scene_stage) cudaFreeHost(h_scene_stage);
-        if (scene_stage_ev) cudaEventDestroy(scene_stage_ev);
+        cudaSetDevice(device);   // (the members free their device memory after this)
         destroy_host_tset();
     }
     void destroy_host_tset();
@@ -357,15 +373,22 @@ struct SceneFilter { bool on; float cx, cy, lo, hi; };
 // SceneBatch builds on a stream of its own, so stream order alone does not put a call after a queued build of the same map.
 // The caller holds m->search_mutex.
 static fdcm_status map_wait(const fdcm_dt3* m, cudaStream_t s) {
-    if (m->ev_written) CUDA_TRY(cudaStreamWaitEvent(s, m->ev_written, 0));
+    if (m->ev_written.e) CUDA_TRY(cudaStreamWaitEvent(s, m->ev_written.e, 0));
     return FDCM_OK;
 }
 // (the first call comes from the map's first build, before the handle is visible to any other call)
 static fdcm_status map_written(fdcm_dt3* m, cudaStream_t s) {
-    if (!m->ev_written) CUDA_TRY(cudaEventCreateWithFlags(&m->ev_written, cudaEventDisableTiming));
-    CUDA_TRY(cudaEventRecord(m->ev_written, s));
+    CUDA_TRY(m->ev_written.record(s));
     ++m->write_gen;
     return FDCM_OK;
+}
+
+// Opening of a call on map m, for a caller that holds m->search_mutex: the map's device, the caller's stream of it, and
+// that stream ordered after the last write of the map
+static fdcm_status begin_map_call(const fdcm_dt3* m, cudaStream_t* s) {
+    CUDA_TRY(cudaSetDevice(m->device));
+    if (fdcm_status st = get_stream(m->device, s)) return st;
+    return map_wait(m, *s);
 }
 
 // filterInRange (searchstrategies/concentricrange.h:73-84)
@@ -415,16 +438,10 @@ static fdcm_status upload_search_scene(const fdcm_dt3* m, const float* scene, in
     // through pinned staging: the copies queue behind whatever runs on the stream (e.g. the map build) without making the
     // host wait for it, which a copy from pageable memory would
     const size_t need = (size_t)n_scene * 16 + (size_t)ns * 8;
-    if (!m->scene_stage_ev) CUDA_TRY(cudaEventCreateWithFlags(&m->scene_stage_ev, cudaEventDisableTiming));
-    else CUDA_TRY(cudaEventSynchronize(m->scene_stage_ev));   // the staging buffer may still feed the previous upload
-    if (m->h_scene_stage_cap < need) {
-        if (m->h_scene_stage) cudaFreeHost(m->h_scene_stage);
-        m->h_scene_stage = nullptr;
-        m->h_scene_stage_cap = 0;
-        CUDA_TRY(cudaMallocHost(&m->h_scene_stage, need));
-        m->h_scene_stage_cap = need;
-    }
-    unsigned char* st = static_cast<unsigned char*>(m->h_scene_stage);
+    // the staging buffer may still feed the previous upload
+    if (m->scene_stage_ev.e) CUDA_TRY(cudaEventSynchronize(m->scene_stage_ev.e));
+    CUDA_TRY(m->h_scene_stage.reserve(need));
+    unsigned char* st = m->h_scene_stage.as<unsigned char>();
     std::memcpy(st, scene, (size_t)n_scene * 16);
     CUDA_TRY(cudaMemcpyAsync(m->s_scene.p, st, (size_t)n_scene * 16, cudaMemcpyHostToDevice, s));
     if (ns) {
@@ -433,7 +450,7 @@ static fdcm_status upload_search_scene(const fdcm_dt3* m, const float* scene, in
         CUDA_TRY(cudaMemcpyAsync(m->s_sorted_len.p, st + (size_t)n_scene * 16, (size_t)ns * 4, cudaMemcpyHostToDevice, s));
         CUDA_TRY(cudaMemcpyAsync(m->s_sorted_idx.p, st + (size_t)n_scene * 16 + (size_t)ns * 4, (size_t)ns * 4, cudaMemcpyHostToDevice, s));
     }
-    CUDA_TRY(cudaEventRecord(m->scene_stage_ev, s));
+    CUDA_TRY(m->scene_stage_ev.record(s));
     m->s_scene_n = n_scene;
     m->s_sorted_n = ns;
     m->s_filter_on = flt.on;
@@ -677,10 +694,8 @@ static fdcm_status run_build_kernels(fdcm_dt3* m, cudaStream_t s) {
             // far rows under them.
             cudaStream_t sa;
             if (fdcm_status st = get_aux_stream(m->device, &sa)) return st;
-            if (!m->ev_fork) CUDA_TRY(cudaEventCreateWithFlags(&m->ev_fork, cudaEventDisableTiming));
-            if (!m->ev_join) CUDA_TRY(cudaEventCreateWithFlags(&m->ev_join, cudaEventDisableTiming));
-            CUDA_TRY(cudaEventRecord(m->ev_fork, s));
-            CUDA_TRY(cudaStreamWaitEvent(sa, m->ev_fork, 0));
+            CUDA_TRY(m->ev_fork.record(s));
+            CUDA_TRY(cudaStreamWaitEvent(sa, m->ev_fork.e, 0));
             {
                 KernelScope k("dt_row_envelope", (double)dt_band_info_bytes(dm), sa);
                 launch_dt_row_envelope(m->band_info.p, nullptr, dm, m->band_spill.p, m->col_lo, m->col_hi, m->row_lo, m->row_hi, 1, sa);
@@ -696,7 +711,7 @@ static fdcm_status run_build_kernels(fdcm_dt3* m, cudaStream_t s) {
                 launch_dt_fill_propagate(m->planes.as<float>(), dm, m->band_spill.p, m->col_lo, m->col_hi, m->prop, dist == FDCM_L2, ys0, ys1, 0,
                                          0, sa);
             }
-            CUDA_TRY(cudaEventRecord(m->ev_join, sa));
+            CUDA_TRY(m->ev_join.record(sa));
             {
                 KernelScope k("dt_row_envelope_far", (double)dt_band_info_bytes(dm), s);
                 launch_dt_row_envelope(m->band_info.p, nullptr, dm, m->band_spill.p, m->col_lo, m->col_hi, m->row_lo, m->row_hi, 2, s);
@@ -710,7 +725,7 @@ static fdcm_status run_build_kernels(fdcm_dt3* m, cudaStream_t s) {
                 launch_dt_fill_propagate(m->planes.as<float>(), dm, m->band_spill.p, m->col_lo, m->col_hi, m->prop, dist == FDCM_L2, 0, ys0, ys1,
                                          dm.H, s);
             }
-            CUDA_TRY(cudaStreamWaitEvent(s, m->ev_join, 0));
+            CUDA_TRY(cudaStreamWaitEvent(s, m->ev_join.e, 0));
         } else {
             {
                 KernelScope k("dt_row_envelope", (double)dt_band_info_bytes(dm), s);
@@ -771,6 +786,16 @@ static fdcm_status run_build_kernels(fdcm_dt3* m, cudaStream_t s) {
     return FDCM_OK;
 }
 
+// Queues the whole build of a scene into map m on `s`, ordered after the map's last write (none before its first build).
+// (m->search_mutex held, or the handle not yet visible to any other call)
+static fdcm_status queue_build(fdcm_dt3* m, const float* scene, int32_t n_lines, cudaStream_t s) {
+    if (fdcm_status st = map_wait(m, s)) return st;
+    if (fdcm_status st = prepare_and_upload(m, scene, n_lines, s)) return st;
+    if (fdcm_status st = run_build_kernels(m, s)) return st;
+    if (fdcm_status st = upload_build_scene(m, scene, n_lines, s)) return st;
+    return map_written(m, s);
+}
+
 static fdcm_status validate_params(const fdcm_dt3_params* p) {
     if (!p) return fail(FDCM_ERR_INVALID, "params is null");
     if (p->depth < 1 || p->depth > kMaxDepth) return fail(FDCM_ERR_INVALID, "depth must be in 1..64");
@@ -793,10 +818,7 @@ extern "C" fdcm_status fdcm_dt3_build(const float* scene_xyxy, int32_t n_lines, 
     m->params = *params;
     m->device = device;
     m->stage = stage;
-    fdcm_status st = prepare_and_upload(m, scene_xyxy, n_lines, s);
-    if (st == FDCM_OK) st = run_build_kernels(m, s);
-    if (st == FDCM_OK) st = upload_build_scene(m, scene_xyxy, n_lines, s);
-    if (st == FDCM_OK) st = map_written(m, s);
+    fdcm_status st = queue_build(m, scene_xyxy, n_lines, s);
     if (st == FDCM_OK) {
         cudaError_t e = cudaStreamSynchronize(s);
         if (e != cudaSuccess) st = fail(FDCM_ERR_CUDA, std::string("build: ") + cudaGetErrorString(e));
@@ -828,20 +850,14 @@ static void invalidate_map(fdcm_dt3* m) {
 static fdcm_status rebuild_impl(fdcm_dt3* m, const float* scene_xyxy, int32_t n_lines, bool wait) {
     if (!m) return fail(FDCM_ERR_INVALID, "map is null");
     if (n_lines < 0 || (n_lines > 0 && !scene_xyxy)) return fail(FDCM_ERR_INVALID, "bad scene");
+    std::lock_guard<std::mutex> lk(m->search_mutex);   // a search on this handle must not see a half-replaced map
     CUDA_TRY(cudaSetDevice(m->device));
     cudaStream_t s;
     if (fdcm_status st = get_stream(m->device, &s)) return st;
-    std::lock_guard<std::mutex> lk(m->search_mutex);   // a search on this handle must not see a half-replaced map
-    fdcm_status st = map_wait(m, s);   // an earlier build of this map queued on another stream must not overlap this one
-    if (st == FDCM_OK) st = prepare_and_upload(m, scene_xyxy, n_lines, s);
-    if (st == FDCM_OK) st = run_build_kernels(m, s);
-    if (st == FDCM_OK) st = upload_build_scene(m, scene_xyxy, n_lines, s);
-    if (st == FDCM_OK) st = map_written(m, s);
+    fdcm_status st = queue_build(m, scene_xyxy, n_lines, s);
     if (st != FDCM_OK) {
-        const std::string msg = g_last_error;
         cudaStreamSynchronize(s);
         invalidate_map(m);
-        g_last_error = msg;
     }
     if (st == FDCM_OK && wait) {
         cudaError_t e = cudaStreamSynchronize(s);
@@ -863,33 +879,24 @@ extern "C" fdcm_status fdcm_dt3_rebuild_async(fdcm_dt3* m, const float* scene_xy
     return rebuild_impl(m, scene_xyxy, n_lines, false);
 }
 
-extern "C" fdcm_status fdcm_dt3_rerun(fdcm_dt3* m) {
+static fdcm_status rerun_impl(fdcm_dt3* m, bool wait) {
     if (!m) return fail(FDCM_ERR_INVALID, "map is null");
-    CUDA_TRY(cudaSetDevice(m->device));
-    cudaStream_t s;
-    if (fdcm_status st = get_stream(m->device, &s)) return st;
     std::lock_guard<std::mutex> lk(m->search_mutex);
-    fdcm_status st = map_wait(m, s);
+    cudaStream_t s;
+    fdcm_status st = begin_map_call(m, &s);
     if (st == FDCM_OK) st = run_build_kernels(m, s);
     if (st == FDCM_OK) st = map_written(m, s);
-    if (st == FDCM_OK) {
+    if (st == FDCM_OK && wait) {
         cudaError_t e = cudaStreamSynchronize(s);
         if (e != cudaSuccess) st = fail(FDCM_ERR_CUDA, std::string("rerun: ") + cudaGetErrorString(e));
     }
-    prof_resolve();
+    if (wait) prof_resolve();
     return st;
 }
 
-extern "C" fdcm_status fdcm_dt3_rerun_async(fdcm_dt3* m) {
-    if (!m) return fail(FDCM_ERR_INVALID, "map is null");
-    CUDA_TRY(cudaSetDevice(m->device));
-    cudaStream_t s;
-    if (fdcm_status st = get_stream(m->device, &s)) return st;
-    std::lock_guard<std::mutex> lk(m->search_mutex);
-    if (fdcm_status st = map_wait(m, s)) return st;
-    if (fdcm_status st = run_build_kernels(m, s)) return st;
-    return map_written(m, s);
-}
+extern "C" fdcm_status fdcm_dt3_rerun(fdcm_dt3* m) { return rerun_impl(m, true); }
+
+extern "C" fdcm_status fdcm_dt3_rerun_async(fdcm_dt3* m) { return rerun_impl(m, false); }
 
 extern "C" fdcm_status fdcm_dt3_retain(fdcm_dt3* m) {
     if (!m) return fail(FDCM_ERR_INVALID, "map is null");
@@ -927,11 +934,9 @@ extern "C" fdcm_status fdcm_dt3_angles(const fdcm_dt3* m, float* keys) {
 extern "C" fdcm_status fdcm_dt3_download_plane(const fdcm_dt3* m, int32_t plane, float* dst) {
     if (!m || !dst) return fail(FDCM_ERR_INVALID, "null argument");
     if (plane < 0 || plane >= m->dm.D) return fail(FDCM_ERR_INVALID, "plane out of range");
-    CUDA_TRY(cudaSetDevice(m->device));
-    cudaStream_t s;   // a legacy-stream copy would not be ordered after an async rebuild
-    if (fdcm_status st = get_stream(m->device, &s)) return st;
     std::lock_guard<std::mutex> lk(m->search_mutex);
-    if (fdcm_status st = map_wait(m, s)) return st;
+    cudaStream_t s;   // a legacy-stream copy would not be ordered after an async rebuild
+    if (fdcm_status st = begin_map_call(m, &s)) return st;
     const float* src = m->planes.as<float>() + (size_t)plane * m->dm.plane_elems;
     CUDA_TRY(cudaMemcpy2DAsync(dst, (size_t)m->dm.W * 4, src, (size_t)m->dm.pitch * 4, (size_t)m->dm.W * 4, m->dm.H,
                                cudaMemcpyDeviceToHost, s));
@@ -942,11 +947,9 @@ extern "C" fdcm_status fdcm_dt3_download_plane(const fdcm_dt3* m, int32_t plane,
 extern "C" fdcm_status fdcm_dt3_download_mask(const fdcm_dt3* m, int32_t plane, uint8_t* dst) {
     if (!m || !dst) return fail(FDCM_ERR_INVALID, "null argument");
     if (plane < 0 || plane >= m->dm.D) return fail(FDCM_ERR_INVALID, "plane out of range");
-    CUDA_TRY(cudaSetDevice(m->device));
-    cudaStream_t s;
-    if (fdcm_status st = get_stream(m->device, &s)) return st;
     std::lock_guard<std::mutex> lk(m->search_mutex);
-    if (fdcm_status st = map_wait(m, s)) return st;
+    cudaStream_t s;
+    if (fdcm_status st = begin_map_call(m, &s)) return st;
     std::vector<uint32_t> w((size_t)m->dm.H * m->dm.wwords);
     CUDA_TRY(cudaMemcpyAsync(w.data(), m->mask.as<uint32_t>() + (size_t)plane * m->dm.H * m->dm.wwords, w.size() * 4,
                              cudaMemcpyDeviceToHost, s));
@@ -995,16 +998,13 @@ extern "C" fdcm_status fdcm_dt3_evaluate(const fdcm_dt3* m, const float* tmpl_li
     if (n_scores <= 0) return FDCM_OK;
     if (!scores || !translations || (n_lines > 0 && !tmpl_lines)) return fail(FDCM_ERR_INVALID, "null argument");
     if (m->dm.D == 0) return fail(FDCM_ERR_INVALID, "evaluate on an empty feature map");
-    CUDA_TRY(cudaSetDevice(m->device));
-    cudaStream_t s;
-    if (fdcm_status st = get_stream(m->device, &s)) return st;
     std::lock_guard<std::mutex> lk(m->search_mutex);
-    if (fdcm_status st = map_wait(m, s)) return st;
+    cudaStream_t s;
+    if (fdcm_status st = begin_map_call(m, &s)) return st;
     std::vector<int32_t> owner((size_t)n_scores);
     for (int t = 0; t < n_tmpl; ++t)
         for (int i = transl_offsets[t]; i < transl_offsets[t + 1]; ++i) owner[i] = t;
     DevBuf dl, doff, dtr, down, dsc;
-    auto cleanup = [&]() { for (DevBuf* b : {&dl, &doff, &dtr, &down, &dsc}) b->release(); };
     cudaError_t e = cudaSuccess;
     if (e == cudaSuccess) e = dl.reserve(std::max<size_t>(16, (size_t)n_lines * 16));
     if (e == cudaSuccess) e = doff.reserve((size_t)(n_tmpl + 1) * 4);
@@ -1024,7 +1024,6 @@ extern "C" fdcm_status fdcm_dt3_evaluate(const fdcm_dt3* m, const float* tmpl_li
     if (e == cudaSuccess) e = cudaMemcpyAsync(scores, dsc.p, (size_t)n_scores * 4, cudaMemcpyDeviceToHost, s);
     if (e == cudaSuccess) e = cudaStreamSynchronize(s);
     prof_resolve();
-    cleanup();
     if (e != cudaSuccess) return fail(FDCM_ERR_CUDA, std::string("evaluate: ") + cudaGetErrorString(e));
     return FDCM_OK;
 }
@@ -1033,11 +1032,9 @@ extern "C" fdcm_status fdcm_dt3_classify(const fdcm_dt3* m, const float* lines, 
     if (!m || (n > 0 && (!lines || !bins))) return fail(FDCM_ERR_INVALID, "null argument");
     if (n <= 0) return FDCM_OK;
     if (m->dm.D == 0) return fail(FDCM_ERR_INVALID, "classify on an empty feature map");
-    CUDA_TRY(cudaSetDevice(m->device));
-    cudaStream_t s;
-    if (fdcm_status st = get_stream(m->device, &s)) return st;
     std::lock_guard<std::mutex> lk(m->search_mutex);
-    if (fdcm_status st = map_wait(m, s)) return st;
+    cudaStream_t s;
+    if (fdcm_status st = begin_map_call(m, &s)) return st;
     DevBuf dl, db;
     cudaError_t e = dl.reserve((size_t)n * 16);
     if (e == cudaSuccess) e = db.reserve((size_t)n * 4);
@@ -1050,8 +1047,6 @@ extern "C" fdcm_status fdcm_dt3_classify(const fdcm_dt3* m, const float* lines, 
     if (e == cudaSuccess) e = cudaMemcpyAsync(bins, db.p, (size_t)n * 4, cudaMemcpyDeviceToHost, s);
     if (e == cudaSuccess) e = cudaStreamSynchronize(s);
     prof_resolve();
-    dl.release();
-    db.release();
     if (e != cudaSuccess) return fail(FDCM_ERR_CUDA, std::string("classify: ") + cudaGetErrorString(e));
     return FDCM_OK;
 }
@@ -1093,25 +1088,10 @@ struct fdcm_templates {
     uint64_t load_id = 0;             // unique over all loads of all sets: keys the maps' denominator caches
     std::mutex mu;
     // uploads run on the copy stream (they overlap a map build in flight on the main stream); consumers wait on `ready`
-    cudaEvent_t ready = nullptr;
+    LazyEvent ready;
     std::atomic<bool> upload_pending{false};   // (read by searches of other maps sharing the set)
-    void* h_stage = nullptr;          // pinned staging for the small per-search uploads (denominators, hypothesis offsets)
-    size_t h_stage_cap = 0;
-    cudaError_t stage_reserve(size_t bytes) {
-        if (bytes <= h_stage_cap) return cudaSuccess;
-        if (h_stage) cudaFreeHost(h_stage);
-        h_stage = nullptr;
-        h_stage_cap = 0;
-        cudaError_t e = cudaMallocHost(&h_stage, bytes);
-        if (e == cudaSuccess) h_stage_cap = bytes;
-        return e;
-    }
-    ~fdcm_templates() {
-        cudaSetDevice(device);
-        if (ready) cudaEventDestroy(ready);
-        if (h_stage) cudaFreeHost(h_stage);
-        for (DevBuf* b : {&lines, &offs, &argsort, &line_len, &anchors}) b->release();
-    }
+    PinnedBuf h_stage;                // staging for the small per-search uploads (denominators, hypothesis offsets)
+    ~fdcm_templates() { cudaSetDevice(device); }
 };
 
 // small persistent worker pool for the O(#templates) host preparation (std::sort per template)
@@ -1272,10 +1252,12 @@ static void template_host_prep(const float* tl, const int32_t* off, int32_t T, f
 }
 
 // (re)load a template set into an existing object: device buffers grow only, host scratch is reused
-// make the main stream wait for a template upload in flight on the copy stream
-static fdcm_status templates_ready(fdcm_templates* t, cudaStream_t s) {
+// begin_map_call for a call that also reads template set t: the stream also waits for an upload of t in flight on the copy
+// stream
+static fdcm_status begin_tset_call(const fdcm_dt3* m, fdcm_templates* t, cudaStream_t* s) {
+    if (fdcm_status st = begin_map_call(m, s)) return st;
     if (t->upload_pending) {
-        CUDA_TRY(cudaStreamWaitEvent(s, t->ready, 0));
+        CUDA_TRY(cudaStreamWaitEvent(*s, t->ready.e, 0));
         t->upload_pending = false;
     }
     return FDCM_OK;
@@ -1290,7 +1272,6 @@ static fdcm_status templates_load(fdcm_templates* t, const float* tmpl_lines, co
     (void)main_stream;
     cudaStream_t s;
     if (fdcm_status st = get_copy_stream(t->device, &s)) return st;
-    if (!t->ready) CUDA_TRY(cudaEventCreateWithFlags(&t->ready, cudaEventDisableTiming));
     if (n_tmpl < 0 || !tmpl_offsets) return fail(FDCM_ERR_INVALID, "bad template offsets");
     for (int i = 0; i < n_tmpl; ++i)
         if (tmpl_offsets[i + 1] < tmpl_offsets[i]) return fail(FDCM_ERR_INVALID, "template offsets must be non-decreasing");
@@ -1318,7 +1299,7 @@ static fdcm_status templates_load(fdcm_templates* t, const float* tmpl_lines, co
     if (e == cudaSuccess && n) e = cudaMemcpyAsync(t->line_len.p, t->h_line_len.data(), (size_t)n * 4, cudaMemcpyHostToDevice, s);
     if (e == cudaSuccess && n_tmpl) e = cudaMemcpyAsync(t->anchors.p, t->h_anchors.data(), (size_t)n_tmpl * 8, cudaMemcpyHostToDevice, s);
     // no host synchronisation needed: pageable sources are staged by the runtime before the call returns
-    if (e == cudaSuccess) e = cudaEventRecord(t->ready, s);
+    if (e == cudaSuccess) e = t->ready.record(s);
     if (e != cudaSuccess)
         return fail(e == cudaErrorMemoryAllocation ? FDCM_ERR_NOMEM : FDCM_ERR_CUDA,
                     std::string("templates_load: ") + cudaGetErrorString(e));
@@ -1337,7 +1318,7 @@ extern "C" fdcm_status fdcm_templates_create(const float* tmpl_lines, const int3
     if (!t) return fail(FDCM_ERR_NOMEM, "host allocation failed");
     t->device = device;
     fdcm_status st = templates_load(t, tmpl_lines, tmpl_offsets, n_tmpl, s);
-    if (st == FDCM_OK && cudaEventSynchronize(t->ready) != cudaSuccess) st = fail(FDCM_ERR_CUDA, "templates_create: upload failed");
+    if (st == FDCM_OK && cudaEventSynchronize(t->ready.e) != cudaSuccess) st = fail(FDCM_ERR_CUDA, "templates_create: upload failed");
     if (st == FDCM_OK) t->upload_pending = false;
     if (st != FDCM_OK) {
         delete t;
@@ -1425,7 +1406,6 @@ struct fdcm_comm {
     DevBuf gather, merged, merged_n;
     ~fdcm_comm() {
         cudaSetDevice(device);
-        for (DevBuf* b : {&gather, &merged, &merged_n}) b->release();
         if (comm) nccl_api().CommDestroy(comm);
     }
 };
@@ -1583,18 +1563,18 @@ static fdcm_status stage_uploads(const fdcm_dt3* m, fdcm_templates* t, const int
     std::lock_guard<std::mutex> lk(t->mu);
     cudaStream_t cs;
     if (fdcm_status st = get_copy_stream(m->device, &cs)) return st;
-    if (!t->ready) CUDA_TRY(cudaEventCreateWithFlags(&t->ready, cudaEventDisableTiming));
-    else CUDA_TRY(cudaEventSynchronize(t->ready));   // the staging buffer may still feed an earlier upload (other threads)
+    // the staging buffer may still feed an earlier upload (other threads)
+    if (t->ready.e) CUDA_TRY(cudaEventSynchronize(t->ready.e));
     const size_t off_bytes = n_off * 8, den_bytes = (size_t)t->n_tmpl * (1 + scales.size()) * 4;
-    CUDA_TRY(t->stage_reserve(std::max<size_t>(16, off_bytes + den_bytes)));
-    unsigned char* stage = static_cast<unsigned char*>(t->h_stage);
+    CUDA_TRY(t->h_stage.reserve(std::max<size_t>(16, off_bytes + den_bytes)));
+    unsigned char* stage = t->h_stage.as<unsigned char>();
     if (off_bytes) {
         std::memcpy(stage, hyp_off, off_bytes);
         CUDA_TRY(cudaMemcpyAsync(m->s_hyp_off.p, stage, off_bytes, cudaMemcpyHostToDevice, cs));
     }
     if (fdcm_status st = map_denominators(m, t, kind, tau, scales, reinterpret_cast<float*>(stage + off_bytes), cs, d_denom)) return st;
-    CUDA_TRY(cudaEventRecord(t->ready, cs));
-    CUDA_TRY(cudaStreamWaitEvent(s, t->ready, 0));
+    CUDA_TRY(t->ready.record(cs));
+    CUDA_TRY(cudaStreamWaitEvent(s, t->ready.e, 0));
     t->upload_pending = false;   // (this event is recorded after any template upload on the same copy stream)
     return FDCM_OK;
 }
@@ -1624,10 +1604,18 @@ static fdcm_status check_select(const fdcm_select_params* q, int32_t top_k, bool
     return FDCM_OK;
 }
 
+// check_select of a distinct top-K, if any; with caps and radius both off it is the plain top-K (*q becomes nullptr)
+static fdcm_status select_or_plain(const fdcm_select_params** q, int32_t top_k, bool comm) {
+    if (!*q) return FDCM_OK;
+    if (fdcm_status st = check_select(*q, top_k, comm)) return st;
+    if ((*q)->max_per_template == 0 && !((*q)->radius > 0.f)) *q = nullptr;
+    return FDCM_OK;
+}
+
 // Distinct top-K over the records the search kernel just queued on `s`: writes s_topk_out / s_topk_n like the top-K kernels
 // rec_scale: the grid scale of every record (the scaled dense search), or nullptr
-static fdcm_status run_select(const fdcm_dt3* m, const fdcm_templates* t, const fdcm_search_params* p, const fdcm_select_params* q,
-                              int64_t H, cudaStream_t s, const float* rec_scale = nullptr) {
+static fdcm_status run_select(const fdcm_dt3* m, const fdcm_templates* t, int32_t top_k, int32_t tmpl_idx_base,
+                              const fdcm_select_params* q, int64_t H, cudaStream_t s, const float* rec_scale) {
     if (H >= ((int64_t)1 << 31)) return fail(FDCM_ERR_INVALID, "distinct top-K: more than 2^31 - 1 hypotheses");
     SelectLaunch sp;
     sp.rec = m->s_rec.as<fdcm_match>();
@@ -1636,8 +1624,8 @@ static fdcm_status run_select(const fdcm_dt3* m, const fdcm_templates* t, const 
     sp.anchors = t->anchors.as<float2>();
     sp.n_hyp = H;
     sp.n_tmpl = t->n_tmpl;
-    sp.tmpl_idx_base = p->tmpl_idx_base;
-    sp.top_k = p->top_k;
+    sp.tmpl_idx_base = tmpl_idx_base;
+    sp.top_k = top_k;
     sp.cap = q->max_per_template;
     sp.radius_on = q->radius > 0.f;
     sp.r2 = q->radius * q->radius;
@@ -1704,6 +1692,24 @@ static void refine_level_table(const fdcm_refine_params* r, int level, RefineLev
 // at most this many matches per call: the evaluation grid has (2 rot_steps + 1) blocks per match
 static constexpr int64_t kRefineMaxMatches = ((int64_t)1 << 31) / kRefineSide;
 
+// the top-K of a search whose matches are refined
+static fdcm_status check_refine_top_k(int32_t top_k) {
+    if (top_k < 1 || top_k > kRefineMaxMatches)
+        return fail(FDCM_ERR_INVALID, "pose refinement: top_k must be in 1.." + std::to_string(kRefineMaxMatches));
+    return FDCM_OK;
+}
+
+// in[0..n) all name templates of a set of n_tmpl starting at tmpl_idx_base
+static fdcm_status check_match_indices(const fdcm_match* in, int64_t n, int32_t tmpl_idx_base, int32_t n_tmpl) {
+    for (int64_t i = 0; i < n; ++i) {
+        const int64_t t = (int64_t)in[i].tmpl_idx - tmpl_idx_base;
+        if (t < 0 || t >= n_tmpl)
+            return fail(FDCM_ERR_OUT_OF_RANGE, "match " + std::to_string(i) + ": tmpl_idx " + std::to_string(in[i].tmpl_idx) +
+                                                   " outside the template set");
+    }
+    return FDCM_OK;
+}
+
 // Refinement of the n (or *d_n <= n) matches at d_in, queued on `s`; the refined records go to d_out (which may be d_in)
 static fdcm_status run_refine(const fdcm_dt3* m, const fdcm_templates* t, int32_t tmpl_idx_base, const float* d_denom,
                               const fdcm_refine_params* r, const fdcm_match* d_in, const int* d_n, int n, fdcm_match* d_out,
@@ -1741,6 +1747,34 @@ static fdcm_status run_refine(const fdcm_dt3* m, const fdcm_templates* t, int32_
     return FDCM_OK;
 }
 
+// The top_k best of the H records at s_rec / s_valid that a search queued on `s`: the distinct selection (sel) or the plain
+// top-K, the refinement of the result (ref, or nullptr), then its download (merged over the ranks of comm, or nullptr; with
+// counters, also the search's counters).  rec_scale: as in run_select.
+static fdcm_status run_topk(const fdcm_dt3* m, const fdcm_templates* t, int32_t top_k, int32_t tmpl_idx_base, const fdcm_select_params* sel,
+                            const fdcm_refine_params* ref, int64_t H, const float* rec_scale, const float* d_denom, int smem_optin,
+                            fdcm_comm* comm, unsigned long long* counters, cudaStream_t s, fdcm_match* out, int64_t capacity,
+                            int64_t* n_out) {
+    const int k = top_k;
+    CUDA_TRY(m->s_topk_out.reserve((size_t)k * sizeof(fdcm_match)));
+    CUDA_TRY(m->s_topk_n.reserve(4));
+    if (sel) {
+        if (fdcm_status st = run_select(m, t, top_k, tmpl_idx_base, sel, H, s, rec_scale)) return st;
+    } else {
+        const int blocks = topk_ws_blocks(H);
+        CUDA_TRY(m->s_topk_score.reserve((size_t)blocks * k * 4));
+        CUDA_TRY(m->s_topk_idx.reserve((size_t)blocks * k * 8));
+        KernelScope ks("topk", 0.0, s, 2);   // two kernels in this scope
+        launch_topk(m->s_rec.as<fdcm_match>(), m->s_valid.as<uint8_t>(), H, k, m->s_topk_score.as<float>(), m->s_topk_idx.as<int64_t>(),
+                    blocks, m->s_topk_out.as<fdcm_match>(), m->s_topk_n.as<int>(), s);
+    }
+    CUDA_TRY(cudaGetLastError());
+    if (ref)
+        if (fdcm_status st = run_refine(m, t, tmpl_idx_base, d_denom, ref, m->s_topk_out.as<fdcm_match>(), m->s_topk_n.as<int>(), k,
+                                        m->s_topk_out.as<fdcm_match>(), smem_optin, s))
+            return st;
+    return finish_topk(m, comm, k, s, counters, out, capacity, n_out);
+}
+
 // parameters of the match verification (fdcm_match_coverage and the coverage filter)
 static fdcm_status check_coverage(const fdcm_coverage_params* c) {
     if (!c) return fail(FDCM_ERR_INVALID, "cov is null");
@@ -1773,13 +1807,12 @@ static fdcm_status coverage_mask(const fdcm_dt3* m, const fdcm_coverage_params* 
                                    m->cov_dil.as<uint32_t>(), s);
         }
         CUDA_TRY(cudaGetLastError());
-        if (!m->cov_ev) CUDA_TRY(cudaEventCreateWithFlags(&m->cov_ev, cudaEventDisableTiming));
-        CUDA_TRY(cudaEventRecord(m->cov_ev, s));
+        CUDA_TRY(m->cov_ev.record(s));
         m->cov_gen = m->write_gen;
         m->cov_radius = c->radius;
         m->cov_tol = c->bin_tolerance;
     }
-    CUDA_TRY(cudaStreamWaitEvent(s, m->cov_ev, 0));   // a dilation queued by an earlier call on another stream
+    CUDA_TRY(cudaStreamWaitEvent(s, m->cov_ev.e, 0));   // a dilation queued by an earlier call on another stream
     return FDCM_OK;
 }
 
@@ -1818,10 +1851,7 @@ static fdcm_status search_impl(const fdcm_dt3* m, const fdcm_templates* tc, cons
                                const fdcm_coverage_params* cov = nullptr) {
     if (!m || !tc || !p || !n_out) return fail(FDCM_ERR_INVALID, "null argument");
     *n_out = 0;
-    if (sel)
-        if (fdcm_status st = check_select(sel, p->top_k, comm != nullptr)) return st;
-    // caps and radius both off: the selection is the plain top-K
-    if (sel && sel->max_per_template == 0 && !(sel->radius > 0.f)) sel = nullptr;
+    if (fdcm_status st = select_or_plain(&sel, p->top_k, comm != nullptr)) return st;
     if (comm && p->top_k <= 0) return fail(FDCM_ERR_INVALID, "the multi-GPU search needs top_k > 0");
 #define FDCM_NO_LOCAL_MATCHES() do { if (comm) return exchange_empty(m, comm, p->top_k, out, capacity, n_out); return FDCM_OK; } while (0)
     if (p->max_tmpl_lines < 0 || p->max_scene_lines < 0 || p->batch_size < 0 || p->top_k < 0 || p->penalty_kind < 0 ||
@@ -1844,11 +1874,8 @@ static fdcm_status search_impl(const fdcm_dt3* m, const fdcm_templates* tc, cons
     }
     if (t->n_tmpl == 0 || n_scene <= 0 || (m->dm.W == 0 && m->dm.H == 0)) FDCM_NO_LOCAL_MATCHES();
     if (m->stage != 0) return fail(FDCM_ERR_INVALID, "feature map was built with a debug stage");
-    CUDA_TRY(cudaSetDevice(m->device));
     cudaStream_t s;
-    if (fdcm_status st = get_stream(m->device, &s)) return st;
-    if (fdcm_status st = map_wait(m, s)) return st;
-    if (fdcm_status st = templates_ready(t, s)) return st;
+    if (fdcm_status st = begin_tset_call(m, t, &s)) return st;
     int smem_optin = 0;
     if (fdcm_status st = search_smem_optin(m->device, t->max_lines, &smem_optin)) return st;
 
@@ -1943,42 +1970,14 @@ static fdcm_status search_impl(const fdcm_dt3* m, const fdcm_templates* tc, cons
     unsigned long long counters[3] = {0, 0, 0};
     fdcm_status result = FDCM_OK;
     if (p->top_k > 0) {
-        const int k = p->top_k;
-        if (sel) {
-            CUDA_TRY(m->s_topk_out.reserve((size_t)k * sizeof(fdcm_match)));
-            CUDA_TRY(m->s_topk_n.reserve(4));
-            if (fdcm_status st = run_select(m, t, p, sel, H, s)) return st;
-        } else {
-            const int blocks = topk_ws_blocks(H);
-            CUDA_TRY(m->s_topk_score.reserve((size_t)blocks * k * 4));
-            CUDA_TRY(m->s_topk_idx.reserve((size_t)blocks * k * 8));
-            CUDA_TRY(m->s_topk_out.reserve((size_t)k * sizeof(fdcm_match)));
-            CUDA_TRY(m->s_topk_n.reserve(4));
-            {
-                KernelScope ks("topk", 0.0, s, 2);   // two kernels in this scope
-                launch_topk(so.rec, so.valid, H, k, m->s_topk_score.as<float>(), m->s_topk_idx.as<int64_t>(), blocks,
-                            m->s_topk_out.as<fdcm_match>(), m->s_topk_n.as<int>(), s);
-            }
-            CUDA_TRY(cudaGetLastError());
-        }
-        if (ref)
-            if (fdcm_status st = run_refine(m, t, p->tmpl_idx_base, d_denom, ref, m->s_topk_out.as<fdcm_match>(), m->s_topk_n.as<int>(), k,
-                                            m->s_topk_out.as<fdcm_match>(), smem_optin, s))
-                return st;
-        result = finish_topk(m, comm, k, s, counters, out, capacity, n_out);
+        result = run_topk(m, t, p->top_k, p->tmpl_idx_base, sel, ref, H, nullptr, d_denom, smem_optin, comm, counters, s, out, capacity,
+                          n_out);
         if (result != FDCM_OK && result != FDCM_ERR_CAPACITY) return result;
     } else {
         // every match in hypothesis order: download records + flags, compact on the host
-        const size_t need = (size_t)H * sizeof(fdcm_match) + (size_t)H;
-        if (m->h_pinned_cap < need) {
-            if (m->h_pinned) cudaFreeHost(m->h_pinned);
-            m->h_pinned = nullptr;
-            m->h_pinned_cap = 0;
-            CUDA_TRY(cudaMallocHost(&m->h_pinned, need));
-            m->h_pinned_cap = need;
-        }
-        fdcm_match* h_rec = (fdcm_match*)m->h_pinned;
-        uint8_t* h_valid = (uint8_t*)m->h_pinned + (size_t)H * sizeof(fdcm_match);
+        CUDA_TRY(m->h_pinned.reserve((size_t)H * sizeof(fdcm_match) + (size_t)H));
+        fdcm_match* h_rec = m->h_pinned.as<fdcm_match>();
+        uint8_t* h_valid = m->h_pinned.as<uint8_t>() + (size_t)H * sizeof(fdcm_match);
         CUDA_TRY(cudaMemcpyAsync(h_rec, so.rec, (size_t)H * sizeof(fdcm_match), cudaMemcpyDeviceToHost, s));
         CUDA_TRY(cudaMemcpyAsync(h_valid, so.valid, (size_t)H, cudaMemcpyDeviceToHost, s));
         CUDA_TRY(cudaMemcpyAsync(counters, m->s_counters.p, 3 * 8, cudaMemcpyDeviceToHost, s));
@@ -2017,8 +2016,7 @@ extern "C" fdcm_status fdcm_search_refine(const fdcm_dt3* m, const fdcm_template
                                           fdcm_match* out, int64_t capacity, int64_t* n_out) {
     if (fdcm_status st = check_refine(refine)) return st;
     if (!p) return fail(FDCM_ERR_INVALID, "null argument");
-    if (p->top_k < 1 || p->top_k > kRefineMaxMatches)
-        return fail(FDCM_ERR_INVALID, "pose refinement: top_k must be in 1.." + std::to_string(kRefineMaxMatches));
+    if (fdcm_status st = check_refine_top_k(p->top_k)) return st;
     return search_impl(m, tc, scene, n_scene, p, out, capacity, n_out, nullptr, select, refine);
 }
 
@@ -2030,8 +2028,7 @@ extern "C" fdcm_status fdcm_search_verify(const fdcm_dt3* m, const fdcm_template
     if (p->top_k < 1) return fail(FDCM_ERR_INVALID, "verified search: top_k must be >= 1");
     if (refine) {
         if (fdcm_status st = check_refine(refine)) return st;
-        if (p->top_k > kRefineMaxMatches)
-            return fail(FDCM_ERR_INVALID, "pose refinement: top_k must be in 1.." + std::to_string(kRefineMaxMatches));
+        if (fdcm_status st = check_refine_top_k(p->top_k)) return st;
     }
     return search_impl(m, tc, scene, n_scene, p, out, capacity, n_out, nullptr, select, refine, cov->min_coverage > 0.f ? cov : nullptr);
 }
@@ -2048,19 +2045,11 @@ extern "C" fdcm_status fdcm_refine_matches(const fdcm_dt3* m, const fdcm_templat
     if (tc->device != m->device) return fail(FDCM_ERR_INVALID, "templates and feature map live on different devices");
     if (m->stage != 0) return fail(FDCM_ERR_INVALID, "feature map was built with a debug stage");
     if (m->dm.D == 0) return fail(FDCM_ERR_INVALID, "refine on an empty feature map");
-    for (int64_t i = 0; i < n; ++i) {
-        const int64_t t = (int64_t)in[i].tmpl_idx - tmpl_idx_base;
-        if (t < 0 || t >= tc->n_tmpl)
-            return fail(FDCM_ERR_OUT_OF_RANGE, "match " + std::to_string(i) + ": tmpl_idx " + std::to_string(in[i].tmpl_idx) +
-                                                   " outside the template set");
-    }
+    if (fdcm_status st = check_match_indices(in, n, tmpl_idx_base, tc->n_tmpl)) return st;
     fdcm_templates* t = const_cast<fdcm_templates*>(tc);
     std::lock_guard<std::mutex> lk(m->search_mutex);
-    CUDA_TRY(cudaSetDevice(m->device));
     cudaStream_t s;
-    if (fdcm_status st = get_stream(m->device, &s)) return st;
-    if (fdcm_status st = map_wait(m, s)) return st;
-    if (fdcm_status st = templates_ready(t, s)) return st;
+    if (fdcm_status st = begin_tset_call(m, t, &s)) return st;
     int smem_optin = 0;
     if (fdcm_status st = search_smem_optin(m->device, t->max_lines, &smem_optin)) return st;
     CUDA_TRY(m->s_ref_io.reserve((size_t)n * sizeof(fdcm_match)));
@@ -2177,12 +2166,10 @@ static fdcm_status dense_impl(const fdcm_dt3* m, const fdcm_templates* tc, const
     const int S = grid ? (int)scales.size() : 1;
     if (penalty_kind < 0 || penalty_kind > 2) return fail(FDCM_ERR_INVALID, "bad penalty kind");
     if (top_k < 1) return fail(FDCM_ERR_INVALID, "dense search: top_k must be >= 1");
-    if (sel)
-        if (fdcm_status st = check_select(sel, top_k, false)) return st;
-    if (sel && sel->max_per_template == 0 && !(sel->radius > 0.f)) sel = nullptr;   // the plain top-K
+    if (fdcm_status st = select_or_plain(&sel, top_k, false)) return st;
     if (ref) {
         if (fdcm_status st = check_refine(ref)) return st;
-        if (top_k > kRefineMaxMatches) return fail(FDCM_ERR_INVALID, "pose refinement: top_k must be in 1.." + std::to_string(kRefineMaxMatches));
+        if (fdcm_status st = check_refine_top_k(top_k)) return st;
     }
     if (tc->device != m->device) return fail(FDCM_ERR_INVALID, "templates and feature map live on different devices");
     if (m->stage != 0) return fail(FDCM_ERR_INVALID, "feature map was built with a debug stage");
@@ -2191,11 +2178,8 @@ static fdcm_status dense_impl(const fdcm_dt3* m, const fdcm_templates* tc, const
     // The records, their valid flags and the per-template offsets go to the search's buffers, so that the selection runs
     // unchanged; the hypothesis list and the counters of the last fdcm_search (s_hyp, last_n_hyp, last_stats) stay as they are.
     std::lock_guard<std::mutex> lk(m->search_mutex);
-    CUDA_TRY(cudaSetDevice(m->device));
     cudaStream_t s;
-    if (fdcm_status st = get_stream(m->device, &s)) return st;
-    if (fdcm_status st = map_wait(m, s)) return st;
-    if (fdcm_status st = templates_ready(t, s)) return st;
+    if (fdcm_status st = begin_tset_call(m, t, &s)) return st;
     int smem_optin = 0;
     if (fdcm_status st = search_smem_optin(m->device, t->max_lines, &smem_optin)) return st;
     const DenseGrid g = dense_grid(dense, m->shift, m->dm.W, m->dm.H);
@@ -2269,28 +2253,8 @@ static fdcm_status dense_impl(const fdcm_dt3* m, const fdcm_templates* tc, const
     }
     if (cov)
         if (fdcm_status st = run_coverage(m, t, tmpl_idx_base, cov, dl.rec, H, nullptr, dl.valid, s)) return st;
-    const int k = top_k;
-    CUDA_TRY(m->s_topk_out.reserve((size_t)k * sizeof(fdcm_match)));
-    CUDA_TRY(m->s_topk_n.reserve(4));
-    if (sel) {
-        fdcm_search_params sp{};
-        sp.top_k = k;
-        sp.tmpl_idx_base = tmpl_idx_base;
-        if (fdcm_status st = run_select(m, t, &sp, sel, H, s, dl.rec_scale)) return st;
-    } else {
-        const int blocks = topk_ws_blocks(H);
-        CUDA_TRY(m->s_topk_score.reserve((size_t)blocks * k * 4));
-        CUDA_TRY(m->s_topk_idx.reserve((size_t)blocks * k * 8));
-        KernelScope ks("topk", 0.0, s, 2);   // two kernels in this scope
-        launch_topk(dl.rec, dl.valid, H, k, m->s_topk_score.as<float>(), m->s_topk_idx.as<int64_t>(), blocks, m->s_topk_out.as<fdcm_match>(),
-                    m->s_topk_n.as<int>(), s);
-    }
-    CUDA_TRY(cudaGetLastError());
-    if (ref)
-        if (fdcm_status st = run_refine(m, t, tmpl_idx_base, d_denom, ref, m->s_topk_out.as<fdcm_match>(), m->s_topk_n.as<int>(), k,
-                                        m->s_topk_out.as<fdcm_match>(), smem_optin, s))
-            return st;
-    const fdcm_status result = finish_topk(m, nullptr, k, s, nullptr, out, capacity, n_out);
+    const fdcm_status result =
+        run_topk(m, t, top_k, tmpl_idx_base, sel, ref, H, dl.rec_scale, d_denom, smem_optin, nullptr, nullptr, s, out, capacity, n_out);
     prof_resolve();
     return result;
 }
@@ -2332,23 +2296,15 @@ extern "C" fdcm_status fdcm_match_coverage(const fdcm_dt3* m, const fdcm_templat
     if (!in || !coverage) return fail(FDCM_ERR_INVALID, "null argument");
     if (tc->device != m->device) return fail(FDCM_ERR_INVALID, "templates and feature map live on different devices");
     if (m->stage != 0) return fail(FDCM_ERR_INVALID, "feature map was built with a debug stage");
-    for (int64_t i = 0; i < n; ++i) {
-        const int64_t t = (int64_t)in[i].tmpl_idx - tmpl_idx_base;
-        if (t < 0 || t >= tc->n_tmpl)
-            return fail(FDCM_ERR_OUT_OF_RANGE, "match " + std::to_string(i) + ": tmpl_idx " + std::to_string(in[i].tmpl_idx) +
-                                                   " outside the template set");
-    }
+    if (fdcm_status st = check_match_indices(in, n, tmpl_idx_base, tc->n_tmpl)) return st;
     fdcm_templates* t = const_cast<fdcm_templates*>(tc);
     std::lock_guard<std::mutex> lk(m->search_mutex);
     if (m->dm.D == 0 || m->dm.W == 0 || m->dm.H == 0) {   // empty map (rule 2)
         for (int64_t i = 0; i < n; ++i) coverage[i] = NAN;
         return FDCM_OK;
     }
-    CUDA_TRY(cudaSetDevice(m->device));
     cudaStream_t s;
-    if (fdcm_status st = get_stream(m->device, &s)) return st;
-    if (fdcm_status st = map_wait(m, s)) return st;
-    if (fdcm_status st = templates_ready(t, s)) return st;
+    if (fdcm_status st = begin_tset_call(m, t, &s)) return st;
     CUDA_TRY(m->cov_io.reserve((size_t)n * sizeof(fdcm_match)));
     CUDA_TRY(m->cov_out.reserve((size_t)n * 4));
     CUDA_TRY(cudaMemcpyAsync(m->cov_io.p, in, (size_t)n * sizeof(fdcm_match), cudaMemcpyHostToDevice, s));
@@ -2399,12 +2355,11 @@ static fdcm_status fit_grid(const fdcm_dt3* m, float max_distance, cudaStream_t 
                                  m->fit_cnt.as<unsigned long long>(), m->fit_items.as<int32_t>(), s);
         }
         CUDA_TRY(cudaGetLastError());
-        if (!m->fit_ev) CUDA_TRY(cudaEventCreateWithFlags(&m->fit_ev, cudaEventDisableTiming));
-        CUDA_TRY(cudaEventRecord(m->fit_ev, s));
+        CUDA_TRY(m->fit_ev.record(s));
         m->fit_gen = m->write_gen;
         m->fit_md = max_distance;
     }
-    CUDA_TRY(cudaStreamWaitEvent(s, m->fit_ev, 0));   // a grid queued by an earlier call on another stream
+    CUDA_TRY(cudaStreamWaitEvent(s, m->fit_ev.e, 0));   // a grid queued by an earlier call on another stream
     return FDCM_OK;
 }
 
@@ -2420,12 +2375,7 @@ static fdcm_status fit_impl(const fdcm_dt3* m, const fdcm_templates* tc, int32_t
     if (n >= ((int64_t)1 << 34)) return fail(FDCM_ERR_INVALID, "pose fit: at most 2^34 - 1 matches per call");   // (one warp each)
     if (tc->device != m->device) return fail(FDCM_ERR_INVALID, "templates and feature map live on different devices");
     if (m->stage != 0) return fail(FDCM_ERR_INVALID, "feature map was built with a debug stage");
-    for (int64_t i = 0; i < n; ++i) {
-        const int64_t t = (int64_t)in[i].tmpl_idx - tmpl_idx_base;
-        if (t < 0 || t >= tc->n_tmpl)
-            return fail(FDCM_ERR_OUT_OF_RANGE, "match " + std::to_string(i) + ": tmpl_idx " + std::to_string(in[i].tmpl_idx) +
-                                                   " outside the template set");
-    }
+    if (fdcm_status st = check_match_indices(in, n, tmpl_idx_base, tc->n_tmpl)) return st;
     fdcm_templates* t = const_cast<fdcm_templates*>(tc);
     std::lock_guard<std::mutex> lk(m->search_mutex);
     if (m->dm.D == 0 || m->dm.W == 0 || m->dm.H == 0) {   // empty map: every input is invalid (rule 6)
@@ -2436,11 +2386,8 @@ static fdcm_status fit_impl(const fdcm_dt3* m, const fdcm_templates* tc, int32_t
         }
         return FDCM_OK;
     }
-    CUDA_TRY(cudaSetDevice(m->device));
     cudaStream_t s;
-    if (fdcm_status st = get_stream(m->device, &s)) return st;
-    if (fdcm_status st = map_wait(m, s)) return st;
-    if (fdcm_status st = templates_ready(t, s)) return st;
+    if (fdcm_status st = begin_tset_call(m, t, &s)) return st;
     CUDA_TRY(m->fit_in.reserve((size_t)n * sizeof(fdcm_match)));
     CUDA_TRY(m->fit_out.reserve((size_t)n * sizeof(fdcm_match)));
     if (stats) CUDA_TRY(m->fit_st.reserve((size_t)n * sizeof(fdcm_fit_stats)));
@@ -2584,10 +2531,10 @@ extern "C" fdcm_status fdcm_comm_rebuild_broadcast(fdcm_comm* comm, fdcm_dt3* m,
     if (root < 0 || root >= comm->world) return fail(FDCM_ERR_INVALID, "bad root");
     if (n_lines < 0 || (n_lines > 0 && !scene_xyxy)) return fail(FDCM_ERR_INVALID, "bad scene");
     if (m->stage != 0) return fail(FDCM_ERR_INVALID, "feature map was built with a debug stage");
+    std::lock_guard<std::mutex> lk(m->search_mutex);
     CUDA_TRY(cudaSetDevice(m->device));
     cudaStream_t s;
     if (fdcm_status st = get_stream(m->device, &s)) return st;
-    std::lock_guard<std::mutex> lk(m->search_mutex);
     fdcm_status st = map_wait(m, s);
     if (st == FDCM_OK) st = prepare_and_upload(m, scene_xyxy, n_lines, s);
     if (st == FDCM_OK && comm->rank == root) st = run_build_kernels(m, s);
@@ -2600,11 +2547,7 @@ extern "C" fdcm_status fdcm_comm_rebuild_broadcast(fdcm_comm* comm, fdcm_dt3* m,
     if (st == FDCM_OK) st = map_written(m, s);
     if (st == FDCM_OK && cudaStreamSynchronize(s) != cudaSuccess) st = fail(FDCM_ERR_CUDA, "rebuild_broadcast: stream failed");
     prof_resolve();
-    if (st != FDCM_OK) {
-        const std::string msg = g_last_error;
-        invalidate_map(m);
-        g_last_error = msg;
-    }
+    if (st != FDCM_OK) invalidate_map(m);   // (no synchronisation: a failed peer may never finish the collective)
     return st;
 }
 
@@ -2661,19 +2604,12 @@ extern "C" fdcm_status fdcm_scene_batch_destroy(fdcm_scene_batch* b) {
 static fdcm_status batch_queue_build(fdcm_scene_batch* b, int slot, const float* scene, int32_t n_lines) {
     fdcm_dt3* m = b->maps[slot];
     std::lock_guard<std::mutex> lk(m->search_mutex);
-    fdcm_status st = map_wait(m, b->build_stream);
-    if (st == FDCM_OK) st = prepare_and_upload(m, scene, n_lines, b->build_stream);
-    if (st == FDCM_OK) st = run_build_kernels(m, b->build_stream);
-    if (st == FDCM_OK) st = upload_build_scene(m, scene, n_lines, b->build_stream);
-    if (st == FDCM_OK) st = map_written(m, b->build_stream);
+    const fdcm_status st = queue_build(m, scene, n_lines, b->build_stream);
     if (st != FDCM_OK) {
-        const std::string msg = g_last_error;
         cudaStreamSynchronize(b->build_stream);
         invalidate_map(m);
-        g_last_error = msg;
-        return st;
     }
-    return FDCM_OK;
+    return st;
 }
 
 static fdcm_status search_scenes_impl(fdcm_scene_batch* b, const float* scene_lines, const int32_t* scene_offsets, int32_t n_scenes,
@@ -2732,17 +2668,14 @@ extern "C" fdcm_status fdcm_optimize(const fdcm_dt3* m, const float* tmpl_lines,
     if (m->stage != 0) return fail(FDCM_ERR_INVALID, "feature map was built with a debug stage");
     const int64_t n_lines = tmpl_offsets[n_tmpl];
     if (n_lines > 0 && !tmpl_lines) return fail(FDCM_ERR_INVALID, "tmpl_lines is null");
-    CUDA_TRY(cudaSetDevice(m->device));
-    cudaStream_t s;
-    if (fdcm_status st = get_stream(m->device, &s)) return st;
     std::lock_guard<std::mutex> lk(m->search_mutex);
-    if (fdcm_status st = map_wait(m, s)) return st;
+    cudaStream_t s;
+    if (fdcm_status st = begin_map_call(m, &s)) return st;
     int max_lines = 1;
     for (int t = 0; t < n_tmpl; ++t) max_lines = std::max(max_lines, tmpl_offsets[t + 1] - tmpl_offsets[t]);
     int smem_optin = 0;
     if (fdcm_status st = search_smem_optin(m->device, max_lines, &smem_optin)) return st;
     DevBuf dl, doff, dal, drec, dval, dcnt;
-    auto cleanup = [&]() { for (DevBuf* b : {&dl, &doff, &dal, &drec, &dval, &dcnt}) b->release(); };
     std::vector<fdcm_match> rec((size_t)n_tmpl);
     cudaError_t e = dl.reserve(std::max<size_t>(16, (size_t)n_lines * 16));
     if (e == cudaSuccess) e = doff.reserve((size_t)(n_tmpl + 1) * 4);
@@ -2777,7 +2710,6 @@ extern "C" fdcm_status fdcm_optimize(const fdcm_dt3* m, const float* tmpl_lines,
     if (e == cudaSuccess) e = cudaMemcpyAsync(has_value, dval.p, (size_t)n_tmpl, cudaMemcpyDeviceToHost, s);
     if (e == cudaSuccess) e = cudaStreamSynchronize(s);
     prof_resolve();
-    cleanup();
     if (e != cudaSuccess) return fail(FDCM_ERR_CUDA, std::string("optimize: ") + cudaGetErrorString(e));
     for (int t = 0; t < n_tmpl; ++t) {
         if (has_value[t]) {
@@ -2946,7 +2878,6 @@ extern "C" fdcm_status fdcm_debug_dt_rows(const uint16_t* g_rows, int32_t n_rows
     if (e == cudaSuccess) e = cudaMemcpy2DAsync(out, (size_t)n * 4, dp.p, (size_t)dm.pitch * 4, (size_t)n * 4, n_rows, cudaMemcpyDeviceToHost, s);
     if (e == cudaSuccess) e = cudaStreamSynchronize(s);
     prof_resolve();
-    dg.release(); dp.release(); ds.release();
     if (e != cudaSuccess) return fail(FDCM_ERR_CUDA, std::string("debug_dt_rows: ") + cudaGetErrorString(e));
     return FDCM_OK;
 }

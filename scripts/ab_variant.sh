@@ -9,7 +9,8 @@ out=build/ab/$name
 mkdir -p $out
 NVCCFLAGS="-gencode arch=compute_100a,code=sm_100a -std=c++17 -O3 -lineinfo -fmad=false -prec-div=true -prec-sqrt=true -Xcompiler -fPIC,-O3,-fno-math-errno,-ffp-contract=off"
 objs=""
-for f in fdcm_api dt3_kernels dt_band_kernels integral_tma search_kernels; do
+for cu in $(sed -n 's/^SRCS *= *//p' $src/Makefile); do   # every source the library links, as the Makefile lists them
+  f=${cu%.cu}
   if [[ " $* " == *" $f.cu "* ]]; then
     /usr/local/cuda/bin/nvcc $NVCCFLAGS $flags -c $src/$f.cu -o $out/$f.o
     objs="$objs $out/$f.o"
