@@ -2106,13 +2106,6 @@ static fdcm_status check_dense(const fdcm_dense_params* d) {
     return FDCM_OK;
 }
 
-// rule 1: cosine and sine of rotation r
-static void dense_rotation(const fdcm_dense_params* d, int r, float* c, float* s) {
-    const double th = (double)d->rot_start + (double)r * (double)d->rot_step;
-    *c = (float)std::cos(th);
-    *s = (float)std::sin(th);
-}
-
 // scaled dense search, rule 1: the scales s_k of a grid, or FDCM_ERR_INVALID
 static fdcm_status dense_scales(const fdcm_scale_grid* g, std::vector<float>* out) {
     if (!g) return fail(FDCM_ERR_INVALID, "scales is null");
@@ -2130,7 +2123,8 @@ static fdcm_status dense_scales(const fdcm_scale_grid* g, std::vector<float>* ou
     return FDCM_OK;
 }
 
-// scaled dense search, rule 1: the pose matrix entries (a, b) of scale s_k and rotation r
+// rule 1: the pose matrix entries (a, b) of scale s_k and rotation r; at s_k = 1.0f these are (c_r, s_r) of the unscaled
+// search, (float)((double)1.0f * cos th) == (float)cos th
 static void dense_scaled_rotation(const fdcm_dense_params* d, float sk, int r, float* a, float* b) {
     const double th = (double)d->rot_start + (double)r * (double)d->rot_step;
     *a = (float)((double)sk * std::cos(th));
@@ -2201,8 +2195,7 @@ static fdcm_status dense_impl(const fdcm_dt3* m, const fdcm_templates* tc, const
     for (int k = 0; k < S; ++k)
         for (int r = 0; r < dense->rotations; ++r) {
             float* cs = &rot[2 * ((size_t)k * dense->rotations + r)];
-            if (grid) dense_scaled_rotation(dense, scales[(size_t)k], r, cs, cs + 1);
-            else dense_rotation(dense, r, cs, cs + 1);
+            dense_scaled_rotation(dense, grid ? scales[(size_t)k] : 1.0f, r, cs, cs + 1);
         }
     std::copy(scales.begin(), scales.end(), rot.begin() + 2 * SR);
     if (grid) CUDA_TRY(m->s_dense_rs.reserve((size_t)H * 4));
@@ -2460,25 +2453,31 @@ extern "C" fdcm_status fdcm_fit_samples(const float* tl, int32_t n_lines, float 
     return FDCM_OK;
 }
 
-extern "C" fdcm_status fdcm_dense_poses(const fdcm_dense_params* dense, const float anchor[2], const float shift[2], int32_t width,
-                                        int32_t height, int32_t rotation, float* out, int64_t capacity, int64_t* n_out, int32_t grid_wh[2]) {
-    if (fdcm_status st = check_dense(dense)) return st;
-    if (!anchor || !shift || !n_out || !grid_wh) return fail(FDCM_ERR_INVALID, "null argument");
-    if (width < 0 || height < 0) return fail(FDCM_ERR_INVALID, "width and height must be >= 0");
-    if (rotation < 0 || rotation >= dense->rotations) return fail(FDCM_ERR_INVALID, "rotation must be in 0..rotations - 1");
+// the poses of fdcm_dense_poses / fdcm_dense_scaled_poses at scale sk and rotation r, after their argument checks
+static fdcm_status dense_poses(const fdcm_dense_params* dense, float sk, int r, const float anchor[2], const float shift[2], int32_t width,
+                               int32_t height, float* out, int64_t capacity, int64_t* n_out, int32_t grid_wh[2]) {
     const DenseGrid g = dense_grid(dense, shift, width, height);
     grid_wh[0] = g.nx;
     grid_wh[1] = g.ny;
     const int64_t n = (int64_t)g.nx * g.ny;
     *n_out = n;
     if (n > capacity || (n > 0 && !out)) return fail(FDCM_ERR_CAPACITY, "output buffer too small");
-    float c, s;
-    dense_rotation(dense, rotation, &c, &s);
+    float a, b;
+    dense_scaled_rotation(dense, sk, r, &a, &b);
     for (int v = 0; v < g.ny; ++v)
         for (int u = 0; u < g.nx; ++u)
-            dense_pose(c, s, anchor[0], anchor[1], g.lo_x + u * dense->stride, g.lo_y + v * dense->stride, shift[0], shift[1],
+            dense_pose(a, b, anchor[0], anchor[1], g.lo_x + u * dense->stride, g.lo_y + v * dense->stride, shift[0], shift[1],
                        out + 6 * ((size_t)v * g.nx + u));
     return FDCM_OK;
+}
+
+extern "C" fdcm_status fdcm_dense_poses(const fdcm_dense_params* dense, const float anchor[2], const float shift[2], int32_t width,
+                                        int32_t height, int32_t rotation, float* out, int64_t capacity, int64_t* n_out, int32_t grid_wh[2]) {
+    if (fdcm_status st = check_dense(dense)) return st;
+    if (!anchor || !shift || !n_out || !grid_wh) return fail(FDCM_ERR_INVALID, "null argument");
+    if (width < 0 || height < 0) return fail(FDCM_ERR_INVALID, "width and height must be >= 0");
+    if (rotation < 0 || rotation >= dense->rotations) return fail(FDCM_ERR_INVALID, "rotation must be in 0..rotations - 1");
+    return dense_poses(dense, 1.0f, rotation, anchor, shift, width, height, out, capacity, n_out, grid_wh);
 }
 
 extern "C" fdcm_status fdcm_dense_scaled_poses(const fdcm_dense_params* dense, const fdcm_scale_grid* grid, const float anchor[2],
@@ -2491,19 +2490,7 @@ extern "C" fdcm_status fdcm_dense_scaled_poses(const fdcm_dense_params* dense, c
     if (width < 0 || height < 0) return fail(FDCM_ERR_INVALID, "width and height must be >= 0");
     if (scale < 0 || scale >= grid->scales) return fail(FDCM_ERR_INVALID, "scale must be in 0..scales - 1");
     if (rotation < 0 || rotation >= dense->rotations) return fail(FDCM_ERR_INVALID, "rotation must be in 0..rotations - 1");
-    const DenseGrid g = dense_grid(dense, shift, width, height);
-    grid_wh[0] = g.nx;
-    grid_wh[1] = g.ny;
-    const int64_t n = (int64_t)g.nx * g.ny;
-    *n_out = n;
-    if (n > capacity || (n > 0 && !out)) return fail(FDCM_ERR_CAPACITY, "output buffer too small");
-    float a, b;
-    dense_scaled_rotation(dense, scales[(size_t)scale], rotation, &a, &b);
-    for (int v = 0; v < g.ny; ++v)
-        for (int u = 0; u < g.nx; ++u)
-            dense_pose(a, b, anchor[0], anchor[1], g.lo_x + u * dense->stride, g.lo_y + v * dense->stride, shift[0], shift[1],
-                       out + 6 * ((size_t)v * g.nx + u));
-    return FDCM_OK;
+    return dense_poses(dense, scales[(size_t)scale], rotation, anchor, shift, width, height, out, capacity, n_out, grid_wh);
 }
 
 // fdcm_search of this rank's template shard (params->tmpl_idx_base = first global index of the shard) followed by the

@@ -14,7 +14,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 import openfdcm_b200 as fdcm
 from oracle import fdcm_oracle as orc
-from tests.test_gpu_real_assets import load_object
+from tests.helpers import load_object
 
 out = {"parameters": "DefaultSearch(4,10), BatchOptimize(10), depth 30, coeff 5, padding 1.0, L2, ExponentialPenalty(1.5), top-10",
        "reference_claim": "22 FPS (45 ms / scene) on an i7-14700, notebooks/pose_extimation_example.ipynb:244", "objects": {}}

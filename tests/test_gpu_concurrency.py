@@ -14,6 +14,7 @@ import pytest
 import openfdcm_b200 as fdcm
 from openfdcm_b200 import _lib
 from oracle import fdcm_oracle as orc
+from tests.helpers import masks
 from tests.util import F32, plant_instances, synth_scene, synth_templates
 
 pytestmark = pytest.mark.gpu
@@ -47,10 +48,6 @@ def same(a, b):
 
 def planes(fm):
     return np.stack([fm.plane(d) for d in range(fm.depth)])
-
-
-def masks(fm):
-    return np.stack([fm.mask(d) for d in range(fm.depth)])
 
 
 def top10(fm, tset, penalty=PEN, **kw):

@@ -1,5 +1,5 @@
 """Match verification on the device (fdcm_match_coverage, search_topk / search_dense with verify=): byte-equal to the numpy
-model of tests/test_coverage_host.py, which reads the map's own edge masks (Dt3Cuda.mask)."""
+model of tests/models/coverage.py, which reads the map's own edge masks (Dt3Cuda.mask)."""
 import ctypes as C
 import threading
 
@@ -8,18 +8,14 @@ import pytest
 
 import openfdcm_b200 as fdcm
 from openfdcm_b200 import _lib
-from tests.test_coverage_host import Dilated, coverage_model, filter_model
-from tests.test_dense_host import output_model
-from tests.test_gpu_select import load_object, synthetic
+from tests.helpers import load_object, masks, synthetic
+from tests.models.coverage import Dilated, coverage_model, filter_model
+from tests.models.dense import output_model
 from tests.util import F32, synth_scene, synth_templates
 
 pytestmark = pytest.mark.gpu
 
 S, O, P = fdcm.DefaultSearch(4, 4), fdcm.BatchOptimize(10), fdcm.ExponentialPenalty(1.5)
-
-
-def masks(fm):
-    return np.stack([fm.mask(q) for q in range(fm.depth)]) if fm.depth else np.zeros((0, 0, 0), np.uint8)
 
 
 def model(fm, tmpls, matches, cov, tmpl_idx_base=0):

@@ -1,5 +1,5 @@
 """Dense pose-grid search on the device (search_dense, DenseSearch): byte for byte against the numpy model of
-tests/test_dense_host.py, whose pose scores come from the device evaluate (itself bit-exact with the oracle) or, in one
+tests/models/dense.py, whose pose scores come from the device evaluate (itself bit-exact with the oracle) or, in one
 case, from the oracle directly."""
 import ctypes as C
 import itertools
@@ -11,8 +11,8 @@ import pytest
 import openfdcm_b200 as fdcm
 from openfdcm_b200 import _lib
 from oracle import fdcm_oracle as orc
-from tests.test_dense_host import dense_records, output_model, rotate_template
-from tests.test_gpu_select import load_object, synthetic
+from tests.helpers import evaluate_fn, load_object, synthetic
+from tests.models.dense import dense_records, output_model, penalised, rotate_template
 from tests.util import F32, synth_scene
 
 pytestmark = pytest.mark.gpu
@@ -20,34 +20,8 @@ PEN = fdcm.ExponentialPenalty(1.5)
 OPT = fdcm.BatchOptimize(10)
 
 
-def evaluate_fn(fm):
-    """score_fn of the model: fdcm_dt3_evaluate of the rotated template at every translation."""
-    def score(Rt, tr):
-        flat = np.ascontiguousarray(Rt, F32).reshape(-1, 4)
-        off = np.array([0, len(flat)], np.int32)
-        trn = np.ascontiguousarray(tr, F32)
-        troff = np.array([0, len(trn)], np.int32)
-        out = np.zeros(len(trn), F32)
-        _lib.check(_lib.lib().fdcm_dt3_evaluate(fm._h, _lib.ptr(flat), _lib.ptr(off), 1, _lib.ptr(trn), _lib.ptr(troff), _lib.ptr(out)))
-        return out
-    return score
-
-
 def model_records(fm, tmpls, anchors, d, score_fn=None, tmpl_idx_base=0):
     return dense_records(tmpls, anchors, d, fm.get_scene_translation(), fm.width, fm.height, score_fn or evaluate_fn(fm), tmpl_idx_base)
-
-
-def penalised(rec, valid, tmpls, penalty, tmpl_idx_base=0):
-    if penalty is None:
-        return rec
-    lengths = np.asarray(fdcm.get_template_lengths(tmpls), F32)
-    p = rec[valid].copy()
-    p["tmpl_idx"] -= tmpl_idx_base
-    p = fdcm.penalize(penalty, p, lengths)
-    p["tmpl_idx"] += tmpl_idx_base
-    out = rec.copy()
-    out[valid] = p
-    return out
 
 
 def outputs(n_valid):
@@ -61,9 +35,9 @@ def outputs(n_valid):
 
 
 def check_all(fm, tset, tmpls, anchors, d, what, tmpl_idx_base=0):
-    rec, valid = model_records(fm, tmpls, anchors, d, tmpl_idx_base=tmpl_idx_base)
+    rec, valid, _ = model_records(fm, tmpls, anchors, d, tmpl_idx_base=tmpl_idx_base)
     for pen in (None, PEN):
-        prec = penalised(rec, valid, tmpls, pen, tmpl_idx_base)
+        prec = penalised(rec, valid, fdcm.get_template_lengths(tmpls), pen)
         for k, sel in outputs(int(valid.sum())):
             got = fdcm.search_dense(fm, tset, d, pen, k, tmpl_idx_base, select=sel)
             want = output_model(prec, valid, k, anchors, sel, tmpl_idx_base)
@@ -101,9 +75,9 @@ def test_real_assets_bit_exact(obj):
     tset, anchors = fdcm.TemplateSet(tmpls), fdcm.get_template_anchors(tmpls)
     fm = fdcm.build_cuda_featuremap(scenes[0], fdcm.Dt3CudaParameters(30, 5.0, 1.0))
     d = fdcm.DenseSearch(12, stride=8, cell=4)
-    rec, valid = model_records(fm, tmpls, anchors, d)
+    rec, valid, _ = model_records(fm, tmpls, anchors, d)
     for k, sel in ((10, None), (10, fdcm.DistinctMatches(max_per_template=1))):
-        want = output_model(penalised(rec, valid, tmpls, PEN), valid, k, anchors, sel)
+        want = output_model(penalised(rec, valid, fdcm.get_template_lengths(tmpls), PEN), valid, k, anchors, sel)
         assert fdcm.search_dense(fm, tset, d, PEN, k, select=sel).tobytes() == want.tobytes(), f"{obj} {sel}"
 
 
@@ -164,7 +138,7 @@ def test_edge_cases():
     assert len(fdcm.search_dense(fm, tmpls, fdcm.DenseSearch(6, roi=(1e5, 1e5, 2e5, 2e5)))) == 0
     # top_k larger than the number of valid records
     d = fdcm.DenseSearch(6, stride=3, cell=1000)
-    rec, valid = model_records(fm, tmpls, fdcm.get_template_anchors(tmpls), d)
+    rec, valid, _ = model_records(fm, tmpls, fdcm.get_template_anchors(tmpls), d)
     got = fdcm.search_dense(fm, tmpls, d, None, int(valid.sum()) + 1000)
     assert len(got) == int(valid.sum()) and got.tobytes() == output_model(rec, valid, len(got)).tobytes()
 
@@ -198,11 +172,11 @@ def test_long_templates():
     d = fdcm.DenseSearch(2, rot_step=0.3, stride=4, cell=3, roi=(300.0, 200.0, 340.0, 240.0))
     for tmpls in ([long_template(4000, 5), long_template(30, 6)], [np.ascontiguousarray(lines[:, :L])]):
         tset, anchors = fdcm.TemplateSet(tmpls), fdcm.get_template_anchors(tmpls)
-        rec, valid = model_records(fm, tmpls, anchors, d)
+        rec, valid, _ = model_records(fm, tmpls, anchors, d)
         assert valid.any()
         for k, sel in ((5, None), (5, fdcm.DistinctMatches(max_per_template=1))):
             assert fdcm.search_dense(fm, tset, d, PEN, k, select=sel).tobytes() == \
-                output_model(penalised(rec, valid, tmpls, PEN), valid, k, anchors, sel).tobytes()
+                output_model(penalised(rec, valid, fdcm.get_template_lengths(tmpls), PEN), valid, k, anchors, sel).tobytes()
     with pytest.raises(fdcm.FdcmError) as e:
         fdcm.search_dense(fm, [lines], d)
     assert e.value.status == _lib.FDCM_ERR_INVALID and "lines per template" in str(e.value)

@@ -1,5 +1,5 @@
 """Pose fit on the device (fdcm_fit_matches, fit_matches, search_topk / search_dense with fit=): byte-equal to the float64
-model of tests/test_fit_host.py, and the model's recovery properties on the device."""
+model of tests/models/fit.py, and the model's recovery properties on the device."""
 import math
 import threading
 
@@ -8,10 +8,9 @@ import pytest
 
 import openfdcm_b200 as fdcm
 from openfdcm_b200 import _lib
-from tests.test_fit_host import SceneLines, fit_model, house, offset_pose, pose, pose_errors, posed
-from tests.test_gpu_refine import device_scores
-from tests.test_refine_host import rotated, valid_poses
-from tests.test_gpu_select import load_object, synthetic
+from tests.helpers import device_scores, fit_candidates, house, load_object, offset_pose, pose, pose_errors, posed, synthetic
+from tests.models.fit import SceneLines, fit_model
+from tests.models.refine import rotated, valid_poses
 from tests.util import F32, synth_scene, synth_templates
 
 pytestmark = pytest.mark.gpu
@@ -31,25 +30,6 @@ def model(fm, scene, tmpls, matches, fit, penalty=None, tmpl_idx_base=0):
     return out, stats
 
 
-def candidates(fm, tmpls, scene, n=40, seed=0):
-    """Distinct search matches, the same matches moved by up to 2 px and 0.03 rad, and poses off the map."""
-    rec = fdcm.search_topk(fm, tmpls, scene, S, O, P, k=n, select=fdcm.DistinctMatches(max_per_template=2))
-    rng = np.random.default_rng(seed)
-    moved = rec.copy()
-    a = rng.uniform(-0.03, 0.03, len(rec)).astype(F32)
-    c, s = np.cos(a).astype(F32), np.sin(a).astype(F32)
-    T = moved["transform"].copy()
-    moved["transform"][:, 0] = c * T[:, 0] - s * T[:, 3]
-    moved["transform"][:, 1] = c * T[:, 1] - s * T[:, 4]
-    moved["transform"][:, 3] = s * T[:, 0] + c * T[:, 3]
-    moved["transform"][:, 4] = s * T[:, 1] + c * T[:, 4]
-    moved["transform"][:, 2] += rng.uniform(-2, 2, len(rec)).astype(F32)
-    moved["transform"][:, 5] += rng.uniform(-2, 2, len(rec)).astype(F32)
-    off = rec[: min(3, len(rec))].copy()
-    off["transform"][:, 2] += F32(1e5)
-    return np.concatenate([rec, moved, off])
-
-
 def check_fit(fm, scene, tmpls, matches, fit, penalty=None, tmpl_idx_base=0):
     got, gst = fdcm.fit_matches(fm, tmpls, matches, fit, penalty, tmpl_idx_base, return_stats=True)
     want, wst = model(fm, scene, tmpls, matches, fit, penalty, tmpl_idx_base)
@@ -64,7 +44,7 @@ def check_fit(fm, scene, tmpls, matches, fit, penalty=None, tmpl_idx_base=0):
 def test_synthetic_scenes_against_the_model(dist):
     tmpls, scene = synthetic(n_tmpl=10, seed=500)
     fm = fdcm.build_cuda_featuremap(scene, fdcm.Dt3CudaParameters(30, 5.0, 1.5, dist))
-    m = candidates(fm, tmpls, scene, 30)
+    m = fit_candidates(fm, tmpls, scene, 30)
     got, st = check_fit(fm, scene, tmpls, m, fdcm.PoseFit(), P)
     assert np.isnan(got[-3:]["score"]).all() and (st["iterations"][:-3] > 0).any()
     check_fit(fm, scene, tmpls, m[::3], fdcm.PoseFit(iterations=3, max_distance=6.0, sample_step=0.75, bin_tolerance=0, min_inliers=3))
@@ -73,7 +53,7 @@ def test_synthetic_scenes_against_the_model(dist):
 def test_odd_depth_and_tmpl_idx_base():
     tmpls, scene = synthetic(n_tmpl=6, seed=510)
     fm = fdcm.build_cuda_featuremap(scene, fdcm.Dt3CudaParameters(7, 5.0, 1.5))
-    m = candidates(fm, tmpls, scene, 20)
+    m = fit_candidates(fm, tmpls, scene, 20)
     m["tmpl_idx"] += 100
     check_fit(fm, scene, tmpls, m, fdcm.PoseFit(bin_tolerance=2), tmpl_idx_base=100)
 
@@ -83,14 +63,14 @@ def test_literal_path_map():
     scene = synth_scene(3000, 3000, 120, seed=521)
     fm = fdcm.build_cuda_featuremap(scene, fdcm.Dt3CudaParameters(30, 5.0, 1.05))
     assert fm.width > 2897
-    check_fit(fm, scene, tmpls, candidates(fm, tmpls, scene, 12), fdcm.PoseFit(max_distance=16.0))
+    check_fit(fm, scene, tmpls, fit_candidates(fm, tmpls, scene, 12), fdcm.PoseFit(max_distance=16.0))
 
 
 @pytest.mark.parametrize("obj", ["obj_01", "obj_02", "obj_03", "obj_04"])
 def test_real_assets(obj):
     tmpls, scenes = load_object(obj)
     fm = fdcm.build_cuda_featuremap(scenes[0], fdcm.Dt3CudaParameters(30, 5.0, 2.2))
-    check_fit(fm, scenes[0], tmpls, candidates(fm, tmpls, scenes[0], 10, seed=1), fdcm.PoseFit(), P)
+    check_fit(fm, scenes[0], tmpls, fit_candidates(fm, tmpls, scenes[0], 10, seed=1), fdcm.PoseFit(), P)
 
 
 # ---- the model's properties on the device ----------------------------------------------------------------------------
@@ -188,7 +168,7 @@ def test_edge_cases():
     with pytest.raises(fdcm.FdcmError, match="max_distance"):
         fdcm.fit_matches(fm, tset, recs, fdcm.PoseFit(max_distance=17.0))
     # two identical calls are byte-identical
-    m = candidates(fm, tmpls[:4], scene, 20)
+    m = fit_candidates(fm, tmpls[:4], scene, 20)
     a1, s1 = fdcm.fit_matches(fm, tset, m, fit, P, return_stats=True)
     a2, s2 = fdcm.fit_matches(fm, tset, m, fit, P, return_stats=True)
     assert a1.tobytes() == a2.tobytes() and s1.tobytes() == s2.tobytes()
@@ -217,7 +197,7 @@ def test_grid_follows_rebuilds():
     _, scene2 = synthetic(n_tmpl=6, seed=561)
     fm = fdcm.build_cuda_featuremap(scene, fdcm.Dt3CudaParameters(30, 5.0, 1.5))
     fit = fdcm.PoseFit()
-    m = candidates(fm, tmpls, scene, 12)
+    m = fit_candidates(fm, tmpls, scene, 12)
     first, _ = check_fit(fm, scene, tmpls, m, fit)
     fm.rebuild(scene2)
     second, _ = check_fit(fm, scene2, tmpls, m, fit)
@@ -233,7 +213,7 @@ def test_async_rebuild_then_stream_switch():
     fm = fdcm.build_cuda_featuremap(scene2, fdcm.Dt3CudaParameters(30, 5.0, 1.5))
     ref = fdcm.build_cuda_featuremap(scene, fdcm.Dt3CudaParameters(30, 5.0, 1.5))
     fit = fdcm.PoseFit()
-    m = candidates(ref, tmpls, scene, 12)
+    m = fit_candidates(ref, tmpls, scene, 12)
     want = fdcm.fit_matches(ref, tmpls, m, fit)
     fdcm.fit_matches(fm, tmpls, m, fit)   # a cached grid of the old scene
     fm.rebuild(scene, wait=False)
@@ -250,7 +230,7 @@ def test_two_threads_with_different_max_distance_on_one_map():
     tmpls, scene = synthetic(n_tmpl=6, seed=580)
     fm = fdcm.build_cuda_featuremap(scene, fdcm.Dt3CudaParameters(30, 5.0, 1.5))
     tset = fdcm.TemplateSet(tmpls)
-    m = candidates(fm, tmpls, scene, 12)
+    m = fit_candidates(fm, tmpls, scene, 12)
     fits = [fdcm.PoseFit(max_distance=1.5), fdcm.PoseFit(max_distance=8.0)]
     want = [model(fm, scene, tmpls, m, f)[0] for f in fits]
     errors = []
@@ -288,7 +268,7 @@ def test_broadcast_map_on_a_non_root_rank():
     tmpls, scene = synthetic(n_tmpl=6, seed=590)
     _, other = synthetic(n_tmpl=6, seed=591)
     ref = fdcm.build_cuda_featuremap(scene, fdcm.Dt3CudaParameters(30, 5.0, 1.5))
-    m = candidates(ref, tmpls, scene, 12)
+    m = fit_candidates(ref, tmpls, scene, 12)
     want = model(ref, scene, tmpls, m, fdcm.PoseFit())[0]
     uid = fd.Communicator.unique_id()
     out = {}

@@ -13,13 +13,11 @@ import pytest
 
 import openfdcm_b200 as fdcm
 from oracle import fdcm_oracle as orc
-from tests.test_gpu_refine import model as refine_reference
-from tests.test_gpu_search_space import _assert_matches, _check_full_search, _penalized, _topk_ref
-from tests.test_select_host import select_model
+from tests.helpers import DIST, assert_matches, check_full_search, oracle_penalized, refine_reference, topk_ref
+from tests.models.select import select_model
 from tests.util import F32, plant_instances, synth_scene, synth_templates
 
 pytestmark = pytest.mark.gpu
-DIST = {"L2": (fdcm.distance.L2, orc.L2), "L2_SQUARED": (fdcm.distance.L2_SQUARED, orc.L2_SQUARED), "L1": (fdcm.distance.L1, orc.L1)}
 PEN = fdcm.ExponentialPenalty(1.5)
 OPT = fdcm.BatchOptimize(10)
 
@@ -220,11 +218,11 @@ def check_map(g, c, scene, stage=0, planes=None, what=""):
 def check_search(g, c, tmpls, scene, max_t, max_s, batches=(10,), what=""):
     """search_all (hypotheses, counters, every match) for each batch size, and the penalised top-10 of BatchOptimize(10)."""
     for batch in batches:
-        raw, _ = _check_full_search(g, c, tmpls, scene, max_t, max_s, batch)
+        raw, _ = check_full_search(g, c, tmpls, scene, max_t, max_s, batch)
         if batch == 10:
             raw10 = raw
     top = fdcm.search_topk(g, tmpls, scene, fdcm.DefaultSearch(max_t, max_s), OPT, PEN, k=10)
-    _assert_matches(top, _topk_ref(_penalized(raw10, tmpls, PEN), 10), f"{what} top-10")
+    assert_matches(top, topk_ref(oracle_penalized(raw10, tmpls, PEN), 10), f"{what} top-10")
     return raw10
 
 
@@ -388,7 +386,7 @@ def check_step(g, c, scene, tset, tmpls, what):
     planes = range(c.depth) if c.W < 2000 else (0, 7, 14, 22, 29)
     check_map(g, c, scene, planes=planes, what=what)
     top = fdcm.search_topk(g, tset, None, fdcm.DefaultSearch(4, 4), OPT, PEN, k=10)
-    _assert_matches(top, _topk_ref(_penalized(c.search(tmpls, scene, 4, 4, batch=10), tmpls, PEN), 10), f"{what}: top-10")
+    assert_matches(top, topk_ref(oracle_penalized(c.search(tmpls, scene, 4, 4, batch=10), tmpls, PEN), 10), f"{what}: top-10")
 
 
 @pytest.mark.parametrize("dist", list(DIST))
@@ -432,8 +430,8 @@ def test_rebuilds_across_sizes(dist):
     got = fdcm.SceneBatch(params).search_topk(mix, tset, fdcm.DefaultSearch(4, 4), OPT, PEN, k=10)
     assert len(got) == len(mix)
     for i, scene in enumerate(mix):
-        want = _topk_ref(_penalized(oracle(scene).search(tmpls, scene, 4, 4, batch=10), tmpls, PEN), 10)
-        _assert_matches(got[i], want, f"{dist} SceneBatch scene {i}")
+        want = topk_ref(oracle_penalized(oracle(scene).search(tmpls, scene, 4, 4, batch=10), tmpls, PEN), 10)
+        assert_matches(got[i], want, f"{dist} SceneBatch scene {i}")
 
 
 # ---- coverage of the build paths ------------------------------------------------------------------------------------

@@ -15,6 +15,7 @@ import pytest
 
 import openfdcm_b200 as fdcm
 from oracle import fdcm_oracle as orc
+from tests.helpers import DIST
 from tests.util import synth_scene
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -23,8 +24,6 @@ if ROOT not in sys.path:
 import bench  # noqa: E402  (the workload generator of the headline benchmark)
 
 pytestmark = pytest.mark.gpu
-DIST = {"L2": (fdcm.distance.L2, orc.L2), "L2_SQUARED": (fdcm.distance.L2_SQUARED, orc.L2_SQUARED),
-        "L1": (fdcm.distance.L1, orc.L1)}
 
 
 def _compare_all_planes(g, c, what):

@@ -9,11 +9,10 @@ import pytest
 
 import openfdcm_b200 as fdcm
 from oracle import fdcm_oracle as orc
+from tests.helpers import DIST
 from tests.util import F32, load_kats, plant_instances, synth_scene, synth_templates
 
 pytestmark = pytest.mark.gpu
-DIST = {"L2": (fdcm.distance.L2, orc.L2), "L2_SQUARED": (fdcm.distance.L2_SQUARED, orc.L2_SQUARED),
-        "L1": (fdcm.distance.L1, orc.L1)}
 KATS = load_kats()
 
 

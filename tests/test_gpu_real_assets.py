@@ -9,15 +9,9 @@ import pytest
 
 import openfdcm_b200 as fdcm
 from oracle import fdcm_oracle as orc
+from tests.helpers import ASSETS, load_object
 
 pytestmark = pytest.mark.gpu
-ASSETS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "real_assets")
-
-
-def load_object(obj):
-    tm = sorted(glob.glob(os.path.join(ASSETS, obj, "templates", "*.tmpl")), key=lambda p: int(os.path.basename(p)[9:-5]))
-    scenes = sorted(glob.glob(os.path.join(ASSETS, obj, "scene_*", "camera_0.scene")), key=lambda p: int(os.path.basename(os.path.dirname(p))[6:]))
-    return [fdcm.read(p) for p in tm], [fdcm.read(p) for p in scenes]
 
 
 def test_assets_complete():

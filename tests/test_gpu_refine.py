@@ -1,5 +1,5 @@
 """Pose refinement on the device (refine_matches, search_topk(refine=...)): byte for byte against the numpy model of
-tests/test_refine_host.py, whose pose scores come from the device evaluate (itself bit-exact with the oracle) or, in one
+tests/models/refine.py, whose pose scores come from the device evaluate (itself bit-exact with the oracle) or, in one
 case, from the oracle directly.
 
 No test asserts that refinement brings planted instances closer to their known poses: it does not.  The evaluate<Dt3Cpu>
@@ -15,8 +15,8 @@ import pytest
 import openfdcm_b200 as fdcm
 from openfdcm_b200 import _lib
 from oracle import fdcm_oracle as orc
-from tests.test_gpu_select import load_object, synthetic
-from tests.test_refine_host import refine_model, rotated
+from tests.helpers import device_scores, load_object, refine_reference, synthetic
+from tests.models.refine import refine_model, rotated
 from tests.util import F32, synth_scene, synth_templates
 
 pytestmark = pytest.mark.gpu
@@ -30,31 +30,6 @@ def settings():
         yield fdcm.PoseRefinement(levels, n_r, rs, n_t, ts)
 
 
-def device_scores(fm):
-    """score_fn of the model: fdcm_dt3_evaluate of every rotated template at (P2, P5)."""
-    def score(work):
-        recs, tr = [], []
-        for tmpl, poses in work:
-            R = rotated(poses, tmpl)
-            recs += list(R)
-            tr.append(poses[:, [2, 5]])
-        off = np.zeros(len(recs) + 1, np.int32)
-        off[1:] = np.cumsum([r.shape[0] for r in recs])
-        flat = np.ascontiguousarray(np.concatenate(recs) if off[-1] else np.zeros((1, 4), F32), F32)
-        trn = np.ascontiguousarray(np.concatenate(tr), F32)
-        troff = np.arange(len(recs) + 1, dtype=np.int32)
-        out = np.zeros(len(recs), F32)
-        _lib.check(_lib.lib().fdcm_dt3_evaluate(fm._h, _lib.ptr(flat), _lib.ptr(off), len(recs), _lib.ptr(trn), _lib.ptr(troff),
-                                                _lib.ptr(out)))
-        return out
-    return score
-
-
-def model(fm, tmpls, anchors, matches, r, score_fn=None, tmpl_idx_base=0):
-    return refine_model(matches, tmpls, anchors, r, fm.get_scene_translation(), fm.width, fm.height, score_fn or device_scores(fm),
-                        tmpl_idx_base)
-
-
 def centre_scores(fm, tmpls, matches):
     """evaluate of the rotation-only template at (c2, c5) of every match."""
     work = [(tmpls[int(m["tmpl_idx"])], np.asarray(m["transform"], F32).reshape(1, 6)) for m in matches]
@@ -65,7 +40,7 @@ def check_settings(fm, tset, tmpls, anchors, base, what, cases=None):
     lengths = tset.lengths()
     centre = centre_scores(fm, tmpls, base)
     for r in cases or settings():
-        want = model(fm, tmpls, anchors, base, r)
+        want = refine_reference(fm, tmpls, anchors, base, r)
         got = fdcm.refine_matches(fm, tset, base, r)
         assert got.tobytes() == want.tobytes(), f"{what} {r}: got {got} want {want}"
         gotp = fdcm.refine_matches(fm, tset, base, r, penalty=PEN)
@@ -154,7 +129,7 @@ def test_edge_cases():
     T[2] = F32(W - 1) - fm.get_scene_translation()[0] - F32(max(R[:, 0].max(), R[:, 2].max())) - F32(1.5)
     recs[4] = (base[0]["tmpl_idx"], 0.0, T.reshape(6))
     got = fdcm.refine_matches(fm, tset, recs, r)
-    assert got.tobytes() == model(fm, tmpls, anchors, recs, r).tobytes()
+    assert got.tobytes() == refine_reference(fm, tmpls, anchors, recs, r).tobytes()
     assert got[3]["score"] == 0.0 and got[3]["transform"].tobytes() == recs[3]["transform"].tobytes()
     # a NaN transform: no valid pose, score NaN, transform unchanged
     bad = recs[:1].copy()
@@ -188,7 +163,7 @@ def test_template_longer_than_3418_lines():
     for q in range(2):
         recs[q] = (q, 0.0, np.array([math.cos(0.3), -math.sin(0.3), 320.0, math.sin(0.3), math.cos(0.3), 240.0], F32))
     for r in (fdcm.PoseRefinement(2, 1, 0.02, 2, 1.0), fdcm.PoseRefinement(1, 0, 0.0, 1, 1.0)):
-        assert fdcm.refine_matches(fm, tset, recs, r).tobytes() == model(fm, tmpls, anchors, recs, r).tobytes()
+        assert fdcm.refine_matches(fm, tset, recs, r).tobytes() == refine_reference(fm, tmpls, anchors, recs, r).tobytes()
     base = fdcm.search_topk(fm, tset, None, fdcm.DefaultSearch(2, 4), OPT, PEN, k=2)
     r = fdcm.PoseRefinement(1, 1, 0.02, 1, 1.0)
     assert fdcm.search_topk(fm, tset, None, fdcm.DefaultSearch(2, 4), OPT, PEN, k=2, refine=r).tobytes() == \
@@ -217,7 +192,7 @@ def test_template_at_the_search_limit():
     recs = np.zeros(1, fdcm.MATCH_DTYPE)
     recs[0] = (0, 0.0, np.array([math.cos(0.2), -math.sin(0.2), 320.0, math.sin(0.2), math.cos(0.2), 240.0], F32))
     r = fdcm.PoseRefinement(1, 1, 0.02, 1, 1.0)
-    assert fdcm.refine_matches(fm, tset, recs, r).tobytes() == model(fm, tmpls, anchors, recs, r).tobytes()
+    assert fdcm.refine_matches(fm, tset, recs, r).tobytes() == refine_reference(fm, tmpls, anchors, recs, r).tobytes()
     base = fdcm.search_topk(fm, tset, None, fdcm.DefaultSearch(1, 2), OPT, PEN, k=1)
     assert fdcm.search_topk(fm, tset, None, fdcm.DefaultSearch(1, 2), OPT, PEN, k=1, refine=r).tobytes() == \
         fdcm.refine_matches(fm, tset, base, r, penalty=PEN).tobytes()

@@ -1,4 +1,4 @@
-"""Scale as a pose dimension on the device: fdcm_search_dense_scales against the numpy model of tests/test_scale_host.py
+"""Scale as a pose dimension on the device: fdcm_search_dense_scales against the numpy model of tests/models/dense.py
 (scores through fdcm_dt3_evaluate, as tests/test_gpu_dense.py does), byte-identity with the unscaled search at one scale,
 composition with refinement, the coverage filter and the fit, fdcm_fit_matches_scaled against the float64 model, recovery of
 planted scaled instances, edge cases and the interfaces."""
@@ -9,13 +9,9 @@ import pytest
 
 import openfdcm_b200 as fdcm
 from openfdcm_b200 import _lib
-from tests.test_fit_host import SceneLines, house, posed
-from tests.test_gpu_dense import evaluate_fn
-from tests.test_gpu_fit import candidates
-from tests.test_gpu_refine import device_scores
-from tests.test_gpu_select import load_object, synthetic
-from tests.test_scale_host import (fit_model_scaled, scale_error, scale_values, scaled_output_model, scaled_penalised,
-                                   scaled_records, spose)
+from tests.helpers import device_scores, evaluate_fn, fit_candidates, house, load_object, posed, scale_error, spose, synthetic
+from tests.models.dense import dense_records, output_model, penalised, scale_values
+from tests.models.fit import SceneLines, fit_model
 from tests.util import F32, synth_scene, synth_templates
 
 pytestmark = pytest.mark.gpu
@@ -23,8 +19,8 @@ PEN = fdcm.ExponentialPenalty(1.5)
 
 
 def model(fm, tmpls, d, g, tmpl_idx_base=0):
-    return scaled_records(tmpls, fdcm.get_template_anchors(tmpls), d, g, fm.get_scene_translation(), fm.width, fm.height, evaluate_fn(fm),
-                          tmpl_idx_base)
+    return dense_records(tmpls, fdcm.get_template_anchors(tmpls), d, fm.get_scene_translation(), fm.width, fm.height, evaluate_fn(fm),
+                         tmpl_idx_base, g)
 
 
 def check_dense(fm, tset, tmpls, d, g, what, pens=(None, PEN), tmpl_idx_base=0):
@@ -33,12 +29,12 @@ def check_dense(fm, tset, tmpls, d, g, what, pens=(None, PEN), tmpl_idx_base=0):
     lengths = fdcm.get_template_lengths(tmpls)
     n_valid = int(valid.sum())
     for pen in pens:
-        prec = scaled_penalised(rec, valid, g, lengths, pen, d, tmpl_idx_base)
+        prec = penalised(rec, valid, lengths, pen, g)
         for k, sel in ((1, None), (10, None), (min(max(n_valid, 1), 500), None), (10, fdcm.DistinctMatches(max_per_template=1)),
                        (10, fdcm.DistinctMatches(radius=6.0, max_angle=0.3)),
                        (10, fdcm.DistinctMatches(radius=6.0, max_angle=0.3, across_templates=True))):
             got = fdcm.search_dense(fm, tset, d, pen, k, tmpl_idx_base, select=sel, scales=g)
-            want = scaled_output_model(prec, valid, rs, k, anchors, sel, tmpl_idx_base)
+            want = output_model(prec, valid, k, anchors, sel, tmpl_idx_base, rs)
             assert got.tobytes() == want.tobytes(), f"{what} {g} {pen} k={k} {sel}: got {got[:3]} want {want[:3]}"
     return rec, valid
 
@@ -75,9 +71,9 @@ def test_real_assets_bit_exact(obj):
     rec, valid, rs = model(fm, tmpls, d, g)
     anchors, lengths = fdcm.get_template_anchors(tmpls), fdcm.get_template_lengths(tmpls)
     for pen in (PEN, fdcm.DefaultPenalty()):
-        prec = scaled_penalised(rec, valid, g, lengths, pen, d)
+        prec = penalised(rec, valid, lengths, pen, g)
         for sel in (None, fdcm.DistinctMatches(max_per_template=1), fdcm.DistinctMatches(radius=20.0, max_angle=0.2, across_templates=True)):
-            want = scaled_output_model(prec, valid, rs, 10, anchors, sel)
+            want = output_model(prec, valid, 10, anchors, sel, rs=rs)
             got = fdcm.search_dense(fm, tset, d, pen, 10, select=sel, scales=g)
             assert got.tobytes() == want.tobytes(), f"{obj} {pen} {sel}"
 
@@ -125,10 +121,10 @@ def test_composed_refine_fit_and_coverage():
     c = fdcm.match_coverage(fm, tset, rec[valid], cov)
     keep = valid.copy()
     keep[np.flatnonzero(valid)] = c >= F32(0.4)
-    prec = scaled_penalised(rec, keep, g, fdcm.get_template_lengths(tmpls), PEN, d)
+    prec = penalised(rec, keep, fdcm.get_template_lengths(tmpls), PEN, g)
     for s in (None, sel):
         got = fdcm.search_dense(fm, tset, d, PEN, 10, select=s, verify=cov, scales=g)
-        assert got.tobytes() == scaled_output_model(prec, keep, rs, 10, fdcm.get_template_anchors(tmpls), s).tobytes(), s
+        assert got.tobytes() == output_model(prec, keep, 10, fdcm.get_template_anchors(tmpls), s, rs=rs).tobytes(), s
 
 
 # ---- the scaled fit, bit for bit -------------------------------------------------------------------------------------
@@ -136,8 +132,8 @@ def check_fit(fm, scene, tmpls, matches, fit, penalty=None):
     got, gst = fdcm.fit_matches(fm, tmpls, matches, fit, penalty, return_stats=True)
     sc = SceneLines.of(scene, fm.get_scene_translation(), fm.scene_bins(), fm.depth, fm.width, fm.height)
     scores = device_scores(fm)
-    want, wst = fit_model_scaled(sc, tmpls, fdcm.get_template_anchors(tmpls), matches, fit,
-                                 lambda tmpl, F: scores([(tmpl, F.reshape(1, 6))])[0])
+    want, wst = fit_model(sc, tmpls, fdcm.get_template_anchors(tmpls), matches, fit,
+                          lambda tmpl, F: scores([(tmpl, F.reshape(1, 6))])[0])
     if penalty is not None:
         want = fdcm.penalize(penalty, want, fdcm.get_template_lengths(tmpls))
     bad = np.flatnonzero([a.tobytes() != b.tobytes() for a, b in zip(got, want)])
@@ -147,8 +143,8 @@ def check_fit(fm, scene, tmpls, matches, fit, penalty=None):
 
 
 def scaled_candidates(fm, tmpls, scene, n, seed):
-    """candidates() of the rigid fit tests, some of them scaled by up to 6 % about their origin."""
-    m = candidates(fm, tmpls, scene, n, seed)
+    """fit_candidates() of the rigid fit tests, some of them scaled by up to 6 % about their origin."""
+    m = fit_candidates(fm, tmpls, scene, n, seed)
     rng = np.random.default_rng(seed)
     f = rng.uniform(0.94, 1.06, len(m)).astype(F32)
     f[::3] = F32(1)
@@ -259,7 +255,7 @@ def test_denominator_cache_across_scale_grids():
     g4 = fdcm.ScaleGrid(4, 0.8, 1.15)
     want1 = fdcm.search_dense(fm, tset, d, PEN, 20)
     rec, valid, rs = model(fm, tmpls, d, g4)
-    want4 = scaled_output_model(scaled_penalised(rec, valid, g4, fdcm.get_template_lengths(tmpls), PEN, d), valid, rs, 20)
+    want4 = output_model(penalised(rec, valid, fdcm.get_template_lengths(tmpls), PEN, g4), valid, 20)
     for _ in range(2):
         assert fdcm.search_dense(fm, tset, d, PEN, 20, scales=fdcm.ScaleGrid()).tobytes() == want1.tobytes()
         assert fdcm.search_dense(fm, tset, d, PEN, 20, scales=g4).tobytes() == want4.tobytes()

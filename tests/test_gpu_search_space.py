@@ -12,6 +12,7 @@ import pytest
 
 import openfdcm_b200 as fdcm
 from oracle import fdcm_oracle as orc
+from tests.helpers import assert_matches, check_full_search, optimizer, oracle_penalized, topk_ref
 from tests.util import F32, plant_instances, synth_scene, synth_templates
 
 pytestmark = pytest.mark.gpu
@@ -21,48 +22,6 @@ pytestmark = pytest.mark.gpu
 BATCHES = [0, 1, 2, 4, 7, 8, 9, 15, 16, 17, 31, 32, 33, 48, 64, 1000, 100000]
 PENALTIES = [None, fdcm.DefaultPenalty(), fdcm.ExponentialPenalty(0.5), fdcm.ExponentialPenalty(1.5), fdcm.ExponentialPenalty(3.0)]
 PENALTY_IDS = ["none", "default", "exp0.5", "exp1.5", "exp3"]
-
-
-def _opt(batch):
-    return fdcm.BatchOptimize(batch) if batch else fdcm.DefaultOptimize()
-
-
-def _penalized(raw, tmpls, penalty):
-    """penalize() of the oracle: DefaultPenalty divides by the template length, ExponentialPenalty by length ** tau."""
-    if penalty is None:
-        return raw
-    kind = 0 if isinstance(penalty, fdcm.DefaultPenalty) else 1
-    return orc.penalize(kind, penalty.tau, raw, orc.template_lengths(tmpls))
-
-
-def _topk_ref(pen, k, base=0):
-    """Ascending score (NaN ranks as +inf), ties by hypothesis order, template indices offset by base."""
-    key = np.where(np.isnan(pen["score"]), np.inf, pen["score"])
-    want = pen[np.lexsort((np.arange(len(pen)), key))[:k]].copy()
-    want["tmpl_idx"] += base
-    return want
-
-
-def _assert_matches(got, want, what=""):
-    assert len(got) == len(want), what
-    assert np.array_equal(got["tmpl_idx"], want["tmpl_idx"]), what
-    assert np.array_equal(got["score"], want["score"], equal_nan=True), what
-    assert np.array_equal(got["transform"], want["transform"], equal_nan=True), what
-
-
-def _check_full_search(g, c, tmpls, scene, max_t, max_s, batch, penalty=None, tset=None):
-    """search_all against the oracle: hypothesis list, counters and every match in hypothesis order."""
-    got = fdcm.search_all(g, tset or tmpls, scene, fdcm.DefaultSearch(max_t, max_s), _opt(batch), penalty)
-    st = g.last_search_stats()
-    orc.stats_reset()
-    raw, hyp = c.search(tmpls, scene, max_t, max_s, batch=batch, want_hyp=True)
-    evals, lookups = orc.stats_get()
-    assert np.array_equal(g.last_hypotheses(), hyp), "hypothesis list"
-    assert st["n_hypotheses"] == len(hyp)
-    assert (st["n_evaluations"], st["n_lookups"]) == (evals, lookups), "the kernel scored another candidate set"
-    assert st["n_valid"] == len(raw)
-    _assert_matches(got, _penalized(raw, tmpls, penalty), f"batch {batch}")
-    return raw, hyp
 
 
 # ---- workloads ------------------------------------------------------------------------------------------------------
@@ -112,14 +71,14 @@ def random_wl():
 @pytest.mark.parametrize("batch", BATCHES)
 def test_batch_sweep_plateau(batch, plateau):
     g, c, scene, tmpls = plateau
-    _, hyp = _check_full_search(g, c, tmpls, scene, 4, 6, batch)
+    _, hyp = check_full_search(g, c, tmpls, scene, 4, 6, batch)
     assert len(hyp) == 60
 
 
 @pytest.mark.parametrize("batch", BATCHES)
 def test_batch_sweep_spatial_order(batch, random_wl):
     g, c, scene, tset, tmpls = random_wl
-    _, hyp = _check_full_search(g, c, tmpls, scene, 4, 4, batch, tset=tset)
+    _, hyp = check_full_search(g, c, tmpls, scene, 4, 4, batch, tset=tset)
     assert len(hyp) == 4096
 
 
@@ -172,7 +131,7 @@ def optimize_wl():
 @pytest.mark.parametrize("batch", BATCHES)
 def test_optimize_entry_point_batch_sweep(batch, optimize_wl):
     g, c, cases = optimize_wl
-    got = fdcm.optimize(_opt(batch), [t for t, _ in cases], [np.array(v, F32) for _, v in cases], g)
+    got = fdcm.optimize(optimizer(batch), [t for t, _ in cases], [np.array(v, F32) for _, v in cases], g)
     for i, ((t, v), r) in enumerate(zip(cases, got)):
         has, score, tr = c.optimize_one(t, np.array(v, F32), batch)
         assert (r is not None) == has, f"case {i} (align {v})"
@@ -203,11 +162,11 @@ def test_template_sizes(longest, size_wl):
     g, c, scene, big = size_wl
     tmpls = [big[L] for L in SIZES if L <= longest]
     for batch in (10, 0):
-        _check_full_search(g, c, tmpls, scene, 4, 4, batch)
+        check_full_search(g, c, tmpls, scene, 4, 4, batch)
         rng = np.random.default_rng(longest + batch)
         placed = [(t.T.reshape(-1, 2) + np.array([320, 240], F32)).reshape(-1, 4).T.astype(F32) for t in tmpls]
         aligns = [rng.standard_normal(2).astype(F32) for _ in placed]
-        got = fdcm.optimize(_opt(batch), placed, aligns, g)
+        got = fdcm.optimize(optimizer(batch), placed, aligns, g)
         for i, (t, a, r) in enumerate(zip(placed, aligns, got)):
             has, score, tr = c.optimize_one(t, a, batch)
             assert (r is not None) == has, f"template of {t.shape[1]} lines"
@@ -221,7 +180,7 @@ def test_ordinary_templates_next_to_a_long_one(size_wl):
     g, c, scene, big = size_wl
     tmpls = synth_templates(200, 20, 640, seed=4203)
     tmpls.insert(117, big[4000])
-    raw, _ = _check_full_search(g, c, tmpls, scene, 4, 4, 10)
+    raw, _ = check_full_search(g, c, tmpls, scene, 4, 4, 10)
     assert (raw["tmpl_idx"] != 117).sum() > 0
 
 
@@ -254,8 +213,8 @@ def test_template_over_the_shared_memory_limit_is_rejected(size_wl):
             call()
         assert e.value.status == fdcm._lib.FDCM_ERR_INVALID and str(limit) in str(e.value), str(e.value)
     # the map, the template upload path and the search workspace are still usable
-    _check_full_search(g, c, ordinary, scene, 4, 4, 10)
-    _check_full_search(g, c, ordinary + [big[4000]], scene, 4, 4, 10)
+    check_full_search(g, c, ordinary, scene, 4, 4, 10)
+    check_full_search(g, c, ordinary + [big[4000]], scene, 4, 4, 10)
 
 
 # ---- top-k --------------------------------------------------------------------------------------------------------
@@ -275,10 +234,10 @@ def topk_wl():
 
 
 def _check_topk(g, tset, tmpls, scene, max_s, raw, penalty, ks, base):
-    pen = _penalized(raw, tmpls, penalty)
+    pen = oracle_penalized(raw, tmpls, penalty)
     for k in ks:
         got = fdcm.search_topk(g, tset, scene, fdcm.DefaultSearch(2, max_s), fdcm.BatchOptimize(10), penalty, k=k, tmpl_idx_base=base)
-        _assert_matches(got, _topk_ref(pen, k, base), f"k={k}")
+        assert_matches(got, topk_ref(pen, k, base), f"k={k}")
 
 
 @pytest.mark.parametrize("penalty", PENALTIES, ids=PENALTY_IDS)
@@ -288,7 +247,7 @@ def test_topk_shapes(size, penalty, topk_wl):
     tset, tmpls, max_s, raw = sets[size]
     H = len(tmpls) * 2 * max_s * 2
     n_valid = len(raw)
-    pen = _penalized(raw, tmpls, penalty)
+    pen = oracle_penalized(raw, tmpls, penalty)
     assert len(np.unique(pen["score"])) <= n_valid // 2, "the workload must be full of exact ties"
     ks = [1, 2, 31, 32, 33, 1023, 1024, 1025, n_valid - 1, n_valid, n_valid + 1, H + 7]
     _check_topk(g, tset, tmpls, scene, max_s, raw, penalty, ks, base=1000)
@@ -313,9 +272,9 @@ def test_penalty_switches_on_one_template_set(random_wl):
                     None, fdcm.DefaultPenalty()):
         what = "none" if penalty is None else f"{type(penalty).__name__}({penalty.tau})"
         got = fdcm.search_all(g, tset, scene, fdcm.DefaultSearch(4, 4), fdcm.BatchOptimize(10), penalty)
-        _assert_matches(got, _penalized(raw, tmpls, penalty), what)
+        assert_matches(got, oracle_penalized(raw, tmpls, penalty), what)
         top = fdcm.search_topk(g, tset, scene, fdcm.DefaultSearch(4, 4), fdcm.BatchOptimize(10), penalty, k=10)
-        _assert_matches(top, _topk_ref(_penalized(raw, tmpls, penalty), 10), what)
+        assert_matches(top, topk_ref(oracle_penalized(raw, tmpls, penalty), 10), what)
 
 
 # ---- depth and propagation coefficient ------------------------------------------------------------------------------
@@ -330,6 +289,6 @@ def test_depth_and_coeff_through_search(depth, coeff):
     assert g.depth == c.depth == depth
     for d in range(depth):
         assert np.array_equal(g.plane(d), c.plane(d)), f"plane {d}"
-    raw, _ = _check_full_search(g, c, tmpls, scene, 4, 4, 10)
+    raw, _ = check_full_search(g, c, tmpls, scene, 4, 4, 10)
     top = fdcm.search_topk(g, tmpls, scene, fdcm.DefaultSearch(4, 4), fdcm.BatchOptimize(10), fdcm.ExponentialPenalty(1.5), k=10)
-    _assert_matches(top, _topk_ref(_penalized(raw, tmpls, fdcm.ExponentialPenalty(1.5)), 10))
+    assert_matches(top, topk_ref(oracle_penalized(raw, tmpls, fdcm.ExponentialPenalty(1.5)), 10))

@@ -1,6 +1,5 @@
 """Distinct top-K on the device (fdcm_search_select, DistinctMatches): bit-exact against the numpy model of
-tests/test_select_host.py applied to search_all(..., penalty), which is itself bit-exact with the oracle."""
-import glob
+tests/models/select.py applied to search_all(..., penalty), which is itself bit-exact with the oracle."""
 import math
 import os
 import socket
@@ -10,11 +9,11 @@ import pytest
 
 import openfdcm_b200 as fdcm
 from openfdcm_b200._lib import FDCM_ERR_INVALID
-from tests.test_select_host import select_model
+from tests.helpers import load_object, synthetic
+from tests.models.select import select_model
 from tests.util import F32, plant_instances, synth_scene, synth_templates
 
 pytestmark = pytest.mark.gpu
-ASSETS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "real_assets")
 PEN = fdcm.ExponentialPenalty(1.5)
 OPT = fdcm.BatchOptimize(10)
 
@@ -38,22 +37,10 @@ def check(fm, tset, anchors, scene, searcher, cases, what=""):
     return allm
 
 
-def synthetic(n_tmpl=24, n_lines=20, seed=0, w=640, h=480, n_scene=200):
-    tmpls = synth_templates(n_tmpl, n_lines, w, seed=seed + 1)
-    scene = plant_instances(synth_scene(w, h, n_scene, seed=seed + 2), tmpls, w, h, seed=seed + 3, count=6)
-    return tmpls, scene
-
-
 def test_synthetic_scene_bit_exact():
     tmpls, scene = synthetic()
     fm = fdcm.build_cuda_featuremap(scene, fdcm.Dt3CudaParameters(30, 5.0, 1.5))
     check(fm, fdcm.TemplateSet(tmpls), fdcm.get_template_anchors(tmpls), scene, fdcm.DefaultSearch(4, 4), settings(len(tmpls)), "synthetic")
-
-
-def load_object(obj):
-    tm = sorted(glob.glob(os.path.join(ASSETS, obj, "templates", "*.tmpl")), key=lambda p: int(os.path.basename(p)[9:-5]))
-    scenes = sorted(glob.glob(os.path.join(ASSETS, obj, "scene_*", "camera_0.scene")), key=lambda p: int(os.path.basename(os.path.dirname(p))[6:]))
-    return [fdcm.read(p) for p in tm], [fdcm.read(p) for p in scenes]
 
 
 @pytest.mark.parametrize("obj", ["obj_01", "obj_02", "obj_03", "obj_04"])
