@@ -1,6 +1,7 @@
 """Helpers of more than one test module: the real assets and the synthetic workload of the device tests, the score
-functions the models take from the device evaluate, the parity hook of the dense poses, the oracle references of the
-search, and the poses and scenes of the fit tests."""
+functions the models take from the device evaluate, the models' inputs taken from the CPU oracle instead (scores, edge
+masks, scene bins), the parity hook of the dense poses, the oracle references of the search, the poses and scenes of the
+fit tests, and the map-geometry generators (tiny maps, the exact / literal boundary, scenes far from the origin)."""
 import ctypes as C
 import glob
 import math
@@ -92,6 +93,34 @@ def device_scores(fm):
                                                 _lib.ptr(out)))
         return out
     return score
+
+
+# ---- the CPU oracle as the models' inputs ----------------------------------------------------------------------------
+def oracle_scores(c):
+    """score_fn of the dense model from an oracle map c (orc.Dt3Cpu): evaluate of the rotated template at every
+    translation."""
+    def score(Rt, tr):
+        return c.evaluate(np.ascontiguousarray(np.asarray(Rt, F32).reshape(-1, 4).T), np.asarray(tr, F32).reshape(-1, 2))
+    return score
+
+
+def oracle_pose_score(c):
+    """score_fn of the fit model from an oracle map c: evaluate of the template posed by F at (F2, F5)."""
+    def score(tmpl, F):
+        F = np.asarray(F, F32).reshape(6)
+        return c.evaluate(np.ascontiguousarray(rotated(F[None], tmpl)[0].T), F[[2, 5]].reshape(1, 2))[0]
+    return score
+
+
+def oracle_masks(c):
+    """The edge masks (D, H, W) of a stage-1 oracle map c: its zero pixels."""
+    return np.stack([c.plane(d) == 0 for d in range(c.depth)]).astype(np.uint8) if c.depth else np.zeros((0, 0, 0), np.uint8)
+
+
+def oracle_bins(c, scene):
+    """The scene bins of an oracle map c: closest_orientation of every shifted scene line."""
+    ts = shifted_scene(scene, c.shift)
+    return np.array([orc.closest_orientation(c.keys, ts[:, i]) for i in range(ts.shape[1])], np.int32)
 
 
 def refine_reference(fm, tmpls, anchors, matches, r, score_fn=None, tmpl_idx_base=0):
@@ -223,3 +252,88 @@ def one_match(T, t=0):
     m = np.zeros(1, _lib.MATCH_DTYPE)
     m["tmpl_idx"], m["transform"] = t, T
     return m
+
+
+# ---- the map geometry: tiny maps, the exact / literal boundary, scenes far from the origin -------------------------
+def pinned_scene(side, n, seed):
+    """n random lines in [0, side-1]^2 with lengths 0..side (a third of them on integer coordinates) plus two 1-px lines
+    at the corners that pin the extent: at padding 1 the map side is exactly `side`.  Side 1: one point line."""
+    if side == 1:
+        return np.zeros((4, 1), F32)
+    rng = np.random.default_rng(seed)
+    p1 = rng.uniform(0, side - 1, (2, n))
+    ang = rng.uniform(0, 2 * math.pi, n)
+    ln = rng.uniform(0, side, n)
+    p2 = np.clip(p1 + ln * np.stack([np.cos(ang), np.sin(ang)]), 0, side - 1)
+    lines = np.concatenate([p1, p2])
+    lines[:, : n // 3] = np.round(lines[:, : n // 3])
+    pins = np.array([[0, 0, 1, 0], [side - 2, side - 1, side - 1, side - 1]], np.float64).T
+    return np.ascontiguousarray(np.concatenate([lines, pins], axis=1), F32)
+
+
+def map_templates(side, seed, n=6):
+    """Templates scaled to a map of `side` px: lines of 1..side px about the origin, one template holding a zero-length
+    line, one larger than the map (every hypothesis of it is nullopt)."""
+    rng = np.random.default_rng(seed)
+    out = []
+    for _ in range(n):
+        k = int(rng.integers(1, 6))
+        c = rng.uniform(-side / 4, side / 4, (2, k))
+        ang = rng.uniform(0, math.pi, k)
+        ln = rng.uniform(1, side, k) if side > 1 else np.ones(k)
+        d = 0.5 * ln * np.stack([np.cos(ang), np.sin(ang)])
+        out.append(np.ascontiguousarray(np.concatenate([c - d, c + d]), F32))
+    out[1] = np.ascontiguousarray(np.concatenate([out[1], np.array([[0.5], [0.25], [0.5], [0.25]], F32)], axis=1), F32)
+    big = 2.0 * side + 5.0
+    out.append(np.array([[-big / 2, 0, big / 2, 0], [0, -big / 3, 0, big / 3]], F32).T.copy())
+    return out
+
+
+def shifted_scene(scene, shift):
+    """The scene in map coordinates, as the host computes it: scene + shift in fp32 (core/math.h:352-354)."""
+    return (np.asarray(scene, F32).T.reshape(-1, 2) + np.asarray(shift, F32)).reshape(-1, 4).T.astype(F32)
+
+
+def host_geometry(scene, padding):
+    """scene_centered_translation (host_math.hpp) in fp32: shift = req/2 - (mx+mn)/2, side = ceil(req + 1)."""
+    pts = np.asarray(scene, F32).T.reshape(-1, 2)
+    mn, mx = pts.min(axis=0), pts.max(axis=0)
+    d = (mx - mn).astype(F32)
+    req = F32(max(F32(1), F32(padding))) * F32(max(d[0], d[1]))
+    shift = (req / F32(2) - (mx + mn) / F32(2)).astype(F32)
+    return shift, int(math.ceil(float(req + F32(1))))
+
+
+# offsets with fractional parts; per offset: the seed of a 3-line scene and (seed, scale) of a synthetic scene whose
+# shifted end points leave the map at padding 1.0 (chosen on the CPU, asserted by check_generators)
+FAR = {1e3: (1234.56, -987.31), 3e4: (-29999.37, 30123.71), 1e5: (-99999.63, 50000.21)}
+FAR_SMALL_SEED = {1e3: 8, 3e4: 0, 1e5: 14}
+FAR_SYNTH = {1e3: (104, 1.1), 3e4: (100, 1.2), 1e5: (100, 0.9)}
+
+
+def far_small_scene(offset, seed):
+    """3 random lines within an extent of 50..900 px, moved to the offset."""
+    rng = np.random.default_rng(seed)
+    ext = rng.uniform(50, 900)
+    lines = rng.uniform(0, ext, (4, 3)) + np.array(FAR[offset] * 2, np.float64).reshape(4, 1)
+    tmpls = synth_templates(6, 5, max(ext, 100.0), seed=seed + 1, max_len=max(8.0, ext / 4))
+    return np.ascontiguousarray(lines, F32), tmpls
+
+
+def far_synthetic_scene(offset, seed, scale):
+    """The 640x480 synthetic scene with planted templates, without its corner lines, scaled and moved to the offset."""
+    tmpls = synth_templates(10, 12, 640, seed=seed + 1)
+    scene = plant_instances(synth_scene(640, 480, 120, seed=seed)[:, :-2], tmpls, 640, 480, seed=seed + 2)
+    scene = scene.astype(np.float64) * scale + np.array(FAR[offset] * 2, np.float64).reshape(4, 1)
+    return np.ascontiguousarray(scene, F32), [np.ascontiguousarray(t * F32(scale), F32) for t in tmpls]
+
+
+def far_scene(offset, source):
+    if source == "small":
+        return far_small_scene(offset, FAR_SMALL_SEED[offset])
+    seed, scale = FAR_SYNTH[offset]
+    return far_synthetic_scene(offset, seed, scale)
+
+
+TINY = [1, 2, 3, 5, 8, 31, 32, 33, 64, 65, 129, 160, 161, 164, 165]
+BOUNDARY = [2896, 2897, 2898]
