@@ -497,6 +497,41 @@ fdcm_status fdcm_fit_matches_scaled(const fdcm_dt3* map, const fdcm_templates* t
                                     float penalty_tau, const fdcm_fit_params* fit, const fdcm_fit_scale* scale, const fdcm_match* in,
                                     int64_t n, fdcm_match* out, fdcm_fit_stats* stats);
 
+/* ---- scale in the line-alignment search (beyond the reference) -------------------------------------------------------
+ * fdcm_search over a grid of template scales: exactly the search of the scaled copies of the templates, expressed in the
+ * original templates.  Rules, in fp32 without contraction, for a set of T templates and a grid of S scales:
+ *   1. Scales.  s_k, k = 0..S-1, as in scaled dense rule 1 (the same computation, checks and FDCM_DENSE_MAX_SCALES).
+ *   2. Copies.  Copy C_v, v = t * S + k, is template t with every coordinate of every line multiplied by s_k, one fp32
+ *      multiply each: (s_k*x1, s_k*y1, s_k*x2, s_k*y2).
+ *   3. Hypotheses and raw results: exactly those of fdcm_search on the set {C_0 .. C_{T*S-1}} in v order with the same
+ *      params: DefaultSearch on each copy's own line lengths (a scaled copy pairs with scene lines of its own length),
+ *      BatchOptimize / DefaultOptimize, ConcentricRange, the hypothesis order, validity, the raw score and the copy transform
+ *      M = (r00 r01 tx; r10 r11 ty).  fdcm_search_last_hypotheses and fdcm_search_last_stats report this copy search: the
+ *      first field of a hypothesis is v + tmpl_idx_base.
+ *   4. Record of a valid hypothesis of C_v: tmpl_idx = t + tmpl_idx_base; transform = (s_k*r00, s_k*r01, tx, s_k*r10,
+ *      s_k*r11, ty), one fp32 multiply each: the pose of template t, of the form of the dense grid's (s cos, s sin) poses;
+ *      score = the raw score, divided when a penalty is given by the penalty denominator of getTemplateLengths(C_v), the
+ *      copy's own length (host powf like the search).  That length is deliberately not scaled dense rule 3's len_t * s_k:
+ *      the two differ by rounding only, and with the copy's own length the records are penalize(search(copies)) bit for bit.
+ *   5. Output.  top_k == 0: every valid record in hypothesis order, like fdcm_search.  top_k > 0: the top_k best in
+ *      (score, h) order; with select the walk of fdcm_search_select with scaled dense rule 4 (the angle test
+ *      Ta0*Tb0 + Ta3*Tb3 >= cos_thr * (s_a * s_b), the anchor of template t posed by the record's transform,
+ *      max_per_template counting a template over all its scales).  With cov and min_coverage > 0 the coverage filter of
+ *      rule 6 of the match verification runs on the records of rule 4, before the top-K or the selection.  With refine the
+ *      selected records are refined, scoring with the search's denominator of t (the unscaled length) like scaled dense
+ *      rule 5: the result equals fdcm_refine_matches of the unrefined output.  select, refine and cov need top_k > 0.
+ *   6. S == 1 with scale_start == 1: byte-identical to fdcm_search, fdcm_search_select, fdcm_search_refine or
+ *      fdcm_search_verify (records, hypothesis list and stats): s*x and s*r are exact for s = 1.0f.
+ *   7. Invalid input fails with FDCM_ERR_INVALID: everything fdcm_search_verify rejects, everything fdcm_search_dense_scales
+ *      rejects about the grid (a null scales too), T * S or the copies' line count of 2^31 or more, and a selection over
+ *      2^31 or more hypotheses counted over the copies.  A set whose copies give no hypothesis gives no matches.
+ * Cost: the search of T * S templates (S times the hypotheses); the copies are prepared on the host and uploaded once per
+ * (map, template set load, grid) and kept on the map. */
+fdcm_status fdcm_search_scales(const fdcm_dt3* map, const fdcm_templates* templates, const float* scene_xyxy, int32_t n_scene,
+                               const fdcm_search_params* params, const fdcm_scale_grid* scales,
+                               const fdcm_select_params* select, const fdcm_refine_params* refine,
+                               const fdcm_coverage_params* cov, fdcm_match* out, int64_t capacity, int64_t* n_out);
+
 /* optimize(optimizer, templates, alignments, featuremap) (matching/optimizestrategy.h:62-64; BatchOptimize:
  * batchoptimize.cpp:6-123, batch_size == 0: DefaultOptimize, defaultoptimize.cpp:6-93).  The templates are used
  * as given (already aligned); alignments: n_tmpl (x,y) pairs.  Outputs per template: has_value (0 = nullopt),

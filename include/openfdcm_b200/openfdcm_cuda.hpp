@@ -496,6 +496,51 @@ inline std::vector<Match> searchDense(const Dt3Cuda& fm, const std::vector<LineA
     return detail::search_dense(fm, templates, dense, FDCM_PENALTY_EXPONENTIAL, pen.tau, k, select, refine, &c, &scales);
 }
 
+// line-alignment search over a scale grid (rules of fdcm_search_scales): the search of every template scaled by every
+// s_k, each match expressed in its original template (tmplIdx), with the scale in the rotation part of its transform
+namespace detail {
+inline std::vector<Match> search_scales(const DefaultSearch& s, int batch, int penalty_kind, float tau, const Dt3Cuda& fm,
+                                        const std::vector<LineArray>& templates, const LineArray& scene, int k, const ScaleGrid& scales,
+                                        const DistinctMatches* select, const PoseRefinement* refine, const EdgeCoverage* verify) {
+    std::vector<float> flat;
+    std::vector<int32_t> off;
+    pack(templates, flat, off);
+    fdcm_templates* ts = nullptr;
+    check(fdcm_templates_create(flat.data(), off.data(), (int32_t)templates.size(), fm.info().device, &ts));
+    const std::unique_ptr<fdcm_templates, fdcm_status (*)(fdcm_templates*)> owner(ts, fdcm_templates_release);
+    const fdcm_search_params p{(int32_t)s.max_tmpl_lines, (int32_t)s.max_scene_lines, batch, penalty_kind, tau, k, 0, 0, 0.f, 0.f, 0.f, 0.f};
+    const fdcm_scale_grid g{scales.scales, scales.start, scales.ratio};
+    fdcm_select_params q{};
+    if (select) q = fdcm_select_params{select->maxPerTemplate, select->radius, select->maxAngle, select->acrossTemplates ? 1 : 0};
+    fdcm_refine_params r{};
+    if (refine) r = refine_params(*refine);
+    fdcm_coverage_params c{};
+    if (verify) c = coverage_params(*verify);
+    int64_t cap = k > 0 ? k : 0;   // k == 0: every hypothesis of every copy may match
+    if (k <= 0)
+        for (const auto& t : templates)
+            cap += 2 * (int64_t)std::max(scales.scales, 0) * (int64_t)std::min<size_t>(t.size() / 4, (size_t)s.max_tmpl_lines) *
+                   (int64_t)s.max_scene_lines;
+    std::vector<fdcm_match> rec((size_t)std::max<int64_t>(cap, 1));
+    int64_t n = 0;
+    check(fdcm_search_scales(fm.handle(), ts, scene.data(), (int32_t)(scene.size() / 4), &p, &g, select ? &q : nullptr, refine ? &r : nullptr,
+                             verify ? &c : nullptr, rec.data(), (int64_t)rec.size(), &n));
+    return to_matches(rec, n);
+}
+}   // namespace detail
+// every match of the scaled copies in hypothesis order, nullopt hypotheses dropped
+inline std::vector<Match> search(const DefaultMatch&, const DefaultSearch& s, const BatchOptimize& o, const Dt3Cuda& fm,
+                                 const std::vector<LineArray>& templates, const LineArray& scene, const ScaleGrid& scales) {
+    return detail::search_scales(s, (int)o.batchSize, FDCM_PENALTY_NONE, 0.f, fm, templates, scene, 0, scales, nullptr, nullptr, nullptr);
+}
+// fused search over a scale grid [-> coverage filter] -> top-k (or distinct top-k) [-> pose refinement] on the device
+inline std::vector<Match> searchTopK(const DefaultSearch& s, const BatchOptimize& o, const ExponentialPenalty& pen, const Dt3Cuda& fm,
+                                     const std::vector<LineArray>& templates, const LineArray& scene, int k, const ScaleGrid& scales,
+                                     const DistinctMatches* select = nullptr, const PoseRefinement* refine = nullptr,
+                                     const EdgeCoverage* verify = nullptr) {
+    return detail::search_scales(s, (int)o.batchSize, FDCM_PENALTY_EXPONENTIAL, pen.tau, fm, templates, scene, k, scales, select, refine, verify);
+}
+
 // pose fit (beyond the reference; rules of fdcm_fit_matches): per match, up to `iterations` Gauss-Newton steps of oriented
 // point-to-line least squares of the template's samples against the build scene's line segments (nearest scene line within
 // maxDistance pixels on an orientation plane within binTolerance planes).  It needs scene lines near the pose, uses no

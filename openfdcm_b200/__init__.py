@@ -450,7 +450,7 @@ class PoseFit:
 
 
 def _search_raw(featuremap, templates, scene, searcher, optimizer, penalty=None, top_k=0, tmpl_idx_base=0, select=None, refine=None,
-                verify=None):
+                verify=None, scales=None):
     if not isinstance(featuremap, Dt3Cuda):
         raise TypeError("the CUDA search needs a Dt3Cuda feature map (build_cuda_featuremap)")
     tset = templates if isinstance(templates, TemplateSet) else TemplateSet(templates, featuremap.device)
@@ -463,12 +463,20 @@ def _search_raw(featuremap, templates, scene, searcher, optimizer, penalty=None,
                           searcher.low_boundary if conc else 0.0, searcher.high_boundary if conc else 0.0)
     if tset.n_tmpl == 0:
         return np.zeros(0, MATCH_DTYPE)
-    cap = int(top_k) if top_k > 0 or select is not None else 2 * tset.n_tmpl * max(1, min(searcher.max_tmpl_lines, tset.max_lines)) * max(
+    # top_k == 0: every hypothesis may match (with scales, every hypothesis of every copy)
+    copies = 1 if scales is None else int(scales.scales)
+    cap = int(top_k) if top_k > 0 or select is not None else 2 * tset.n_tmpl * copies * max(1, min(searcher.max_tmpl_lines, tset.max_lines)) * max(
         1, searcher.max_scene_lines)
     out = np.zeros(max(cap, 1), MATCH_DTYPE)
     n = C.c_int64(0)
     n_scene = _lib.FDCM_SCENE_RESIDENT if s is None else s.shape[0]
-    if verify is not None:
+    if scales is not None:
+        sp = None if select is None else C.byref(select._params())
+        rp = None if refine is None else C.byref(refine._params())
+        vp = None if verify is None else C.byref(verify._params())
+        check(lib().fdcm_search_scales(featuremap._h, tset._h, ptr(s), n_scene, C.byref(p), C.byref(scales._params()), sp, rp, vp, ptr(out),
+                                       out.shape[0], C.byref(n)))
+    elif verify is not None:
         sp = None if select is None else C.byref(select._params())
         rp = None if refine is None else C.byref(refine._params())
         check(lib().fdcm_search_verify(featuremap._h, tset._h, ptr(s), n_scene, C.byref(p), sp, rp, C.byref(verify._params()), ptr(out),
@@ -492,17 +500,22 @@ def search(matcher, searcher, optimizer, featuremap, templates, scene):
 
 
 def search_topk(featuremap, templates, scene, searcher, optimizer, penalty=None, k=10, tmpl_idx_base=0, *, select=None, refine=None,
-                verify=None, fit=None):
+                verify=None, fit=None, scales=None):
     """Fused search -> penalize -> top-k on the device; returns a MATCH_DTYPE record array (ascending score).
     select: a DistinctMatches for the distinct top-k (the kept matches in acceptance order, also ascending score).
     refine: a PoseRefinement applied to the selected matches on the device, equal to refine_matches of the unrefined
     result (same order: re-rank with sort_matches); it lowers the score, not the pose error (see PoseRefinement).
     verify: an EdgeCoverage whose min_coverage > 0 drops every match of lower (or NaN) coverage before the selection.
     fit: a PoseFit applied last (after select / refine / verify), equal to fit_matches of the unfitted result; the fitted
-    list is not re-selected or re-sorted, so two distinct matches may converge on one instance."""
+    list is not re-selected or re-sorted, so two distinct matches may converge on one instance.
+    scales: a ScaleGrid (fdcm_search_scales): the search of every template scaled by every s_k (its own line lengths pair
+    with the scene's), each match expressed in its original template: tmpl_idx names the template and the transform's
+    rotation part carries the scale.  A penalty divides by the scaled copy's length; select's max_per_template counts a
+    template over all its scales; refine scores with the unscaled length; fit with a scale_range fits the scale too.
+    None: the unscaled search."""
     if fit is not None and not isinstance(templates, TemplateSet) and isinstance(featuremap, Dt3Cuda):
         templates = TemplateSet(templates, featuremap.device)
-    out = _search_raw(featuremap, templates, scene, searcher, optimizer, penalty, k, tmpl_idx_base, select, refine, verify).copy()
+    out = _search_raw(featuremap, templates, scene, searcher, optimizer, penalty, k, tmpl_idx_base, select, refine, verify, scales).copy()
     return out if fit is None else fit_matches(featuremap, templates, out, fit, penalty, tmpl_idx_base)
 
 
@@ -599,9 +612,11 @@ def fit_matches(featuremap, templates, matches, fit=None, penalty=None, tmpl_idx
     return (out, stats[: rec.shape[0]].copy()) if return_stats else out
 
 
-def search_all(featuremap, templates, scene, searcher, optimizer, penalty=None, tmpl_idx_base=0):
-    """Every match (hypothesis order) as a MATCH_DTYPE record array, optionally penalised on the device."""
-    return _search_raw(featuremap, templates, scene, searcher, optimizer, penalty, 0, tmpl_idx_base).copy()
+def search_all(featuremap, templates, scene, searcher, optimizer, penalty=None, tmpl_idx_base=0, scales=None):
+    """Every match (hypothesis order) as a MATCH_DTYPE record array, optionally penalised on the device.
+    scales: a ScaleGrid, as in search_topk: the matches of the scaled copies, copy by copy (template t's copies in scale
+    order), in their original templates."""
+    return _search_raw(featuremap, templates, scene, searcher, optimizer, penalty, 0, tmpl_idx_base, scales=scales).copy()
 
 
 class SceneBatch:

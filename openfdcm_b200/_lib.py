@@ -124,6 +124,8 @@ SIGNATURES = {
                                           C.c_int32, _P, C.c_int64, C.POINTER(C.c_int64), _P]),
     "fdcm_fit_matches_scaled": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_float, C.POINTER(FitParams), C.POINTER(FitScaleParams), _P,
                                           C.c_int64, _P, _P]),
+    "fdcm_search_scales": (C.c_int, [_P, _P, _P, C.c_int32, C.POINTER(SearchParams), C.POINTER(ScaleGridParams), C.POINTER(SelectParams),
+                                     C.POINTER(RefineParams), C.POINTER(CoverageParams), _P, C.c_int64, C.POINTER(C.c_int64)]),
     "fdcm_fit_samples": (C.c_int, [_P, C.c_int32, C.c_float, _P, C.c_int64, C.POINTER(C.c_int64)]),
     "fdcm_optimize": (C.c_int, [_P, _P, _P, C.c_int32, _P, C.c_int32, _P, _P, _P]),
     "fdcm_search_host": (C.c_int, [_P, _P, _P, C.c_int32, _P, C.c_int32, C.POINTER(SearchParams), _P, C.c_int64,

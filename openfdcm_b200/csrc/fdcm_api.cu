@@ -326,7 +326,16 @@ struct fdcm_dt3 {
     // (t, k) at t * S + k); empty: the T per-template ones only
     mutable std::vector<float> denom_scales;
     mutable DevBuf s_dense_keys, s_dense_rot;   // dense pose-grid search (records: s_rec / s_valid / s_hyp_off)
-    mutable DevBuf s_dense_rs;                  // scaled dense search: the grid scale of every record
+    mutable DevBuf s_dense_rs;                  // scaled dense and line searches: the grid scale of every record
+    // line search over a scale grid: the scaled copies of the last set searched with a grid on this map, for (the set's
+    // load_id, the s_k), with their penalty denominators for (cp_kind, cp_tau).  Per map for the reason of s_denom; the set
+    // itself stays read-only, so maps sharing it can search it with different grids at the same time.
+    mutable DevBuf cp_lines, cp_offs, cp_argsort, cp_len, cp_denom;
+    mutable uint64_t cp_set = 0;
+    mutable std::vector<float> cp_scales;
+    mutable std::vector<float> cp_lengths;      // getTemplateLengths of every copy
+    mutable int cp_kind = -1;
+    mutable float cp_tau = 0.f;
     // match verification: the dilated edge mask of (cov_radius, cov_tol) for the map write cov_gen (0: none), its scratch and
     // the standalone call's buffers; cov_ev is recorded after the dilation, which later calls on any stream wait on
     uint64_t write_gen = 0;         // incremented by every write of the map (map_written)
@@ -1579,6 +1588,85 @@ static fdcm_status stage_uploads(const fdcm_dt3* m, fdcm_templates* t, const int
     return FDCM_OK;
 }
 
+// fdcm_search_scales rule 2: the copies C_v, v = t * S + k, of set t on the map's buffers, unless the map holds them for
+// (t's load, scales) already, and their penalty denominators of (kind, tau) (those of getTemplateLengths(C_v), host powf).
+// The copies take the host preparation of a set's load, so their length order is std::sort's.  The set keeps no host copy
+// of its lines, so a new grid first downloads them.  Uploads go through the set's pinned staging on the copy stream, and
+// `s` waits for them.  (m->search_mutex held)
+static fdcm_status copy_set(const fdcm_dt3* m, fdcm_templates* t, const std::vector<float>& scales, int kind, float tau, cudaStream_t s) {
+    const size_t S = scales.size(), T = (size_t)t->n_tmpl, n = (size_t)t->n_lines, TS = T * S, N = n * S;
+    const bool fresh = m->cp_set != t->load_id || m->cp_scales != scales;
+    const bool denom = kind != FDCM_PENALTY_NONE && (fresh || m->cp_kind != kind || m->cp_tau != tau);
+    if (!fresh && !denom) return FDCM_OK;
+    std::lock_guard<std::mutex> lk(t->mu);
+    cudaStream_t cs;
+    if (fdcm_status st = get_copy_stream(m->device, &cs)) return st;
+    if (t->ready.e) CUDA_TRY(cudaEventSynchronize(t->ready.e));   // (the staging may still feed an earlier upload)
+    std::vector<float> lines, len, anchors;
+    std::vector<int32_t> offs, argsort;
+    if (fresh) {
+        m->cp_set = 0;
+        m->cp_kind = -1;
+        CUDA_TRY(t->h_stage.reserve(std::max<size_t>(16, n * 16)));
+        if (n) {
+            CUDA_TRY(cudaMemcpyAsync(t->h_stage.p, t->lines.p, n * 16, cudaMemcpyDeviceToHost, cs));
+            CUDA_TRY(cudaStreamSynchronize(cs));
+        }
+        const float* tl = t->h_stage.as<float>();
+        lines.resize(N * 4);
+        offs.assign(TS + 1, 0);
+        for (size_t i = 0; i < T; ++i) {
+            const int32_t l0 = t->offsets[i], L = t->offsets[i + 1] - l0;
+            for (size_t k = 0; k < S; ++k) {
+                const size_t v = i * S + k;
+                offs[v + 1] = offs[v] + L;
+                const float* src = tl + 4 * (size_t)l0;
+                float* dst = lines.data() + 4 * (size_t)offs[v];
+                for (size_t j = 0; j < 4 * (size_t)L; ++j) dst[j] = scales[k] * src[j];   // one fp32 multiply
+            }
+        }
+        len.resize(std::max<size_t>(N, 1));
+        argsort.resize(std::max<size_t>(N, 1));
+        anchors.resize(2 * std::max<size_t>(TS, 1));   // (not used: the selection poses the anchor of the original template)
+        template_host_prep(lines.data(), offs.data(), (int32_t)TS, len.data(), argsort.data(), anchors.data(), m->cp_lengths);
+        CUDA_TRY(m->cp_lines.reserve(std::max<size_t>(16, N * 16)));
+        CUDA_TRY(m->cp_offs.reserve((TS + 1) * 4));
+        CUDA_TRY(m->cp_argsort.reserve(std::max<size_t>(4, N * 4)));
+        CUDA_TRY(m->cp_len.reserve(std::max<size_t>(4, N * 4)));
+    }
+    if (denom) CUDA_TRY(m->cp_denom.reserve(std::max<size_t>(4, TS * 4)));
+    // staging: lines, argsort, lengths, offsets (a new grid), then the denominators
+    const size_t geo = fresh ? N * 24 + (TS + 1) * 4 : 0;
+    CUDA_TRY(t->h_stage.reserve(std::max<size_t>(16, geo + (denom ? TS * 4 : 0))));
+    unsigned char* stage = t->h_stage.as<unsigned char>();
+    if (fresh) {
+        const std::pair<void*, size_t> parts[4] = {{lines.data(), N * 16}, {argsort.data(), N * 4}, {len.data(), N * 4}, {offs.data(), (TS + 1) * 4}};
+        void* const dst[4] = {m->cp_lines.p, m->cp_argsort.p, m->cp_len.p, m->cp_offs.p};
+        size_t off = 0;
+        for (int i = 0; i < 4; ++i) {
+            if (parts[i].second == 0) continue;
+            std::memcpy(stage + off, parts[i].first, parts[i].second);
+            CUDA_TRY(cudaMemcpyAsync(dst[i], stage + off, parts[i].second, cudaMemcpyHostToDevice, cs));
+            off += parts[i].second;
+        }
+    }
+    if (denom && TS) {
+        float* d = reinterpret_cast<float*>(stage + geo);
+        for (size_t v = 0; v < TS; ++v) d[v] = penalty_denominator(kind, tau, m->cp_lengths[v]);
+        CUDA_TRY(cudaMemcpyAsync(m->cp_denom.p, d, TS * 4, cudaMemcpyHostToDevice, cs));
+    }
+    CUDA_TRY(t->ready.record(cs));
+    CUDA_TRY(cudaStreamWaitEvent(s, t->ready.e, 0));
+    t->upload_pending = false;
+    m->cp_set = t->load_id;
+    m->cp_scales = scales;
+    if (denom) {
+        m->cp_kind = kind;
+        m->cp_tau = tau;
+    }
+    return FDCM_OK;
+}
+
 // The search kernel stages the longest template of a set in shared memory, at least one warp's worth per block: a set
 // holding a template longer than one warp can stage within the device's per-block opt-in limit cannot be searched.
 static fdcm_status search_smem_optin(int device, int max_lines, int* smem_optin) {
@@ -1843,12 +1931,19 @@ static fdcm_status run_coverage(const fdcm_dt3* m, const fdcm_templates* t, int3
     return FDCM_OK;
 }
 
+static fdcm_status dense_scales(const fdcm_scale_grid* g, std::vector<float>* out);
+
 // sel: distinct top-K (fdcm_search_select); ref: pose refinement of the top-K (fdcm_search_refine); cov: the coverage filter
-// before the selection (fdcm_search_verify, min_coverage > 0); nullptr when not asked
+// before the selection (fdcm_search_verify, min_coverage > 0); grid: the scale grid of fdcm_search_scales; nullptr when not
+// asked
 static fdcm_status search_impl(const fdcm_dt3* m, const fdcm_templates* tc, const float* scene, int32_t n_scene,
                                const fdcm_search_params* p, fdcm_match* out, int64_t capacity, int64_t* n_out, fdcm_comm* comm,
                                const fdcm_select_params* sel, const fdcm_refine_params* ref = nullptr,
-                               const fdcm_coverage_params* cov = nullptr) {
+                               const fdcm_coverage_params* cov = nullptr, const fdcm_scale_grid* grid = nullptr) {
+    std::vector<float> scales;   // empty: the unscaled search
+    if (grid)
+        if (fdcm_status st = dense_scales(grid, &scales)) return st;
+    const int S = grid ? (int)scales.size() : 1;
     if (!m || !tc || !p || !n_out) return fail(FDCM_ERR_INVALID, "null argument");
     *n_out = 0;
     if (fdcm_status st = select_or_plain(&sel, p->top_k, comm != nullptr)) return st;
@@ -1858,6 +1953,8 @@ static fdcm_status search_impl(const fdcm_dt3* m, const fdcm_templates* tc, cons
         p->penalty_kind > 2)
         return fail(FDCM_ERR_INVALID, "bad search parameters");
     if (tc->device != m->device) return fail(FDCM_ERR_INVALID, "templates and feature map live on different devices");
+    if (grid && ((int64_t)tc->n_tmpl * S > INT32_MAX || tc->n_lines * S > INT32_MAX))
+        return fail(FDCM_ERR_INVALID, "scaled search: at most 2^31 - 1 copies and copy lines (templates or lines x scales)");
     fdcm_templates* t = const_cast<fdcm_templates*>(tc);
     std::lock_guard<std::mutex> lk(m->search_mutex);
     m->last_n_hyp = 0;
@@ -1890,15 +1987,23 @@ static fdcm_status search_impl(const fdcm_dt3* m, const fdcm_templates* tc, cons
     n_scene = m->s_sorted_n;   // the lines that take part in the length matching
     if (n_scene <= 0) FDCM_NO_LOCAL_MATCHES();   // concentricrange.cpp:37-38
     const int nS = std::min<int>(n_scene, p->max_scene_lines);
-    std::vector<int64_t> hyp_off((size_t)t->n_tmpl + 1, 0);
-    for (int i = 0; i < t->n_tmpl; ++i) {
-        const int L = t->offsets[(size_t)i + 1] - t->offsets[(size_t)i];
-        hyp_off[(size_t)i + 1] = hyp_off[(size_t)i] + 2LL * std::min(L, p->max_tmpl_lines) * nS;
+    // hypothesis offsets of the searched set (the copies of a scale grid, v = t * S + k, each with template t's count); with
+    // a grid they follow the T + 1 per-template offsets of the selection, hyp_off[t] = that of copy t * S
+    const size_t T = (size_t)t->n_tmpl, TS = T * S, lead = grid ? T + 1 : 0;
+    std::vector<int64_t> hyp_off(lead + TS + 1, 0);
+    int64_t* copy_off = hyp_off.data() + lead;
+    for (size_t v = 0; v < TS; ++v) {
+        const size_t i = v / S;
+        const int L = t->offsets[i + 1] - t->offsets[i];
+        copy_off[v + 1] = copy_off[v] + 2LL * std::min(L, p->max_tmpl_lines) * nS;
     }
-    const int64_t H = hyp_off[(size_t)t->n_tmpl];
+    for (size_t i = 0; i < lead; ++i) hyp_off[i] = copy_off[i * S];
+    const int64_t H = copy_off[TS];
     m->last_n_hyp = H;
     m->last_stats.n_hypotheses = H;
     if (H == 0) FDCM_NO_LOCAL_MATCHES();
+    // (the selection's limit, before the copies' records are allocated)
+    if (grid && sel && H >= ((int64_t)1 << 31)) return fail(FDCM_ERR_INVALID, "distinct top-K: more than 2^31 - 1 hypotheses");
 #undef FDCM_NO_LOCAL_MATCHES
 
     // ---- workspace ----
@@ -1908,17 +2013,21 @@ static fdcm_status search_impl(const fdcm_dt3* m, const fdcm_templates* tc, cons
     CUDA_TRY(m->s_hyp.reserve((size_t)H * 16));
     CUDA_TRY(m->s_counters.reserve(3 * 8));
 
-    const float* d_denom = nullptr;
+    if (grid) {
+        CUDA_TRY(m->s_dense_rs.reserve((size_t)H * 4));
+        if (fdcm_status st = copy_set(m, t, scales, p->penalty_kind, p->penalty_tau, s)) return st;
+    }
+    const float* d_denom = nullptr;   // of the set's templates: the search's, and with a grid the refinement's
     if (fdcm_status st = stage_uploads(m, t, hyp_off.data(), hyp_off.size(), p->penalty_kind, p->penalty_tau, s, &d_denom)) return st;
     CUDA_TRY(cudaMemsetAsync(m->s_counters.p, 0, 3 * 8, s));
 
     TemplatesView tv;
-    tv.lines = t->lines.as<float4>();
-    tv.offsets = t->offs.as<int32_t>();
-    tv.argsort = t->argsort.as<int32_t>();
-    tv.line_len = t->line_len.as<float>();
-    tv.denom = d_denom;
-    tv.n_tmpl = t->n_tmpl;
+    tv.lines = grid ? m->cp_lines.as<float4>() : t->lines.as<float4>();
+    tv.offsets = grid ? m->cp_offs.as<int32_t>() : t->offs.as<int32_t>();
+    tv.argsort = grid ? m->cp_argsort.as<int32_t>() : t->argsort.as<int32_t>();
+    tv.line_len = grid ? m->cp_len.as<float>() : t->line_len.as<float>();
+    tv.denom = grid && d_denom ? m->cp_denom.as<float>() : d_denom;
+    tv.n_tmpl = (int32_t)TS;
     tv.max_lines = std::max(1, t->max_lines);
     SceneView sv;
     sv.lines = m->s_scene.as<float4>();
@@ -1930,7 +2039,7 @@ static fdcm_status search_impl(const fdcm_dt3* m, const fdcm_templates* tc, cons
     sl.max_scene_lines = p->max_scene_lines;
     sl.batch = p->batch_size > 0 ? p->batch_size : 1;   // DefaultOptimize == batches of one (defaultoptimize.cpp:49-64)
     sl.tmpl_idx_base = p->tmpl_idx_base;
-    sl.hyp_off = m->s_hyp_off.as<int64_t>();
+    sl.hyp_off = m->s_hyp_off.as<int64_t>() + lead;
     sl.n_hyp = H;
     sl.direct_align = nullptr;
     SearchOutputs so;
@@ -1964,13 +2073,27 @@ static fdcm_status search_impl(const fdcm_dt3* m, const fdcm_templates* tc, cons
         KernelScope k("search", 0.0, s);
         CUDA_TRY(launch_search(map_view(m), m->table_dev, tv, sv, sl, so, smem_optin, s));
     }
+    const float* rec_scale = grid ? m->s_dense_rs.as<float>() : nullptr;
+    if (grid) {
+        // rule 4, before the coverage filter: it poses the original template
+        ScaleRemapLaunch rl;
+        rl.rec = so.rec;
+        rl.valid = so.valid;
+        rl.rec_scale = m->s_dense_rs.as<float>();
+        rl.n_hyp = H;
+        rl.scales = S;
+        rl.tmpl_idx_base = p->tmpl_idx_base;
+        std::copy(scales.begin(), scales.end(), rl.scale);
+        KernelScope k("search_scale_remap", (double)H * (1 + 2 * sizeof(fdcm_match) + 4), s);
+        launch_search_scale_remap(rl, s);
+    }
     if (cov)
         if (fdcm_status st = run_coverage(m, t, p->tmpl_idx_base, cov, so.rec, H, nullptr, so.valid, s)) return st;
 
     unsigned long long counters[3] = {0, 0, 0};
     fdcm_status result = FDCM_OK;
     if (p->top_k > 0) {
-        result = run_topk(m, t, p->top_k, p->tmpl_idx_base, sel, ref, H, nullptr, d_denom, smem_optin, comm, counters, s, out, capacity,
+        result = run_topk(m, t, p->top_k, p->tmpl_idx_base, sel, ref, H, rec_scale, d_denom, smem_optin, comm, counters, s, out, capacity,
                           n_out);
         if (result != FDCM_OK && result != FDCM_ERR_CAPACITY) return result;
     } else {
@@ -2031,6 +2154,24 @@ extern "C" fdcm_status fdcm_search_verify(const fdcm_dt3* m, const fdcm_template
         if (fdcm_status st = check_refine_top_k(p->top_k)) return st;
     }
     return search_impl(m, tc, scene, n_scene, p, out, capacity, n_out, nullptr, select, refine, cov->min_coverage > 0.f ? cov : nullptr);
+}
+
+extern "C" fdcm_status fdcm_search_scales(const fdcm_dt3* m, const fdcm_templates* tc, const float* scene, int32_t n_scene,
+                                          const fdcm_search_params* p, const fdcm_scale_grid* scales, const fdcm_select_params* select,
+                                          const fdcm_refine_params* refine, const fdcm_coverage_params* cov, fdcm_match* out,
+                                          int64_t capacity, int64_t* n_out) {
+    if (!scales) return fail(FDCM_ERR_INVALID, "scales is null");
+    if (!p) return fail(FDCM_ERR_INVALID, "null argument");
+    if ((select || refine || cov) && p->top_k < 1)
+        return fail(FDCM_ERR_INVALID, "scaled search: select, refine and cov need top_k >= 1");
+    if (cov)
+        if (fdcm_status st = check_coverage(cov)) return st;
+    if (refine) {
+        if (fdcm_status st = check_refine(refine)) return st;
+        if (fdcm_status st = check_refine_top_k(p->top_k)) return st;
+    }
+    return search_impl(m, tc, scene, n_scene, p, out, capacity, n_out, nullptr, select, refine, cov && cov->min_coverage > 0.f ? cov : nullptr,
+                       scales);
 }
 
 extern "C" fdcm_status fdcm_refine_matches(const fdcm_dt3* m, const fdcm_templates* tc, int32_t tmpl_idx_base, int32_t penalty_kind,

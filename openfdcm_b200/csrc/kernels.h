@@ -119,6 +119,17 @@ void launch_search_order(const TemplatesView& tv, const SceneView& sv, const Sea
 int search_max_template_lines(int smem_optin);
 cudaError_t launch_search(const MapView& map, const SlopeTableDev& table, const TemplatesView& tv, const SceneView& sv,
                           const SearchLaunch& sl, const SearchOutputs& out, int smem_optin, cudaStream_t s);
+// the line search over a scale grid (fdcm_search_scales): after launch_search on the copies, every valid record is remapped
+// in place to its original template and scaled pose, and its grid scale goes to rec_scale (the selection's angle test)
+struct ScaleRemapLaunch {
+    fdcm_match* rec;             // n_hyp records of the copy search
+    const uint8_t* valid;        // n_hyp flags
+    float* rec_scale;            // n_hyp grid scales, written for the valid records
+    int64_t n_hyp;
+    int32_t scales, tmpl_idx_base;
+    float scale[FDCM_DENSE_MAX_SCALES];   // s_k
+};
+void launch_search_scale_remap(const ScaleRemapLaunch& p, cudaStream_t s);
 
 // top-K smallest (score, index) among valid records; returns via d_out (k records) and d_n_out
 void launch_topk(const fdcm_match* d_rec, const uint8_t* d_valid, int64_t n, int k, float* d_ws_score, int64_t* d_ws_idx,

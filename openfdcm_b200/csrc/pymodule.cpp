@@ -275,10 +275,13 @@ PYBIND11_MODULE(_openfdcm_cuda, m) {
     m.def("search_topk",
           [](const Dt3Cuda& featuremap, const std::vector<LinesIn>& templates, const LinesIn& scene, const DefaultSearch& searcher,
              const BatchOptimize& optimizer, const ExponentialPenalty& penalty, int k, const std::optional<DistinctMatches>& select,
-             const std::optional<PoseRefinement>& refine, const std::optional<EdgeCoverage>& verify) {
+             const std::optional<PoseRefinement>& refine, const std::optional<EdgeCoverage>& verify, const std::optional<ScaleGrid>& scales) {
               const auto t = to_templates(templates);
               const auto s = to_lines(scene);
               py::gil_scoped_release release;
+              if (scales)
+                  return searchTopK(searcher, optimizer, penalty, featuremap, t, s, k, *scales, select ? &*select : nullptr,
+                                    refine ? &*refine : nullptr, verify ? &*verify : nullptr);
               if (verify)
                   return searchTopK(searcher, optimizer, penalty, featuremap, t, s, k, select ? &*select : nullptr, refine ? &*refine : nullptr,
                                     *verify);
@@ -288,10 +291,11 @@ PYBIND11_MODULE(_openfdcm_cuda, m) {
               return searchTopK(searcher, optimizer, penalty, featuremap, t, s, k);
           },
           "featuremap"_a, "templates"_a, "scene"_a, "searcher"_a, "optimizer"_a, "penalty"_a, "k"_a = 10, py::kw_only(), "select"_a = py::none(),
-          "refine"_a = py::none(), "verify"_a = py::none(),
+          "refine"_a = py::none(), "verify"_a = py::none(), "scales"_a = py::none(),
           "Fused search -> penalize -> top-k on the device (ascending score); select: DistinctMatches for the distinct top-k; "
           "refine: PoseRefinement of the selected matches (not re-sorted; it minimises the score, which was measured to increase the "
-          "error against known poses); verify: EdgeCoverage whose min_coverage > 0 drops matches of lower coverage before the selection");
+          "error against known poses); verify: EdgeCoverage whose min_coverage > 0 drops matches of lower coverage before the selection; "
+          "scales: a ScaleGrid, the search of every template scaled by every grid scale, each match in its original template");
 
     m.def("refine_matches",
           [](const Dt3Cuda& featuremap, const std::vector<LinesIn>& templates, const std::vector<Match>& matches, const PoseRefinement& refine,

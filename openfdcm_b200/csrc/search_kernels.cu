@@ -382,6 +382,27 @@ cudaError_t launch_search(const MapView& map, const SlopeTableDev& table, const 
     return cudaGetLastError();
 }
 
+// fdcm_search_scales rule 4: a valid record of copy v = t * scales + k becomes a record of template t posed at scale s_k
+__global__ void search_scale_remap_kernel(const __grid_constant__ ScaleRemapLaunch p) {
+    const long long h = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (h >= p.n_hyp || !p.valid[h]) return;
+    fdcm_match m = p.rec[h];
+    const int v = m.tmpl_idx - p.tmpl_idx_base, t = v / p.scales, k = v - t * p.scales;
+    const float s = p.scale[k];
+    m.tmpl_idx = t + p.tmpl_idx_base;
+    m.transform[0] = s * m.transform[0];
+    m.transform[1] = s * m.transform[1];
+    m.transform[3] = s * m.transform[3];
+    m.transform[4] = s * m.transform[4];
+    p.rec[h] = m;
+    p.rec_scale[h] = s;
+}
+
+void launch_search_scale_remap(const ScaleRemapLaunch& p, cudaStream_t s) {
+    if (p.n_hyp <= 0) return;
+    search_scale_remap_kernel<<<(unsigned)((p.n_hyp + 255) / 256), 256, 0, s>>>(p);
+}
+
 // =============================================================================================
 // K7: top-K.  K rounds of a block-wide arg-min over keys (score, index) strictly greater than the
 // previously selected key: deterministic, ties broken by hypothesis order.
